@@ -9,14 +9,15 @@ configs[1]: 4096 envs of 14x14 per GPU, Logs/14-sized constants, actions from th
 ACTION stream, auto-reset on done).  Prints one JSON line (rank 0); DESIGN.md section 5 explains
 every field.
 
-  value         device-resident throughput, steady state: R back-to-back K-step regions (R = `repeats`, chosen so
-                that the timed region lasts >= 0.3 s whatever K is), launched `launch.steps_per_launch` steps at a
-                time with one un-timed launch queued in front of the first event so that the GPU never idles inside
-                the region; CUDA events on the launching stream, max over ranks.  Obs/reward/done of EVERY step are
-                written to HBM into a buffer larger than L2.  ms_per_step = region / (R * K).
+  value         device-resident throughput: exactly K = --steps timed steps, launched `launch.steps_per_launch` steps
+                at a time (the last launch shorter when that does not divide K), after `warmup` un-timed steps (W
+                rounded up to whole launches, the last of them queued in front of the first event so that the GPU
+                never idles inside the region); CUDA events on the launching stream, max over ranks.  Obs/reward/done
+                of EVERY step are written to HBM.  ms_per_step = region / K.  Every other timed region of the line
+                (e2e, per_step_launch, secondary, via_torch) is K steps too, each behind un-timed warm-up steps.
   e2e           the same metric through the host-buffer C-ABI call (wf_step_host, page-locked host buffers): per
                 step actions H2D, step, obs + reward + done D2H, all inside the timed region; wall clock over
-                R_e * K steps.  `session` says whether the handle's persistent step-server kernel was used.
+                K steps.  `session` says whether the handle's persistent step-server kernel was used.
   per_step_launch   one wf_step per step with device-resident actions (Python loop, and CUDA graph).
   roofline      dominant kernel.  `achieved` / `frac` count the bytes THIS layout must move per env-step
                 (`bytes_per_unit`); `survey_accounting` is the same throughput in SURVEY.md 8(d)'s byte-per-cell
@@ -25,14 +26,19 @@ every field.
                 `python_ref`: the UNMODIFIED Python reference in os.cpu_count() processes (oracle/ref_bench.py).
   secondary     (default workload only) c4 (256x256 stencil stress), c5 (1024x1024, 64 envs/GPU) and c3 (8192
                 envs/GPU, the reference's DQN network in the loop), each measured the same way with its own roofline.
---impl reference times the reference's own Python step (oracle/_ref snapshot or /root/reference) on all host
+--impl reference times the reference's own Python step (oracle/_ref snapshot or the reference tree) on all host
 cores, and the C port beside it; its line carries "impl": "reference".
+
+--dump-outputs DIR writes, after the timed steps, what the timed path returned for its last step: per workload
+<workload>_reward.npy (float64) and <workload>_done.npy (float32) of every env and <workload>_obs.npy (float32) of the
+envs listed in <workload>_obs_env_index.npy (all of them, or a fixed seeded sample so that the files stay within
+64 MiB in all).  The step count is fixed by --warmup / --steps and every input is seeded, so two builds of the
+project run with the same arguments can be compared file by file.
 """
 from __future__ import annotations
 
 import argparse
 import json
-import math
 import os
 import subprocess
 import sys
@@ -64,7 +70,7 @@ WORKLOADS = {
 BYTES_PER_CELL_UPDATE = 15  # SURVEY.md 8(d): 6 B state read + 6 B state write + 3 B uint8 observation
 CPU_BASELINE_SECONDS = 10.0  # bounded sample of the cpu_baseline (port) leg
 PYTHON_REF_STEPS = 20        # bounded sample of the python_ref leg: the workload's envs (at most 4096) x this many steps
-TIMED_REGION_S = 0.3         # every timed region lasts at least this long
+DUMP_BYTES = 64 << 20        # --dump-outputs writes at most this much in all
 C3_POLICY = os.path.join(ROOT, "bench_inputs", "c3_policy_sarsa9_14s.npz")
 
 
@@ -81,12 +87,28 @@ def load_peaks():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
-def plan_repeats(K: int, chunk: int, us_per_step: float, target_s: float = None) -> int:
-    """R back-to-back K-step regions: R * K steps are a whole number of `chunk`-step launches and last >= target_s."""
-    target_s = TIMED_REGION_S if target_s is None else target_s
-    unit = chunk // math.gcd(chunk, K)
-    need = max(1, math.ceil(target_s * 1e6 / (K * max(us_per_step, 1e-3))))
-    return -(-need // unit) * unit
+def launch_sizes(steps: int, chunk: int) -> list:
+    """`steps` steps as launches of `chunk` steps, the last one shorter when `chunk` does not divide `steps`."""
+    return [chunk] * (steps // chunk) + ([steps % chunk] if steps % chunk else [])
+
+
+def warmup_steps(W: int, chunk: int) -> int:
+    """The un-timed steps in front of a timed region: W rounded up to whole launches, at least one."""
+    return max(1, -(-W // chunk)) * chunk
+
+
+def last_step_outputs(obs, reward, done, budget: int) -> dict:
+    """What a caller of the timed path received for its last step, as float32 / float64 numpy arrays of at most
+    `budget` bytes: reward and done of every env, and the observation of as many envs as fit (a fixed seeded sample
+    when not all of them do, listed in obs_env_index)."""
+    import numpy as np
+    import torch
+    N = reward.shape[0]
+    keep = min(N, max(1, (budget - 20 * N) // (obs[0].numel() * 4)))  # 20 B per env: reward, done, index
+    idx = np.arange(N) if keep == N else np.sort(np.random.default_rng(0).choice(N, keep, replace=False))
+    sel = obs.index_select(0, torch.as_tensor(idx, device=obs.device))
+    return {"reward": reward.double().cpu().numpy(), "done": done.float().cpu().numpy(),
+            "obs": sel.float().cpu().numpy(), "obs_env_index": idx.astype(np.float64)}
 
 
 class ClockSampler:
@@ -230,31 +252,27 @@ class Dist:
             self.dist.destroy_process_group()
 
 
-def timed_region(D: Dist, launch, K: int, chunk: int, warm_launches: int):
-    """Steady-state timing of `launch()` (= `chunk` steps): calibrate, pick R (the same on every rank), then time
-    R * K steps with one un-timed launch queued in front of the first event.  Returns (ms, R, n_launches)."""
+def timed_region(D: Dist, launch, K: int, chunk: int, W: int):
+    """Time exactly K steps of `launch(n)` (n <= chunk steps per call) after warmup_steps(W, chunk) un-timed steps, the
+    last `chunk` of them queued in front of the first event.  Returns (ms, n_launches) of the region."""
     torch = D.torch
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    for _ in range(max(1, warm_launches)):
-        launch()
+    for _ in range(warmup_steps(W, chunk) // chunk - 1):
+        launch(chunk)
     D.barrier()
-    ev0.record(); launch(); launch(); ev1.record()
-    torch.cuda.synchronize()
-    us_step = D.max_over_ranks(ev0.elapsed_time(ev1) * 1e3 / (2 * chunk))
-    R = plan_repeats(K, chunk, us_step)
-    n_launch = R * K // chunk
-    D.barrier()
-    launch()          # un-timed: the GPU is busy when ev0 is reached, so no host launch latency sits in the region
+    launch(chunk)     # un-timed: the GPU is busy when ev0 is reached, so no host launch latency sits in the region
     ev0.record()
-    for _ in range(n_launch):
-        launch()
+    sizes = launch_sizes(K, chunk)
+    for n in sizes:
+        launch(n)
     ev1.record()
     D.barrier()
-    return D.max_over_ranks(ev0.elapsed_time(ev1)), R, n_launch
+    return D.max_over_ranks(ev0.elapsed_time(ev1)), len(sizes)
 
 
-def measure(D: Dist, name: str, K: int, Wm: int, chunk_arg: int, with_e2e: bool, with_per_step: bool):
-    """Time workload `name` on this rank's GPU; every rank calls this, results are max-reduced."""
+def measure(D: Dist, name: str, K: int, Wm: int, chunk_arg: int, with_e2e: bool, with_per_step: bool, dump_budget: int = 0):
+    """Time workload `name` on this rank's GPU; every rank calls this, results are max-reduced.  dump_budget > 0: keep
+    the last timed step's outputs (last_step_outputs) as res["outputs"]."""
     import numpy as np
     torch = D.torch
     from wildfire_control_python_b200 import BatchedForestFire
@@ -268,57 +286,54 @@ def measure(D: Dist, name: str, K: int, Wm: int, chunk_arg: int, with_e2e: bool,
     obs_buf = torch.empty((chunk, N, W, H, 3), dtype=torch.uint8, device=dev)
     rew_buf = torch.empty((chunk, N), dtype=torch.float64, device=dev)
     done_buf = torch.empty((chunk, N), dtype=torch.uint8, device=dev)
-    out = (obs_buf, rew_buf, done_buf)
 
-    def launch():
-        env.rollout(chunk, actions=None, out=out)
+    def launch(n):
+        env.rollout(n, actions=None, out=(obs_buf[:n], rew_buf[:n], done_buf[:n]))
 
     launches0 = env.launch_count
-    ms_max, R, n_launch = timed_region(D, launch, K, chunk, -(-max(Wm, 3) // chunk))
-    res = {"name": name, "wl": wl, "N": N, "W": W, "H": H, "K": K, "repeats": R, "chunk": chunk, "ms": ms_max,
-           "launches": int(n_launch), "launches_total": int(env.launch_count - launches0),
-           "value": world * N * R * K / (ms_max * 1e-3), "obs_mb": obs_buf.numel() / 1e6, "family": env.kernel_family,
+    ms_max, n_launch = timed_region(D, launch, K, chunk, Wm)
+    res = {"name": name, "wl": wl, "N": N, "W": W, "H": H, "K": K, "warmup": warmup_steps(Wm, chunk), "chunk": chunk,
+           "ms": ms_max, "launches": int(n_launch), "launches_total": int(env.launch_count - launches0),
+           "value": world * N * K / (ms_max * 1e-3), "obs_mb": obs_buf.numel() / 1e6, "family": env.kernel_family,
            "state_bytes": env.state_bytes_per_env, "tile_geometry": list(env.tile_geometry)}
+    if dump_budget:
+        last = launch_sizes(K, chunk)[-1] - 1
+        res["outputs"] = last_step_outputs(obs_buf[last], rew_buf[last], done_buf[last], dump_budget)
 
     if with_per_step:
-        Kp = 2000
         g = torch.Generator(device=dev).manual_seed(99 + rank)
-        acts = torch.randint(0, 4, (Kp, N), dtype=torch.int32, device=dev, generator=g)
+        acts = torch.randint(0, 4, (K, N), dtype=torch.int32, device=dev, generator=g)
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        for k in range(3):
-            env.step(acts[k])
         D.barrier()
+        for k in range(res["warmup"]):
+            env.step(acts[k % K])
         ev0.record()
-        for k in range(Kp):
+        for k in range(K):
             env.step(acts[k])
         ev1.record()
         D.barrier()
         t2 = D.max_over_ranks(ev0.elapsed_time(ev1))
-        per_step = {"value": world * N * Kp / (t2 * 1e-3), "unit": "env-steps/s", "steps": Kp, "us_per_step": t2 * 1e3 / Kp,
+        per_step = {"value": world * N * K / (t2 * 1e-3), "unit": "env-steps/s", "steps": K, "us_per_step": t2 * 1e3 / K,
                     "issue": "python loop over BatchedForestFire.step, actions resident in HBM"}
         try:  # the same per-step launches replayed from a CUDA graph (no host work between launches)
-            Kg = 200
             side = torch.cuda.Stream(device=dev)
             side.wait_stream(torch.cuda.current_stream(dev))
             with torch.cuda.stream(side):
-                env.step(acts[0]); env.step(acts[1])
+                env.step(acts[0])
                 g2 = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(g2, stream=side):
-                    for k in range(Kg):
+                    for k in range(K):
                         env.step(acts[k])
             torch.cuda.current_stream(dev).wait_stream(side)
-            g2.replay()
             D.barrier()
-            reps = 50
-            g2.replay()
+            g2.replay()  # un-timed, queued in front of the first event
             ev0.record()
-            for _ in range(reps):
-                g2.replay()
+            g2.replay()
             ev1.record()
             D.barrier()
             t3 = D.max_over_ranks(ev0.elapsed_time(ev1))
-            per_step["cuda_graph"] = {"value": world * N * Kg * reps / (t3 * 1e-3), "unit": "env-steps/s", "steps": Kg * reps,
-                                      "us_per_step": t3 * 1e3 / (Kg * reps),
+            per_step["cuda_graph"] = {"value": world * N * K / (t3 * 1e-3), "unit": "env-steps/s", "steps": K,
+                                      "us_per_step": t3 * 1e3 / K,
                                       "note": "obs written to the same buffer every step (may stay in L2)"}
         except Exception as exc:  # a convenience measurement, never the headline
             per_step["cuda_graph"] = {"error": repr(exc)[:200]}
@@ -331,25 +346,18 @@ def measure(D: Dist, name: str, K: int, Wm: int, chunk_arg: int, with_e2e: bool,
             session = False
             if hasattr(env, "host_session") and not os.environ.get("WF_BENCH_NO_SESSION"):
                 session = bool(env.host_session(True, persistent_obs=persistent_obs))
-            for k in range(8):
-                env.step_host(host_actions[k])
-            t0 = time.perf_counter()
-            for k in range(32):
-                env.step_host(host_actions[k])
-            us_step = D.max_over_ranks((time.perf_counter() - t0) * 1e6 / 32)
-            Re = max(1, math.ceil(TIMED_REGION_S * 1e6 / (K * us_step)))
-            Ke = Re * K
-            D.barrier()
-            t0 = time.perf_counter()
-            for k in range(Ke):
+            D.barrier()  # before the warm-up: a synchronise would wait until the resident step server parks
+            for k in range(res["warmup"]):
                 env.step_host(host_actions[k & 511])
-            torch.cuda.synchronize()
-            te = D.max_over_ranks(time.perf_counter() - t0)
+            t0 = time.perf_counter()
+            for k in range(K):
+                env.step_host(host_actions[k & 511])
+            te = D.max_over_ranks(time.perf_counter() - t0)  # each call returns with its results in the host arrays
             if session:
                 env.host_session(False)
-            return session, Re, Ke, te
+            return session, te
 
-        session, Re, Ke, te = time_e2e(False)
+        session, te = time_e2e(False)
         obs_bytes = N * W * H * 3
         if env.host_threads:  # packed path: one record of ceil(e * W*H*3 / 32) words per e envs (e = 2 if W <= 16 else 1)
             epw = 2 if W <= 16 else 1
@@ -360,9 +368,9 @@ def measure(D: Dist, name: str, K: int, Wm: int, chunk_arg: int, with_e2e: bool,
                 d2h = records * rec_words * 4 + N * 8 + N
         else:
             d2h = obs_bytes + N * 8 + N
-        res["e2e"] = {"value": world * N * Ke / te, "unit": "env-steps/s", "h2d_bytes_per_step": N * 4,
+        res["e2e"] = {"value": world * N * K / te, "unit": "env-steps/s", "h2d_bytes_per_step": N * 4,
                       "d2h_bytes_per_step": d2h, "obs_bytes_delivered_per_step": obs_bytes,
-                      "steps": K, "repeats": Re, "us_per_step": te * 1e6 / Ke,
+                      "steps": K, "us_per_step": te * 1e6 / K,
                       "host_threads": env.host_threads, "session": session,
                       "api": ("wf_step_host, page-locked host buffers: actions/reward/done zero-copy; observation sent as a bit "
                               "stream and expanded to the caller's uint8 [N][W][H][3] array by the library's host threads"
@@ -374,17 +382,17 @@ def measure(D: Dist, name: str, K: int, Wm: int, chunk_arg: int, with_e2e: bool,
             # The same call with wf_host_session mode 2 (a vectorised Gym env's copy=False convention: step_host hands out
             # the same array every call and the caller does not write to it): only the elements that changed cross PCIe and
             # are patched in place.  Reported beside the headline, which re-delivers the whole array every step.
-            _, Rp, Kp, tp = time_e2e(True)
+            _, tp = time_e2e(True)
             ctas = ((N + epw - 1) // epw + 3) // 4
             res["e2e"]["persistent_obs"] = {
-                "value": world * N * Kp / tp, "unit": "env-steps/s", "us_per_step": tp * 1e6 / Kp, "repeats": Rp,
+                "value": world * N * K / tp, "unit": "env-steps/s", "us_per_step": tp * 1e6 / K,
                 "d2h_bytes_per_step": ctas * 128,
                 "note": "wf_host_session(env, 2): one 128-byte change-list block per 8 envs + the full record (160 B) of every "
                         "pair of envs with more than 13 changed elements (about 4 % of them per step: resets, large fire ticks); "
                         "the array is complete and equal to the headline's after every call (tests/test_host_api_gpu.py)"}
     res["stats"] = env.stats()
     env.close()
-    del obs_buf, rew_buf, done_buf, out, env
+    del obs_buf, rew_buf, done_buf, env
     torch.cuda.empty_cache()
     return res
 
@@ -405,18 +413,37 @@ def load_c3_policy(torch, dev, W, H, n_actions):
     return (w1, b1, w2, b2), "random-weight network"
 
 
-def measure_policy(D: Dist, name: str, K: int, Wm: int):
+def measure_policy(D: Dist, name: str, K: int, Wm: int, dump_budget: int = 0):
     """configs[2]: the reference's DQN network picks the actions (DQN.py:188-233).  Headline: the network evaluated
-    INSIDE the step kernel (WF_POLICY_MLP); beside it the same policy through torch ops, one wf_step per step, the
-    whole step (obs -> float -> MLP -> epsilon-greedy -> wf_step) captured in a CUDA graph."""
+    INSIDE the step kernel (WF_POLICY_MLP); beside it, afterwards, the same policy through torch ops, one wf_step per
+    step, the whole step (obs -> float -> MLP -> epsilon-greedy -> wf_step) captured in CUDA graphs."""
     torch = D.torch
     from wildfire_control_python_b200 import BatchedForestFire
     wl = WORKLOADS[name]
     dev, rank, world = D.dev, D.rank, D.world
     N, W, H = wl["n_envs"], wl["meta"]["width"], wl["meta"]["height"]
     env = BatchedForestFire(N, device=dev, auto_reset=True, seed=0, env_id_base=rank * N, **wl["meta"])
-    obs = env.reset()
+    env.reset()
     (w1, b1, w2, b2), policy_name = load_c3_policy(torch, dev, W, H, env.n_actions)
+    # The policy evaluated INSIDE the step kernel (WF_POLICY_MLP): first layer kept incrementally as a sum of weight rows
+    # of the observation bits, `chunk` steps per launch, obs/reward/done of every step still written.
+    chunk = wl["chunk"]
+    env.set_policy_mlp(w1, b1, w2, b2, eps=0.1)
+    out = (torch.empty((chunk, N, W, H, 3), dtype=torch.uint8, device=dev), torch.empty((chunk, N), dtype=torch.float64, device=dev),
+           torch.empty((chunk, N), dtype=torch.uint8, device=dev))
+    l0 = env.launch_count
+    ms, n_launch = timed_region(D, lambda n: env.rollout(n, policy="mlp", out=tuple(o[:n] for o in out)), K, chunk, Wm)
+    res = {"name": name, "wl": wl, "N": N, "W": W, "H": H, "K": K, "warmup": warmup_steps(Wm, chunk), "chunk": chunk, "ms": ms,
+           "launches": int(n_launch), "launches_total": int(env.launch_count - l0), "value": world * N * K / (ms * 1e-3),
+           "obs_mb": out[0].numel() / 1e6, "family": env.kernel_family, "state_bytes": env.state_bytes_per_env,
+           "tile_geometry": [0, 0],
+           "policy": f"MLP 588-50(sigmoid)-4 = {policy_name}, eps-greedy 0.1, evaluated inside the step kernel (WF_POLICY_MLP); "
+                     "`via_torch` is the same policy through torch ops"}
+    if dump_budget:
+        last = launch_sizes(K, chunk)[-1] - 1
+        res["outputs"] = last_step_outputs(out[0][last], out[1][last], out[2][last], dump_budget)
+
+    obs = env.observe()
     actions = torch.zeros(N, dtype=torch.int32, device=dev)
 
     def one_step():
@@ -430,33 +457,24 @@ def measure_policy(D: Dist, name: str, K: int, Wm: int):
     for _ in range(3):
         one_step()
     G_STEPS = 16
+    graphs = {}
     side = torch.cuda.Stream(device=dev)
     side.wait_stream(torch.cuda.current_stream(dev))
     with torch.cuda.stream(side):
         one_step()
-        graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(graph, stream=side):
-            for _ in range(G_STEPS):
-                one_step()
+        for n in {G_STEPS, *launch_sizes(K, G_STEPS)}:
+            graphs[n] = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(graphs[n], stream=side):
+                for _ in range(n):
+                    one_step()
     torch.cuda.current_stream(dev).wait_stream(side)
-    ms_torch, R_t, n_t = timed_region(D, graph.replay, K, G_STEPS, 2)
-    via_torch = {"value": world * N * R_t * K / (ms_torch * 1e-3), "unit": "env-steps/s", "steps": K, "repeats": R_t,
-                 "us_per_step": ms_torch * 1e3 / (R_t * K),
-                 "how": "obs -> float -> torch MLP -> eps-greedy -> wf_step, 16 steps per CUDA-graph replay"}
-    # The same policy evaluated INSIDE the step kernel (WF_POLICY_MLP): first layer kept incrementally as a sum of
-    # weight rows of the observation bits, `chunk` steps per launch, obs/reward/done of every step still written.
-    chunk = wl["chunk"]
-    env.set_policy_mlp(w1, b1, w2, b2, eps=0.1)
-    out = (torch.empty((chunk, N, W, H, 3), dtype=torch.uint8, device=dev), torch.empty((chunk, N), dtype=torch.float64, device=dev),
-           torch.empty((chunk, N), dtype=torch.uint8, device=dev))
-    l0 = env.launch_count
-    ms, R, n_launch = timed_region(D, lambda: env.rollout(chunk, policy="mlp", out=out), K, chunk, -(-max(Wm, 3) // chunk))
-    res = {"name": name, "wl": wl, "N": N, "W": W, "H": H, "K": K, "repeats": R, "chunk": chunk, "ms": ms,
-           "launches": int(n_launch), "launches_total": int(env.launch_count - l0), "value": world * N * R * K / (ms * 1e-3),
-           "obs_mb": out[0].numel() / 1e6, "family": env.kernel_family, "state_bytes": env.state_bytes_per_env,
-           "tile_geometry": [0, 0], "stats": env.stats(), "via_torch": via_torch,
-           "policy": f"MLP 588-50(sigmoid)-4 = {policy_name}, eps-greedy 0.1, evaluated inside the step kernel (WF_POLICY_MLP); "
-                     "`via_torch` is the same policy through torch ops"}
+    for g in graphs.values():  # a graph's first replay uploads it: keep that out of the region
+        g.replay()
+    ms_torch, _ = timed_region(D, lambda n: graphs[n].replay(), K, G_STEPS, Wm)
+    res["via_torch"] = {"value": world * N * K / (ms_torch * 1e-3), "unit": "env-steps/s", "steps": K,
+                        "us_per_step": ms_torch * 1e3 / K,
+                        "how": "obs -> float -> torch MLP -> eps-greedy -> wf_step, 16 steps per CUDA-graph replay"}
+    res["stats"] = env.stats()
     env.close()
     del out, env
     torch.cuda.empty_cache()
@@ -510,8 +528,8 @@ def roofline_of(res, world):
 def launch_info(res):
     return {"steps_per_launch": res["chunk"], "kernel_family": res["family"],
             "tile_threads_x_cluster": res["tile_geometry"] if res["family"] == "tile" else None,
-            "timing": f"{res['repeats']} back-to-back {res['K']}-step regions = {res['launches']} launches in one CUDA-event "
-                      "interval, one un-timed launch queued in front",
+            "timing": f"{res['K']} steps = {res['launches']} launches in one CUDA-event interval, after {res['warmup']} "
+                      "un-timed steps whose last launch is queued in front",
             "l2": f"outputs of one launch ({res['obs_mb']:.0f} MB obs) exceed the 126 MB L2; "
                   + ("state is register/L2 resident by design" if res["family"] == "warp"
                      else f"state ({res['state_bytes'] * res['N'] / 1e6:.0f} MB) exceeds L2 too")}
@@ -519,8 +537,8 @@ def launch_info(res):
 
 def secondary_entry(sec, world):
     e = {"workload": WORKLOADS[sec["name"]]["desc"], "config": workload_config(sec["name"]), "value": sec["value"],
-         "unit": "env-steps/s", "steps": sec["K"], "repeats": sec["repeats"],
-         "ms_per_step": sec["ms"] / (sec["repeats"] * sec["K"]),
+         "unit": "env-steps/s", "steps": sec["K"], "repeats": 1, "warmup": sec["warmup"],
+         "ms_per_step": sec["ms"] / sec["K"],
          "cell_updates_per_sec_per_gpu": sec["value"] * sec["W"] * sec["H"] / world, "gpu_launches": sec["launches"],
          "launch": launch_info(sec), "roofline": roofline_of(sec, world)}
     if "via_torch" in sec:
@@ -530,23 +548,33 @@ def secondary_entry(sec, world):
 
 def run_ours(args, wl):
     D = Dist(args.gpus)
+    secondary = []
+    if args.workload == "c2" and not args.no_secondary and not args.only_value:
+        secondary = [s for s in args.secondary.split(",") if s]
+    # rank 0's outputs only; every workload of the line gets the same share
+    budget = DUMP_BYTES // (1 + len(secondary)) if args.dump_outputs and D.rank == 0 else 0
     secs = []
     with ClockSampler(D.local) as clk:
         if wl.get("policy"):
-            res = measure_policy(D, args.workload, args.steps, args.warmup)
+            res = measure_policy(D, args.workload, args.steps, args.warmup, budget)
         else:
-            res = measure(D, args.workload, args.steps, args.warmup, args.chunk, not args.only_value, not args.only_value)
-        if args.workload == "c2" and not args.no_secondary and not args.only_value:
-            for name in [s for s in args.secondary.split(",") if s]:
-                if WORKLOADS[name].get("policy"):
-                    secs.append(measure_policy(D, name, args.steps, args.warmup))
-                else:
-                    secs.append(measure(D, name, args.steps, args.warmup, 0, False, False))
+            res = measure(D, args.workload, args.steps, args.warmup, args.chunk, not args.only_value, not args.only_value, budget)
+        for name in secondary:
+            if WORKLOADS[name].get("policy"):
+                secs.append(measure_policy(D, name, args.steps, args.warmup, budget))
+            else:
+                secs.append(measure(D, name, args.steps, args.warmup, 0, False, False, budget))
     clocks = clk.summary()
     if D.rank != 0:
         D.close()
         return
     world, W, H, K = D.world, res["W"], res["H"], res["K"]
+    if budget:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for r in [res] + secs:
+            for key, arr in r["outputs"].items():
+                np.save(os.path.join(args.dump_outputs, f"{r['name']}_{key}.npy"), arr)
 
     cpu_baseline = None
     if world == 1 and not args.only_value:
@@ -559,7 +587,7 @@ def run_ours(args, wl):
     config["l2"] = launch_info(res)["l2"]
     line = {
         "metric": "env_steps_per_sec", "value": res["value"], "unit": "env-steps/s", "n_gpus": world, "steps": K,
-        "repeats": res["repeats"], "warmup": max(args.warmup, 3), "ms_per_step": res["ms"] / (res["repeats"] * K),
+        "repeats": 1, "warmup": res["warmup"], "ms_per_step": res["ms"] / K,
         "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "u32-bitplanes+u8", "data": "synthetic",
         "config": config, "launch": launch_info(res),
@@ -582,7 +610,6 @@ def run_ours(args, wl):
 
 
 def main():
-    global TIMED_REGION_S
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=2048)
@@ -593,12 +620,15 @@ def main():
     ap.add_argument("--secondary", default="c4,c5,c3", help="workloads measured beside the default one (comma separated)")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary measurements in the default line")
     ap.add_argument("--no-python-ref", action="store_true", help="skip the Python-reference leg of cpu_baseline")
-    ap.add_argument("--min-region-s", type=float, default=TIMED_REGION_S,
-                    help="minimum length of every timed region (profiling runs under ncu: 0 = the fewest launches)")
     ap.add_argument("--only-value", action="store_true",
                     help="profiling runs: only the fused-rollout measurement (no per-step, e2e, CPU baseline legs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs of every measured workload to DIR/<workload>_<array>.npy")
     args = ap.parse_args()
-    TIMED_REGION_S = args.min_region_s
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what --impl ours computed")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, wl)

@@ -1,12 +1,12 @@
 #!/usr/bin/env python
-"""Turn the ncu artefacts brought back in gpurun_out/ into the tracked summaries under profiles/.
+"""Turn the ncu artefacts that tools/profile_round.sh writes to profile_out/ into the tracked summaries under profiles/.
 
 usage: python profiles/summarize.py r02
 Reads (whatever exists):
-  gpurun_out/launches_bench.csv (and launches_c2/c4/c5.csv)   `ncu --metrics gpu__time_duration.sum ...` launch lists
-  gpurun_out/prof_c2.ncu-rep                      `ncu --set full` capture of wf::warp_kernel (c2, 256 steps per launch)
-  gpurun_out/prof_c4.ncu-rep, prof_c5.ncu-rep     captures of wf::tile_rollout_kernel (c4 / c5, 16 steps per launch)
-  gpurun_out/prof_c3.ncu-rep                      capture of wf::warp_kernel<..., MLP> (c3, 64 steps per launch; tools/profile_c3.sh)
+  profile_out/launches_bench.csv (and launches_c2/c4/c5.csv)   `ncu --metrics gpu__time_duration.sum ...` launch lists
+  profile_out/prof_c2.ncu-rep                      `ncu --set full` capture of wf::warp_kernel (c2, 256 steps per launch)
+  profile_out/prof_c4.ncu-rep, prof_c5.ncu-rep     captures of wf::tile_rollout_kernel (c4 / c5, 16 steps per launch)
+  profile_out/prof_c3.ncu-rep                      capture of wf::warp_kernel<..., MLP> (c3, 64 steps per launch; tools/profile_c3.sh)
 Writes profiles/<round>_*.{csv,txt,json} and profiles/ncu_traffic.json (DRAM bytes per STEP, read by bench.py).
 """
 import collections
@@ -18,7 +18,7 @@ import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-GO = os.path.join(ROOT, "gpurun_out")
+GO = os.path.join(ROOT, "profile_out")
 PR = os.path.join(ROOT, "profiles")
 
 KEEP = ["gpu__time_duration.sum", "dram__bytes_read.sum", "dram__bytes_write.sum", "dram__throughput.avg.pct_of_peak_sustained_elapsed",

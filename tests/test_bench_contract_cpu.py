@@ -34,16 +34,16 @@ class _NoClocks:
         return {"sm_mhz": 1965, "sm_max_mhz": 1965, "reasons": [], "samples": 3}
 
 
-def _canned(name, K):
+def _canned(name, K, Wm=5):
     wl = bench.WORKLOADS[name]
     N, W, H = wl["n_envs"], wl["meta"]["width"], wl["meta"]["height"]
     chunk = wl["chunk"]
     us = 2.5 if W <= 32 else 50.0
-    R = bench.plan_repeats(K, chunk, us)
-    ms = us * 1e-3 * R * K
+    ms = us * 1e-3 * K
     fam = "warp" if W <= 32 else "tile"
-    out = {"name": name, "wl": wl, "N": N, "W": W, "H": H, "K": K, "repeats": R, "chunk": chunk, "ms": ms,
-           "launches": R * K // chunk, "launches_total": R * K // chunk + 4, "value": N * R * K / (ms * 1e-3),
+    n_launch = len(bench.launch_sizes(K, chunk))
+    out = {"name": name, "wl": wl, "N": N, "W": W, "H": H, "K": K, "warmup": bench.warmup_steps(Wm, chunk), "chunk": chunk,
+           "ms": ms, "launches": n_launch, "launches_total": n_launch + 4, "value": N * K / (ms * 1e-3),
            "obs_mb": chunk * N * W * H * 3 / 1e6, "family": fam, "state_bytes": 1280 if fam == "warp" else 409664,
            "tile_geometry": [0, 0] if fam == "warp" else [256, 1],
            "stats": {"env_steps": N * K, "episodes": 1, "deaths": 1, "contained": 0, "burnouts": 0, "ticks": N * K},
@@ -55,12 +55,12 @@ def _canned(name, K):
     return out
 
 
-def test_plan_repeats_fills_the_region_with_whole_launches():
-    for K, chunk, us in [(20, 256, 2.3), (20, 16, 75.0), (2048, 256, 2.3), (7, 64, 10.0), (20000, 256, 2.3), (1, 256, 2.0)]:
-        R = bench.plan_repeats(K, chunk, us, 0.3)
-        assert (R * K) % chunk == 0 and R * K * us * 1e-6 >= 0.3
-        assert (R - chunk) * K * us * 1e-6 < 0.3 or R <= chunk  # not more than one rounding unit too long
-    assert bench.plan_repeats(20, 256, 2.3, 0.0) == 64  # the fewest whole launches (profiling runs)
+def test_launch_sizes_time_exactly_the_requested_steps():
+    for K, chunk in [(20, 256), (20, 16), (2048, 256), (7, 64), (20000, 256), (1, 256), (64, 64), (65, 64)]:
+        sizes = bench.launch_sizes(K, chunk)
+        assert sum(sizes) == K and all(0 < n <= chunk for n in sizes)
+        assert len(sizes) == -(-K // chunk) and sizes[:-1] == [chunk] * (len(sizes) - 1)  # the fewest launches, all full but the last
+    assert bench.warmup_steps(5, 256) == 256 and bench.warmup_steps(0, 16) == 16 and bench.warmup_steps(33, 16) == 48
 
 
 @pytest.mark.parametrize("argv", [[], ["--workload", "c4", "--steps", "64", "--warmup", "8"], ["--steps", "20", "--warmup", "5"],
@@ -71,9 +71,10 @@ def test_bench_line_has_the_contract_keys(monkeypatch, capsys, argv):
     monkeypatch.setattr(bench, "ClockSampler", _NoClocks)
     monkeypatch.setattr(bench, "CPU_BASELINE_SECONDS", 0.2)
     monkeypatch.setattr(bench, "python_ref_baseline", lambda wl, steps, warmup, budget_s=60.0: None)
-    monkeypatch.setattr(bench, "measure", lambda D, name, K, Wm, chunk, e2e, per_step: {
-        k: v for k, v in _canned(name, K).items() if (k != "e2e" or e2e) and (k != "per_step" or per_step)})
-    monkeypatch.setattr(bench, "measure_policy", lambda D, name, K, Wm: {k: v for k, v in _canned(name, K).items() if k not in ("e2e", "per_step")})
+    monkeypatch.setattr(bench, "measure", lambda D, name, K, Wm, chunk, e2e, per_step, dump_budget=0: {
+        k: v for k, v in _canned(name, K, Wm).items() if (k != "e2e" or e2e) and (k != "per_step" or per_step)})
+    monkeypatch.setattr(bench, "measure_policy", lambda D, name, K, Wm, dump_budget=0: {
+        k: v for k, v in _canned(name, K, Wm).items() if k not in ("e2e", "per_step")})
     monkeypatch.setattr(sys, "argv", ["bench.py"] + argv)
     bench.main()
     line = json.loads(capsys.readouterr().out.strip().splitlines()[-1])
@@ -89,7 +90,10 @@ def test_bench_line_has_the_contract_keys(monkeypatch, capsys, argv):
     assert line["warmup"] >= 3 and line["gpu_launches"] >= 1
     assert line["steps"] == (int(argv[argv.index("--steps") + 1]) if "--steps" in argv else 2048)
     assert line["value"] == pytest.approx(wl["n_envs"] / (line["ms_per_step"] * 1e-3))
-    assert line["ms_per_step"] * line["steps"] * line["repeats"] >= 300.0  # the timed region lasted >= 0.3 s
+    chunk = line["launch"]["steps_per_launch"]
+    assert line["repeats"] == 1 and line["gpu_launches"] == len(bench.launch_sizes(line["steps"], chunk))  # --steps steps timed
+    assert line["ms_per_step"] * line["steps"] == pytest.approx(_canned(name, line["steps"])["ms"])
+    assert line["warmup"] == bench.warmup_steps(int(argv[argv.index("--warmup") + 1]) if "--warmup" in argv else 256, chunk)
     r = line["roofline"]
     assert r["bound"] == "hbm" and r["unit"] == "GB/s" and r["frac"] == pytest.approx(r["achieved"] / r["peak"])
     assert r["achieved"] == pytest.approx(line["value"] * r["bytes_per_unit"] / 1e9)
@@ -133,3 +137,51 @@ def test_reference_arm_line(monkeypatch, capsys):
         assert cb["kind"] == "port"
     assert line["e2e"] == {"value": line["value"], "unit": "env-steps/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert line["gpu_launches"] == 0 and line["higher_is_better"] is True
+
+
+def test_dump_outputs_writes_every_workload_within_64_mib(monkeypatch, capsys, tmp_path):
+    """--dump-outputs DIR: reward, done and observations of the last timed step of every workload of the line as float32 /
+    float64 .npy files, 64 MiB in all; workloads whose observations do not fit keep a fixed seeded sample of envs."""
+    import numpy as np
+    import torch
+
+    def with_outputs(name, K, Wm, budget):
+        res = _canned(name, K, Wm)
+        N, W, H = res["N"], res["W"], res["H"]
+        g = torch.Generator().manual_seed(len(name))
+        obs = torch.randint(0, 2, (1, W, H, 3), dtype=torch.uint8, generator=g).expand(N, -1, -1, -1)
+        reward = torch.arange(N, dtype=torch.float64) - 0.5
+        done = (torch.arange(N) % 3 == 0).to(torch.uint8)
+        assert budget > 0
+        res["outputs"] = bench.last_step_outputs(obs, reward, done, budget)
+        return res
+
+    monkeypatch.setattr(bench, "Dist", _FakeDist)
+    monkeypatch.setattr(bench, "ClockSampler", _NoClocks)
+    monkeypatch.setattr(bench, "CPU_BASELINE_SECONDS", 0.2)
+    monkeypatch.setattr(bench, "python_ref_baseline", lambda wl, steps, warmup, budget_s=60.0: None)
+    monkeypatch.setattr(bench, "measure", lambda D, name, K, Wm, chunk, e2e, per_step, dump_budget=0: {
+        k: v for k, v in with_outputs(name, K, Wm, dump_budget).items() if (k != "e2e" or e2e) and (k != "per_step" or per_step)})
+    monkeypatch.setattr(bench, "measure_policy", lambda D, name, K, Wm, dump_budget=0: {
+        k: v for k, v in with_outputs(name, K, Wm, dump_budget).items() if k not in ("e2e", "per_step")})
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "20", "--warmup", "5", "--dump-outputs", str(tmp_path / "out")])
+    bench.main()
+    assert json.loads(capsys.readouterr().out.strip().splitlines()[-1])["steps"] == 20
+    files = sorted(p.name for p in (tmp_path / "out").iterdir())
+    assert files == sorted(f"{w}_{a}.npy" for w in ("c2", "c3", "c4", "c5") for a in ("obs", "reward", "done", "obs_env_index"))
+    assert sum(p.stat().st_size for p in (tmp_path / "out").iterdir()) <= 64 << 20
+    for w in ("c2", "c3", "c4", "c5"):
+        wl = bench.WORKLOADS[w]
+        N, W, H = wl["n_envs"], wl["meta"]["width"], wl["meta"]["height"]
+        a = {k: np.load(tmp_path / "out" / f"{w}_{k}.npy") for k in ("obs", "reward", "done", "obs_env_index")}
+        assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+        assert a["reward"].dtype == np.float64 and np.array_equal(a["reward"], np.arange(N) - 0.5)
+        assert np.array_equal(a["done"], (np.arange(N) % 3 == 0).astype(np.float32))
+        idx = a["obs_env_index"].astype(np.int64)
+        assert a["obs"].shape == (len(idx), W, H, 3) and np.all(np.diff(idx) > 0) and 0 <= idx[0] and idx[-1] < N
+        assert (len(idx) == N) == (w == "c2")  # c2's 4096 observations fit whole; the others are sampled
+    # the sample is a function of the shapes and the budget only
+    obs = torch.zeros((100, 4, 4, 3), dtype=torch.uint8)
+    one = bench.last_step_outputs(obs, torch.zeros(100, dtype=torch.float64), torch.zeros(100, dtype=torch.uint8), 20 * 100 + 10 * 192)
+    two = bench.last_step_outputs(obs, torch.zeros(100, dtype=torch.float64), torch.zeros(100, dtype=torch.uint8), 20 * 100 + 10 * 192)
+    assert len(one["obs_env_index"]) == 10 and np.array_equal(one["obs_env_index"], two["obs_env_index"])

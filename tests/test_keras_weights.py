@@ -14,6 +14,7 @@ import os
 import numpy as np
 import pytest
 
+from oracle import ref_harness
 from wildfire_control_python_b200.keras_h5 import H5Error, canonical_dense_names, read_h5_datasets, read_keras_weights
 
 HERE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "keras")
@@ -49,10 +50,11 @@ def test_layer_renumbering():
     assert sorted(canonical_dense_names(w)) == ["dense_1/bias:0", "dense_1/kernel:0", "dense_2/bias:0", "dense_2/kernel:0"]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/Models"), reason="reference tree not present on this box")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(ref_harness.REF_ROOT, "Models")),
+                    reason="the original project's Models/ tree is not reachable (WF_REFERENCE_ROOT)")
 def test_every_model_of_the_reference_tree_parses():
     n = 0
-    for f in sorted(glob.glob("/root/reference/Models/*/*")):
+    for f in sorted(glob.glob(os.path.join(ref_harness.REF_ROOT, "Models", "*", "*"))):
         if open(f, "rb").read(8) != b"\x89HDF\r\n\x1a\n":
             continue  # three stray non-HDF5 files ("... (1)") sit in Models/14-sized
         w = read_keras_weights(f)

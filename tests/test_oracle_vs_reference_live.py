@@ -1,17 +1,19 @@
 """Live differential test: the C oracle against the UNMODIFIED Python reference, step by step.
 
-Runs only where the reference tree exists (the build container; `/root/reference` does not travel to
-the GPU box -- there the committed golden trajectories of tests/golden/ stand in).  It is the pytest
-face of `python -m oracle.validate_oracle` (69 000 steps over 23 scenarios, run by hand): a bounded
+Runs only where the reference is reachable (oracle/ref_harness.py: the tree named by WF_REFERENCE_ROOT, or
+the snapshot `make -C oracle ref REF=<tree>` leaves in oracle/_ref/); elsewhere the committed golden
+trajectories of tests/golden/ stand in (tests/test_oracle_golden.py).  It is the pytest face of
+`python -m oracle.validate_oracle` (69 000 steps over 23 scenarios, run by hand): a bounded
 number of steps of every scenario, every plane / scalar / observation / reward / done compared, and
 for the `walk_*` scenarios the reference's own `DQN.choose_randomwalk_action` against the oracle's
 restatement, action by action.
 """
-import os
-
 import pytest
 
-pytestmark = pytest.mark.skipif(not os.path.isdir("/root/reference/Simulation"), reason="reference tree not present on this box")
+from oracle import ref_harness
+
+pytestmark = pytest.mark.skipif(not ref_harness.reference_available(),
+                                reason="the original project is not reachable (WF_REFERENCE_ROOT or oracle/_ref)")
 
 
 def _scenarios():
