@@ -33,7 +33,8 @@
 extern "C" {
 #endif
 
-#define WF_ABI_VERSION 2 /* 2: + wf_reset_host, wf_host_session(_active), wf_get/set_a_iter, wf_tile_geometry, wf_apply_change_blocks (additions only) */
+#define WF_ABI_VERSION 2 /* 2: + wf_reset_host, wf_host_session(_active), wf_get/set_a_iter, wf_tile_geometry, wf_apply_change_blocks;
+                            later, still 2: + WF_OBS_BITS, wf_unpack_obs_bits (additions only) */
 
 enum {
     WF_OK = 0,
@@ -43,8 +44,15 @@ enum {
 };
 
 /* Observation element type written by wf_reset / wf_step / wf_rollout / wf_step_host / wf_get_obs: the 0 / 1 values of
- * World.get_state (environment.py:399-402) as uint8, float32, or bfloat16 (1.0 = 0x3F80) for a bf16 learner. */
-enum { WF_OBS_U8 = 0, WF_OBS_F32 = 1, WF_OBS_BF16 = 2 };
+ * World.get_state (environment.py:399-402) as uint8, float32, or bfloat16 (1.0 = 0x3F80) for a bf16 learner, or packed
+ * one bit per element (WF_OBS_BITS, 8x smaller than uint8):
+ *   - every env takes ceil(W*H*3 / 32) little-endian uint32 words and starts on a word boundary: obs is [N][words]
+ *     ([K][N][words] for a rollout) in place of [N][W][H][3];
+ *   - element k = (x*H + y)*3 + c (the order of [W][H][3], i.e. Keras' Flatten) is bit k % 32 of word k / 32;
+ *   - the padding bits after element W*H*3 - 1 are zero.
+ * On a little-endian host np.unpackbits(obs.view(np.uint8), axis=-1, bitorder="little")[..., :W*H*3] is the uint8
+ * observation; on the device wf_unpack_obs_bits gathers and expands rows. */
+enum { WF_OBS_U8 = 0, WF_OBS_F32 = 1, WF_OBS_BF16 = 2, WF_OBS_BITS = 3 };
 
 /* Cell types -- Simulation/utility.py:128-140. */
 enum { WF_GRASS = 0, WF_FIRE = 1, WF_BURNT = 2, WF_DIRT = 3, WF_WATER = 4 };
@@ -158,6 +166,8 @@ int wf_set_policy_mlp(wf_env* env, const float* kernel1_host, const float* bias1
  * WF_HOST_TIMING=1 prints the launch / sync / expand split when the handle is destroyed; WF_HOST_GRAPH=1
  * (a_speed == 1 only) issues kernel + copy as one CUDA graph: 40.0-40.6 against 42.1 us per C2 step, tools/e2e_ab.py).
  * Fastest: wf_host_session below (23 us; 19 us with a persistent observation array), which also lifts the page-locked requirement.
+ * WF_OBS_BITS (both families): the kernel writes the packed observation to a staging buffer (or, with WF_HOST_MODE=direct,
+ * straight into page-locked obs_host) and one cudaMemcpyAsync brings it over; no host thread expands anything.
  * The device alias of each page-locked buffer is looked up once and re-validated every 1024 calls: a caller that
  * unpins or frees a buffer must not hand the same ADDRESS back as a different kind of memory within that window
  * (pass a new address, or destroy the handle). */
@@ -188,6 +198,10 @@ int wf_step_host(wf_env* env, const int32_t* actions_host, void* obs_host, int32
  * asks for every record in full whenever it differs, on the first step after the kernel was (re)started and hence after
  * every other entry point used in between.  What it cannot detect is the caller overwriting the array: then the patched
  * elements are right and the others stay as the caller left them until their record next travels in full.
+ * WF_OBS_BITS calls are served by the session too (uint8 and bits calls may alternate): the host threads copy each record's
+ * envs into obs_host [N][words], re-aligning the second env of a two-env record.  In mode 2 the changed elements are
+ * patched as bits in place (a host thread owns whole envs, so no two threads share a word); a call whose dtype differs
+ * from the previous call's asks for every record in full, like a new array.
  * Returns WF_ERR_INVALID for the tile family.  wf_host_session_active: 0 off, 1 on (kernel parked), 2 kernel resident. */
 int wf_host_session(wf_env* env, int32_t on);
 int wf_host_session_active(const wf_env* env);
@@ -232,6 +246,13 @@ int wf_set_a_iter(wf_env* env, int32_t a_iter);
 int wf_set_fire_to(wf_env* env, const int32_t* cells_dev, void* stream);
 /* World.get_state() without stepping. */
 int wf_get_obs(wf_env* env, void* obs_dev, int32_t obs_dtype, void* stream);
+
+/* Unpack WF_OBS_BITS rows to [n_out][W][H][3] u8 / f32 / bf16 (out_dtype WF_OBS_U8 / F32 / BF16): row i of out = bits row
+ * index[i] of bits_dev [n_rows][ceil(W*H*3 / 32)] (index_dev: n_out int64, NULL = rows 0..n_out-1) -- a minibatch drawn
+ * from a packed replay buffer.  An index outside [0, n_rows) yields an all-zero observation (never an out-of-bounds read).
+ * Needs no handle: runs on the current device, asynchronously on `stream`.  out_dev 16-byte aligned. */
+int wf_unpack_obs_bits(const uint32_t* bits_dev, int64_t n_rows, const int64_t* index_dev, int64_t n_out,
+                       int32_t width, int32_t height, void* out_dev, int32_t out_dtype, void* stream);
 
 /* Heat quanta table: coef[wind_id][4] float64 (host pointer), n_wind entries (1 or 27). */
 int wf_get_wind_table(const wf_env* env, double* coef_host, double* speed_host,

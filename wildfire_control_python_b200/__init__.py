@@ -6,10 +6,11 @@ launch; ``ForestFire`` is the single-env facade with the reference's attribute s
 The compute lives in ``libwildfire_b200.so`` (csrc/, sm_100a) behind include/wildfire.h.
 """
 from . import _lib
+from ._lib import obs_bits_words
 from .constants import METADATA, grass, layer, make_metadata, types
 
 __all__ = ["BatchedForestFire", "ForestFire", "METADATA", "grass", "layer", "types", "make_metadata", "build",
-           "DQN", "DQN_SARSA", "DQN_DUEL", "DQN_BOTH"]
+           "DQN", "DQN_SARSA", "DQN_DUEL", "DQN_BOTH", "obs_bits_words", "unpack_obs"]
 
 
 def build(force: bool = False, verbose: bool = False) -> str:
@@ -20,6 +21,9 @@ def __getattr__(name):  # torch is imported lazily so that `import wildfire_cont
     if name == "BatchedForestFire":
         from .batched import BatchedForestFire
         return BatchedForestFire
+    if name == "unpack_obs":
+        from .batched import unpack_obs
+        return unpack_obs
     if name == "ForestFire":
         from .compat import ForestFire
         return ForestFire

@@ -16,11 +16,16 @@ LIB_PATH = os.environ.get("WILDFIRE_B200_LIB") or os.path.join(HERE, "libwildfir
 CSRC = os.path.join(HERE, "csrc")
 
 WF_OK, WF_ERR_INVALID, WF_ERR_CUDA, WF_ERR_STATE = 0, -1, -2, -3
-WF_OBS_U8, WF_OBS_F32, WF_OBS_BF16 = 0, 1, 2
+WF_OBS_U8, WF_OBS_F32, WF_OBS_BF16, WF_OBS_BITS = 0, 1, 2, 3
 WF_POLICY_STREAM, WF_POLICY_WALK, WF_POLICY_MLP = 0, 1, 2
 WF_NSCALARS = 16
 (S_ALIVE, S_AX, S_AY, S_DEAD, S_DIGGING, S_VISIBLE, S_RUNNING, S_FIRE_AT_BORDER, S_LATCHED, S_EPISODE, S_T,
  S_WIND_ID, S_WIND_X, S_WIND_Y, S_N_BURNING, S_RESERVED) = range(16)
+
+
+def obs_bits_words(width: int, height: int) -> int:
+    """uint32 words of one env's WF_OBS_BITS observation: ceil(W*H*3 / 32) (include/wildfire.h)."""
+    return (int(width) * int(height) * 3 + 31) // 32
 
 
 class WfConfig(C.Structure):
@@ -110,6 +115,8 @@ def lib():
     L.wf_apply_change_blocks.argtypes = [vp, vp, C.c_int32, vp, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_double,
                                          C.c_double, C.c_int32]
     L.wf_apply_change_blocks.restype = C.c_int
+    L.wf_unpack_obs_bits.argtypes = [vp, C.c_int64, vp, C.c_int64, C.c_int32, C.c_int32, vp, C.c_int32, vp]
+    L.wf_unpack_obs_bits.restype = C.c_int
     L.wf_state_bytes_per_env.argtypes = [vp]
     L.wf_state_bytes_per_env.restype = C.c_int64
     for name in ("wf_create", "wf_reset", "wf_step", "wf_rollout", "wf_rollout_policy", "wf_set_policy_mlp", "wf_step_host", "wf_get_state", "wf_set_state",
@@ -129,4 +136,5 @@ EXPORTED_SYMBOLS = [
     "wf_reset", "wf_step", "wf_rollout", "wf_rollout_policy", "wf_set_policy_mlp", "wf_step_host", "wf_get_state", "wf_set_state", "wf_set_fire_to",
     "wf_get_obs", "wf_get_wind_table", "wf_stats", "wf_stats_reset", "wf_philox_kat", "wf_launch_count",
     "wf_state_bytes_per_env", "wf_host_threads", "wf_expand_packed_obs", "wf_apply_change_blocks", "wf_get_a_iter", "wf_set_a_iter", "wf_reset_host", "wf_tile_geometry", "wf_host_session", "wf_host_session_active",
+    "wf_unpack_obs_bits",
 ]

@@ -50,6 +50,38 @@ def config_from_metadata(m: dict) -> "_lib.WfConfig":
     return cfg
 
 
+_UNPACK_CODES = {torch.uint8: _lib.WF_OBS_U8, torch.float32: _lib.WF_OBS_F32, torch.bfloat16: _lib.WF_OBS_BF16}
+
+
+def unpack_obs(bits: torch.Tensor, width: int, height: int, index=None, dtype: torch.dtype = torch.float32) -> torch.Tensor:
+    """``"bits"`` observations -> ``[n, W, H, 3]`` of ``dtype`` (uint8, float32 or bfloat16) on the device, by
+    ``wf_unpack_obs_bits`` on the current stream.
+
+    ``bits``: ``[rows, words]`` int32 CUDA tensor (a ``[K, N, words]`` rollout: ``.view(-1, words)``).  ``index``: optional
+    ``[n]`` row numbers (repeats and any order allowed; a row outside ``[0, rows)`` gives an all-zero observation), e.g. a
+    minibatch drawn from a packed replay buffer; ``None`` = every row.  ``unpack_obs(...).flatten(1)`` feeds the reference's
+    networks unchanged.
+    """
+    if dtype not in _UNPACK_CODES:
+        raise ValueError("dtype must be torch.uint8, torch.float32 or torch.bfloat16")
+    words = _lib.obs_bits_words(width, height)
+    if not (isinstance(bits, torch.Tensor) and bits.is_cuda and bits.dtype == torch.int32 and bits.dim() == 2
+            and bits.shape[1] == words):
+        raise ValueError(f"bits must be an int32 CUDA tensor of shape [rows, {words}]")
+    bits = bits.contiguous()
+    idx = None
+    if index is not None:
+        idx = torch.as_tensor(index, device=bits.device).to(torch.int64).contiguous()
+        if idx.dim() != 1:
+            raise ValueError("index must be one-dimensional")
+    n = bits.shape[0] if idx is None else idx.shape[0]
+    with torch.cuda.device(bits.device):
+        out = torch.empty((n, int(width), int(height), 3), dtype=dtype, device=bits.device)
+        _lib.check(_lib.lib().wf_unpack_obs_bits(_ptr(bits), bits.shape[0], _ptr(idx), n, int(width), int(height), _ptr(out),
+                                                 _UNPACK_CODES[dtype], C.c_void_p(torch.cuda.current_stream(bits.device).cuda_stream)))
+    return out
+
+
 class BatchedForestFire:
     """``n_envs`` reference environments on one GPU.
 
@@ -62,9 +94,13 @@ class BatchedForestFire:
     Observations are ``[N, W, H, 3]`` (x is the slow axis, exactly ``World.get_state``'s layout,
     environment.py:399-402) so ``obs.flatten(1)`` feeds the reference's ``Flatten`` + ``Dense``
     networks unchanged (DQN.py:209-212).
+
+    ``obs_dtype="bits"``: observations are packed one bit per element (``WF_OBS_BITS``, include/wildfire.h),
+    ``[N, obs_bits_words(W, H)]`` ``torch.int32`` tensors holding the uint32 bit patterns, 8x smaller than uint8;
+    ``unpack_obs`` turns rows of them back into ``[n, W, H, 3]`` on the device.
     """
 
-    def __init__(self, n_envs: int, device=None, obs_dtype: torch.dtype = torch.uint8, **metadata):
+    def __init__(self, n_envs: int, device=None, obs_dtype=torch.uint8, **metadata):
         if not torch.cuda.is_available():
             raise _lib.WildfireError("BatchedForestFire needs a CUDA device (no CPU fallback)")
         self.METADATA = make_metadata(**metadata)
@@ -76,11 +112,12 @@ class BatchedForestFire:
         self.device = dev
         self.width, self.height = int(m["width"]), int(m["height"])
         self.n_actions = int(m["n_actions"])
-        codes = {torch.uint8: _lib.WF_OBS_U8, torch.float32: _lib.WF_OBS_F32, torch.bfloat16: _lib.WF_OBS_BF16}
+        codes = {torch.uint8: _lib.WF_OBS_U8, torch.float32: _lib.WF_OBS_F32, torch.bfloat16: _lib.WF_OBS_BF16, "bits": _lib.WF_OBS_BITS}
         if obs_dtype not in codes:
-            raise ValueError("obs_dtype must be torch.uint8, torch.float32 or torch.bfloat16")
+            raise ValueError('obs_dtype must be torch.uint8, torch.float32, torch.bfloat16 or "bits"')
         self.obs_dtype = obs_dtype
         self._obs_code = codes[obs_dtype]
+        self.obs_bits = self._obs_code == _lib.WF_OBS_BITS
 
         L = _lib.lib()
         self._cfg = config_from_metadata(m)
@@ -91,7 +128,7 @@ class BatchedForestFire:
 
         N, W, H = self.n_envs, self.width, self.height
         with torch.cuda.device(self.device):
-            self._obs = torch.empty((N, W, H, 3), dtype=obs_dtype, device=self.device)
+            self._obs = torch.empty(self._obs_shape(N), dtype=self._obs_torch_dtype, device=self.device)
             self._reward = torch.empty((N,), dtype=torch.float64, device=self.device)
             self._done = torch.empty((N,), dtype=torch.uint8, device=self.device)
         self._done_bool = self._done.view(torch.bool)
@@ -122,6 +159,18 @@ class BatchedForestFire:
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
+    @property
+    def obs_words(self) -> int:
+        """int32 words per env of a ``"bits"`` observation (``obs_bits_words(width, height)``)."""
+        return _lib.obs_bits_words(self.width, self.height)
+
+    def _obs_shape(self, *lead):
+        return (*lead, self.obs_words) if self.obs_bits else (*lead, self.width, self.height, 3)
+
+    @property
+    def _obs_torch_dtype(self):
+        return torch.int32 if self.obs_bits else self.obs_dtype
+
     def _as_i32(self, t, shape):
         if not (isinstance(t, torch.Tensor) and t.dtype == torch.int32 and t.is_cuda and t.is_contiguous()):
             t = torch.as_tensor(t, device=self.device).to(torch.int32).contiguous()
@@ -134,7 +183,7 @@ class BatchedForestFire:
         """``ForestFire.reset()`` (forest_fire.py:52-54) for every env, or those with ``mask[n] != 0``.
 
         ``starts``: optional ``[N, 2]`` int agent start cells (negative x = draw from the stream).
-        Returns the observation batch ``[N, W, H, 3]``.
+        Returns the observation batch ``[N, W, H, 3]`` (``"bits"``: ``[N, words]``).
         """
         m = None
         if mask is not None:
@@ -169,7 +218,8 @@ class BatchedForestFire:
         demonstration / Baseline policy ``DQN.choose_randomwalk_action``, DQN.py:353-389) or ``"mlp"``
         (the Q-network given to ``set_policy_mlp``, eps-greedy, evaluated inside the step kernel).
         ``out``: optional ``(obs_or_None, reward, done_u8)`` buffers to write into.
-        Returns ``(obs [K,N,W,H,3] or None, reward [K,N], done [K,N])`` (+ ``actions [K,N]`` if asked).
+        Returns ``(obs [K,N,W,H,3] or None, reward [K,N], done [K,N])`` (+ ``actions [K,N]`` if asked);
+        with ``obs_dtype="bits"`` obs is ``[K, N, words]`` int32.
         """
         K, N = int(k_steps), self.n_envs
         a = None if actions is None else self._as_i32(actions, (K, N))
@@ -177,9 +227,11 @@ class BatchedForestFire:
         with torch.cuda.device(self.device):
             if out is not None:
                 o, r, d = out
+                if self.obs_bits and o is not None and (tuple(o.shape) != self._obs_shape(K, N) or o.dtype != torch.int32
+                                                        or not o.is_contiguous()):
+                    raise ValueError(f"out obs must be a contiguous int32 tensor of shape {self._obs_shape(K, N)}")
             else:
-                o = (torch.empty((K, N, self.width, self.height, 3), dtype=self.obs_dtype, device=self.device)
-                     if obs else None)
+                o = torch.empty(self._obs_shape(K, N), dtype=self._obs_torch_dtype, device=self.device) if obs else None
                 r = torch.empty((K, N), dtype=torch.float64, device=self.device)
                 d = torch.empty((K, N), dtype=torch.uint8, device=self.device)
             L = _lib.lib()
@@ -212,15 +264,18 @@ class BatchedForestFire:
         """Host-buffer step through ``wf_step_host``: H2D actions, step, D2H obs/reward/done, sync.
 
         Uses page-locked staging arrays owned by this object; returns numpy views of them (numpy has no
-        bfloat16: with ``obs_dtype=torch.bfloat16`` the observation is the pinned torch tensor itself).
+        bfloat16: with ``obs_dtype=torch.bfloat16`` the observation is the pinned torch tensor itself;
+        ``"bits"``: a ``uint32`` ``[N, words]`` array).
         """
         if self._host is None:
-            N, W, H = self.n_envs, self.width, self.height
+            N = self.n_envs
             t = dict(actions=torch.empty((N,), dtype=torch.int32).pin_memory(),
-                     obs=torch.empty((N, W, H, 3), dtype=self.obs_dtype).pin_memory(),
+                     obs=torch.empty(self._obs_shape(N), dtype=self._obs_torch_dtype).pin_memory(),
                      reward=torch.empty((N,), dtype=torch.float64).pin_memory(),
                      done=torch.empty((N,), dtype=torch.uint8).pin_memory())
-            self._host = dict(tensors=t, np_actions=t["actions"].numpy(), np_obs=t["obs"] if self.obs_dtype == torch.bfloat16 else t["obs"].numpy(),
+            np_obs = (t["obs"] if self.obs_dtype == torch.bfloat16 else
+                      t["obs"].numpy().view(np.uint32) if self.obs_bits else t["obs"].numpy())
+            self._host = dict(tensors=t, np_actions=t["actions"].numpy(), np_obs=np_obs,
                               np_reward=t["reward"].numpy(), np_done=t["done"].numpy().view(np.bool_),
                               ptrs=tuple(t[k].data_ptr() for k in ("actions", "obs", "reward", "done")),
                               fn=_lib.lib().wf_step_host)

@@ -30,7 +30,7 @@ bool hostpool_expand_session(HostPool* p, const uint32_t* packed, uint8_t* out, 
                              int64_t env_bits, int64_t envs_per_record, int64_t n_envs, const volatile uint32_t* flags,
                              uint32_t seq, int64_t records_per_slice, double* reward, uint8_t* done, double default_reward,
                              double death_penalty, double contained_bonus, double cells, int64_t timeout_ns, int64_t sectors,
-                             const uint32_t* full_area, int64_t full_stride);
+                             const uint32_t* full_area, int64_t full_stride, bool out_bits);
 int hostpool_default_threads();
 double hostpool_first_flag_seconds(const HostPool* p);
 }  // namespace wf
@@ -131,6 +131,7 @@ struct wf_env {
         uint32_t* full_dev;
         int full_stride;
         const void* frame_ptr;      // the caller's observation array as of the last step served (nullptr: not in step with it)
+        int32_t frame_dtype;        // ... and its obs_dtype (WF_OBS_U8 or WF_OBS_BITS)
         int64_t full_frames;        // steps that asked for every record in full
         int64_t launches, steps, relaunch_races;
     } sess;
@@ -271,6 +272,83 @@ __global__ void get_obs_kernel(DevState s, void* obs, int dtype) {
         } else {
             float* o = static_cast<float*>(obs) + 3 * i;
             o[0] = (float)a; o[1] = (float)f; o[2] = (float)d;
+        }
+    }
+}
+
+// wf_get_obs with WF_OBS_BITS: one thread per output word (padding bits after the env's last element stay 0).
+__global__ void get_obs_bits_kernel(DevState s, uint32_t* obs) {
+    const int nbits = s.W * s.H * 3;
+    const int64_t wpe = obs_bits_words(s.W, s.H), words = (int64_t)s.N * wpe;
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < words; i += (int64_t)gridDim.x * blockDim.x) {
+        const int env = (int)(i / wpe), k0 = (int)(i - env * wpe) * 32;
+        const int32_t* sc = s.scal + (size_t)env * WF_NSCALARS;
+        const int aidx = sc[WF_S_VISIBLE] ? (sc[WF_S_AX] * s.H + sc[WF_S_AY]) * 3 : -1;  // the agent_pos element
+        uint32_t v = 0u;
+        for (int b = 0; b < 32 && k0 + b < nbits; ++b) {
+            const int k = k0 + b, cell = k / 3, c = k - 3 * cell, x = cell / s.H, y = cell - x * s.H;
+            uint32_t bit;
+            if (c == 0) bit = k == aidx ? 1u : 0u;
+            else if (c == 1) bit = (s.planes[word_index(s, P_F, env, x, y >> 5)] >> (y & 31)) & 1u;
+            else bit = ((s.planes[word_index(s, P_I, env, x, y >> 5)] >> (y & 31)) & 1u) ^ 1u;
+            v |= bit << b;
+        }
+        obs[i] = v;
+    }
+}
+
+// wf_unpack_obs_bits: one warp per output row.  Lane l expands 16-bit chunk c = l + 32 t of the row into 16 elements with
+// 16-byte stores (uint8: two look-ups in the byte -> 8 bytes table); rows whose elements are not 16-byte aligned (e.g.
+// 14x14x3 = 588 bytes) and a row's ragged tail are written element by element.
+__device__ __forceinline__ uint32_t unpack_bf16_pair(uint32_t bytes, uint32_t sel) {  // two 0/1 bytes -> two bfloat16
+    return __byte_perm(bytes, 0u, sel) * (uint32_t)kBf16One;
+}
+__global__ void unpack_obs_bits_kernel(const uint32_t* __restrict__ bits, int64_t n_rows, const int64_t* __restrict__ index,
+                                       int64_t n_out, int W, int H, void* out, int dtype) {
+    __shared__ uint2 tab8[256];  // bit i of the index -> byte i
+    for (int v = threadIdx.x; v < 256; v += blockDim.x)
+        tab8[v] = make_uint2(((v & 15u) * 0x00204081u) & 0x01010101u, (((v >> 4) & 15u) * 0x00204081u) & 0x01010101u);
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const int nbits = W * H * 3;
+    const int64_t wpe = obs_bits_words(W, H);
+    const int esz = obs_elem_bytes(dtype);
+    const bool vec = ((int64_t)nbits * esz) % 16 == 0;  // every row starts 16-byte aligned (out is)
+    const int nfull = vec ? nbits / 16 : 0;             // whole 16-element chunks
+    const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    for (int64_t i = blockIdx.x * (int64_t)(blockDim.x >> 5) + (threadIdx.x >> 5); i < n_out; i += warps) {
+        const int64_t r = index ? index[i] : i;
+        const bool ok = r >= 0 && r < n_rows;
+        const uint16_t* src = reinterpret_cast<const uint16_t*>(bits + (ok ? r : 0) * wpe);
+        auto chunk = [&](int c) -> uint32_t { return ok ? (uint32_t)__ldg(src + c) : 0u; };
+        auto bit = [&](int k) -> uint32_t { return ok ? (__ldg(bits + r * wpe + (k >> 5)) >> (k & 31)) & 1u : 0u; };
+        if (dtype == WF_OBS_U8) {
+            uint8_t* o = static_cast<uint8_t*>(out) + i * nbits;
+            for (int c = lane; c < nfull; c += 32) {
+                const uint32_t b = chunk(c);
+                const uint2 lo = tab8[b & 255u], hi = tab8[b >> 8];
+                reinterpret_cast<uint4*>(o)[c] = make_uint4(lo.x, lo.y, hi.x, hi.y);
+            }
+            for (int k = 16 * nfull + lane; k < nbits; k += 32) o[k] = (uint8_t)bit(k);
+        } else if (dtype == WF_OBS_BF16) {  // 8 elements (one byte of bits) per 16-byte store
+            uint16_t* o = static_cast<uint16_t*>(out) + i * nbits;
+            const uint8_t* s8 = reinterpret_cast<const uint8_t*>(src);
+            for (int c = lane; c < 2 * nfull; c += 32) {
+                const uint2 t = tab8[ok ? __ldg(s8 + c) : 0];
+                reinterpret_cast<uint4*>(o)[c] = make_uint4(unpack_bf16_pair(t.x, 0x4140u), unpack_bf16_pair(t.x, 0x4342u),
+                                                            unpack_bf16_pair(t.y, 0x4140u), unpack_bf16_pair(t.y, 0x4342u));
+            }
+            for (int k = 16 * nfull + lane; k < nbits; k += 32) o[k] = bit(k) ? kBf16One : (uint16_t)0;
+        } else {  // 4 elements (one nibble) per 16-byte store
+            float* o = static_cast<float*>(out) + i * nbits;
+            const uint8_t* s8 = reinterpret_cast<const uint8_t*>(src);
+            constexpr uint32_t ONE = 0x3F800000u;
+            for (int c = lane; c < 4 * nfull; c += 32) {
+                const uint32_t nib = ok ? ((uint32_t)__ldg(s8 + (c >> 1)) >> ((c & 1) * 4)) : 0u;
+                reinterpret_cast<uint4*>(o)[c] =
+                    make_uint4((nib & 1u) ? ONE : 0u, (nib & 2u) ? ONE : 0u, (nib & 4u) ? ONE : 0u, (nib & 8u) ? ONE : 0u);
+            }
+            for (int k = 16 * nfull + lane; k < nbits; k += 32) o[k] = bit(k) ? 1.0f : 0.0f;
         }
     }
 }
@@ -503,7 +581,7 @@ int wf_apply_change_blocks(const uint32_t* blocks_host, const uint32_t* full_are
     HostPool* p = hostpool_create(threads);
     const bool ok = hostpool_expand_session(p, blocks_host, obs_host, records, rec_words, env_bits, epw, n_envs, flag, 1u, records,
                                             reward_host, done_host, default_reward, death_penalty, contained_bonus,
-                                            (double)(width * height), 1000000000, 0, full_area_host, full_stride);
+                                            (double)(width * height), 1000000000, 0, full_area_host, full_stride, false);
     hostpool_destroy(p);
     return ok ? WF_OK : fail(WF_ERR_STATE, "wf_apply_change_blocks: timed out");
 }
@@ -534,9 +612,12 @@ static void note_dev_call(wf_env* e, cudaStream_t st) {
     e->dev_pending = true;
 }
 
+static bool public_obs_dtype(int32_t dtype) {
+    return dtype == WF_OBS_U8 || dtype == WF_OBS_F32 || dtype == WF_OBS_BF16 || dtype == WF_OBS_BITS;
+}
 static int check_obs(const void* obs, int32_t dtype) {
-    if (dtype != WF_OBS_U8 && dtype != WF_OBS_F32 && dtype != WF_OBS_BF16 && dtype != kObsPacked)
-        return fail(WF_ERR_INVALID, "obs_dtype must be WF_OBS_U8, WF_OBS_F32 or WF_OBS_BF16");
+    if (!public_obs_dtype(dtype) && dtype != kObsPacked)
+        return fail(WF_ERR_INVALID, "obs_dtype must be WF_OBS_U8, WF_OBS_F32, WF_OBS_BF16 or WF_OBS_BITS");
     if (obs && (reinterpret_cast<uintptr_t>(obs) & 15u)) return fail(WF_ERR_INVALID, "obs pointer must be 16-byte aligned");
     return WF_OK;
 }
@@ -713,11 +794,11 @@ static int ensure_obs_staging(wf_env* e, size_t obs_bytes) {
 // ForestFire.reset() for a caller that only has host memory (INTEGRATION.md section 3).
 int wf_reset_host(wf_env* e, const uint8_t* mask_host, const wf_init* init_host, void* obs_host, int32_t obs_dtype) {
     if (!e) return fail(WF_ERR_INVALID, "null handle");
-    if (obs_dtype != WF_OBS_U8 && obs_dtype != WF_OBS_F32 && obs_dtype != WF_OBS_BF16) return fail(WF_ERR_INVALID, "bad obs_dtype");
+    if (!public_obs_dtype(obs_dtype)) return fail(WF_ERR_INVALID, "bad obs_dtype");
     WF_ON_DEVICE(e);
     WF_QUIESCE(e);
     const DevState& s = e->st;
-    const size_t obs_bytes = (size_t)s.N * s.W * s.H * 3 * obs_elem_bytes(obs_dtype);
+    const size_t obs_bytes = obs_step_bytes(s.N, s.W, s.H, obs_dtype);
     if (int rc = host_prologue(e)) return rc;
     if ((mask_host || init_host) && !e->h_mask) {
         WF_CUDA(cudaMalloc(&e->h_mask, (size_t)s.N));
@@ -770,7 +851,8 @@ static int session_launch(wf_env* e) {
     return WF_OK;
 }
 
-static int session_step(wf_env* e, const int32_t* actions_host, void* obs_host, double* reward_host, uint8_t* done_host) {
+static int session_step(wf_env* e, const int32_t* actions_host, void* obs_host, int32_t obs_dtype, double* reward_host,
+                        uint8_t* done_host) {
     wf_env::Session& ss = e->sess;
     const DevState& s = e->st;
     const int epw = 32 / s.RS;
@@ -826,13 +908,13 @@ static int session_step(wf_env* e, const int32_t* actions_host, void* obs_host, 
         if (int rc = session_launch(e)) {
             ss.wanted = false;  // e.g. the batch is too large for a cooperative launch: the launch-per-step path serves it
             cudaGetLastError();
-            return wf_step_host(e, actions_host, obs_host, WF_OBS_U8, reward_host, done_host);
+            return wf_step_host(e, actions_host, obs_host, obs_dtype, reward_host, done_host);
         }
     }
     volatile uint32_t* ctl = ss.ctl;
     uint64_t db_flags = 0;
-    if (ss.persistent_obs) {  // another array than last step's (or none yet): ask for every record in full
-        const bool want_full = ss.frame_ptr != obs_host;
+    if (ss.persistent_obs) {  // another array or dtype than last step's (or none yet): ask for every record in full
+        const bool want_full = ss.frame_ptr != obs_host || ss.frame_dtype != obs_dtype;
         db_flags = want_full ? 1u : 0u;
         ss.full_frames += want_full ? 1 : 0;
         ss.frame_ptr = nullptr;  // (until this step has been delivered)
@@ -881,9 +963,13 @@ static int session_step(wf_env* e, const int32_t* actions_host, void* obs_host, 
         const bool ok = hostpool_expand_session(e->pool, ss.rec, static_cast<uint8_t*>(obs_host), records, rec_words, env_bits, epw,
                                                 s.N, ss.ctl + 32, ss.seq, rps, reward_host, done_host, e->cfg.default_reward,
                                                 e->cfg.death_penalty, e->cfg.contained_bonus, (double)(s.W * s.H), 200000,
-                                                ss.persistent_obs ? 0 : ss.sectors, ss.persistent_obs ? ss.full : nullptr, ss.full_stride);
+                                                ss.persistent_obs ? 0 : ss.sectors, ss.persistent_obs ? ss.full : nullptr, ss.full_stride,
+                                                obs_dtype == WF_OBS_BITS);
         if (ok) {
-            if (ss.persistent_obs) ss.frame_ptr = obs_host;
+            if (ss.persistent_obs) {
+                ss.frame_ptr = obs_host;
+                ss.frame_dtype = obs_dtype;
+            }
             ss.t_wait += std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count();
             e->a_iter = advance_a_iter(e, 1);  // (after the step: a relaunch below must start from the phase before it)
             return WF_OK;
@@ -934,11 +1020,12 @@ int wf_host_session_active(const wf_env* e) { return e ? (e->sess.wanted ? (e->s
 int wf_step_host(wf_env* e, const int32_t* actions_host, void* obs_host, int32_t obs_dtype, double* reward_host,
                  uint8_t* done_host) {
     if (!e || !actions_host) return fail(WF_ERR_INVALID, "null argument");
-    if (obs_dtype != WF_OBS_U8 && obs_dtype != WF_OBS_F32 && obs_dtype != WF_OBS_BF16) return fail(WF_ERR_INVALID, "bad obs_dtype");
+    if (!public_obs_dtype(obs_dtype)) return fail(WF_ERR_INVALID, "bad obs_dtype");
     WF_ON_DEVICE(e);
     const DevState& s = e->st;
-    const size_t obs_bytes = (size_t)s.N * s.W * s.H * 3 * obs_elem_bytes(obs_dtype);
-    if (e->sess.wanted && !e->tile && obs_host && obs_dtype == WF_OBS_U8) return session_step(e, actions_host, obs_host, reward_host, done_host);
+    const size_t obs_bytes = obs_step_bytes(s.N, s.W, s.H, obs_dtype);
+    if (e->sess.wanted && !e->tile && obs_host && (obs_dtype == WF_OBS_U8 || obs_dtype == WF_OBS_BITS))
+        return session_step(e, actions_host, obs_host, obs_dtype, reward_host, done_host);
     WF_QUIESCE(e);
     if (int rc = host_prologue(e)) return rc;
 
@@ -1135,9 +1222,35 @@ int wf_get_obs(wf_env* e, void* obs_dev, int32_t obs_dtype, void* stream) {
     WF_QUIESCE(e);
     const DevState& s = e->st;
     note_dev_call(e, static_cast<cudaStream_t>(stream));
-    get_obs_kernel<<<grid_for((size_t)s.N * s.W * s.H), 256, 0, static_cast<cudaStream_t>(stream)>>>(s, obs_dev, obs_dtype);
+    if (obs_dtype == WF_OBS_BITS)
+        get_obs_bits_kernel<<<grid_for((size_t)s.N * obs_bits_words(s.W, s.H)), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+            s, static_cast<uint32_t*>(obs_dev));
+    else
+        get_obs_kernel<<<grid_for((size_t)s.N * s.W * s.H), 256, 0, static_cast<cudaStream_t>(stream)>>>(s, obs_dev, obs_dtype);
     WF_CUDA(cudaGetLastError());
     e->launches += 1;
+    return WF_OK;
+}
+
+int wf_unpack_obs_bits(const uint32_t* bits_dev, int64_t n_rows, const int64_t* index_dev, int64_t n_out, int32_t width,
+                       int32_t height, void* out_dev, int32_t out_dtype, void* stream) {
+    if (out_dtype != WF_OBS_U8 && out_dtype != WF_OBS_F32 && out_dtype != WF_OBS_BF16)
+        return fail(WF_ERR_INVALID, "wf_unpack_obs_bits: out_dtype must be WF_OBS_U8, WF_OBS_F32 or WF_OBS_BF16");
+    if (width < 1 || height < 1) return fail(WF_ERR_INVALID, "wf_unpack_obs_bits: width and height must be >= 1");
+    if (n_out < 0 || n_rows < 0) return fail(WF_ERR_INVALID, "wf_unpack_obs_bits: n_out and n_rows must be >= 0");
+    if (n_out > 0 && (!out_dev || (n_rows > 0 && !bits_dev)))
+        return fail(WF_ERR_INVALID, "wf_unpack_obs_bits: null argument");
+    if (reinterpret_cast<uintptr_t>(out_dev) & 15u) return fail(WF_ERR_INVALID, "wf_unpack_obs_bits: out must be 16-byte aligned");
+    if (reinterpret_cast<uintptr_t>(bits_dev) & 3u) return fail(WF_ERR_INVALID, "wf_unpack_obs_bits: bits must be 4-byte aligned");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+        return fail(WF_ERR_CUDA, "no CUDA device: libwildfire_b200 has no CPU fallback");
+    if (n_out == 0) return WF_OK;
+    constexpr int kRowsPerBlock = 8;  // one warp per row
+    const int64_t blocks = std::min<int64_t>((n_out + kRowsPerBlock - 1) / kRowsPerBlock, 148 * 16);
+    unpack_obs_bits_kernel<<<(int)blocks, 32 * kRowsPerBlock, 0, static_cast<cudaStream_t>(stream)>>>(
+        bits_dev, n_rows, index_dev, n_out, width, height, out_dev, out_dtype);
+    WF_CUDA(cudaGetLastError());
     return WF_OK;
 }
 

@@ -60,6 +60,12 @@ constexpr uint32_t kDeltaFullBit = 0x8000u;
 
 // Bytes per observation element of a public obs_dtype (WF_OBS_U8 / WF_OBS_F32 / WF_OBS_BF16).
 __host__ __device__ __forceinline__ int obs_elem_bytes(int dtype) { return dtype == WF_OBS_F32 ? 4 : dtype == WF_OBS_BF16 ? 2 : 1; }
+// WF_OBS_BITS: uint32 words per env (include/wildfire.h: element k = (x*H + y)*3 + c is bit k % 32 of word k / 32).
+__host__ __device__ __forceinline__ int64_t obs_bits_words(int W, int H) { return ((int64_t)W * H * 3 + 31) / 32; }
+// Bytes of one step's observation block of N envs in a public obs_dtype (WF_OBS_U8 / F32 / BF16 / BITS).
+__host__ __device__ __forceinline__ size_t obs_step_bytes(int64_t N, int W, int H, int dtype) {
+    return dtype == WF_OBS_BITS ? (size_t)N * obs_bits_words(W, H) * 4 : (size_t)N * W * H * 3 * obs_elem_bytes(dtype);
+}
 constexpr uint16_t kBf16One = 0x3F80u;  // 1.0 in bfloat16
 
 enum Plane : int { P_G = 0, P_F, P_BT, P_D, P_WT, P_B, P_I, P_FU0 };  // + FB fuel planes (+ S0, S1, R for tiles)

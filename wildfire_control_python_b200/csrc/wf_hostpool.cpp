@@ -42,6 +42,7 @@ struct ExpandJob {
                                 // is complete in full_area[record * full_stride] instead
     int64_t sectors;            // session, != 0: each record is `sectors` self-validating 32-byte sectors (7 payload words + tag =
                                 // seq ^ hash), no flags: a record is taken as soon as all its sectors validate
+    bool out_bits;              // session: `out` is WF_OBS_BITS, uint32 [n_envs][ceil(env_bits / 32)], instead of bytes
 };
 
 static inline uint32_t sector_hash(const uint32_t* w) {  // == wf_common.cuh
@@ -189,9 +190,19 @@ static void apply_delta_records(const ExpandJob& j, int64_t r0, int64_t r1) {
 #endif
         const uint32_t hdr = blk[0];
         const int count = (int)(hdr & 0xffu);
-        uint8_t* out = j.out + 4 * b * rec_elems;
         const uint16_t* e = reinterpret_cast<const uint16_t*>(blk) + kFirstEntry;
-        for (int k = 0; k < count; ++k) out[e[k] >> 1] = (uint8_t)(e[k] & 1u);
+        if (j.out_bits) {  // the block's envs are whole envs of this thread: no other thread writes their words
+            const int64_t wpe = (j.env_bits + 31) / 32;
+            uint32_t* out = reinterpret_cast<uint32_t*>(j.out);
+            for (int k = 0; k < count; ++k) {
+                const int64_t g = 4 * b * rec_elems + (e[k] >> 1), env = g / j.env_bits, bit = g - env * j.env_bits;
+                uint32_t& w = out[env * wpe + (bit >> 5)];
+                w = (w & ~(1u << (bit & 31))) | ((uint32_t)(e[k] & 1u) << (bit & 31));
+            }
+        } else {
+            uint8_t* out = j.out + 4 * b * rec_elems;
+            for (int k = 0; k < count; ++k) out[e[k] >> 1] = (uint8_t)(e[k] & 1u);
+        }
         for (int w = 0; w < 4; ++w) {
             const int64_t r = 4 * b + w;
             if (r >= j.records) break;
@@ -208,8 +219,30 @@ static void apply_delta_records(const ExpandJob& j, int64_t r0, int64_t r1) {
     }
 }
 
+// WF_OBS_BITS: the envs of one record -> their own words (env k's stream starts at record bit k * env_bits: re-aligned to a
+// word boundary, padding bits cleared).
+static void copy_bits_one(const ExpandJob& j, const uint32_t* rec, int64_t env0, int64_t nenv) {
+    const int64_t wpe = (j.env_bits + 31) / 32;
+    const int tail = (int)(j.env_bits & 31);
+    uint32_t* out = reinterpret_cast<uint32_t*>(j.out) + env0 * wpe;
+    for (int64_t k = 0; k < nenv; ++k, out += wpe) {
+        const int64_t w0 = (k * j.env_bits) >> 5;
+        const int sh = (int)((k * j.env_bits) & 31);
+        for (int64_t q = 0; q < wpe; ++q) {
+            const uint32_t lo = rec[w0 + q], hi = w0 + q + 1 < j.rec_words ? rec[w0 + q + 1] : 0u;
+            uint32_t v = sh ? (lo >> sh) | (hi << (32 - sh)) : lo;
+            if (q == wpe - 1 && tail) v &= (1u << tail) - 1u;
+            out[q] = v;
+        }
+    }
+}
+
 // The observation bits of one record -> the bytes of its envs.
 static void expand_one(const ExpandJob& j, const uint32_t* rec, int64_t env0, int64_t nenv) {
+    if (j.out_bits) {
+        copy_bits_one(j, rec, env0, nenv);
+        return;
+    }
 #if defined(__x86_64__)
     static const bool bmi2 = __builtin_cpu_supports("bmi2");
     static const bool avx2 = bmi2 && __builtin_cpu_supports("avx2") && !getenv("WF_HOST_NO_AVX2");
@@ -384,13 +417,14 @@ void hostpool_expand(HostPool* p, const uint32_t* packed, uint8_t* out, int64_t 
     j.recs_per_block = 1; j.block_stride = rec_words;
     p->run(j);
 }
-// Session step: thread t waits for flags[16 * t] == seq, then expands records [t * records_per_slice, ...) and decodes
-// their status words into reward / done.  false: a flag did not come within timeout_ns.
+// Session step: thread t waits for flags[16 * t] == seq, then expands records [t * records_per_slice, ...) -- or, out_bits,
+// copies them into WF_OBS_BITS rows -- and decodes their status words into reward / done.  false: a flag did not come within
+// timeout_ns.
 bool hostpool_expand_session(HostPool* p, const uint32_t* packed, uint8_t* out, int64_t records, int64_t rec_words,
                              int64_t env_bits, int64_t envs_per_record, int64_t n_envs, const volatile uint32_t* flags,
                              uint32_t seq, int64_t records_per_slice, double* reward, uint8_t* done, double default_reward,
                              double death_penalty, double contained_bonus, double cells, int64_t timeout_ns, int64_t sectors,
-                             const uint32_t* full_area, int64_t full_stride) {
+                             const uint32_t* full_area, int64_t full_stride, bool out_bits) {
     ExpandJob j{};
     j.packed = packed; j.out = out; j.records = records; j.rec_words = rec_words; j.env_bits = env_bits;
     j.envs_per_record = envs_per_record; j.n_envs = n_envs; j.rec_stride = rec_words + 1;
@@ -401,6 +435,7 @@ bool hostpool_expand_session(HostPool* p, const uint32_t* packed, uint8_t* out, 
     j.default_reward = default_reward; j.death_penalty = death_penalty; j.contained_bonus = contained_bonus; j.cells = cells;
     j.timeout_ns = timeout_ns;
     j.full_area = full_area; j.full_stride = full_stride;
+    j.out_bits = out_bits;
     return p->run(j);
 }
 double hostpool_first_flag_seconds(const HostPool* p) { return p ? p->first_flag_seconds() : 0.0; }

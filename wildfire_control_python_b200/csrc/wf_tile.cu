@@ -786,10 +786,13 @@ __device__ __forceinline__ void emit_obs_slice(const Env& e, void* obs_step, int
     // cluster of 2).  384 words per warp exist whenever the wide path does (HW % 4 == 0 <=> VW == 4).
     uint32_t* stage = stage_all + warp * ((HW & 3) == 0 ? 384 : 96);  // 32 words x 96 bits
     const uint16_t* stage16 = reinterpret_cast<const uint16_t*>(stage);
+    // WF_OBS_BITS: the env's words.  With H % 32 == 0 word i's 96-bit stream is exactly output words 3i .. 3i+2.
+    uint32_t* const obits = static_cast<uint32_t*>(obs_step) + (size_t)e.env * obs_bits_words(W, H);
     int g_first = e.lo;
     if ((H & 31) == 0 && (HW & 3) == 0) {
-        // Two instantiations, so that the uint8 loop carries no per-iteration test of the element type.
-        auto wide = [&](auto is_u8) {
+        // One instantiation per element type, so that the loop carries no per-iteration test of it.
+        // kind: 0 uint8, 1 bfloat16 / float32, 2 WF_OBS_BITS
+        auto wide = [&](auto kind) {
             // Wide path: a warp takes 128 consecutive words (12 KB of output) per iteration with two 128-bit
             // loads per lane, issued one iteration ahead so that the expansion never waits on HBM.
             uint32_t* stage4 = stage_all + warp * 384;  // 128 words x 96 bits
@@ -831,7 +834,14 @@ __device__ __forceinline__ void emit_obs_slice(const Env& e, void* obs_step, int
                     st[2] = (p[2] >> 16) | (p[3] << 8);
                 }
                 __syncwarp();
-                if constexpr (decltype(is_u8)::value) {
+                if constexpr (decltype(kind)::value == 2) {
+                    // the staged stream as it is: 384 words, 12 bytes per plane word (HW % 4 == 0 and the groups start at
+                    // multiples of 4 words, so the destination is 16-byte aligned)
+                    uint4* o = reinterpret_cast<uint4*>(obits + 3 * (size_t)g);
+                    const uint4* s4 = reinterpret_cast<const uint4*>(stage4);
+#pragma unroll
+                    for (int it = 0; it < 3; ++it) __stcs(&o[it * 32 + lane], s4[it * 32 + lane]);
+                } else if constexpr (decltype(kind)::value == 0) {
                     uint4* o = reinterpret_cast<uint4*>(static_cast<uint8_t*>(obs_step) + (((size_t)e.env * W) * H + (size_t)32 * g) * 3);
 #pragma unroll 8
                     for (int it = 0; it < 24; ++it) {
@@ -848,7 +858,9 @@ __device__ __forceinline__ void emit_obs_slice(const Env& e, void* obs_step, int
             }
             g_first = e.lo + n128 * 128;  // the slice's tail (< 128 words) takes the narrow path
         };
-        if (obs_dtype == WF_OBS_U8) wide(std::true_type{}); else wide(std::false_type{});
+        if (obs_dtype == WF_OBS_U8) wide(std::integral_constant<int, 0>{});
+        else if (obs_dtype == WF_OBS_BITS) wide(std::integral_constant<int, 2>{});
+        else wide(std::integral_constant<int, 1>{});
     }
     const bool fast_ok = (H & 31) == 0;
     for (int g = g_first + warp * 32; g < e.hi; g += nwarps * 32) {
@@ -869,7 +881,30 @@ __device__ __forceinline__ void emit_obs_slice(const Env& e, void* obs_step, int
                 const int ncell = min(32, H - 32 * w);
                 const size_t e0 = (((size_t)e.env * W + x) * H + 32 * w) * 3;  // first output element of this word
                 const uint32_t r[3] = {r0, r1, r2};
-                if (obs_dtype == WF_OBS_U8) {
+                if (obs_dtype == WF_OBS_BITS) {
+                    // bits [b0, b1) of the env's stream; the env's last word also clears the padding after its last
+                    // element.  A word shared with a neighbouring thread -- or with another CTA of the cluster -- is
+                    // updated as clear-then-set over this thread's own bits only, which is right in any order and needs
+                    // no zeroed output.
+                    const int b0 = (int)(e0 - (size_t)e.env * W * H * 3), sh = b0 & 31, w0 = b0 >> 5;
+                    int b1 = b0 + 3 * ncell;
+                    if (x == W - 1 && w == HW - 1) b1 = (b1 + 31) & ~31;
+                    const int nq = ((b1 - 1) >> 5) - w0 + 1;  // <= 4 words
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) {
+                        if (q < nq) {
+                            const uint32_t v = __funnelshift_l(q > 0 ? r[q - 1] : 0u, q < 3 ? r[q] : 0u, sh);
+                            const int wb = 32 * (w0 + q), lo = max(b0, wb) - wb, n = min(b1, wb + 32) - wb - lo;
+                            const uint32_t m = n == 32 ? 0xffffffffu : ((1u << n) - 1u) << lo;
+                            if (m == 0xffffffffu) {
+                                obits[w0 + q] = v;
+                            } else {
+                                atomicAnd(&obits[w0 + q], ~m);
+                                atomicOr(&obits[w0 + q], v & m);
+                            }
+                        }
+                    }
+                } else if (obs_dtype == WF_OBS_U8) {
                     uint8_t* o8 = static_cast<uint8_t*>(obs_step) + e0;
                     for (int b = 0; b < 3 * ncell; ++b) o8[b] = (uint8_t)((r[b >> 5] >> (b & 31)) & 1u);
                 } else if (obs_dtype == WF_OBS_BF16) {
@@ -883,7 +918,11 @@ __device__ __forceinline__ void emit_obs_slice(const Env& e, void* obs_step, int
         }
         if (fast_ok && g + 31 < e.hi) {  // warp-uniform
             __syncwarp();
-            if (obs_dtype == WF_OBS_U8) {
+            if (obs_dtype == WF_OBS_BITS) {  // 32 plane words = 96 output words
+                uint32_t* o = obits + 3 * (size_t)g;
+#pragma unroll
+                for (int it = 0; it < 3; ++it) __stcs(&o[it * 32 + lane], stage[it * 32 + lane]);
+            } else if (obs_dtype == WF_OBS_U8) {
                 uint4* o = reinterpret_cast<uint4*>(static_cast<uint8_t*>(obs_step) + (((size_t)e.env * W) * H + (size_t)32 * g) * 3);
 #pragma unroll
                 for (int it = 0; it < 6; ++it) {
@@ -1744,7 +1783,7 @@ static TilePar make_par(const TileState* t, const DevState& s, int obs_dtype) {
     p.cells = s.W * s.H;
     p.pstride = (size_t)s.N * s.RS * s.HW;
     p.env_words = (size_t)s.RS * s.HW;
-    p.step_bytes = (size_t)s.N * s.W * s.H * 3 * obs_elem_bytes(obs_dtype);
+    p.step_bytes = obs_step_bytes(s.N, s.W, s.H, obs_dtype);
     p.overlap = t->overlap ? 1 : 0;
     return p;
 }

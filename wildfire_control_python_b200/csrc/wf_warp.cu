@@ -154,7 +154,8 @@ __device__ void reset_rows(Rows<FB>& r, Agent& a, const DevState& s, const StepC
 // 4-byte words of the output (coalesced 64/128-byte stores, ~7 instructions per word).
 constexpr int kStreamWords = 100;  // 3*32*32/32 = 96 words + spill-over of the last row's funnel shift
 
-template <int L, bool SRV = false>
+// OB: the WF_OBS_BITS instantiation (dtype == WF_OBS_BITS); the other element types never see its code.
+template <int L, bool SRV = false, bool OB = false>
 __device__ __forceinline__ void emit_obs(void* obs_step, int dtype, uint32_t arow, uint32_t frow, uint32_t freerow,
                                          uint32_t* stream, const uint32_t* spread3, const uint2* tab8, int lane, int sub,
                                          int x, int W, int H, int env0, int n_valid, uint32_t status16 = 0u) {
@@ -204,6 +205,20 @@ __device__ __forceinline__ void emit_obs(void* obs_step, int dtype, uint32_t aro
         } else {
             uint32_t* rec = static_cast<uint32_t*>(obs_step) + (size_t)(env0 / EPW) * rec_words;
             for (int w = lane; w < nw; w += 32) rec[w] = stream[w];
+        }
+        return;
+    }
+    if constexpr (OB) {
+        // The public format starts every env on a word boundary: output word j of env e (e = 0 or 1) is stream bits
+        // e * nbits + 32 j ..., with the bits past the env's last element cleared.  The warp's envs are n_valid * wpe
+        // consecutive output words, stored coalesced.
+        const int wpe = (nbits + 31) >> 5, tail = nbits & 31;
+        uint32_t* o = static_cast<uint32_t*>(obs_step) + (size_t)env0 * wpe;
+        for (int w = lane; w < n_valid * wpe; w += 32) {
+            const int e = w >= wpe ? 1 : 0, j = w - e * wpe, b = e * nbits + 32 * j;
+            uint32_t v = __funnelshift_r(stream[b >> 5], stream[(b >> 5) + 1], b & 31);
+            if (j == wpe - 1 && tail) v &= (1u << tail) - 1u;
+            o[w] = v;
         }
         return;
     }
@@ -274,7 +289,7 @@ __device__ __forceinline__ void st_release_gpu(uint32_t* p, uint32_t v) {
     asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
 
-template <int L, int FB, bool UNI, bool MLP, bool SRV>
+template <int L, int FB, bool UNI, bool MLP, bool SRV, bool OB>
 __device__ __forceinline__ void warp_body(const DevState& s, const StepCfg& c, const WarpIO& io, const SrvCtl& srv) {
     constexpr int EPW = 32 / L;  // envs per warp
     constexpr uint32_t FULL = 0xffffffffu;
@@ -358,7 +373,7 @@ __device__ __forceinline__ void warp_body(const DevState& s, const StepCfg& c, c
         }
         __syncwarp();
         if (io.obs != nullptr) {
-            emit_obs<L>(io.obs, io.obs_dtype, (a.vis && x == a.ax) ? (1u << a.ay) : 0u, r.F, ~r.I & validmask,
+            emit_obs<L, false, OB>(io.obs, io.obs_dtype, (a.vis && x == a.ax) ? (1u << a.ay) : 0u, r.F, ~r.I & validmask,
                         stream_warp, spread3, tab8, lane, sub, x, W, H, env0, n_valid);
         }
     } else {
@@ -892,9 +907,9 @@ __device__ __forceinline__ void warp_body(const DevState& s, const StepCfg& c, c
             } else if (io.obs != nullptr) {
                 const size_t step_bytes =
                     io.obs_dtype == kObsPacked ? (size_t)((s.N + EPW - 1) / EPW) * ((EPW * W * H * 3 + 31) >> 5) * 4
-                                               : (size_t)s.N * W * H * 3 * obs_elem_bytes(io.obs_dtype);
+                    : OB ? obs_step_bytes(s.N, W, H, WF_OBS_BITS) : (size_t)s.N * W * H * 3 * obs_elem_bytes(io.obs_dtype);
                 const int srv_stride = ((EPW * W * H * 3 + 31) >> 5) + 1;  // words per record incl. the status word
-                emit_obs<L, SRV>(SRV ? static_cast<void*>(srv_block + warp * srv_stride) : static_cast<char*>(io.obs) + (size_t)k * step_bytes,
+                emit_obs<L, SRV, OB>(SRV ? static_cast<void*>(srv_block + warp * srv_stride) : static_cast<char*>(io.obs) + (size_t)k * step_bytes,
                                  io.obs_dtype, (a.vis && x == a.ax) ? (1u << a.ay) : 0u, r.F, ~r.I & validmask, stream_warp, spread3, tab8,
                                  lane, sub, x, W, H, env0, n_valid, SRV ? (rkind | (done ? 8u : 0u) | (rcnt << 4)) : 0u);
             }
@@ -1020,19 +1035,21 @@ __device__ __forceinline__ void warp_body(const DevState& s, const StepCfg& c, c
 // registers a step costs 3.3 instead of 2.3 us).  ptxas lands there by itself and schedules better that way than under an
 // explicit cap (__launch_bounds__(128, 4): 115 registers, 2.52 us per step; A/B on one box, tools/build_variant.sh
 // -DWF_WARP_MINBLOCKS); the build checks the register count (csrc/Makefile, `make check-regs`).
-template <int L, int FB, bool UNI, bool MLP>
+// OB: WF_OBS_BITS observations -- a separate instantiation, because any extra code in the observation path of the C2 kernel
+// moves ptxas's schedule (with the bits path behind a run-time test the uint8 step took 2.15 instead of 1.97 us, same box).
+template <int L, int FB, bool UNI, bool MLP, bool OB>
 #ifdef WF_WARP_MINBLOCKS
 __global__ void __launch_bounds__(kWarpsPerBlock * 32, (MLP && !UNI) ? 8 / kWarpsPerBlock : 16 / kWarpsPerBlock)
 #else
 __global__ void __launch_bounds__(kWarpsPerBlock * 32)
 #endif
 warp_kernel(DevState s, StepCfg c, WarpIO io) {
-    warp_body<L, FB, UNI, MLP, false>(s, c, io, SrvCtl{});
+    warp_body<L, FB, UNI, MLP, false, OB>(s, c, io, SrvCtl{});
 }
 // The step server must be resident as a whole (cooperative launch): 128 registers at most.
 template <int L, int FB, bool UNI>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32, 16 / kWarpsPerBlock) warp_server_kernel(DevState s, StepCfg c, WarpIO io, SrvCtl srv) {
-    warp_body<L, FB, UNI, false, true>(s, c, io, srv);
+    warp_body<L, FB, UNI, false, true, false>(s, c, io, srv);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1045,7 +1062,12 @@ cudaError_t launch_warp_family(const DevState& s, const StepCfg& c, const WarpIO
     if (s.HB != 0 && (s.HB != kHitBits || s.FB != 5)) return cudaErrorInvalidValue;
     const bool mlp = io.policy == WF_POLICY_MLP && io.actions == nullptr && !io.reset_mode;
     if (mlp && (io.mlp.hid < 1 || io.mlp.hid > kHidMax || io.mlp.n_actions > kActMax)) return cudaErrorInvalidValue;
-#define WF_LAUNCH(LL, FF, UU, MM) warp_kernel<LL, FF, UU, MM><<<grid, block, 0, stream>>>(s, c, io)
+    const bool ob = io.obs != nullptr && io.obs_dtype == WF_OBS_BITS;
+#define WF_LAUNCH(LL, FF, UU, MM)                                                   \
+    do {                                                                            \
+        if (ob) warp_kernel<LL, FF, UU, MM, true><<<grid, block, 0, stream>>>(s, c, io);  \
+        else warp_kernel<LL, FF, UU, MM, false><<<grid, block, 0, stream>>>(s, c, io);    \
+    } while (0)
     if (mlp) {
         if (L == 16 && s.FB == 5 && s.HB) WF_LAUNCH(16, 5, true, true);
         else if (L == 32 && s.FB == 5 && s.HB) WF_LAUNCH(32, 5, true, true);

@@ -51,7 +51,7 @@ def gather_stats(local: Dict[str, int], device: Optional[torch.device] = None) -
 class ShardedForestFire:
     """This rank's slice of a global batch of ``n_total`` environments (one CUDA device per rank)."""
 
-    def __init__(self, n_total: int, device=None, **metadata):
+    def __init__(self, n_total: int, device=None, obs_dtype=torch.uint8, **metadata):
         from .batched import BatchedForestFire
         self.rank, self.world_size = dist_info()
         self.n_total = int(n_total)
@@ -60,7 +60,7 @@ class ShardedForestFire:
             raise ValueError("more ranks than environments")
         metadata = dict(metadata)
         metadata["env_id_base"] = int(metadata.get("env_id_base", 0)) + self.env_id_base
-        self.local = BatchedForestFire(self.n_local, device=device, **metadata)
+        self.local = BatchedForestFire(self.n_local, device=device, obs_dtype=obs_dtype, **metadata)
 
     def __getattr__(self, name):  # reset / step / rollout / get_state ... act on the local slice
         return getattr(self.local, name)
