@@ -34,7 +34,8 @@ extern "C" {
 #endif
 
 #define WF_ABI_VERSION 2 /* 2: + wf_reset_host, wf_host_session(_active), wf_get/set_a_iter, wf_tile_geometry, wf_apply_change_blocks;
-                            later, still 2: + WF_OBS_BITS, wf_unpack_obs_bits (additions only) */
+                            later, still 2: + WF_OBS_BITS, wf_unpack_obs_bits; + wf_set_policy_mlp_dev, wf_replay_fit
+                            (additions only) */
 
 enum {
     WF_OK = 0,
@@ -155,6 +156,15 @@ int wf_rollout_policy(wf_env* env, int32_t k_steps, int32_t policy, int32_t* act
  * hidden <= 64, n_actions <= 8. */
 int wf_set_policy_mlp(wf_env* env, const float* kernel1_host, const float* bias1_host, const float* kernel2_host,
                       const float* bias2_host, int32_t hidden, double eps);
+/* wf_set_policy_mlp from DEVICE tensors in nn.Linear orientation: weight1_dev [hidden][W*H*3], bias1_dev [hidden],
+ * weight2_dev [n_actions][hidden], bias2_dev [n_actions] (float32).  The repack into the kernel's layout runs as a kernel
+ * on `stream`: no host copy and no synchronisation, so a refresh queued behind a rollout on the same stream sees the
+ * weights that rollout's predecessors left and the next rollout on that stream sees the new ones.  The first call of a
+ * handle allocates the packed buffer (as wf_set_policy_mlp does), later calls overwrite it in place: a rollout still
+ * running on ANOTHER stream must be ordered by the caller.  The packed buffer is byte-identical to wf_set_policy_mlp's
+ * for the same weights (the empty-map sum is accumulated in float64 in the same order), so rollouts are too. */
+int wf_set_policy_mlp_dev(wf_env* env, const float* weight1_dev, const float* bias1_dev, const float* weight2_dev,
+                          const float* bias2_dev, int32_t hidden, double eps, void* stream);
 
 /* Host-buffer variant of wf_step (what a CPU-side caller of the reference would bind):
  * copies actions H2D, steps, copies obs/reward/done D2H and synchronises.  Buffers should
@@ -253,6 +263,52 @@ int wf_get_obs(wf_env* env, void* obs_dev, int32_t obs_dtype, void* stream);
  * Needs no handle: runs on the current device, asynchronously on `stream`.  out_dev 16-byte aligned. */
 int wf_unpack_obs_bits(const uint32_t* bits_dev, int64_t n_rows, const int64_t* index_dev, int64_t n_out,
                        int32_t width, int32_t height, void* out_dev, int32_t out_dtype, void* stream);
+
+/* ---- learning: n_replays consecutive DQN.replay updates (DQN.py:156-185, DQN_SARSA.py:103-132) in one launch ----
+ * The Q-network is Flatten(W, H, 3) -> Dense(hidden, sigmoid) -> Dense(n_actions) (DQN.make_network, DQN.py:209-233), or
+ * the dueling head (DQN_DUEL.py:18-48) with a value stream Flatten -> Dense(hidden, sigmoid) -> Dense(1) and
+ * q = v + (a - mean a).  Its parameters are ONE flat float32 buffer in torch.nn.utils.parameters_to_vector(model.parameters())
+ * order, nn.Linear orientation (weight[out][in]), n_in = width * height * 3:
+ *   dense_1.weight [hidden][n_in] | dense_1.bias [hidden] | dense_2.weight [n_actions][hidden] | dense_2.bias [n_actions]
+ *   dueling head, then: dense_3.weight [hidden][n_in] | dense_3.bias [hidden] | dense_4.weight [1][hidden] | dense_4.bias [1]
+ * i.e. (hidden * (n_in + 1 + n_actions) + n_actions) floats, plus (hidden * (n_in + 2) + 1) for the dueling head.  The
+ * target network and Adam's first and second moments m and v use the same layout. */
+typedef struct wf_mlp_shape {
+    int32_t width, height; /* observation grid of the warp family: 10 <= height <= width <= 32 */
+    int32_t hidden;        /* 1..64 units per stream */
+    int32_t n_actions;     /* 1..8 */
+    int32_t dueling;       /* 0: plain head, 1: dueling head */
+    int32_t batch;         /* transitions per replay, 1..256 */
+} wf_mlp_shape;
+
+/* Hyper-parameters of wf_replay_fit: the reference's gamma and Keras 2's Adam(lr, clipvalue) (agents.KerasAdam). */
+typedef struct wf_fit_params {
+    double gamma;
+    double lr, beta_1, beta_2, epsilon; /* epsilon is added to sqrt(v) of the uncorrected second moment (Keras) */
+    double clipvalue;                   /* every gradient element is clipped to +-clipvalue first (> 0; INFINITY: none) */
+    int64_t adam_t;                     /* updates made before this call: replay r uses t = adam_t + r + 1 */
+    int32_t target_every;               /* the model is copied into the target every target_every replays (>= 1) ... */
+    int32_t phase;                      /* ... after the replay that brings this counter (1..target_every) to zero:
+                                           the reference's until_sync */
+} wf_fit_params;
+
+/* Replay r (0 <= r < n_replays) is one fit_batch on transitions i = r * batch .. r * batch + batch - 1:
+ *   s = frames row s_row[i], s' = frames row sp_row[i] (frames_dev [n_frames][ceil(W*H*3 / 32)] WF_OBS_BITS rows);
+ *   target = Q_target(s) with entry action[i] replaced by reward[i] if done[i] else
+ *            reward[i] + gamma * (max_a Q_target(s', a), or Q_target(s', next_action[i]) when next_action_dev != NULL);
+ *   loss = mean over batch x n_actions of (Q_model(s) - target)^2; one clipped Keras Adam step on every parameter;
+ *   then the model is copied into the target if the replay brings the until_sync counter to zero.
+ * Out-of-range inputs never cause an out-of-bounds access: a row outside [0, n_frames) is an all-zero observation (as in
+ * wf_unpack_obs_bits); an action outside [0, n_actions) replaces no entry (the sample's target is Q_target(s)); a next
+ * action outside [0, n_actions) bootstraps nothing (the target entry is reward[i], as for a terminal transition).
+ * loss_dev [n_replays] may be NULL.  Runs as ONE thread-block cluster on the current device, asynchronously on `stream`;
+ * each CTA owns a slice of the hidden units and the result is deterministic (no floating-point atomics).
+ * Needs no handle; without a CUDA device it fails with WF_ERR_CUDA (no CPU fallback). */
+int wf_replay_fit(const wf_mlp_shape* shape, const wf_fit_params* params, int32_t n_replays, float* params_dev,
+                  float* target_dev, float* adam_m_dev, float* adam_v_dev, const uint32_t* frames_dev, int64_t n_frames,
+                  const int64_t* s_row_dev, const int64_t* sp_row_dev, const int32_t* action_dev,
+                  const int32_t* next_action_dev, const float* reward_dev, const uint8_t* done_dev, float* loss_dev,
+                  void* stream);
 
 /* Heat quanta table: coef[wind_id][4] float64 (host pointer), n_wind entries (1 or 27). */
 int wf_get_wind_table(const wf_env* env, double* coef_host, double* speed_host,

@@ -10,7 +10,7 @@ from ._lib import obs_bits_words
 from .constants import METADATA, grass, layer, make_metadata, types
 
 __all__ = ["BatchedForestFire", "ForestFire", "METADATA", "grass", "layer", "types", "make_metadata", "build",
-           "DQN", "DQN_SARSA", "DQN_DUEL", "DQN_BOTH", "obs_bits_words", "unpack_obs"]
+           "DQN", "DQN_SARSA", "DQN_DUEL", "DQN_BOTH", "obs_bits_words", "unpack_obs", "pack_obs"]
 
 
 def build(force: bool = False, verbose: bool = False) -> str:
@@ -21,9 +21,9 @@ def __getattr__(name):  # torch is imported lazily so that `import wildfire_cont
     if name == "BatchedForestFire":
         from .batched import BatchedForestFire
         return BatchedForestFire
-    if name == "unpack_obs":
-        from .batched import unpack_obs
-        return unpack_obs
+    if name in ("unpack_obs", "pack_obs"):
+        from . import batched
+        return getattr(batched, name)
     if name == "ForestFire":
         from .compat import ForestFire
         return ForestFire

@@ -44,6 +44,24 @@ class WfInit(C.Structure):
     _fields_ = [("ax", C.c_int32), ("ay", C.c_int32)]
 
 
+class WfMlpShape(C.Structure):
+    _fields_ = [("width", C.c_int32), ("height", C.c_int32), ("hidden", C.c_int32), ("n_actions", C.c_int32),
+                ("dueling", C.c_int32), ("batch", C.c_int32)]
+
+
+class WfFitParams(C.Structure):
+    _fields_ = [("gamma", C.c_double), ("lr", C.c_double), ("beta_1", C.c_double), ("beta_2", C.c_double),
+                ("epsilon", C.c_double), ("clipvalue", C.c_double), ("adam_t", C.c_int64), ("target_every", C.c_int32),
+                ("phase", C.c_int32)]
+
+
+def mlp_param_count(width: int, height: int, hidden: int, n_actions: int, dueling: bool) -> int:
+    """Floats of wf_replay_fit's flat parameter buffer (include/wildfire.h): parameters_to_vector(model.parameters())."""
+    n_in = int(width) * int(height) * 3
+    n = hidden * (n_in + 1 + n_actions) + n_actions
+    return n + (hidden * (n_in + 2) + 1 if dueling else 0)
+
+
 class WildfireError(RuntimeError):
     pass
 
@@ -88,6 +106,11 @@ def lib():
     L.wf_rollout.argtypes = [vp, C.c_int32, i32p, vp, C.c_int32, f64p, u8p, vp]
     L.wf_rollout_policy.argtypes = [vp, C.c_int32, C.c_int32, i32p, vp, C.c_int32, f64p, u8p, vp]
     L.wf_set_policy_mlp.argtypes = [vp, vp, vp, vp, vp, C.c_int32, C.c_double]
+    L.wf_set_policy_mlp_dev.argtypes = [vp, vp, vp, vp, vp, C.c_int32, C.c_double, vp]
+    L.wf_set_policy_mlp_dev.restype = C.c_int
+    L.wf_replay_fit.argtypes = [C.POINTER(WfMlpShape), C.POINTER(WfFitParams), C.c_int32, vp, vp, vp, vp, vp, C.c_int64,
+                                vp, vp, vp, vp, vp, vp, vp, vp]
+    L.wf_replay_fit.restype = C.c_int
     L.wf_step_host.argtypes = [vp, i32p, vp, C.c_int32, f64p, u8p]
     L.wf_reset_host.argtypes = [vp, u8p, vp, vp, C.c_int32]
     L.wf_host_session.argtypes = [vp, C.c_int32]
@@ -136,5 +159,5 @@ EXPORTED_SYMBOLS = [
     "wf_reset", "wf_step", "wf_rollout", "wf_rollout_policy", "wf_set_policy_mlp", "wf_step_host", "wf_get_state", "wf_set_state", "wf_set_fire_to",
     "wf_get_obs", "wf_get_wind_table", "wf_stats", "wf_stats_reset", "wf_philox_kat", "wf_launch_count",
     "wf_state_bytes_per_env", "wf_host_threads", "wf_expand_packed_obs", "wf_apply_change_blocks", "wf_get_a_iter", "wf_set_a_iter", "wf_reset_host", "wf_tile_geometry", "wf_host_session", "wf_host_session_active",
-    "wf_unpack_obs_bits",
+    "wf_unpack_obs_bits", "wf_set_policy_mlp_dev", "wf_replay_fit",
 ]

@@ -21,6 +21,7 @@ Keras is not a dependency; weights are saved as ``.npz`` with Keras' layer names
 """
 from __future__ import annotations
 
+import ctypes
 import json
 import os
 import math
@@ -609,26 +610,156 @@ class DQN:
         for _ in range(0, max_steps, chunk):
             _, rew, done = env.rollout(chunk, policy="mlp", obs=False)
             rew, done = rew.cpu().numpy(), done.cpu().numpy()
-            c = carry[None, :] + np.cumsum(rew, axis=0)
-            e_idx, k_idx = np.nonzero(done.T)  # episode ends, sorted by env then step
-            at_end = c[k_idx, e_idx]
+            e_idx, k_idx, ret, carry = _episode_ends(carry, rew, done)
             same = np.r_[False, e_idx[1:] == e_idx[:-1]]
-            ret = at_end - np.where(same, np.r_[0.0, at_end[:-1]], 0.0)
             first = np.r_[True, ~same[1:]] if len(e_idx) else np.zeros(0, bool)
             rank = np.arange(len(e_idx)) - np.maximum.accumulate(np.where(first, np.arange(len(e_idx)), 0))
             slot = n_done[e_idx] + rank
             keep = slot < episodes_per_env
             returns[e_idx[keep], slot[keep]] = ret[keep]
             died[e_idx[keep], slot[keep]] = rew[k_idx[keep], e_idx[keep]] == death_penalty
-            last = np.zeros(n_envs)
-            if len(e_idx):
-                is_last = np.r_[e_idx[1:] != e_idx[:-1], True]
-                last[e_idx[is_last]] = at_end[is_last]
-            carry = c[-1] - last
             n_done += np.bincount(e_idx, minlength=n_envs)
             if (n_done >= episodes_per_env).all():
                 return returns.flatten(), died.flatten()
         raise RuntimeError("evaluate_batched: some episodes did not finish")
+
+    # ------------------------------------------------------------------ batched learning on the device
+    def _flat_shape(self, batch):
+        from . import _lib
+        W, H = self.obs_shape[0], self.obs_shape[1]
+        return _lib.WfMlpShape(width=W, height=H, hidden=self.model.dense_1.out_features, n_actions=self.action_size,
+                               dueling=int(hasattr(self.model, "dense_3")), batch=int(batch))
+
+    def fit_batches_fused(self, frames, s_row, sp_row, a, ap, r, d, n_replays, phase=None):
+        """``n_replays`` consecutive ``fit_batch`` updates in ONE launch of ``wf_replay_fit`` (include/wildfire.h), the
+        same rule (targets from the target network, MSE, clipped Keras Adam) on packed observations.
+
+        ``frames``: ``[n_frames, words]`` int32 CUDA tensor of ``WF_OBS_BITS`` rows (``pack_obs`` / ``obs_dtype="bits"``);
+        ``s_row`` / ``sp_row``: int64 row numbers of S and S'; ``a`` / ``ap``: actions and next actions (``ap`` is used by
+        the on-policy learners only); ``r``: rewards; ``d``: done flags -- each of length ``n_replays * batch``, replay i
+        taking entries ``i * batch ...``.  A row outside ``frames`` is an all-zero observation, an action outside
+        ``[0, n_actions)`` replaces no target entry, an out-of-range next action bootstraps nothing.
+        The target network is refreshed every ``target_update`` replays as in ``learn``: ``phase`` (default: carried over
+        from the previous call, starting at ``target_update``) is the number of replays left until the next refresh.
+        ``model``, ``target`` and the optimiser's ``t``, ``m``, ``v`` are updated in place; returns the ``[n_replays]``
+        float32 losses (a device tensor: nothing is synchronised)."""
+        from torch.nn.utils import parameters_to_vector
+        from . import _lib
+        from .batched import _ptr
+        if self.device.type != "cuda":
+            raise _lib.WildfireError("fit_batches_fused needs a CUDA device (no CPU fallback)")
+        n_replays = int(n_replays)
+        if n_replays < 1 or len(s_row) % n_replays:
+            raise ValueError("the number of transitions must be a positive multiple of n_replays")
+        batch = len(s_row) // n_replays
+        dev = self.device
+        frames = frames.to(dev).contiguous()
+        if frames.dtype != torch.int32 or frames.dim() != 2:
+            raise ValueError("frames must be an int32 [n_frames, words] tensor")
+        cols = [torch.as_tensor(x, device=dev).to(dt).contiguous()
+                for x, dt in ((s_row, torch.int64), (sp_row, torch.int64), (a, torch.int32), (ap, torch.int32),
+                              (r, torch.float32), (d, torch.uint8))]
+        if any(c.shape != (n_replays * batch,) for c in cols):
+            raise ValueError("s_row, sp_row, a, ap, r and d must be one-dimensional and of the same length")
+        s_row, sp_row, a, ap, r, d = cols
+        params = list(self.model.parameters())
+        states = [self.optimizer.state[p] for p in params]
+        t0 = states[0]["t"] if states[0] else 0
+        with torch.no_grad():
+            flat = parameters_to_vector(params).contiguous()
+            tgt = parameters_to_vector(self.target.parameters()).contiguous()
+            m = parameters_to_vector([st["m"] for st in states]) if t0 else torch.zeros_like(flat)
+            v = parameters_to_vector([st["v"] for st in states]) if t0 else torch.zeros_like(flat)
+        group = self.optimizer.param_groups[0]
+        te = int(self.target_update_freq)
+        phase = int(getattr(self, "_until_sync", te) if phase is None else phase)
+        hp = _lib.WfFitParams(gamma=float(self.gamma), lr=group["lr"], beta_1=group["beta_1"], beta_2=group["beta_2"],
+                              epsilon=group["epsilon"], clipvalue=math.inf if group["clipvalue"] is None else group["clipvalue"],
+                              adam_t=t0, target_every=te, phase=phase)
+        loss = torch.empty(n_replays, dtype=torch.float32, device=dev)
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib().wf_replay_fit(
+                ctypes.byref(self._flat_shape(batch)), ctypes.byref(hp), n_replays, _ptr(flat), _ptr(tgt), _ptr(m), _ptr(v),
+                _ptr(frames), frames.shape[0], _ptr(s_row), _ptr(sp_row), _ptr(a), _ptr(ap) if self._SARSA else None,
+                _ptr(r), _ptr(d), _ptr(loss), ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
+        with torch.no_grad():
+            off = 0
+            for p, tp, st in zip(params, self.target.parameters(), states):
+                n = p.numel()
+                p.copy_(flat[off:off + n].view_as(p))
+                tp.copy_(tgt[off:off + n].view_as(p))
+                st["m"] = m[off:off + n].view_as(p).clone()
+                st["v"] = v[off:off + n].view_as(p).clone()
+                st["t"] = t0 + n_replays
+                off += n
+        self._until_sync = (phase - n_replays - 1) % te + 1
+        return loss
+
+    def learn_batched(self, n_episodes, n_envs=1024, k_steps=16, replays_per_launch=None, batch_size=None, seed=0):
+        """``learn`` over ``n_envs`` CUDA environments at once: the envs act with the eps-greedy Q-network evaluated inside
+        the step kernel (``rollout(policy="mlp")``, ``k_steps`` steps per launch), each rollout writes its packed
+        observations straight into a device replay ring, and after every launch ``replays_per_launch`` (default
+        ``k_steps``) replays of ``batch_size`` (default METADATA's) transitions run as one ``fit_batches_fused`` launch.
+        The in-kernel policy is refreshed on the device before every launch, with eps = min + (max - min) *
+        exp(-rate * episodes completed so far) (``decay_epsilon``).
+
+        Replay memory: the ring (``_PackedReplayRing``) holds at least the last ``memory_size`` transitions of every env
+        together (whole launches, at least two), plus every transition already in ``self.memory`` (demonstrations from ``collect_memories(_batched)``, kept for
+        the whole run like the reference's unbounded post-demonstration deque).  Each replay draws its batch uniformly
+        without replacement from both, on the device, from a generator seeded with ``seed``; replays start once more
+        than a batch of transitions exists.  The target network is refreshed every ``target_update`` replays.
+
+        Runs until ``n_episodes`` episodes have ended (over all envs, in order of their last step, then env) and logs those
+        in the reference's format (``total_rewards``, ``agent_deaths``, ``n_episodes``, ``init_memories``,
+        ``total_time``; ``write_data``).  Per-episode ``maps`` and ``agent_pos`` are not recorded: the envs run on the
+        device and are not rendered.  One small device-to-host read per launch (rewards and done flags).
+        ``eps_per_launch`` / ``episodes_before_launch`` record the schedule.  Grids up to 32x32 only (the in-kernel
+        policy).  Returns the number of environment steps simulated."""
+        from .batched import BatchedForestFire
+        from .constants import DQN_DEFAULTS as _D
+        t_run = time.time()
+        W, H = self.obs_shape[0], self.obs_shape[1]
+        if W > 32 or H > 32:
+            raise ValueError("learn_batched runs the in-kernel policy: grids up to 32x32 only")
+        N, K = int(n_envs), int(k_steps)
+        R = K if replays_per_launch is None else int(replays_per_launch)
+        B = int(self.METADATA["batch_size"] if batch_size is None else batch_size)
+        keys = {k: v for k, v in self.METADATA.items() if k not in _D and k not in ("debug", "a_speed_iter", "seed", "auto_reset")}
+        env = BatchedForestFire(N, device=self.device, obs_dtype="bits", auto_reset=True, seed=seed, **keys)
+        death_penalty = float(self.METADATA["death_penalty"])
+        gen = torch.Generator(device=env.device).manual_seed(int(seed))
+        self._until_sync = self.target_update_freq
+        self.logs["n_episodes"] = n_episodes
+        self.eps_per_launch, self.episodes_before_launch = [], []
+        rewards, deaths = [], []
+        carry = np.zeros(N)
+        done_eps = 0
+        try:
+            ring = _PackedReplayRing(env, K, int(self.METADATA["memory_size"]), self.memory, self._SARSA)
+            while len(rewards) < n_episodes:
+                self.eps = self.min_eps + (self.max_eps - self.min_eps) * np.exp(-self.eps_decay_rate * done_eps)
+                self.eps_per_launch.append(float(self.eps))
+                self.episodes_before_launch.append(done_eps)
+                net = self.model
+                env.set_policy_mlp_dev(net.dense_1.weight, net.dense_1.bias, net.dense_2.weight, net.dense_2.bias, eps=self.eps)
+                rew, done = ring.launch()
+                if R > 0 and ring.n_sampleable > B:
+                    self.fit_batches_fused(ring.frames, *ring.gather(ring.sample(R, B, gen)), R)
+                rd = torch.stack((rew, done.double())).cpu().numpy()
+                e_idx, k_idx, ret, carry = _episode_ends(carry, rd[0], rd[1] != 0)
+                order = np.lexsort((e_idx, k_idx))
+                for i in order[: n_episodes - len(rewards)]:
+                    rewards.append(float(ret[i]))
+                    deaths.append(bool(rd[0][k_idx[i], e_idx[i]] == death_penalty))
+                done_eps += len(e_idx)
+            steps = ring.steps
+        finally:
+            env.close()
+        self.logs["total_rewards"] = rewards
+        self.logs["agent_deaths"] = deaths
+        self.logs["total_time"] = round(time.time() - t_run, 3)
+        self.write_data()
+        return steps * N
 
     def save_model(self, name):  # DQN.py:441-443
         path = os.path.join(self.out_dir, "Models", name)
@@ -650,6 +781,97 @@ class DQN:
             self.set_weights({k: z[k] for k in z.files})
         if self.verbose:
             print("Model loaded!")
+
+
+class _PackedReplayRing:
+    """The device replay memory of ``DQN.learn_batched``: every rollout of a ``"bits"`` env writes its observations,
+    actions, rewards and done flags straight into the next ``K`` slots of a ``[T][N]`` ring; transitions are addressed by
+    rows of one ``frames`` table, ``[ring T*N | the frames before the first step N | demonstration s D | s' D]``.
+
+    Transition (t, n) of global step t and env n: s = the frame of step t - 1 (after an auto-reset already the new
+    episode's start; the reset frame for t = 0), a / r / done / s' of step t, a' = the action of step t + 1 (so an
+    on-policy transition becomes sampleable one step later).  Held after ``steps`` steps: t in [lo, hi) with
+    lo = max(0, steps - T + 1) (s of step lo is the oldest frame the ring holds) and hi = steps (steps - 1 with a').
+    T is the smallest multiple of K, and at least 2K, for which T - 1 (T - 2 with a') steps of all envs hold
+    ``memory_size`` transitions.  The demonstrations (``ReplayMemory`` entries, uint8) are packed once and kept."""
+
+    def __init__(self, env, k_steps, memory_size, demos, on_policy):
+        from .batched import pack_obs
+        self.env, self.K, self.N, self.on_policy = env, int(k_steps), env.n_envs, bool(on_policy)
+        K, N, dev, words = self.K, self.N, env.device, env.obs_words
+        need = -(-int(memory_size) // N) + 1 + int(self.on_policy)
+        self.T = T = max(2, -(-need // K)) * K
+        self.D = D = len(demos)
+        self.frames = torch.zeros((T * N + N + 2 * D, words), dtype=torch.int32, device=dev)
+        self.ring = self.frames[: T * N].view(T, N, words)
+        self.acts = torch.zeros((T, N), dtype=torch.int32, device=dev)
+        self.rews = torch.zeros((T, N), dtype=torch.float64, device=dev)
+        self.dones = torch.zeros((T, N), dtype=torch.uint8, device=dev)
+        if D:
+            self.frames[T * N + N:T * N + N + D] = pack_obs(demos._s[:D])
+            self.frames[T * N + N + D:] = pack_obs(demos._sp[:D])
+            self.demo = (demos._a[:D].to(torch.int32), demos._ap[:D].to(torch.int32), demos._r[:D].float(),
+                         demos._d[:D].to(torch.uint8))
+        self.steps = 0
+        self.frames[T * N:T * N + N] = env.reset()
+
+    def launch(self):
+        """One ``rollout(K, policy="mlp")`` into the next K slots; returns its rewards [K, N] and done flags [K, N]."""
+        sl = slice(self.steps % self.T, self.steps % self.T + self.K)
+        _, _, _, chosen = self.env.rollout(self.K, policy="mlp", return_actions=True,
+                                           out=(self.ring[sl], self.rews[sl], self.dones[sl]))
+        self.acts[sl] = chosen
+        self.steps += self.K
+        return self.rews[sl], self.dones[sl]
+
+    @property
+    def window(self):
+        """Global steps [lo, hi) whose transitions are held."""
+        return max(0, self.steps - self.T + 1), self.steps - int(self.on_policy)
+
+    @property
+    def n_sampleable(self):
+        lo, hi = self.window
+        return max(0, hi - lo) * self.N + self.D
+
+    def sample(self, n_batches, batch, gen):
+        """``n_batches`` batches, each drawn uniformly without replacement from the sampleable transitions: [n * batch]."""
+        return torch.rand((n_batches, self.n_sampleable), device=self.frames.device, generator=gen).topk(batch, dim=1).indices.flatten()
+
+    def gather(self, k):
+        """Transitions k (0 .. n_sampleable - 1: ring transitions (t, n) in order of t then n, then the demonstrations) as
+        ``fit_batches_fused``'s (s_row, sp_row, a, ap, r, d)."""
+        T, N, D = self.T, self.N, self.D
+        lo, hi = self.window
+        nv = max(0, hi - lo) * N
+        ring_k = k.clamp(max=max(nv - 1, 0))
+        t, n = lo + ring_k // N, ring_k % N
+        slot, prev, nxt = t % T, (t - 1) % T, (t + 1) % T
+        s_row = torch.where(t == 0, T * N + n, prev * N + n)
+        sp_row = slot * N + n
+        a, ap, r, d = self.acts[slot, n], self.acts[nxt, n], self.rews[slot, n].float(), self.dones[slot, n]
+        if D:
+            is_demo = k >= nv
+            j = (k - nv).clamp(min=0, max=D - 1)
+            s_row = torch.where(is_demo, T * N + N + j, s_row)
+            sp_row = torch.where(is_demo, T * N + N + D + j, sp_row)
+            a, ap, r, d = (torch.where(is_demo, x[j], y) for x, y in zip(self.demo, (a, ap, r, d)))
+        return s_row, sp_row, a, ap, r, d
+
+
+def _episode_ends(carry, rew, done):
+    """Episodes that end within a [K, N] chunk of rewards and done flags: (env, step, return) of each, sorted by env then
+    step, and the new carry (reward of each env's running episode at the end of the chunk; ``carry`` is the one before)."""
+    c = carry[None, :] + np.cumsum(rew, axis=0)
+    e_idx, k_idx = np.nonzero(done.T)  # episode ends, sorted by env then step
+    at_end = c[k_idx, e_idx]
+    same = np.r_[False, e_idx[1:] == e_idx[:-1]]
+    ret = at_end - np.where(same, np.r_[0.0, at_end[:-1]], 0.0)
+    last = np.zeros(len(carry))
+    if len(e_idx):
+        is_last = np.r_[e_idx[1:] != e_idx[:-1], True]
+        last[e_idx[is_last]] = at_end[is_last]
+    return e_idx, k_idx, ret, c[-1] - last
 
 
 def _jsonable(o):

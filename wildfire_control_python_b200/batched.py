@@ -82,6 +82,21 @@ def unpack_obs(bits: torch.Tensor, width: int, height: int, index=None, dtype: t
     return out
 
 
+def pack_obs(obs: torch.Tensor) -> torch.Tensor:
+    """The inverse of ``unpack_obs``: ``[..., W, H, 3]`` 0/1 observations (any dtype, any device) -> ``[..., words]`` int32
+    in the ``WF_OBS_BITS`` layout (include/wildfire.h: element k = (x*H + y)*3 + c is bit k % 32 of word k // 32, zero
+    padding).  Plain torch, for packing stored uint8 memories once (e.g. demonstrations) into a packed replay buffer."""
+    if obs.dim() < 3 or obs.shape[-1] != 3:
+        raise ValueError("obs must have shape [..., W, H, 3]")
+    lead, W, H = tuple(obs.shape[:-3]), int(obs.shape[-3]), int(obs.shape[-2])
+    words = _lib.obs_bits_words(W, H)
+    flat = (obs.reshape(*lead, W * H * 3) != 0).to(torch.int64)
+    flat = torch.nn.functional.pad(flat, (0, words * 32 - W * H * 3)).reshape(*lead, words, 32)
+    shifts = torch.arange(32, device=obs.device, dtype=torch.int64)
+    packed = (flat << shifts).sum(-1)  # < 2**32: the uint32 pattern; as int32 with the same bits
+    return torch.where(packed >= 2**31, packed - 2**32, packed).to(torch.int32)
+
+
 class BatchedForestFire:
     """``n_envs`` reference environments on one GPU.
 
@@ -259,6 +274,26 @@ class BatchedForestFire:
                              f"{self.n_actions} network")
         _lib.check(_lib.lib().wf_set_policy_mlp(self._h, k1.ctypes.data, b1.ctypes.data, k2.ctypes.data, b2.ctypes.data,
                                                 hidden, float(eps)))
+
+    def set_policy_mlp_dev(self, weight1, bias1, weight2, bias2, eps: float = 0.0):
+        """``set_policy_mlp`` from float32 CUDA tensors in ``nn.Linear`` orientation (``weight1`` ``[hidden, W*H*3]``,
+        ``weight2`` ``[n_actions, hidden]``), repacked by a kernel on the current stream: no host copy, no synchronisation
+        (``wf_set_policy_mlp_dev``).  Rollouts queued after it on the same stream use the new weights, and they act
+        exactly as after ``set_policy_mlp`` with the same weights.  For a dueling head pass the advantage stream."""
+        ts = []
+        for t in (weight1, bias1, weight2, bias2):
+            if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float32 and t.device == self.device):
+                raise ValueError(f"set_policy_mlp_dev takes float32 tensors on {self.device}")
+            ts.append(t.detach().contiguous())
+        w1, b1, w2, b2 = ts
+        hidden = int(b1.shape[0]) if b1.dim() == 1 else -1
+        if (b1.dim() != 1 or tuple(w1.shape) != (hidden, self.width * self.height * 3)
+                or tuple(w2.shape) != (self.n_actions, hidden) or tuple(b2.shape) != (self.n_actions,)):
+            raise ValueError(f"weight shapes {[tuple(t.shape) for t in ts]} do not fit a {self.width}x{self.height}x3 -> "
+                             f"hidden -> {self.n_actions} network in nn.Linear orientation")
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().wf_set_policy_mlp_dev(self._h, _ptr(w1), _ptr(b1), _ptr(w2), _ptr(b2), hidden, float(eps),
+                                                        self._stream()))
 
     def step_host(self, actions):
         """Host-buffer step through ``wf_step_host``: H2D actions, step, D2H obs/reward/done, sync.

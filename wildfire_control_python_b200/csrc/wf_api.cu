@@ -40,6 +40,9 @@ static int fail(int code, const std::string& msg) {
     g_err = msg;
     return code;
 }
+namespace wf {  // the error text of the entry points in other translation units (wf_learn.cu)
+int api_fail(int code, const std::string& msg) { return fail(code, msg); }
+}  // namespace wf
 #define WF_CUDA(expr)                                                                         \
     do {                                                                                      \
         cudaError_t _e = (expr);                                                              \
@@ -294,6 +297,38 @@ __global__ void get_obs_bits_kernel(DevState s, uint32_t* obs) {
             v |= bit << b;
         }
         obs[i] = v;
+    }
+}
+
+// wf_set_policy_mlp_dev: wf_set_policy_mlp's host repack, one thread per float of the packed buffer, from nn.Linear-oriented
+// weights (w1 [hidden][n_in], w2 [A][hidden]).  Every float of the buffer is written (padding 0, missing actions' bias
+// -inf), and `base` is summed in float64 in the host's order, so the buffer is byte-identical to the host path's.
+__global__ void pack_policy_mlp_kernel(float* __restrict__ out, const float* __restrict__ w1, const float* __restrict__ b1,
+                                       const float* __restrict__ w2, const float* __restrict__ b2, int n_in, int cells,
+                                       int hidden, int A, int L) {
+    const int hpl = 64 / L;
+    const size_t n_w1 = (size_t)n_in * 64, total = n_w1 + 64 + 512 + 8;
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        float v = 0.0f;
+        if (i < n_w1) {  // w1 [n_in][64]: unit j sits at (j % L) * hpl + j / L
+            const int f = (int)(i / 64), pos = (int)(i % 64);
+            const int j = (pos % hpl) * L + pos / hpl;
+            if (j < hidden) v = w1[(size_t)j * n_in + f];
+        } else if (i < n_w1 + 64) {  // base: bias1 + the all-free empty map (channel 2 of every cell)
+            const int j = (int)(i - n_w1);
+            if (j < hidden) {
+                double acc = b1[j];
+                for (int cell = 0; cell < cells; ++cell) acc += w1[(size_t)j * n_in + cell * 3 + 2];
+                v = (float)acc;
+            }
+        } else if (i < n_w1 + 64 + 512) {  // w2 [2][64][4]: action b of unit j at (b / 4) * 256 + j * 4 + b % 4
+            const int k = (int)(i - n_w1 - 64), j = (k % 256) / 4, b = (k / 256) * 4 + k % 4;
+            if (j < hidden && b < A) v = w2[(size_t)b * hidden + j];
+        } else {
+            const int b = (int)(i - n_w1 - 64 - 512);
+            v = b < A ? b2[b] : -INFINITY;
+        }
+        out[i] = v;
     }
 }
 
@@ -726,6 +761,33 @@ int wf_set_policy_mlp(wf_env* e, const float* k1, const float* b1, const float* 
     e->mlp = MlpPolicy{};
     WF_CUDA(cudaMalloc(&e->mlp_dev, total * sizeof(float)));
     WF_CUDA(cudaMemcpy(e->mlp_dev, h, total * sizeof(float), cudaMemcpyHostToDevice));
+    e->mlp.w1 = e->mlp_dev;
+    e->mlp.base = e->mlp_dev + n_w1;
+    e->mlp.w2 = e->mlp.base + 64;
+    e->mlp.b2 = e->mlp.w2 + 512;
+    e->mlp.hid = hidden;
+    e->mlp.n_actions = A;
+    e->mlp.eps_u32 = eps >= 1.0 ? 0xffffffffu : (uint32_t)(eps * 4294967296.0);
+    return WF_OK;
+}
+
+int wf_set_policy_mlp_dev(wf_env* e, const float* w1, const float* b1, const float* w2, const float* b2, int32_t hidden,
+                          double eps, void* stream) {
+    if (!e || !w1 || !b1 || !w2 || !b2) return fail(WF_ERR_INVALID, "null argument");
+    if (hidden < 1 || hidden > 64) return fail(WF_ERR_INVALID, "hidden must be in 1..64");
+    if (e->cfg.n_actions > 8) return fail(WF_ERR_INVALID, "WF_POLICY_MLP supports at most 8 actions");
+    if (!(eps >= 0.0 && eps <= 1.0)) return fail(WF_ERR_INVALID, "eps must be in [0, 1]");
+    for (const float* p : {w1, b1, w2, b2})
+        if (reinterpret_cast<uintptr_t>(p) & 3u) return fail(WF_ERR_INVALID, "weights must be 4-byte aligned");
+    WF_ON_DEVICE(e);
+    WF_QUIESCE(e);
+    const DevState& s = e->st;
+    const int n_in = s.W * s.H * 3, A = e->cfg.n_actions;
+    const size_t n_w1 = (size_t)n_in * 64, total = n_w1 + 64 + 2 * 64 * 4 + 8;  // the layout of wf_set_policy_mlp
+    if (!e->mlp_dev) WF_CUDA(cudaMalloc(&e->mlp_dev, total * sizeof(float)));
+    pack_policy_mlp_kernel<<<(int)std::min<size_t>((total + 255) / 256, 148 * 16), 256, 0, static_cast<cudaStream_t>(stream)>>>(e->mlp_dev, w1, b1, w2, b2, n_in,
+                                                                                          s.W * s.H, hidden, A, s.RS);
+    WF_CUDA(cudaGetLastError());
     e->mlp.w1 = e->mlp_dev;
     e->mlp.base = e->mlp_dev + n_w1;
     e->mlp.w2 = e->mlp.base + 64;
