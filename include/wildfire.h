@@ -34,8 +34,8 @@ extern "C" {
 #endif
 
 #define WF_ABI_VERSION 2 /* 2: + wf_reset_host, wf_host_session(_active), wf_get/set_a_iter, wf_tile_geometry, wf_apply_change_blocks;
-                            later, still 2: + WF_OBS_BITS, wf_unpack_obs_bits; + wf_set_policy_mlp_dev, wf_replay_fit
-                            (additions only) */
+                            later, still 2: + WF_OBS_BITS, wf_unpack_obs_bits; + wf_set_policy_mlp_dev, wf_replay_fit;
+                            + wf_set_policy_mlp_nets_dev, wf_replay_fit_many (additions only) */
 
 enum {
     WF_OK = 0,
@@ -309,6 +309,43 @@ int wf_replay_fit(const wf_mlp_shape* shape, const wf_fit_params* params, int32_
                   const int64_t* s_row_dev, const int64_t* sp_row_dev, const int32_t* action_dev,
                   const int32_t* next_action_dev, const float* reward_dev, const uint8_t* done_dev, float* loss_dev,
                   void* stream);
+
+/* ---- populations: up to 64 independent learners in one launch -------------------------------------------------------
+ * One learner of wf_replay_fit_many: its own flat model, target and Adam moments (the layout above), its own transitions
+ * ([n_replays * batch] each, as for wf_replay_fit; next_action NULL = the DQN target, max_a Q_target(s', a)), its own loss
+ * ([n_replays] or NULL) and its own hyper-parameters, Adam step and target-sync phase. */
+typedef struct wf_fit_learner {
+    float *params, *target, *adam_m, *adam_v;
+    const int64_t *s_row, *sp_row;
+    const int32_t *action, *next_action;
+    const float* reward;
+    const uint8_t* done;
+    float* loss;
+    wf_fit_params hp;
+} wf_fit_learner;
+
+/* wf_replay_fit for n_learners (1..64) learners of one network shape and batch size (learners_host: a host array,
+ * read before the call returns), in ONE launch: one thread-block cluster per learner.  The frames table is shared and
+ * its row numbers are global, so each learner may use any rows (e.g. its own demonstrations).  Every learner is checked
+ * as wf_replay_fit checks its arguments (misaligned pointers included) and follows its out-of-range rules.  The
+ * cluster size is the one wf_replay_fit uses on this device, so each learner's result is bit-identical to a
+ * wf_replay_fit call on that learner alone; clusters beyond those the GPU holds at once run in later waves.
+ * wf_replay_fit is this call with one learner. */
+int wf_replay_fit_many(const wf_mlp_shape* shape, int32_t n_learners, const wf_fit_learner* learners_host,
+                       int32_t n_replays, const uint32_t* frames_dev, int64_t n_frames, void* stream);
+
+/* The in-kernel policy (WF_POLICY_MLP) with n_nets (1..64) networks: env n acts with network n / (N / n_nets).
+ * N must be a multiple of n_nets and the group size N / n_nets a multiple of 8 (whole CTAs of the warp family, so each CTA
+ * uses one network).  params_dev: [n_nets][P] float32 in the flat layout of wf_replay_fit above (P floats per network,
+ * dueling included); the policy reads dense_1 / dense_2 (the advantage stream of a dueling head), so the buffer that
+ * wf_replay_fit(_many) writes is read as it is.  eps_host: n_nets exploration rates in [0, 1] (host; read before the call
+ * returns).  shape: the handle's grid and n_actions; batch is ignored.  Like wf_set_policy_mlp_dev, the repack runs as a
+ * kernel on `stream` with no host copy and no synchronisation, and each network's packed block is byte-identical to the
+ * one wf_set_policy_mlp(_dev) produces for the same weights and eps (those calls write network 0, one group covering every
+ * env).  A call with more networks than any call before it on the handle reallocates the packed buffer (which waits for
+ * the device). */
+int wf_set_policy_mlp_nets_dev(wf_env* env, const wf_mlp_shape* shape, int32_t n_nets, const float* params_dev,
+                               const double* eps_host, void* stream);
 
 /* Heat quanta table: coef[wind_id][4] float64 (host pointer), n_wind entries (1 or 27). */
 int wf_get_wind_table(const wf_env* env, double* coef_host, double* speed_host,

@@ -10,7 +10,7 @@ from ._lib import obs_bits_words
 from .constants import METADATA, grass, layer, make_metadata, types
 
 __all__ = ["BatchedForestFire", "ForestFire", "METADATA", "grass", "layer", "types", "make_metadata", "build",
-           "DQN", "DQN_SARSA", "DQN_DUEL", "DQN_BOTH", "obs_bits_words", "unpack_obs", "pack_obs"]
+           "DQN", "DQN_SARSA", "DQN_DUEL", "DQN_BOTH", "learn_population", "obs_bits_words", "unpack_obs", "pack_obs"]
 
 
 def build(force: bool = False, verbose: bool = False) -> str:
@@ -27,7 +27,7 @@ def __getattr__(name):  # torch is imported lazily so that `import wildfire_cont
     if name == "ForestFire":
         from .compat import ForestFire
         return ForestFire
-    if name in ("DQN", "DQN_SARSA", "DQN_DUEL", "DQN_BOTH"):
+    if name in ("DQN", "DQN_SARSA", "DQN_DUEL", "DQN_BOTH", "learn_population"):
         from . import agents
         return getattr(agents, name)
     raise AttributeError(name)

@@ -55,6 +55,16 @@ class WfFitParams(C.Structure):
                 ("phase", C.c_int32)]
 
 
+class WfFitLearner(C.Structure):
+    """``wf_fit_learner``: one learner of ``wf_replay_fit_many`` (device pointers travel as integers)."""
+    _fields_ = [("params", C.c_void_p), ("target", C.c_void_p), ("adam_m", C.c_void_p), ("adam_v", C.c_void_p),
+                ("s_row", C.c_void_p), ("sp_row", C.c_void_p), ("action", C.c_void_p), ("next_action", C.c_void_p),
+                ("reward", C.c_void_p), ("done", C.c_void_p), ("loss", C.c_void_p), ("hp", WfFitParams)]
+
+
+MAX_LEARNERS = 64  # wf_replay_fit_many's n_learners and wf_set_policy_mlp_nets_dev's n_nets
+
+
 def mlp_param_count(width: int, height: int, hidden: int, n_actions: int, dueling: bool) -> int:
     """Floats of wf_replay_fit's flat parameter buffer (include/wildfire.h): parameters_to_vector(model.parameters())."""
     n_in = int(width) * int(height) * 3
@@ -111,6 +121,10 @@ def lib():
     L.wf_replay_fit.argtypes = [C.POINTER(WfMlpShape), C.POINTER(WfFitParams), C.c_int32, vp, vp, vp, vp, vp, C.c_int64,
                                 vp, vp, vp, vp, vp, vp, vp, vp]
     L.wf_replay_fit.restype = C.c_int
+    L.wf_replay_fit_many.argtypes = [C.POINTER(WfMlpShape), C.c_int32, C.POINTER(WfFitLearner), C.c_int32, vp, C.c_int64, vp]
+    L.wf_replay_fit_many.restype = C.c_int
+    L.wf_set_policy_mlp_nets_dev.argtypes = [vp, C.POINTER(WfMlpShape), C.c_int32, vp, C.POINTER(C.c_double), vp]
+    L.wf_set_policy_mlp_nets_dev.restype = C.c_int
     L.wf_step_host.argtypes = [vp, i32p, vp, C.c_int32, f64p, u8p]
     L.wf_reset_host.argtypes = [vp, u8p, vp, vp, C.c_int32]
     L.wf_host_session.argtypes = [vp, C.c_int32]
@@ -159,5 +173,5 @@ EXPORTED_SYMBOLS = [
     "wf_reset", "wf_step", "wf_rollout", "wf_rollout_policy", "wf_set_policy_mlp", "wf_step_host", "wf_get_state", "wf_set_state", "wf_set_fire_to",
     "wf_get_obs", "wf_get_wind_table", "wf_stats", "wf_stats_reset", "wf_philox_kat", "wf_launch_count",
     "wf_state_bytes_per_env", "wf_host_threads", "wf_expand_packed_obs", "wf_apply_change_blocks", "wf_get_a_iter", "wf_set_a_iter", "wf_reset_host", "wf_tile_geometry", "wf_host_session", "wf_host_session_active",
-    "wf_unpack_obs_bits", "wf_set_policy_mlp_dev", "wf_replay_fit",
+    "wf_unpack_obs_bits", "wf_set_policy_mlp_dev", "wf_replay_fit", "wf_replay_fit_many", "wf_set_policy_mlp_nets_dev",
 ]

@@ -695,7 +695,8 @@ class DQN:
         self._until_sync = (phase - n_replays - 1) % te + 1
         return loss
 
-    def learn_batched(self, n_episodes, n_envs=1024, k_steps=16, replays_per_launch=None, batch_size=None, seed=0):
+    def learn_batched(self, n_episodes, n_envs=1024, k_steps=16, replays_per_launch=None, batch_size=None, seed=0,
+                      replay_seed=None):
         """``learn`` over ``n_envs`` CUDA environments at once: the envs act with the eps-greedy Q-network evaluated inside
         the step kernel (``rollout(policy="mlp")``, ``k_steps`` steps per launch), each rollout writes its packed
         observations straight into a device replay ring, and after every launch ``replays_per_launch`` (default
@@ -706,7 +707,8 @@ class DQN:
         Replay memory: the ring (``_PackedReplayRing``) holds at least the last ``memory_size`` transitions of every env
         together (whole launches, at least two), plus every transition already in ``self.memory`` (demonstrations from ``collect_memories(_batched)``, kept for
         the whole run like the reference's unbounded post-demonstration deque).  Each replay draws its batch uniformly
-        without replacement from both, on the device, from a generator seeded with ``seed``; replays start once more
+        without replacement from both, on the device, from a generator seeded with ``replay_seed`` (default: ``seed``, the
+        envs' Philox key); replays start once more
         than a batch of transitions exists.  The target network is refreshed every ``target_update`` replays.
 
         Runs until ``n_episodes`` episodes have ended (over all envs, in order of their last step, then env) and logs those
@@ -727,7 +729,7 @@ class DQN:
         keys = {k: v for k, v in self.METADATA.items() if k not in _D and k not in ("debug", "a_speed_iter", "seed", "auto_reset")}
         env = BatchedForestFire(N, device=self.device, obs_dtype="bits", auto_reset=True, seed=seed, **keys)
         death_penalty = float(self.METADATA["death_penalty"])
-        gen = torch.Generator(device=env.device).manual_seed(int(seed))
+        gen = torch.Generator(device=env.device).manual_seed(int(seed if replay_seed is None else replay_seed))
         self._until_sync = self.target_update_freq
         self.logs["n_episodes"] = n_episodes
         self.eps_per_launch, self.episodes_before_launch = [], []
@@ -784,34 +786,46 @@ class DQN:
 
 
 class _PackedReplayRing:
-    """The device replay memory of ``DQN.learn_batched``: every rollout of a ``"bits"`` env writes its observations,
-    actions, rewards and done flags straight into the next ``K`` slots of a ``[T][N]`` ring; transitions are addressed by
-    rows of one ``frames`` table, ``[ring T*N | the frames before the first step N | demonstration s D | s' D]``.
+    """The device replay memory of ``DQN.learn_batched`` and ``learn_population``: every rollout of a ``"bits"`` env writes
+    its observations, actions, rewards and done flags straight into the next ``K`` slots of a ``[T][N]`` ring; transitions
+    are addressed by rows of one ``frames`` table, ``[ring T*N | the frames before the first step N | per group j:
+    demonstration s D_j | s' D_j]``.
 
+    The N envs form ``groups`` equal column groups of G = N / groups envs, one per learner: group j's transitions are
+    those of envs j*G ... j*G + G - 1, plus its own demonstrations.  ``learn_batched`` is the one-group case.
     Transition (t, n) of global step t and env n: s = the frame of step t - 1 (after an auto-reset already the new
     episode's start; the reset frame for t = 0), a / r / done / s' of step t, a' = the action of step t + 1 (so an
     on-policy transition becomes sampleable one step later).  Held after ``steps`` steps: t in [lo, hi) with
     lo = max(0, steps - T + 1) (s of step lo is the oldest frame the ring holds) and hi = steps (steps - 1 with a').
-    T is the smallest multiple of K, and at least 2K, for which T - 1 (T - 2 with a') steps of all envs hold
-    ``memory_size`` transitions.  The demonstrations (``ReplayMemory`` entries, uint8) are packed once and kept."""
+    T is the smallest multiple of K, and at least 2K, for which T - 1 (T - 2 with a') steps of a group's G envs hold
+    ``memory_size`` transitions.  The demonstrations (``ReplayMemory`` entries, uint8; ``demos``: one memory per group, or
+    one memory for one group) are packed once and kept."""
 
-    def __init__(self, env, k_steps, memory_size, demos, on_policy):
+    def __init__(self, env, k_steps, memory_size, demos, on_policy, groups=1):
         from .batched import pack_obs
         self.env, self.K, self.N, self.on_policy = env, int(k_steps), env.n_envs, bool(on_policy)
+        if not isinstance(demos, (list, tuple)):
+            demos = [demos]
+        if len(demos) != groups or self.N % groups:
+            raise ValueError("need one demonstration memory per group and equal groups of envs")
+        self.G = G = self.N // groups
         K, N, dev, words = self.K, self.N, env.device, env.obs_words
-        need = -(-int(memory_size) // N) + 1 + int(self.on_policy)
+        need = -(-int(memory_size) // G) + 1 + int(self.on_policy)
         self.T = T = max(2, -(-need // K)) * K
-        self.D = D = len(demos)
-        self.frames = torch.zeros((T * N + N + 2 * D, words), dtype=torch.int32, device=dev)
+        self.D = [len(m) for m in demos]
+        self.demo_base = [T * N + N + 2 * sum(self.D[:j]) for j in range(groups)]  # first row of group j's demo s
+        self.frames = torch.zeros((T * N + N + 2 * sum(self.D), words), dtype=torch.int32, device=dev)
         self.ring = self.frames[: T * N].view(T, N, words)
         self.acts = torch.zeros((T, N), dtype=torch.int32, device=dev)
         self.rews = torch.zeros((T, N), dtype=torch.float64, device=dev)
         self.dones = torch.zeros((T, N), dtype=torch.uint8, device=dev)
-        if D:
-            self.frames[T * N + N:T * N + N + D] = pack_obs(demos._s[:D])
-            self.frames[T * N + N + D:] = pack_obs(demos._sp[:D])
-            self.demo = (demos._a[:D].to(torch.int32), demos._ap[:D].to(torch.int32), demos._r[:D].float(),
-                         demos._d[:D].to(torch.uint8))
+        self.demo = []
+        for m, D, base in zip(demos, self.D, self.demo_base):
+            if D:
+                self.frames[base:base + D] = pack_obs(m._s[:D])
+                self.frames[base + D:base + 2 * D] = pack_obs(m._sp[:D])
+            self.demo.append((m._a[:D].to(torch.int32), m._ap[:D].to(torch.int32), m._r[:D].float(),
+                              m._d[:D].to(torch.uint8)) if D else None)
         self.steps = 0
         self.frames[T * N:T * N + N] = env.reset()
 
@@ -829,34 +843,194 @@ class _PackedReplayRing:
         """Global steps [lo, hi) whose transitions are held."""
         return max(0, self.steps - self.T + 1), self.steps - int(self.on_policy)
 
+    def sampleable(self, group=0):
+        """Transitions group ``group`` can draw from: its envs' held transitions and its demonstrations."""
+        lo, hi = self.window
+        return max(0, hi - lo) * self.G + self.D[group]
+
     @property
     def n_sampleable(self):
-        lo, hi = self.window
-        return max(0, hi - lo) * self.N + self.D
+        return self.sampleable(0)
 
-    def sample(self, n_batches, batch, gen):
-        """``n_batches`` batches, each drawn uniformly without replacement from the sampleable transitions: [n * batch]."""
-        return torch.rand((n_batches, self.n_sampleable), device=self.frames.device, generator=gen).topk(batch, dim=1).indices.flatten()
+    def sample(self, n_batches, batch, gen, group=0):
+        """``n_batches`` batches, each drawn uniformly without replacement from the group's sampleable transitions:
+        [n * batch]."""
+        return torch.rand((n_batches, self.sampleable(group)), device=self.frames.device, generator=gen).topk(batch, dim=1).indices.flatten()
 
-    def gather(self, k):
-        """Transitions k (0 .. n_sampleable - 1: ring transitions (t, n) in order of t then n, then the demonstrations) as
-        ``fit_batches_fused``'s (s_row, sp_row, a, ap, r, d)."""
-        T, N, D = self.T, self.N, self.D
+    def gather(self, k, group=0):
+        """Transitions k of group ``group`` (0 .. sampleable - 1: its ring transitions (t, n) in order of t then n, then
+        its demonstrations) as ``fit_batches_fused``'s (s_row, sp_row, a, ap, r, d), rows of the shared ``frames``."""
+        T, N, G, D = self.T, self.N, self.G, self.D[group]
         lo, hi = self.window
-        nv = max(0, hi - lo) * N
+        nv = max(0, hi - lo) * G
         ring_k = k.clamp(max=max(nv - 1, 0))
-        t, n = lo + ring_k // N, ring_k % N
+        t, n = lo + ring_k // G, ring_k % G + group * G
         slot, prev, nxt = t % T, (t - 1) % T, (t + 1) % T
         s_row = torch.where(t == 0, T * N + n, prev * N + n)
         sp_row = slot * N + n
         a, ap, r, d = self.acts[slot, n], self.acts[nxt, n], self.rews[slot, n].float(), self.dones[slot, n]
         if D:
+            base = self.demo_base[group]
             is_demo = k >= nv
             j = (k - nv).clamp(min=0, max=D - 1)
-            s_row = torch.where(is_demo, T * N + N + j, s_row)
-            sp_row = torch.where(is_demo, T * N + N + D + j, sp_row)
-            a, ap, r, d = (torch.where(is_demo, x[j], y) for x, y in zip(self.demo, (a, ap, r, d)))
+            s_row = torch.where(is_demo, base + j, s_row)
+            sp_row = torch.where(is_demo, base + D + j, sp_row)
+            a, ap, r, d = (torch.where(is_demo, x[j], y) for x, y in zip(self.demo[group], (a, ap, r, d)))
         return s_row, sp_row, a, ap, r, d
+
+
+# METADATA keys the learners of one learn_population may set differently: the learning rate, the discount, the target
+# refresh interval and the eps schedule.  Everything else (the environment, memory_size, batch_size) must agree.
+_POPULATION_FREE_KEYS = ("alpha", "gamma", "target_update", "max_eps", "min_eps", "eps_decay_rate")
+
+
+def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replays_per_launch=None, batch_size=None, seed=0):
+    """``DQN.learn_batched`` for M = len(agents) independent learners (1 to 64) at once on one GPU, with one rollout launch
+    and one ``wf_replay_fit_many`` launch per iteration for all of them.
+
+    The agents must be of one class and share the network shape, the environment METADATA, ``memory_size`` and the batch
+    size; their initial weights, demonstrations already in ``agent.memory``, ``alpha``, ``gamma``, ``target_update`` and
+    eps schedule may differ.  One ``"bits"`` handle of M * ``envs_per_learner`` auto-reset envs with Philox key ``seed``
+    runs them all: learner j's envs are the j-th group of ``envs_per_learner`` (a multiple of 8), acting with learner j's
+    network and eps (``set_policy_mlp_flat_dev``).  The replay ring (``_PackedReplayRing``) keeps one column group and
+    the demonstrations per learner; learner j draws its batches from its own window with its own generator, seeded with
+    ``seed + j``.  The stacked [M, P] model, target and Adam moments are the state during the run and are written back
+    into each agent (modules, ``KerasAdam`` m, v and t, ``_until_sync``) at the end.
+
+    Learner j logs its first ``n_episodes`` episodes exactly as ``learn_batched`` does (``eps_per_launch`` and
+    ``episodes_before_launch`` included) and stops replaying after the launch in which it reaches them; its envs keep
+    stepping, ignored, until every learner has finished.  Then each agent calls ``write_data()``.  Agent j's result is
+    that of ``agent.learn_batched(n_episodes, envs_per_learner, k_steps, replays_per_launch, batch_size, seed=seed,
+    replay_seed=seed + j)`` with METADATA ``env_id_base = j * envs_per_learner``, byte for byte.
+    Returns the env-step count of each learner (what ``learn_batched`` returns)."""
+    from torch.nn.utils import parameters_to_vector
+    from . import _lib
+    from .batched import BatchedForestFire, _ptr
+    from .constants import DQN_DEFAULTS as _D
+    agents = list(agents)
+    M = len(agents)
+    if not 1 <= M <= _lib.MAX_LEARNERS:
+        raise ValueError(f"learn_population takes 1 to {_lib.MAX_LEARNERS} agents, got {M}")
+    a0 = agents[0]
+    if any(type(a) is not type(a0) for a in agents):
+        raise ValueError("learn_population: every agent must be of the same class")
+    shared = lambda a: {k: v for k, v in a.METADATA.items() if k not in _POPULATION_FREE_KEYS}
+    if any(shared(a) != shared(a0) for a in agents):
+        raise ValueError("learn_population: the agents' METADATA (environment, memory_size, batch_size) must agree")
+    shapes = lambda a: [tuple(p.shape) for p in a.model.parameters()]
+    if any(shapes(a) != shapes(a0) for a in agents):
+        raise ValueError("learn_population: every agent must have the same network shape")
+    W, H = a0.obs_shape[0], a0.obs_shape[1]
+    if W > 32 or H > 32:
+        raise ValueError("learn_population runs the in-kernel policy: grids up to 32x32 only")
+    G, K = int(envs_per_learner), int(k_steps)
+    if G < 8 or G % 8:
+        raise ValueError("envs_per_learner must be a positive multiple of 8")
+    if any(a.device != a0.device for a in agents):
+        raise ValueError("learn_population: every agent must be on the same device")
+    if a0.device.type != "cuda":
+        raise _lib.WildfireError("learn_population needs a CUDA device (no CPU fallback)")
+    t_run = time.time()
+    N = M * G
+    R = K if replays_per_launch is None else int(replays_per_launch)
+    B = int(a0.METADATA["batch_size"] if batch_size is None else batch_size)
+    sarsa, dueling = a0._SARSA, hasattr(a0.model, "dense_3")
+    hidden = a0.model.dense_1.out_features
+    keys = {k: v for k, v in a0.METADATA.items() if k not in _D and k not in ("debug", "a_speed_iter", "seed", "auto_reset")}
+    env = BatchedForestFire(N, device=a0.device, obs_dtype="bits", auto_reset=True, seed=seed, **keys)
+    dev = env.device
+    death_penalty = float(a0.METADATA["death_penalty"])
+    gens = [torch.Generator(device=dev).manual_seed(int(seed) + j) for j in range(M)]
+    # the stacked state, as DQN.fit_batches_fused flattens it
+    with torch.no_grad():
+        adam_t = [(a.optimizer.state[next(a.model.parameters())] or {}).get("t", 0) for a in agents]
+        P = torch.stack([parameters_to_vector(a.model.parameters()) for a in agents]).contiguous()
+        Tg = torch.stack([parameters_to_vector(a.target.parameters()) for a in agents]).contiguous()
+        Mm = torch.stack([parameters_to_vector([a.optimizer.state[p]["m"] for p in a.model.parameters()]) if t else
+                          torch.zeros(P.shape[1], device=dev) for a, t in zip(agents, adam_t)]).contiguous()
+        Vv = torch.stack([parameters_to_vector([a.optimizer.state[p]["v"] for p in a.model.parameters()]) if t else
+                          torch.zeros(P.shape[1], device=dev) for a, t in zip(agents, adam_t)]).contiguous()
+    until_sync = [int(a.target_update_freq) for a in agents]
+    rewards, deaths = [[] for _ in agents], [[] for _ in agents]
+    carry = [np.zeros(G) for _ in agents]
+    done_eps, steps, finished = [0] * M, [0] * M, [False] * M
+    for a in agents:
+        a.logs["n_episodes"] = n_episodes
+        a.eps_per_launch, a.episodes_before_launch = [], []
+    shape = a0._flat_shape(B)
+    stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+    try:
+        ring = _PackedReplayRing(env, K, int(a0.METADATA["memory_size"]), [a.memory for a in agents], sarsa, groups=M)
+        while not all(finished):
+            for j, a in enumerate(agents):
+                if not finished[j]:
+                    a.eps = a.min_eps + (a.max_eps - a.min_eps) * np.exp(-a.eps_decay_rate * done_eps[j])
+                    a.eps_per_launch.append(float(a.eps))
+                    a.episodes_before_launch.append(done_eps[j])
+            env.set_policy_mlp_flat_dev(P, hidden, dueling, [float(a.eps) for a in agents])
+            rew, done = ring.launch()
+            fit = [j for j in range(M) if not finished[j] and R > 0 and ring.sampleable(j) > B]
+            if fit:
+                keep, desc = [], (_lib.WfFitLearner * len(fit))()
+                for i, j in enumerate(fit):
+                    a = agents[j]
+                    cols = [x.to(dt).contiguous() for x, dt in zip(ring.gather(ring.sample(R, B, gens[j], j), j),
+                                                                   (torch.int64, torch.int64, torch.int32, torch.int32,
+                                                                    torch.float32, torch.uint8))]
+                    keep.append(cols)
+                    grp = a.optimizer.param_groups[0]
+                    te = int(a.target_update_freq)
+                    hp = _lib.WfFitParams(gamma=float(a.gamma), lr=grp["lr"], beta_1=grp["beta_1"], beta_2=grp["beta_2"],
+                                          epsilon=grp["epsilon"],
+                                          clipvalue=math.inf if grp["clipvalue"] is None else grp["clipvalue"],
+                                          adam_t=adam_t[j], target_every=te, phase=until_sync[j])
+                    desc[i] = _lib.WfFitLearner(P[j].data_ptr(), Tg[j].data_ptr(), Mm[j].data_ptr(), Vv[j].data_ptr(),
+                                                cols[0].data_ptr(), cols[1].data_ptr(), cols[2].data_ptr(),
+                                                cols[3].data_ptr() if sarsa else None, cols[4].data_ptr(),
+                                                cols[5].data_ptr(), None, hp)
+                with torch.cuda.device(dev):
+                    _lib.check(_lib.lib().wf_replay_fit_many(ctypes.byref(shape), len(fit), desc, R, _ptr(ring.frames),
+                                                             ring.frames.shape[0], stream))
+                for j in fit:
+                    adam_t[j] += R
+                    te = int(agents[j].target_update_freq)
+                    until_sync[j] = (until_sync[j] - R - 1) % te + 1
+            rd = torch.stack((rew, done.double())).cpu().numpy()
+            for j in range(M):
+                if finished[j]:
+                    continue
+                cols = slice(j * G, (j + 1) * G)
+                e_idx, k_idx, ret, carry[j] = _episode_ends(carry[j], rd[0][:, cols], rd[1][:, cols] != 0)
+                order = np.lexsort((e_idx, k_idx))
+                for i in order[: n_episodes - len(rewards[j])]:
+                    rewards[j].append(float(ret[i]))
+                    deaths[j].append(bool(rd[0][k_idx[i], j * G + e_idx[i]] == death_penalty))
+                done_eps[j] += len(e_idx)
+                if len(rewards[j]) >= n_episodes:
+                    finished[j], steps[j] = True, ring.steps * G
+    finally:
+        env.close()
+    total_time = round(time.time() - t_run, 3)
+    with torch.no_grad():
+        for j, a in enumerate(agents):
+            params = list(a.model.parameters())
+            off = 0
+            for p, tp in zip(params, a.target.parameters()):
+                n = p.numel()
+                p.copy_(P[j, off:off + n].view_as(p))
+                tp.copy_(Tg[j, off:off + n].view_as(p))
+                if adam_t[j]:
+                    st = a.optimizer.state[p]
+                    st["m"] = Mm[j, off:off + n].view_as(p).clone()
+                    st["v"] = Vv[j, off:off + n].view_as(p).clone()
+                    st["t"] = adam_t[j]
+                off += n
+            a._until_sync = until_sync[j]
+            a.logs["total_rewards"] = rewards[j]
+            a.logs["agent_deaths"] = deaths[j]
+            a.logs["total_time"] = total_time
+            a.write_data()
+    return steps
 
 
 def _episode_ends(carry, rew, done):

@@ -295,6 +295,31 @@ class BatchedForestFire:
             _lib.check(_lib.lib().wf_set_policy_mlp_dev(self._h, _ptr(w1), _ptr(b1), _ptr(w2), _ptr(b2), hidden, float(eps),
                                                         self._stream()))
 
+    def set_policy_mlp_flat_dev(self, params, hidden: int, dueling: bool, eps):
+        """One in-kernel Q-network per group of envs (``wf_set_policy_mlp_nets_dev``): ``params`` is a float32 CUDA tensor
+        ``[M, P]`` of M networks in the flat ``parameters_to_vector`` layout of ``wf_replay_fit`` (``mlp_param_count``;
+        a dueling head acts with its advantage stream), ``eps`` M exploration rates.  Env n acts with network
+        ``n // (n_envs // M)``; ``n_envs`` must be a multiple of M and ``n_envs // M`` a multiple of 8.  Repacked by a
+        kernel on the current stream like ``set_policy_mlp_dev``, and network j acts exactly as ``set_policy_mlp_dev``
+        with the same weights and ``eps[j]`` would."""
+        if not (isinstance(params, torch.Tensor) and params.is_cuda and params.dtype == torch.float32
+                and params.device == self.device and params.dim() == 2):
+            raise ValueError(f"set_policy_mlp_flat_dev takes a float32 [M, P] tensor on {self.device}")
+        M = int(params.shape[0])
+        eps = [float(e) for e in eps]
+        if len(eps) != M:
+            raise ValueError(f"eps has {len(eps)} entries for {M} networks")
+        P = _lib.mlp_param_count(self.width, self.height, int(hidden), self.n_actions, bool(dueling))
+        if params.shape[1] != P:
+            raise ValueError(f"params has {params.shape[1]} floats per network, a {self.width}x{self.height}x3 -> {hidden} -> "
+                             f"{self.n_actions} network{' with a dueling head' if dueling else ''} has {P}")
+        params = params.detach().contiguous()
+        shape = _lib.WfMlpShape(width=self.width, height=self.height, hidden=int(hidden), n_actions=self.n_actions,
+                                dueling=int(bool(dueling)), batch=1)
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().wf_set_policy_mlp_nets_dev(self._h, C.byref(shape), M, _ptr(params),
+                                                             (C.c_double * M)(*eps), self._stream()))
+
     def step_host(self, actions):
         """Host-buffer step through ``wf_step_host``: H2D actions, step, D2H obs/reward/done, sync.
 

@@ -78,7 +78,8 @@ struct wf_env {
     int32_t a_iter;  // METADATA['a_speed_iter']: one per handle, not reset by reset() (Q8)
     int64_t launches;
     TileState* tstate;
-    float* mlp_dev;      // WF_POLICY_MLP weights: w1 | base | w2 | b2
+    float* mlp_dev;      // WF_POLICY_MLP weights: per network w1 | base | w2 | b2 | threshold
+    int32_t mlp_cap;     // network blocks mlp_dev holds
     MlpPolicy mlp;       // device pointers into mlp_dev (hid == 0: not set)
     // wf_step_host staging
     cudaStream_t hstream;
@@ -300,14 +301,20 @@ __global__ void get_obs_bits_kernel(DevState s, uint32_t* obs) {
     }
 }
 
-// wf_set_policy_mlp_dev: wf_set_policy_mlp's host repack, one thread per float of the packed buffer, from nn.Linear-oriented
-// weights (w1 [hidden][n_in], w2 [A][hidden]).  Every float of the buffer is written (padding 0, missing actions' bias
-// -inf), and `base` is summed in float64 in the host's order, so the buffer is byte-identical to the host path's.
+// wf_set_policy_mlp_dev / wf_set_policy_mlp_nets_dev: wf_set_policy_mlp's host repack, one thread per float of a network's
+// packed block (network blockIdx.y), from nn.Linear-oriented weights (w1 [hidden][n_in], w2 [A][hidden]; network k's at
+// in_stride floats after network k - 1's).  Every float of the block is written (padding 0, missing actions' bias -inf),
+// and `base` is summed in float64 in the host's order, so each block is byte-identical to the host path's.
+struct MlpThresholds {
+    uint32_t v[kMlpMaxNets];  // explore threshold of every network (mlp_eps_threshold)
+};
 __global__ void pack_policy_mlp_kernel(float* __restrict__ out, const float* __restrict__ w1, const float* __restrict__ b1,
-                                       const float* __restrict__ w2, const float* __restrict__ b2, int n_in, int cells,
-                                       int hidden, int A, int L) {
-    const int hpl = 64 / L;
-    const size_t n_w1 = (size_t)n_in * 64, total = n_w1 + 64 + 512 + 8;
+                                       const float* __restrict__ w2, const float* __restrict__ b2, size_t in_stride,
+                                       int n_in, int cells, int hidden, int A, int L, const MlpThresholds eps) {
+    const int hpl = 64 / L, net = blockIdx.y;
+    const size_t n_w1 = (size_t)n_in * 64, total = mlp_net_floats(n_in);
+    out += net * total;
+    w1 += net * in_stride, b1 += net * in_stride, w2 += net * in_stride, b2 += net * in_stride;
     for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         float v = 0.0f;
         if (i < n_w1) {  // w1 [n_in][64]: unit j sits at (j % L) * hpl + j / L
@@ -324,9 +331,11 @@ __global__ void pack_policy_mlp_kernel(float* __restrict__ out, const float* __r
         } else if (i < n_w1 + 64 + 512) {  // w2 [2][64][4]: action b of unit j at (b / 4) * 256 + j * 4 + b % 4
             const int k = (int)(i - n_w1 - 64), j = (k % 256) / 4, b = (k / 256) * 4 + k % 4;
             if (j < hidden && b < A) v = w2[(size_t)b * hidden + j];
-        } else {
+        } else if (i < n_w1 + 64 + 512 + 8) {
             const int b = (int)(i - n_w1 - 64 - 512);
             v = b < A ? b2[b] : -INFINITY;
+        } else if (i == n_w1 + 64 + 512 + 8) {
+            v = __uint_as_float(eps.v[net]);
         }
         out[i] = v;
     }
@@ -728,6 +737,32 @@ int wf_rollout_policy(wf_env* e, int32_t k_steps, int32_t policy, int32_t* actio
     return rollout_impl(e, k_steps, nullptr, policy, actions_out_dev, obs_dev, obs_dtype, reward_dev, done_dev, stream);
 }
 
+// Explore threshold of eps: a 32-bit draw below it explores.
+static uint32_t mlp_eps_threshold(double eps) { return eps >= 1.0 ? 0xffffffffu : (uint32_t)(eps * 4294967296.0); }
+
+// The handle's packed buffer holds at least n_nets network blocks; network 0's pointers, one group covering every env.
+static int mlp_reserve(wf_env* e, int n_nets, int hidden) {
+    const int n_in = e->st.W * e->st.H * 3;
+    const size_t per = mlp_net_floats(n_in);
+    if (!e->mlp_dev || e->mlp_cap < n_nets) {
+        cudaFree(e->mlp_dev);
+        e->mlp_dev = nullptr;
+        e->mlp_cap = 0;
+        e->mlp = MlpPolicy{};
+        WF_CUDA(cudaMalloc(&e->mlp_dev, per * n_nets * sizeof(float)));
+        e->mlp_cap = n_nets;
+    }
+    e->mlp.w1 = e->mlp_dev;
+    e->mlp.base = e->mlp_dev + (size_t)n_in * 64;
+    e->mlp.w2 = e->mlp.base + 64;
+    e->mlp.b2 = e->mlp.w2 + 512;
+    e->mlp.hid = hidden;
+    e->mlp.n_actions = e->cfg.n_actions;
+    e->mlp.group_envs = 1 << 30;  // one network for every env (a multiple of any CTA's envs)
+    e->mlp.net_stride = (int32_t)per;
+    return WF_OK;
+}
+
 int wf_set_policy_mlp(wf_env* e, const float* k1, const float* b1, const float* k2, const float* b2, int32_t hidden,
                       double eps) {
     if (!e || !k1 || !b1 || !k2 || !b2) return fail(WF_ERR_INVALID, "null argument");
@@ -738,9 +773,9 @@ int wf_set_policy_mlp(wf_env* e, const float* k1, const float* b1, const float* 
     WF_QUIESCE(e);
     const DevState& s = e->st;
     const int n_in = s.W * s.H * 3, A = e->cfg.n_actions;
-    // device layout (MlpPolicy): w1 [n_in][64] permuted for the lanes | base [64] | w2 [2][64][4] | b2 [8]
+    // device layout (MlpPolicy): w1 [n_in][64] permuted for the lanes | base [64] | w2 [2][64][4] | b2 [8] | threshold [8]
     const int L = s.RS, hpl = 64 / L;
-    const size_t n_w1 = (size_t)n_in * 64, total = n_w1 + 64 + 2 * 64 * 4 + 8;
+    const size_t n_w1 = (size_t)n_in * 64, total = mlp_net_floats(n_in);
     std::vector<float> hbuf(total, 0.0f);
     float* h = hbuf.data();
     for (int f = 0; f < n_in; ++f)
@@ -756,18 +791,29 @@ int wf_set_policy_mlp(wf_env* e, const float* k1, const float* b1, const float* 
         for (int b = 0; b < A; ++b) w2[(size_t)(b / 4) * 256 + j * 4 + (b & 3)] = k2[(size_t)j * A + b];
     float* bias2 = w2 + 512;
     for (int b = 0; b < 8; ++b) bias2[b] = b < A ? b2[b] : -INFINITY;
+    const uint32_t thr = mlp_eps_threshold(eps);
+    std::memcpy(bias2 + 8, &thr, sizeof(thr));
     cudaFree(e->mlp_dev);
     e->mlp_dev = nullptr;
-    e->mlp = MlpPolicy{};
-    WF_CUDA(cudaMalloc(&e->mlp_dev, total * sizeof(float)));
+    if (int rc = mlp_reserve(e, 1, hidden)) return rc;
     WF_CUDA(cudaMemcpy(e->mlp_dev, h, total * sizeof(float), cudaMemcpyHostToDevice));
-    e->mlp.w1 = e->mlp_dev;
-    e->mlp.base = e->mlp_dev + n_w1;
-    e->mlp.w2 = e->mlp.base + 64;
-    e->mlp.b2 = e->mlp.w2 + 512;
-    e->mlp.hid = hidden;
-    e->mlp.n_actions = A;
-    e->mlp.eps_u32 = eps >= 1.0 ? 0xffffffffu : (uint32_t)(eps * 4294967296.0);
+    return WF_OK;
+}
+
+// Queues the repack of n_nets networks (network k's weights at k * in_stride floats after w1 / b1 / w2 / b2) into the
+// handle's packed buffer on `stream`.
+static int pack_policy_nets(wf_env* e, int n_nets, const float* w1, const float* b1, const float* w2, const float* b2,
+                            size_t in_stride, int hidden, const double* eps, void* stream) {
+    MlpThresholds thr{};
+    for (int k = 0; k < n_nets; ++k) thr.v[k] = mlp_eps_threshold(eps[k]);
+    if (int rc = mlp_reserve(e, n_nets, hidden)) return rc;
+    const DevState& s = e->st;
+    const int n_in = s.W * s.H * 3;
+    const size_t total = mlp_net_floats(n_in);
+    const dim3 grid((unsigned)std::min<size_t>((total + 255) / 256, 148 * 16), (unsigned)n_nets);
+    pack_policy_mlp_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(e->mlp_dev, w1, b1, w2, b2, in_stride, n_in,
+                                                                                  s.W * s.H, hidden, e->cfg.n_actions, s.RS, thr);
+    WF_CUDA(cudaGetLastError());
     return WF_OK;
 }
 
@@ -781,20 +827,39 @@ int wf_set_policy_mlp_dev(wf_env* e, const float* w1, const float* b1, const flo
         if (reinterpret_cast<uintptr_t>(p) & 3u) return fail(WF_ERR_INVALID, "weights must be 4-byte aligned");
     WF_ON_DEVICE(e);
     WF_QUIESCE(e);
-    const DevState& s = e->st;
-    const int n_in = s.W * s.H * 3, A = e->cfg.n_actions;
-    const size_t n_w1 = (size_t)n_in * 64, total = n_w1 + 64 + 2 * 64 * 4 + 8;  // the layout of wf_set_policy_mlp
-    if (!e->mlp_dev) WF_CUDA(cudaMalloc(&e->mlp_dev, total * sizeof(float)));
-    pack_policy_mlp_kernel<<<(int)std::min<size_t>((total + 255) / 256, 148 * 16), 256, 0, static_cast<cudaStream_t>(stream)>>>(e->mlp_dev, w1, b1, w2, b2, n_in,
-                                                                                          s.W * s.H, hidden, A, s.RS);
-    WF_CUDA(cudaGetLastError());
-    e->mlp.w1 = e->mlp_dev;
-    e->mlp.base = e->mlp_dev + n_w1;
-    e->mlp.w2 = e->mlp.base + 64;
-    e->mlp.b2 = e->mlp.w2 + 512;
-    e->mlp.hid = hidden;
-    e->mlp.n_actions = A;
-    e->mlp.eps_u32 = eps >= 1.0 ? 0xffffffffu : (uint32_t)(eps * 4294967296.0);
+    return pack_policy_nets(e, 1, w1, b1, w2, b2, 0, hidden, &eps, stream);
+}
+
+int wf_set_policy_mlp_nets_dev(wf_env* e, const wf_mlp_shape* shape, int32_t n_nets, const float* params_dev,
+                               const double* eps_host, void* stream) {
+    if (!e || !shape || !params_dev || !eps_host) return fail(WF_ERR_INVALID, "wf_set_policy_mlp_nets_dev: null argument");
+    if (n_nets < 1 || n_nets > kMlpMaxNets) return fail(WF_ERR_INVALID, "wf_set_policy_mlp_nets_dev: n_nets must be in 1..64");
+    const wf_mlp_shape& sh = *shape;
+    if (sh.hidden < 1 || sh.hidden > 64) return fail(WF_ERR_INVALID, "wf_set_policy_mlp_nets_dev: hidden must be in 1..64");
+    if (sh.n_actions < 1 || sh.n_actions > 8) return fail(WF_ERR_INVALID, "wf_set_policy_mlp_nets_dev: n_actions must be in 1..8");
+    if (sh.dueling != 0 && sh.dueling != 1) return fail(WF_ERR_INVALID, "wf_set_policy_mlp_nets_dev: dueling must be 0 or 1");
+    if (sh.height < 10 || sh.width < sh.height || sh.width > 32)
+        return fail(WF_ERR_INVALID, "wf_set_policy_mlp_nets_dev: the grid must satisfy 10 <= height <= width <= 32");
+    for (int k = 0; k < n_nets; ++k)
+        if (!(eps_host[k] >= 0.0 && eps_host[k] <= 1.0)) return fail(WF_ERR_INVALID, "wf_set_policy_mlp_nets_dev: eps must be in [0, 1]");
+    if (reinterpret_cast<uintptr_t>(params_dev) & 3u) return fail(WF_ERR_INVALID, "wf_set_policy_mlp_nets_dev: params must be 4-byte aligned");
+    if (e->tile) return fail(WF_ERR_INVALID, "WF_POLICY_MLP is implemented for grids up to 32x32 (warp family) only");
+    if (sh.width != e->cfg.width || sh.height != e->cfg.height || sh.n_actions != e->cfg.n_actions)
+        return fail(WF_ERR_INVALID, "wf_set_policy_mlp_nets_dev: the shape's grid and n_actions must be the handle's");
+    if (e->N % n_nets != 0) return fail(WF_ERR_INVALID, "wf_set_policy_mlp_nets_dev: n_envs must be a multiple of n_nets");
+    const int group = e->N / n_nets;
+    if (group % 8 != 0) return fail(WF_ERR_INVALID, "wf_set_policy_mlp_nets_dev: n_envs / n_nets must be a multiple of 8");
+    WF_ON_DEVICE(e);
+    WF_QUIESCE(e);
+    // the flat layout of wf_replay_fit: dense_1.weight | dense_1.bias | dense_2.weight | dense_2.bias | (dueling) ...
+    const int n_in = sh.width * sh.height * 3, hid = sh.hidden, A = sh.n_actions;
+    const size_t P = (size_t)hid * (n_in + 1 + A) + A + (sh.dueling ? (size_t)hid * (n_in + 2) + 1 : 0);
+    const float* w1 = params_dev;
+    const float* b1 = w1 + (size_t)hid * n_in;
+    const float* w2 = b1 + hid;
+    const float* b2 = w2 + (size_t)A * hid;
+    if (int rc = pack_policy_nets(e, n_nets, w1, b1, w2, b2, P, hid, eps_host, stream)) return rc;
+    e->mlp.group_envs = group;
     return WF_OK;
 }
 

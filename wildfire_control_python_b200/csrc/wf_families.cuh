@@ -4,17 +4,22 @@
 
 namespace wf {
 
-// Q-network of WF_POLICY_MLP, device pointers (owned by the handle).  Everything is padded to 64 hidden units and
-// 8 actions (zero weights; -inf bias for the missing actions), so the kernel has no bounds tests.
+// Q-networks of WF_POLICY_MLP, device pointers into network 0's block (owned by the handle).  Everything is padded to 64
+// hidden units and 8 actions (zero weights; -inf bias for the missing actions), so the kernel has no bounds tests.
+// Network k's block starts net_stride floats after network k - 1's; env n acts with network n / group_envs.
 struct MlpPolicy {
     const float* w1;    // [n_in][64]: hidden unit j = x + L*i of a row sits at x*(64/L) + i (L = lanes per env), i.e. the
                         // units one lane accumulates are adjacent: one 16- or 8-byte load per changed input bit
     const float* base;  // [64]: bias1 + sum over cells of w1[(cell, channel 2)] -- the all-free, no-fire, no-agent map
     const float* w2;    // [2][64] float4: actions 0..3 and 4..7 of every hidden unit
-    const float* b2;    // [8]
+    const float* b2;    // [8], then [8]: the explore threshold (uint32 bits: explore iff a 32-bit draw is below it), 0 x 7
     int32_t hid, n_actions;
-    uint32_t eps_u32;   // explore iff a 32-bit draw is below this
+    int32_t group_envs; // envs per network: a multiple of the envs of one CTA, so a CTA's envs share one network
+    int32_t net_stride; // floats per network block
 };
+constexpr int kMlpMaxNets = 64;
+// Floats of one network's block: w1 | base [64] | w2 [2][64][4] | b2 [8] | threshold + padding [8].
+__host__ __device__ inline size_t mlp_net_floats(int n_in) { return (size_t)n_in * 64 + 64 + 512 + 16; }
 
 // Step-server session (wf_host_session): the warp kernel stays resident and is driven from the host through
 // flags in mapped page-locked memory -- no launch and no stream synchronise per step.

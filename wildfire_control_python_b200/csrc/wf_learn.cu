@@ -1,6 +1,8 @@
-// wf_learn.cu -- wf_replay_fit (include/wildfire.h): n_replays consecutive DQN.replay / fit_batch updates
-// (DQN.py:156-185, DQN_SARSA.py:103-132; the rule agents.py pins to tests/golden/agents/n1_replay.npz) in ONE launch of
-// one thread-block cluster.
+// wf_learn.cu -- wf_replay_fit / wf_replay_fit_many (include/wildfire.h): n_replays consecutive DQN.replay / fit_batch
+// updates (DQN.py:156-185, DQN_SARSA.py:103-132; the rule agents.py pins to tests/golden/agents/n1_replay.npz) for each of
+// up to 64 independent learners in ONE launch: one thread-block cluster per learner (learner = cluster index).  A
+// cluster reads only its learner's descriptor, so its result does not depend on the other learners; with the same
+// cluster size it is bit-identical to a launch of that learner alone (wf_replay_fit is the one-learner case).
 //
 // Work split.  The network's hidden units (hidden, or 2 * hidden for the dueling head: advantage units first, then value
 // units) are dealt out to the CTAs of the cluster in contiguous slices.  A CTA reads and writes only its own units' first-
@@ -33,14 +35,13 @@ namespace {
 constexpr int kThreads = 512;
 constexpr int kMaxBatch = 256, kMaxHidden = 64, kMaxActions = 8, kOut = kMaxActions + 1;
 constexpr int kMaxUnits = 16;  // units per CTA: 2 * kMaxHidden over a cluster of at least 8 CTAs
+constexpr int kMaxLearners = 64;
 
-struct FitArgs {
+struct FitLearner {  // one learner's buffers and hyper-parameters (wf_fit_learner, scalars prepared for the kernel)
     float* P;  // model
     float* T;  // target
     float* M;  // Adam m
     float* V;  // Adam v
-    const uint32_t* frames;
-    int64_t n_frames;
     const int64_t* s_row;
     const int64_t* sp_row;
     const int32_t* action;
@@ -48,13 +49,19 @@ struct FitArgs {
     const float* reward;
     const uint8_t* done;
     float* loss;
-    int n_replays;
-    int n_in, words, hid, A, duel, B;
-    int off_b1, off_w2, off_b2, off_w3, off_b3, off_w4, off_b4;
     float gamma, b1, omb1, b2, omb2, eps, clip;
     double lr, beta_1, beta_2;
     int64_t adam_t;
     int target_every, phase;
+};
+
+struct FitArgs {  // in the kernel's parameter block (~10 KB of the 32 KB limit)
+    const uint32_t* frames;
+    int64_t n_frames;
+    int n_replays;
+    int n_in, words, hid, A, duel, B;
+    int off_b1, off_w2, off_b2, off_w3, off_b3, off_w4, off_b4;
+    FitLearner learner[kMaxLearners];
 };
 
 struct Smem {
@@ -74,18 +81,19 @@ struct Smem {
 __device__ __forceinline__ float sigmoidf(float z) { return 1.0f / (1.0f + expf(-z)); }
 
 // Keras 2 Adam on one element (agents.KerasAdam.step): clip, moments, p -= lr_t * m / (sqrt(v) + epsilon).
-__device__ __forceinline__ float adam(const FitArgs& a, float lr_t, float p, float g, float& m, float& v) {
+__device__ __forceinline__ float adam(const FitLearner& a, float lr_t, float p, float g, float& m, float& v) {
     g = fminf(fmaxf(g, -a.clip), a.clip);
     m = m * a.b1 + a.omb1 * g;
     v = v * a.b2 + a.omb2 * g * g;
     return p + (-lr_t) * (m / (sqrtf(v) + a.eps));
 }
 
-__global__ void __launch_bounds__(kThreads) replay_fit_kernel(const FitArgs a) {
+__global__ void __launch_bounds__(kThreads) replay_fit_kernel(const __grid_constant__ FitArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Smem& S = *reinterpret_cast<Smem*>(smem_raw);
     cg::cluster_group cluster = cg::this_cluster();
     const int rank = (int)cluster.block_rank(), cs = (int)cluster.num_blocks();
+    const FitLearner& l = a.learner[blockIdx.x / cs];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = kThreads / 32;
     const int A = a.A, A1 = A + 1, B = a.B, hid = a.hid, n_in = a.n_in;
     const int n_units = hid * (a.duel ? 2 : 1);
@@ -101,30 +109,30 @@ __global__ void __launch_bounds__(kThreads) replay_fit_kernel(const FitArgs a) {
         const int o = tid;
         const bool has = o < A || a.duel;
         const int off = o < A ? a.off_b2 + o : a.off_b4;
-        S.ob[0][o] = has ? a.P[off] : 0.0f;
-        S.ob[1][o] = has ? a.T[off] : 0.0f;
-        S.ob[2][o] = has ? a.M[off] : 0.0f;
-        S.ob[3][o] = has ? a.V[off] : 0.0f;
+        S.ob[0][o] = has ? l.P[off] : 0.0f;
+        S.ob[1][o] = has ? l.T[off] : 0.0f;
+        S.ob[2][o] = has ? l.M[off] : 0.0f;
+        S.ob[3][o] = has ? l.V[off] : 0.0f;
     }
-    int until_sync = a.phase;
+    int until_sync = l.phase;
 
     for (int r = 0; r < a.n_replays; ++r) {
         const int buf = r & 1;
         const int64_t i0 = (int64_t)r * B;
         for (int b = tid; b < B; b += kThreads) {
-            S.row[0][b] = a.s_row[i0 + b];
-            S.row[1][b] = a.sp_row[i0 + b];
-            S.act[b] = a.action[i0 + b];
-            S.nact[b] = a.next_action ? a.next_action[i0 + b] : 0;
-            S.rew[b] = a.reward[i0 + b];
-            S.dn[b] = a.done[i0 + b];
+            S.row[0][b] = l.s_row[i0 + b];
+            S.row[1][b] = l.sp_row[i0 + b];
+            S.act[b] = l.action[i0 + b];
+            S.nact[b] = l.next_action ? l.next_action[i0 + b] : 0;
+            S.rew[b] = l.reward[i0 + b];
+            S.dn[b] = l.done[i0 + b];
         }
         __syncthreads();
 
         // ---- forward: model(s), target(s), target(s'); one warp per (pass, sample), lanes over the input bits
         for (int item = warp; item < 3 * B; item += nwarps) {
             const int p = item / B, b = item - p * B;
-            const float* W = p == 0 ? a.P : a.T;
+            const float* W = p == 0 ? l.P : l.T;
             const int64_t row = S.row[p == 2 ? 1 : 0][b];
             const bool ok = row >= 0 && row < a.n_frames;
             const uint32_t* bits = a.frames + (ok ? row : 0) * a.words;
@@ -182,12 +190,12 @@ __global__ void __launch_bounds__(kThreads) replay_fit_kernel(const FitArgs a) {
             const int act = S.act[b], nact = S.nact[b];
             float upd = S.rew[b];
             if (!S.dn[b]) {
-                if (a.next_action) {
-                    if (nact >= 0 && nact < A) upd = S.rew[b] + a.gamma * qv[2][nact];
+                if (l.next_action) {
+                    if (nact >= 0 && nact < A) upd = S.rew[b] + l.gamma * qv[2][nact];
                 } else {
                     float best = qv[2][0];
                     for (int o = 1; o < A; ++o) best = fmaxf(best, qv[2][o]);
-                    upd = S.rew[b] + a.gamma * best;
+                    upd = S.rew[b] + l.gamma * best;
                 }
             }
             float se = 0.0f, dsum = 0.0f, dq[kMaxActions];
@@ -210,19 +218,19 @@ __global__ void __launch_bounds__(kThreads) replay_fit_kernel(const FitArgs a) {
         }
         __syncthreads();
 
-        if (rank == 0 && tid == 0 && a.loss) {
+        if (rank == 0 && tid == 0 && l.loss) {
             float s = 0.0f;
             for (int b = 0; b < B; ++b) s += S.sqerr[b];
-            a.loss[r] = s * inv_n;
+            l.loss[r] = s * inv_n;
         }
         // ---- back through the second layer into this CTA's units (reads the second layer before it is updated)
         for (int k = tid; k < B * nu; k += kThreads) {
             const int b = k / nu, u = k - b * nu, g = g0 + u;
             float dh = 0.0f;
             if (g < hid) {
-                for (int o = 0; o < A; ++o) dh += S.dout[b][o] * a.P[w2_off(g, o)];
+                for (int o = 0; o < A; ++o) dh += S.dout[b][o] * l.P[w2_off(g, o)];
             } else {
-                dh = S.dout[b][A] * a.P[w2_off(g, A)];
+                dh = S.dout[b][A] * l.P[w2_off(g, A)];
             }
             const float hv = S.h[b][u];
             S.dz[b][u] = dh * hv * (1.0f - hv);
@@ -230,10 +238,10 @@ __global__ void __launch_bounds__(kThreads) replay_fit_kernel(const FitArgs a) {
         __syncthreads();
 
         // ---- Adam on every parameter this CTA owns (+ the shared output biases, redundantly), then the target copy
-        const int64_t t = a.adam_t + r + 1;
-        const float lr_t = (float)(a.lr * sqrt(1.0 - pow(a.beta_2, (double)t)) / (1.0 - pow(a.beta_1, (double)t)));
+        const int64_t t = l.adam_t + r + 1;
+        const float lr_t = (float)(l.lr * sqrt(1.0 - pow(l.beta_2, (double)t)) / (1.0 - pow(l.beta_1, (double)t)));
         const bool sync = --until_sync == 0;
-        if (sync) until_sync = a.target_every;
+        if (sync) until_sync = l.target_every;
         for (int k = tid; k < nu * n_in; k += kThreads) {  // first-layer rows
             const int u = k / n_in, f = k - u * n_in;
             const int off = w1_off(g0 + u) + f;
@@ -244,12 +252,12 @@ __global__ void __launch_bounds__(kThreads) replay_fit_kernel(const FitArgs a) {
                 const int64_t row = S.row[0][b];
                 if (row >= 0 && row < a.n_frames && (__ldg(a.frames + row * a.words + w) & bit)) g += S.dz[b][u];
             }
-            float m = a.M[off], v = a.V[off];
-            const float p = adam(a, lr_t, a.P[off], g, m, v);
-            a.P[off] = p;
-            a.M[off] = m;
-            a.V[off] = v;
-            if (sync) a.T[off] = p;
+            float m = l.M[off], v = l.V[off];
+            const float p = adam(l, lr_t, l.P[off], g, m, v);
+            l.P[off] = p;
+            l.M[off] = m;
+            l.V[off] = v;
+            if (sync) l.T[off] = p;
         }
         for (int k = tid; k < nu * (1 + A1); k += kThreads) {  // first-layer biases and second-layer columns
             const int u = k / (1 + A1), c = k - u * (1 + A1), g = g0 + u;
@@ -264,18 +272,18 @@ __global__ void __launch_bounds__(kThreads) replay_fit_kernel(const FitArgs a) {
                 off = w2_off(g, o);
                 for (int b = 0; b < B; ++b) gr += S.dout[b][o] * S.h[b][u];
             }
-            float m = a.M[off], v = a.V[off];
-            const float p = adam(a, lr_t, a.P[off], gr, m, v);
-            a.P[off] = p;
-            a.M[off] = m;
-            a.V[off] = v;
-            if (sync) a.T[off] = p;
+            float m = l.M[off], v = l.V[off];
+            const float p = adam(l, lr_t, l.P[off], gr, m, v);
+            l.P[off] = p;
+            l.M[off] = m;
+            l.V[off] = v;
+            if (sync) l.T[off] = p;
         }
         if (tid < A1 && (tid < A || a.duel)) {  // output biases: every CTA, identically
             const int o = tid;
             float gr = 0.0f;
             for (int b = 0; b < B; ++b) gr += S.dout[b][o];
-            S.ob[0][o] = adam(a, lr_t, S.ob[0][o], gr, S.ob[2][o], S.ob[3][o]);
+            S.ob[0][o] = adam(l, lr_t, S.ob[0][o], gr, S.ob[2][o], S.ob[3][o]);
             if (sync) S.ob[1][o] = S.ob[0][o];
         }
         __syncthreads();
@@ -283,10 +291,10 @@ __global__ void __launch_bounds__(kThreads) replay_fit_kernel(const FitArgs a) {
 
     if (rank == 0 && tid < A1 && (tid < A || a.duel)) {
         const int o = tid, off = o < A ? a.off_b2 + o : a.off_b4;
-        a.P[off] = S.ob[0][o];
-        a.T[off] = S.ob[1][o];
-        a.M[off] = S.ob[2][o];
-        a.V[off] = S.ob[3][o];
+        l.P[off] = S.ob[0][o];
+        l.T[off] = S.ob[1][o];
+        l.M[off] = S.ob[2][o];
+        l.V[off] = S.ob[3][o];
     }
     cluster.sync();  // no CTA leaves while a peer may still read its partial sums
 }
@@ -326,48 +334,47 @@ int cluster_size_for(int device, size_t smem, cudaError_t* err) {
     return 0;
 }
 
-}  // namespace
-
-extern "C" int wf_replay_fit(const wf_mlp_shape* shape, const wf_fit_params* hp, int32_t n_replays, float* params_dev,
-                             float* target_dev, float* adam_m_dev, float* adam_v_dev, const uint32_t* frames_dev,
-                             int64_t n_frames, const int64_t* s_row_dev, const int64_t* sp_row_dev,
-                             const int32_t* action_dev, const int32_t* next_action_dev, const float* reward_dev,
-                             const uint8_t* done_dev, float* loss_dev, void* stream) {
-    if (!shape || !hp || !params_dev || !target_dev || !adam_m_dev || !adam_v_dev || !frames_dev || !s_row_dev ||
-        !sp_row_dev || !action_dev || !reward_dev || !done_dev)
-        return api_fail(WF_ERR_INVALID, "wf_replay_fit: null argument");
-    const wf_mlp_shape& sh = *shape;
-    if (sh.height < 10 || sh.width < sh.height || sh.width > 32)
-        return api_fail(WF_ERR_INVALID, "wf_replay_fit: the grid must satisfy 10 <= height <= width <= 32");
-    if (sh.hidden < 1 || sh.hidden > kMaxHidden) return api_fail(WF_ERR_INVALID, "wf_replay_fit: hidden must be in 1..64");
-    if (sh.n_actions < 1 || sh.n_actions > kMaxActions)
-        return api_fail(WF_ERR_INVALID, "wf_replay_fit: n_actions must be in 1..8");
-    if (sh.dueling != 0 && sh.dueling != 1) return api_fail(WF_ERR_INVALID, "wf_replay_fit: dueling must be 0 or 1");
-    if (sh.batch < 1 || sh.batch > kMaxBatch) return api_fail(WF_ERR_INVALID, "wf_replay_fit: batch must be in 1..256");
-    if (n_replays < 1) return api_fail(WF_ERR_INVALID, "wf_replay_fit: n_replays must be >= 1");
-    if (n_frames < 0) return api_fail(WF_ERR_INVALID, "wf_replay_fit: n_frames must be >= 0");
+// Refuses a learner whose pointers or hyper-parameters wf_replay_fit would refuse; `who` prefixes the message.
+int check_learner(const std::string& who, const wf_fit_learner& l) {
+    if (!l.params || !l.target || !l.adam_m || !l.adam_v || !l.s_row || !l.sp_row || !l.action || !l.reward || !l.done)
+        return api_fail(WF_ERR_INVALID, who + ": null argument");
+    const wf_fit_params* hp = &l.hp;
     if (hp->target_every < 1 || hp->phase < 1 || hp->phase > hp->target_every)
-        return api_fail(WF_ERR_INVALID, "wf_replay_fit: need target_every >= 1 and 1 <= phase <= target_every");
-    if (hp->adam_t < 0) return api_fail(WF_ERR_INVALID, "wf_replay_fit: adam_t must be >= 0");
+        return api_fail(WF_ERR_INVALID, who + ": need target_every >= 1 and 1 <= phase <= target_every");
+    if (hp->adam_t < 0) return api_fail(WF_ERR_INVALID, who + ": adam_t must be >= 0");
     if (!(hp->clipvalue > 0.0) || !std::isfinite(hp->gamma) || !std::isfinite(hp->lr) || !(hp->beta_1 >= 0.0 && hp->beta_1 < 1.0) ||
         !(hp->beta_2 >= 0.0 && hp->beta_2 < 1.0) || !(hp->epsilon >= 0.0))
-        return api_fail(WF_ERR_INVALID, "wf_replay_fit: bad hyper-parameter (need clipvalue > 0, 0 <= beta < 1, epsilon >= 0)");
-    for (const void* p : {(const void*)params_dev, (const void*)target_dev, (const void*)adam_m_dev, (const void*)adam_v_dev,
-                          (const void*)frames_dev})
-        if (reinterpret_cast<uintptr_t>(p) & 3u) return api_fail(WF_ERR_INVALID, "wf_replay_fit: buffers must be 4-byte aligned");
-    for (const void* p : {(const void*)action_dev, (const void*)next_action_dev, (const void*)reward_dev})
-        if (reinterpret_cast<uintptr_t>(p) & 3u) return api_fail(WF_ERR_INVALID, "wf_replay_fit: buffers must be 4-byte aligned");
-    if ((reinterpret_cast<uintptr_t>(s_row_dev) | reinterpret_cast<uintptr_t>(sp_row_dev)) & 7u)
-        return api_fail(WF_ERR_INVALID, "wf_replay_fit: s_row and sp_row must be 8-byte aligned");
+        return api_fail(WF_ERR_INVALID, who + ": bad hyper-parameter (need clipvalue > 0, 0 <= beta < 1, epsilon >= 0)");
+    for (const void* p : {(const void*)l.params, (const void*)l.target, (const void*)l.adam_m, (const void*)l.adam_v,
+                          (const void*)l.action, (const void*)l.next_action, (const void*)l.reward, (const void*)l.loss})
+        if (reinterpret_cast<uintptr_t>(p) & 3u) return api_fail(WF_ERR_INVALID, who + ": buffers must be 4-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(l.s_row) | reinterpret_cast<uintptr_t>(l.sp_row)) & 7u)
+        return api_fail(WF_ERR_INVALID, who + ": s_row and sp_row must be 8-byte aligned");
+    return WF_OK;
+}
+
+// wf_replay_fit_many after the caller's null checks; `name` is the entry point the messages name.
+int replay_fit_impl(const char* name, const wf_mlp_shape& sh, int32_t n_learners, const wf_fit_learner* learners,
+                    int32_t n_replays, const uint32_t* frames_dev, int64_t n_frames, void* stream) {
+    const std::string fn(name);
+    if (n_learners < 1 || n_learners > kMaxLearners) return api_fail(WF_ERR_INVALID, fn + ": n_learners must be in 1..64");
+    if (sh.height < 10 || sh.width < sh.height || sh.width > 32)
+        return api_fail(WF_ERR_INVALID, fn + ": the grid must satisfy 10 <= height <= width <= 32");
+    if (sh.hidden < 1 || sh.hidden > kMaxHidden) return api_fail(WF_ERR_INVALID, fn + ": hidden must be in 1..64");
+    if (sh.n_actions < 1 || sh.n_actions > kMaxActions) return api_fail(WF_ERR_INVALID, fn + ": n_actions must be in 1..8");
+    if (sh.dueling != 0 && sh.dueling != 1) return api_fail(WF_ERR_INVALID, fn + ": dueling must be 0 or 1");
+    if (sh.batch < 1 || sh.batch > kMaxBatch) return api_fail(WF_ERR_INVALID, fn + ": batch must be in 1..256");
+    if (n_replays < 1) return api_fail(WF_ERR_INVALID, fn + ": n_replays must be >= 1");
+    if (n_frames < 0) return api_fail(WF_ERR_INVALID, fn + ": n_frames must be >= 0");
+    if (reinterpret_cast<uintptr_t>(frames_dev) & 3u) return api_fail(WF_ERR_INVALID, fn + ": buffers must be 4-byte aligned");
+    for (int j = 0; j < n_learners; ++j)
+        if (int rc = check_learner(n_learners == 1 ? fn : fn + ": learner " + std::to_string(j), learners[j])) return rc;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
         return api_fail(WF_ERR_CUDA, "no CUDA device: libwildfire_b200 has no CPU fallback");
 
     FitArgs a{};
-    a.P = params_dev, a.T = target_dev, a.M = adam_m_dev, a.V = adam_v_dev;
-    a.frames = frames_dev, a.n_frames = n_frames;
-    a.s_row = s_row_dev, a.sp_row = sp_row_dev, a.action = action_dev, a.next_action = next_action_dev;
-    a.reward = reward_dev, a.done = done_dev, a.loss = loss_dev, a.n_replays = n_replays;
+    a.frames = frames_dev, a.n_frames = n_frames, a.n_replays = n_replays;
     a.n_in = sh.width * sh.height * 3;
     a.words = (int)wf::obs_bits_words(sh.width, sh.height);
     a.hid = sh.hidden, a.A = sh.n_actions, a.duel = sh.dueling, a.B = sh.batch;
@@ -378,33 +385,60 @@ extern "C" int wf_replay_fit(const wf_mlp_shape* shape, const wf_fit_params* hp,
     a.off_b3 = a.off_w3 + a.hid * a.n_in;
     a.off_w4 = a.off_b3 + a.hid;
     a.off_b4 = a.off_w4 + a.hid;
-    // scalars as torch applies them to float32 tensors (KerasAdam.step): cast once to float
-    a.gamma = (float)hp->gamma;
-    a.b1 = (float)hp->beta_1, a.omb1 = (float)(1.0 - hp->beta_1);
-    a.b2 = (float)hp->beta_2, a.omb2 = (float)(1.0 - hp->beta_2);
-    a.eps = (float)hp->epsilon, a.clip = (float)hp->clipvalue;
-    a.lr = hp->lr, a.beta_1 = hp->beta_1, a.beta_2 = hp->beta_2;
-    a.adam_t = hp->adam_t, a.target_every = hp->target_every, a.phase = hp->phase;
+    for (int j = 0; j < n_learners; ++j) {
+        const wf_fit_learner& in = learners[j];
+        const wf_fit_params* hp = &in.hp;
+        FitLearner& l = a.learner[j];
+        l.P = in.params, l.T = in.target, l.M = in.adam_m, l.V = in.adam_v;
+        l.s_row = in.s_row, l.sp_row = in.sp_row, l.action = in.action, l.next_action = in.next_action;
+        l.reward = in.reward, l.done = in.done, l.loss = in.loss;
+        // scalars as torch applies them to float32 tensors (KerasAdam.step): cast once to float
+        l.gamma = (float)hp->gamma;
+        l.b1 = (float)hp->beta_1, l.omb1 = (float)(1.0 - hp->beta_1);
+        l.b2 = (float)hp->beta_2, l.omb2 = (float)(1.0 - hp->beta_2);
+        l.eps = (float)hp->epsilon, l.clip = (float)hp->clipvalue;
+        l.lr = hp->lr, l.beta_1 = hp->beta_1, l.beta_2 = hp->beta_2;
+        l.adam_t = hp->adam_t, l.target_every = hp->target_every, l.phase = hp->phase;
+    }
 
     const size_t smem = sizeof(Smem);
     int device = 0;
     cudaError_t err = cudaGetDevice(&device);
     const int cs = err == cudaSuccess ? cluster_size_for(device, smem, &err) : 0;
-    if (err != cudaSuccess) return api_fail(WF_ERR_CUDA, std::string("wf_replay_fit: ") + cudaGetErrorString(err));
-    if (cs == 0) return api_fail(WF_ERR_CUDA, "wf_replay_fit: no thread-block cluster of 8 or 16 CTAs fits this device");
+    if (err != cudaSuccess) return api_fail(WF_ERR_CUDA, fn + ": " + cudaGetErrorString(err));
+    if (cs == 0) return api_fail(WF_ERR_CUDA, fn + ": no thread-block cluster of 8 or 16 CTAs fits this device");
     cudaLaunchConfig_t cfg = {};
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = cs;
     attr[0].val.clusterDim.y = 1;
     attr[0].val.clusterDim.z = 1;
-    cfg.gridDim = dim3(cs);
+    cfg.gridDim = dim3(cs * n_learners);  // one cluster per learner: clusters beyond what the GPU holds run in later waves
     cfg.blockDim = dim3(kThreads);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = static_cast<cudaStream_t>(stream);
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     err = cudaLaunchKernelEx(&cfg, replay_fit_kernel, a);
-    if (err != cudaSuccess) return api_fail(WF_ERR_CUDA, std::string("wf_replay_fit: ") + cudaGetErrorString(err));
+    if (err != cudaSuccess) return api_fail(WF_ERR_CUDA, fn + ": " + cudaGetErrorString(err));
     return WF_OK;
+}
+
+}  // namespace
+
+extern "C" int wf_replay_fit_many(const wf_mlp_shape* shape, int32_t n_learners, const wf_fit_learner* learners_host,
+                                  int32_t n_replays, const uint32_t* frames_dev, int64_t n_frames, void* stream) {
+    if (!shape || !learners_host || !frames_dev) return api_fail(WF_ERR_INVALID, "wf_replay_fit_many: null argument");
+    return replay_fit_impl("wf_replay_fit_many", *shape, n_learners, learners_host, n_replays, frames_dev, n_frames, stream);
+}
+
+extern "C" int wf_replay_fit(const wf_mlp_shape* shape, const wf_fit_params* hp, int32_t n_replays, float* params_dev,
+                             float* target_dev, float* adam_m_dev, float* adam_v_dev, const uint32_t* frames_dev,
+                             int64_t n_frames, const int64_t* s_row_dev, const int64_t* sp_row_dev,
+                             const int32_t* action_dev, const int32_t* next_action_dev, const float* reward_dev,
+                             const uint8_t* done_dev, float* loss_dev, void* stream) {
+    if (!shape || !hp || !frames_dev) return api_fail(WF_ERR_INVALID, "wf_replay_fit: null argument");
+    const wf_fit_learner l{params_dev, target_dev, adam_m_dev, adam_v_dev, s_row_dev, sp_row_dev, action_dev, next_action_dev,
+                           reward_dev, done_dev, loss_dev, *hp};
+    return replay_fit_impl("wf_replay_fit", *shape, 1, &l, n_replays, frames_dev, n_frames, stream);
 }

@@ -305,7 +305,9 @@ __device__ __forceinline__ void warp_body(const DevState& s, const StepCfg& c, c
     // the 4-byte-per-lane stores of unaligned 152-byte records (which cost ~25 us per step on the link)
     __shared__ __align__(16) uint32_t srv_block[SRV ? kWarpsPerBlock * 97 + 31 + 96 : 1];  // (+ slack: the sector copy reads 7-word groups)
     __shared__ float4 mlp_w2[MLP ? 2 * kHidMax : 1];  // second layer (MlpPolicy::w2), read every step
-    __shared__ float mlp_b2[kActMax];
+    __shared__ float mlp_b2[MLP ? kActMax + 1 : kActMax];  // + the explore threshold (uint32 bits)
+    // WF_POLICY_MLP: this CTA's envs all act with one network (MlpPolicy::group_envs is a multiple of the CTA's envs)
+    const size_t mlp_off = MLP ? (size_t)((int)blockIdx.x * (kWarpsPerBlock * (32 / L)) / io.mlp.group_envs) * io.mlp.net_stride : 0;
     for (int v = threadIdx.x; v < 256; v += blockDim.x) {
         uint32_t o = 0u;
 #pragma unroll
@@ -314,8 +316,8 @@ __device__ __forceinline__ void warp_body(const DevState& s, const StepCfg& c, c
         tab8[v] = make_uint2(((v & 15u) * 0x00204081u) & 0x01010101u, (((v >> 4) & 15u) * 0x00204081u) & 0x01010101u);
     }
     if (MLP) {
-        for (int v = threadIdx.x; v < 2 * kHidMax; v += blockDim.x) mlp_w2[v] = reinterpret_cast<const float4*>(io.mlp.w2)[v];
-        if (threadIdx.x < kActMax) mlp_b2[threadIdx.x] = io.mlp.b2[threadIdx.x];
+        for (int v = threadIdx.x; v < 2 * kHidMax; v += blockDim.x) mlp_w2[v] = reinterpret_cast<const float4*>(io.mlp.w2 + mlp_off)[v];
+        if (threadIdx.x <= kActMax) mlp_b2[threadIdx.x] = io.mlp.b2[mlp_off + threadIdx.x];
     }
     __syncthreads();
 
@@ -361,7 +363,7 @@ __device__ __forceinline__ void warp_body(const DevState& s, const StepCfg& c, c
     uint32_t pA = 0u, pF = 0u, pFree = validmask;  // the empty map: what `base` stands for
     if (MLP) {
 #pragma unroll
-        for (int i = 0; i < HPL; ++i) hacc[i] = (double)io.mlp.base[x + L * i];
+        for (int i = 0; i < HPL; ++i) hacc[i] = (double)io.mlp.base[mlp_off + x + L * i];
     }
 
     if (io.reset_mode) {
@@ -507,7 +509,7 @@ __device__ __forceinline__ void warp_body(const DevState& s, const StepCfg& c, c
                     }
                     code = __shfl_sync(FULL, code, sub * L + owner);
                     if (mine) {
-                        const float* wrow = io.mlp.w1 + (size_t)(code >> 1) * kHidMax + x * HPL;
+                        const float* wrow = io.mlp.w1 + mlp_off + (size_t)(code >> 1) * kHidMax + x * HPL;
                         const uint32_t flip = (code & 1u) ? 0u : 0x80000000u;  // bit cleared: subtract the row
                         float wv[HPL];
                         if (HPL == 4) {
@@ -564,7 +566,7 @@ __device__ __forceinline__ void warp_body(const DevState& s, const StepCfg& c, c
                     ablk_idx = a.t >> 1;
                 }
                 const uint32_t u0 = (a.t & 1u) ? ablk[2] : ablk[0], u1 = (a.t & 1u) ? ablk[3] : ablk[1];
-                action = (u0 < io.mlp.eps_u32) ? (int)(u1 % (uint32_t)c.n_actions) : greedy;
+                action = (u0 < __float_as_uint(mlp_b2[kActMax])) ? (int)(u1 % (uint32_t)c.n_actions) : greedy;
             } else if (io.policy == WF_POLICY_WALK) {
                 // DQN.choose_randomwalk_action (DQN.py:353-389): walk clockwise round the fire origin,
                 // re-draw (at most 11 times) while the move would step onto a burning cell.
@@ -1061,7 +1063,9 @@ cudaError_t launch_warp_family(const DevState& s, const StepCfg& c, const WarpIO
     const dim3 grid((s.N + envs_per_block - 1) / envs_per_block), block(kWarpsPerBlock * 32);
     if (s.HB != 0 && (s.HB != kHitBits || s.FB != 5)) return cudaErrorInvalidValue;
     const bool mlp = io.policy == WF_POLICY_MLP && io.actions == nullptr && !io.reset_mode;
-    if (mlp && (io.mlp.hid < 1 || io.mlp.hid > kHidMax || io.mlp.n_actions > kActMax)) return cudaErrorInvalidValue;
+    if (mlp && (io.mlp.hid < 1 || io.mlp.hid > kHidMax || io.mlp.n_actions > kActMax || io.mlp.group_envs < 1 ||
+                io.mlp.group_envs % envs_per_block != 0))
+        return cudaErrorInvalidValue;
     const bool ob = io.obs != nullptr && io.obs_dtype == WF_OBS_BITS;
 #define WF_LAUNCH(LL, FF, UU, MM)                                                   \
     do {                                                                            \
