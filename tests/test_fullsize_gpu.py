@@ -159,17 +159,7 @@ def _rollout_against_oracle(gpu, orc, steps, chunk, policy, check_state_every):
     return events
 
 
-@pytest.fixture(params=["overlapped", "phased", "fused"])
-def tile_pass(request, monkeypatch):
-    """The three step structures of the tile kernel: the default (tick, then observation, with finish / the next agent phase /
-    cluster barrier Y overlapped with the observation), the strictly phased flow (WF_TILE_OVERLAP=0) and the opt-in fused
-    pass (WF_TILE_FUSED=1: the tick of step k emits the observation of step k-1 in the same cp.async-staged sweep)."""
-    monkeypatch.setenv("WF_TILE_FUSED", "1" if request.param == "fused" else "0")
-    monkeypatch.setenv("WF_TILE_OVERLAP", "0" if request.param == "phased" else "1")
-    return request.param
-
-
-def test_c4_production_geometry_matches_oracle(monkeypatch, tile_pass):
+def test_c4_production_geometry_matches_oracle(monkeypatch):
     """C4 (256x256, wind [0.85,(1,0)], 32 extra ignitions) on the geometry its 1024-env batch runs with: 256 threads,
     cluster of 1.  300 ticks in 16-step launches: several ignition generations, burn-outs, deaths and auto-resets."""
     geom = _production_geometry(monkeypatch, 256, 1024)
@@ -185,7 +175,7 @@ def test_c4_production_geometry_matches_oracle(monkeypatch, tile_pass):
     assert ev["done"] >= 1  # at least one in-kernel reset happened
 
 
-def test_c5_production_geometry_matches_oracle(monkeypatch, tile_pass):
+def test_c5_production_geometry_matches_oracle(monkeypatch):
     """C5 (1024x1024, no wind, 256 extra ignitions) on the geometry its 64-env batch runs with: 16 CTAs of 128 threads
     per env (8 of 256 where the device cannot hold a cluster of 16).  272 ticks in 16-step launches (14 ignition generations of the 19-tick delay; the first fires burn out at tick 20)."""
     geom = _production_geometry(monkeypatch, 1024, 64)
@@ -200,7 +190,7 @@ def test_c5_production_geometry_matches_oracle(monkeypatch, tile_pass):
     _rollout_against_oracle(gpu, orc, 272, 16, "stream", 136)
 
 
-def test_c5_geometry_walk_policy_contains_burns_out_and_resets(monkeypatch, tile_pass):
+def test_c5_geometry_walk_policy_contains_burns_out_and_resets(monkeypatch):
     """1024x1024 on the C5 geometry with the reference's heuristic walk policy (DQN.py:353-389): the bulldozer rings
     the fire (containment bonus, environment.py:342-377 -- the reach plane is cut by the closing dig and re-flooded by
     the whole cluster), the ring burns out (burn-out reward), the env resets inside the kernel and does it again."""

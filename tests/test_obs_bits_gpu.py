@@ -86,13 +86,6 @@ def test_warp_family_bits_equal_uint8(W, H, N, cfg):
 
 # ---------------------------------------------------------------------------------------------
 # tile family
-@pytest.fixture(params=["overlapped", "phased", "fused"])
-def tile_pass(request, monkeypatch):
-    monkeypatch.setenv("WF_TILE_FUSED", "1" if request.param == "fused" else "0")
-    monkeypatch.setenv("WF_TILE_OVERLAP", "0" if request.param == "phased" else "1")
-    return request.param
-
-
 def _tile_run(monkeypatch, W, H, N, T, CS, steps, chunk, want_done, **cfg):
     monkeypatch.setenv("WF_TILE_T", str(T))
     monkeypatch.setenv("WF_TILE_CS", str(CS))
@@ -113,19 +106,19 @@ def _tile_run(monkeypatch, W, H, N, T, CS, steps, chunk, want_done, **cfg):
     return a.tile_geometry
 
 
-def test_tile_c4_production_geometry(monkeypatch, tile_pass):
+def test_tile_c4_production_geometry(monkeypatch):
     geom = _tile_run(monkeypatch, 256, 256, 4, 256, 1, 96, 16, False, wind=[0.85, (1, 0)], extra_ignitions=32)
     assert geom == (256, 1)
 
 
 @pytest.mark.parametrize("T,CS", [(256, 8), (128, 16)])
-def test_tile_1024_clusters(monkeypatch, tile_pass, T, CS):
+def test_tile_1024_clusters(monkeypatch, T, CS):
     geom = _tile_run(monkeypatch, 1024, 1024, 2, T, CS, 32, 16, False, extra_ignitions=64)
     assert geom[1] > 1
 
 
 @pytest.mark.parametrize("W,H,T,CS", [(100, 70, 128, 4), (48, 33, 128, 2), (40, 40, 128, 2)])
-def test_tile_ragged_sizes_straddle_cta_slices(monkeypatch, tile_pass, W, H, T, CS):
+def test_tile_ragged_sizes_straddle_cta_slices(monkeypatch, W, H, T, CS):
     geom = _tile_run(monkeypatch, W, H, 5, T, CS, 320, 32, True, wind=[0.85, (1, 0)], extra_ignitions=3)
     assert geom[1] == CS
 

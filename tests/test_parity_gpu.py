@@ -411,21 +411,9 @@ def test_tile_cluster_geometries_match_oracle(monkeypatch, T, CS, cfg):
                                  dict(width=128, height=128, seed=712, make_rivers=True, wind="random", a_speed=2, extra_ignitions=3),
                                  dict(width=256, height=128, seed=713, wind=[0.85, (1, 0)], extra_ignitions=9, fuel=40)],
                          ids=["128_toggle", "128_rivers_aspeed2", "256x128_wide_fuel40"])
-def test_tile_fused_pass_matches_oracle(monkeypatch, T, CS, cfg):
-    """WF_TILE_FUSED=1: the tick of step k and the observation of step k-1 in one cp.async-staged sweep (grids whose
-    slices are whole 128-word groups).  Same check as the geometry sweep above."""
-    monkeypatch.setenv("WF_TILE_FUSED", "1")
-    _tile_geometry_case(monkeypatch, T, CS, cfg)
-
-
-@pytest.mark.parametrize("T,CS", [(128, 2), (256, 4), (128, 8)])
-@pytest.mark.parametrize("cfg", [dict(width=64, height=64, seed=721, make_rivers=True, wind="random", extra_ignitions=3),
-                                 dict(width=100, height=70, seed=722, wind=[0.85, (1, 0)], extra_ignitions=6, a_speed=2)],
-                         ids=["64_rivers", "100x70_aspeed2"])
-def test_tile_phased_flow_matches_oracle(monkeypatch, T, CS, cfg):
-    """WF_TILE_OVERLAP=0: the strictly phased step (full cluster barrier Y, finish, then the observation) that the default
-    overlapped flow replaced; kept as the A/B reference."""
-    monkeypatch.setenv("WF_TILE_OVERLAP", "0")
+def test_tile_whole_group_slices_match_oracle(monkeypatch, T, CS, cfg):
+    """Grids whose CTA slices are whole 128-word groups, so the observation runs on the wide path alone: dig toggle,
+    rivers with a_speed 2, and a W > H map with 8 fuel bit-slices.  Same check as the geometry sweep above."""
     _tile_geometry_case(monkeypatch, T, CS, cfg)
 
 

@@ -12,6 +12,7 @@ FLAGS="-O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -lineinfo -Xcompil
 nvcc $FLAGS "$@" -c "${API_SRC:-$src/wf_api.cu}" -o "$out/wf_api.o" &
 nvcc $FLAGS "$@" -c "${WARP_SRC:-$src/wf_warp.cu}" -o "$out/wf_warp.o" &
 nvcc $FLAGS "$@" -c "${TILE_SRC:-$src/wf_tile.cu}" -o "$out/wf_tile.o" &
+nvcc $FLAGS "$@" -c "$src/wf_learn.cu" -o "$out/wf_learn.o" &
 nvcc $FLAGS "$@" -c "$src/wf_hostpool.cpp" -o "$out/wf_hostpool.o" &
 wait
 nvcc --shared -gencode arch=compute_100a,code=sm_100a -ccbin g++ "$out"/*.o -o "build_ab/lib$name.so"

@@ -31,8 +31,8 @@ for _ in range(R):
 e1.record()
 torch.cuda.synchronize()
 L.wf_debug_tile_timing(buf, 0)
-names = ["agent", "barrier X", "tick_slice", "sync", "exchange(Y)", "finish", "sync", "reset", "obs"]
-tot = sum(buf[i] for i in range(9))
+names = ["barrier X", "flood + tick", "CTA barrier", "Y + finish + agent", "observation", "closing sync", "slow + reset"]
+tot = sum(buf[i] for i in range(len(names)))
 print(f"{name} obs={with_obs}: {e0.elapsed_time(e1) * 1e3 / (R * K):.2f} us/step; probe CTA per step:")
 for i, n in enumerate(names):
     print(f"  {n:12s} {buf[i] / (R * K) / 1e3:7.2f} us")

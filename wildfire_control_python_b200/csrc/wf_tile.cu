@@ -37,8 +37,6 @@ namespace wf {
 struct TileState {
     int32_t P_S0, P_S1, P_R;
     int32_t T, CS;  // threads per CTA, CTAs per cluster (one cluster per env)
-    bool fused;     // WF_TILE_FUSED=1 (read by wf_create): the fused pass for the shapes that allow it
-    bool overlap;   // WF_TILE_OVERLAP (read by wf_create): see TilePar::overlap
 };
 
 struct TilePar {  // launch constants, precomputed on the host so the kernel re-reads them from the constant bank
@@ -51,34 +49,7 @@ struct TilePar {  // launch constants, precomputed on the host so the kernel re-
     size_t pstride;      // words between consecutive planes (N * RS * HW)
     size_t env_words;    // words between consecutive envs within a plane (RS * HW)
     size_t step_bytes;   // bytes of one step's observation block [N][W][H][3]
-    int32_t overlap;     // two-phase path: finish / next agent phase / barrier Y overlapped with the observation (WF_TILE_OVERLAP)
 };
-
-// ---------------------------------------------------------------------------------------------
-// Fused pass (kernel instantiations with FU = true): ONE sweep per step over the env's words does the fire tick of
-// step k AND emits the observation of step k-1 (whose planes are exactly what the tick reads), so the latency-bound
-// stencil rides on the bandwidth-bound observation stream instead of being a phase of its own.  A warp owns 128
-// consecutive words per iteration; their seven input words (G, B, S, S of the rows above / below, F, I) are staged in
-// shared memory with cp.async (no registers in flight) one iteration ahead.  Needs HW % 4 == 0, H % 32 == 0, uint8
-// observations and slices of whole 128-word groups; every other shape runs the two-phase path.
-constexpr int kFuIn = 7 * 128;                     // staged input words per warp: G B S U D F I
-constexpr int kFuEdge = kFuIn;                     // + S[g - 1], S[g + 128] (+ 2 pad)
-constexpr int kFuStage = kFuEdge + 4;              // 384 words of observation bit stream
-constexpr int kFuQ = kFuStage + 384;               // 128 queue entries (uint16)
-constexpr int kFuWords = kFuQ + 64;                // per warp; multiple of 4 words
-static_assert(kFuWords % 4 == 0, "16-byte alignment of the per-warp regions");
-
-__device__ __forceinline__ void cp_async16(uint32_t* smem_dst, const uint32_t* gsrc, bool valid = true) {
-    const uint32_t a = (uint32_t)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(a), "l"(gsrc), "r"(valid ? 16 : 0) : "memory");
-}
-__device__ __forceinline__ void cp_async4(uint32_t* smem_dst, const uint32_t* gsrc, bool valid) {
-    const uint32_t a = (uint32_t)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(a), "l"(gsrc), "r"(valid ? 4 : 0) : "memory");
-}
-__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
 
 // Block-wide scratch of the env a CTA is working on (every CTA of the cluster holds the same values).
 struct StepShared {
@@ -90,11 +61,10 @@ struct StepShared {
     int32_t tot[8];       // cluster totals: burning cells, grass cells, ignition on edge, burning touches reach,
                           // a burning cell is a border point (W > H maps only); 5..7 unused
     int32_t reset_now;
-    int32_t obs_vis, obs_ax, obs_ay;  // agent_pos layer of the observation being emitted
     int32_t obs_ctr;                  // next 128-word observation group of this CTA (dynamic distribution)
     uint32_t stat[ST_N];  // this launch's contribution to the handle's statistics (flushed once, at the end)
-    int32_t obs_agent[2][3];  // overlapped flow: agent_pos layer (visible, x, y) after the action of step k, in slot k & 1
-    int32_t slow;             // overlapped flow: this step's reward needs the whole cluster (seed_cells_touch) before it is known
+    int32_t obs_agent[2][3];  // agent_pos layer (visible, x, y) after the action of step k, in slot k & 1
+    int32_t slow;             // this step's reward needs the whole cluster (seed_cells_touch) before it is known
     int32_t keep[3];          // ... and the step's totals (burning, grass, ignition on edge) kept meanwhile
 };
 
@@ -939,239 +909,6 @@ __device__ __forceinline__ void emit_obs_slice(const Env& e, void* obs_step, int
     }
 }
 
-
-// ---------------------------------------------------------------------------------------------
-// The fused pass (see kFuIn above): tick of this step (if do_tick) + observation of the PREVIOUS step (if obs_step),
-// one sweep over this CTA's slice, 128 words per warp and iteration.  Leaves the CTA's partial reductions in red[]
-// like tick_slice.  Per iteration:
-//   wait for the staged inputs -> phase 1 of the tick from shared memory (heat masks, active words compacted into the
-//   warp's queue, S_next := 0) -> every lane picks up one queued word -> the observation bit streams of the group are
-//   built from the staged F / I words -> the NEXT group's inputs are requested (cp.async) -> the queued words run the
-//   active path (their fuel / hit-counter round trips overlap the copies in flight) -> the 12 KB of observation bytes
-//   of the group are expanded and stored.
-struct FusedEntry {  // one queued active word: what the active path needs of the staged inputs
-    int wi, x, w;
-    uint32_t G, B, h0, h1, h2, h3;
-};
-template <int FB>
-__device__ __forceinline__ void fused_slice(const Env& e, const DevState& s, const StepCfg& c, const TilePar& t, const int32_t* sc,
-                                            const StepShared& ss, bool do_tick, bool ticking, int digw, int* red,
-                                            uint32_t* smem_all, const uint32_t* spread3, const uint2* tab8, uint8_t* obs_step,
-                                            int vis, int ax, int ay) {
-    const int W = e.W, H = e.H, HW = e.HW;
-    const int lane = e.tid & 31, warp = e.tid >> 5, nwarps = e.T >> 5;
-    uint32_t* const in = smem_all + warp * kFuWords;
-    uint32_t* const stage = in + kFuStage;
-    uint16_t* const q_idx = reinterpret_cast<uint16_t*>(in + kFuQ);
-    const uint16_t* const stage16 = reinterpret_cast<const uint16_t*>(stage);
-    const unsigned FULL = 0xffffffffu;
-    const uint32_t lt_mask = (1u << lane) - 1u;
-    const size_t pstride = e.pstride;
-    const bool want_touch = !sc[WF_S_FIRE_AT_BORDER] && !sc[WF_S_LATCHED];
-    const int cur = sc[WF_S_RESERVED] & 1;
-    const int scur = cur ? t.P_S1 : t.P_S0, snxt = cur ? t.P_S0 : t.P_S1;
-    const uint32_t digclr = ss.dig_clear_R ? ss.dig_bit : 0u;
-    const int digw_R = ss.dig_word;
-    const uint32_t* const Rp = e.plane(t.P_R);
-    const int wid = sc[WF_S_WIND_ID];
-    const int kmin = s.wind->uniform[wid] ? s.wind->kmin[wid] : -1;
-    const bool do_obs = obs_step != nullptr;
-    const bool need_s = do_tick && ticking;
-    const int aw = (do_obs && vis) ? ax * HW + (ay >> 5) : -1;
-    int my_nb = 0, my_ng = 0, my_edge = 0, my_touch = 0, my_bseed = 0;
-    const int n128 = (e.hi - e.lo) >> 7;
-
-    auto issue = [&](int gi) {  // request the inputs of group gi; every lane copies its own four words of each plane
-        const int g = e.lo + gi * 128, i = g + 4 * lane;
-        const uint32_t* P = e.P0 + i;
-        if (do_tick) {
-            cp_async16(in + 4 * lane, P + P_G * pstride);
-            cp_async16(in + 128 + 4 * lane, P + P_B * pstride);
-        }
-        if (need_s) {
-            const int x = e.row_of(i);
-            const uint32_t* Sc = P + (size_t)scur * pstride;
-            cp_async16(in + 256 + 4 * lane, Sc);
-            cp_async16(in + 384 + 4 * lane, x > 0 ? Sc - HW : Sc, x > 0);          // row above, zeros outside the grid
-            cp_async16(in + 512 + 4 * lane, x < W - 1 ? Sc + HW : Sc, x < W - 1);  // row below
-            if (lane == 0) cp_async4(in + kFuEdge, g > 0 ? Sc - 1 : Sc, g > 0);    // the words next to the group
-            if (lane == 31) cp_async4(in + kFuEdge + 1, i + 4 < e.nwords ? Sc + 4 : Sc, i + 4 < e.nwords);
-        }
-        if (do_obs) {
-            cp_async16(in + 640 + 4 * lane, P + P_F * pstride);
-            cp_async16(in + 768 + 4 * lane, P + P_I * pstride);
-        }
-        cp_async_commit();
-    };
-
-    int gi = warp;
-    if (gi < n128) issue(gi);
-    for (; gi < n128; gi += nwarps) {
-        const int g = e.lo + gi * 128;
-        const int i = g + 4 * lane;
-        cp_async_wait_all();
-        __syncwarp();
-        int nq = 0;
-        if (do_tick) {
-            const int x = e.row_of(i), w0 = i - x * HW;
-            const uint4 g4 = *reinterpret_cast<const uint4*>(in + 4 * lane);
-            const uint4 b4 = *reinterpret_cast<const uint4*>(in + 128 + 4 * lane);
-            uint32_t G[4] = {g4.x, g4.y, g4.z, g4.w};
-            const uint32_t B[4] = {b4.x, b4.y, b4.z, b4.w};
-            if (digw >= i && digw < i + 4) {  // Agent.dig lands in this unit: this thread owns the word
-#pragma unroll
-                for (int k = 0; k < 4; ++k)
-                    if (digw == i + k) G[k] &= ~ss.dig_bit;
-                apply_dig(e, t, digw, ss.dig_bit, ss.dig_clear_R);
-            }
-            if (ticking) {
-                const uint4 s4 = *reinterpret_cast<const uint4*>(in + 256 + 4 * lane);
-                const uint4 u4 = *reinterpret_cast<const uint4*>(in + 384 + 4 * lane);
-                const uint4 d4 = *reinterpret_cast<const uint4*>(in + 512 + 4 * lane);
-                uint32_t S[6];
-                S[1] = s4.x; S[2] = s4.y; S[3] = s4.z; S[4] = s4.w;
-                S[0] = w0 > 0 ? (lane > 0 ? in[256 + 4 * lane - 1] : in[kFuEdge]) : 0u;
-                S[5] = w0 + 4 < HW ? (lane < 31 ? in[256 + 4 * lane + 4] : in[kFuEdge + 1]) : 0u;
-                const uint32_t Sup[4] = {u4.x, u4.y, u4.z, u4.w}, Sdn[4] = {d4.x, d4.y, d4.z, d4.w};
-                bool active[4];
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    const uint32_t a0 = G[k] & ((S[k + 1] >> 1) | (S[k + 2] << 31));  // d = N (0,-1): source at y+1
-                    const uint32_t a1 = G[k] & ((S[k + 1] << 1) | (S[k] >> 31));      // d = S (0,+1): source at y-1
-                    active[k] = (B[k] | a0 | a1 | (G[k] & (Sup[k] | Sdn[k]))) != 0u;
-                    if (!active[k]) my_ng += __popc(G[k]);  // inactive words cannot burn: B == 0
-                }
-                // inactive words have no sources next tick; queued words overwrite their slot below
-                *reinterpret_cast<uint4*>(e.P0 + i + (size_t)snxt * pstride) = make_uint4(0u, 0u, 0u, 0u);
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    const uint32_t m = __ballot_sync(FULL, active[k]);
-                    if (active[k]) q_idx[nq + __popc(m & lt_mask)] = (uint16_t)(4 * lane + k);
-                    nq += __popc(m);
-                }
-            } else {
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    my_nb += __popc(B[k]);
-                    my_ng += __popc(G[k]);
-                    if (B[k] && want_touch) {  // burning border points are judged by seed_cells_touch
-                        const uint32_t sw = seed_word(W, H, x, w0 + k);
-                        if (B[k] & sw) my_bseed = 1;
-                        if ((B[k] & ~sw) && touches_reach(Rp, i + k, B[k] & ~sw, x, w0 + k, W, HW, digw_R, digclr)) my_touch = 1;
-                    }
-                }
-            }
-        }
-        __syncwarp();
-        // ---- a queued word: everything the active path needs of the staged inputs, read before they are overwritten
-        auto read_entry = [&](int it) -> FusedEntry {
-            FusedEntry q;
-            const int off = q_idx[it];
-            q.wi = g + off;
-            q.x = e.row_of(q.wi);
-            q.w = q.wi - q.x * HW;
-            q.G = in[off];
-            q.B = in[128 + off];
-            if (q.wi == digw) q.G &= ~ss.dig_bit;  // the staged copy predates this step's dig
-            const uint32_t sm = in[256 + off];
-            const uint32_t sl = q.w > 0 ? (off > 0 ? in[256 + off - 1] : in[kFuEdge]) : 0u;
-            const uint32_t sr = q.w < HW - 1 ? (off < 127 ? in[256 + off + 1] : in[kFuEdge + 1]) : 0u;
-            q.h0 = q.G & ((sm >> 1) | (sr << 31));
-            q.h1 = q.G & ((sm << 1) | (sl >> 31));
-            q.h2 = q.G & in[384 + off];
-            q.h3 = q.G & in[512 + off];
-            return q;
-        };
-        auto run_entry = [&](FusedEntry& q) {
-            uint32_t* P = e.P0 + q.wi;
-            const uint32_t sn = tick_active_word<FB>(P, pstride, e.FU + (size_t)q.wi * kFuelRec, q.G, q.B, q.h0, q.h1, q.h2, q.h3, s, c,
-                                                     e.hits + ((size_t)q.x * H + 32 * q.w), wid, kmin, edge_word(W, H, q.x, q.w), my_edge);
-            P[(size_t)snxt * pstride] = sn;
-            my_nb += __popc(q.B);
-            my_ng += __popc(q.G);
-            if (q.B && want_touch) {
-                const uint32_t sw = seed_word(W, H, q.x, q.w);
-                if (q.B & sw) my_bseed = 1;
-                if ((q.B & ~sw) && touches_reach(Rp, q.wi, q.B & ~sw, q.x, q.w, W, HW, digw_R, digclr)) my_touch = 1;
-            }
-        };
-        FusedEntry mine;
-        mine.wi = -1;
-        if (nq > 32) {  // rare: more active words than lanes -- run them all before the inputs are recycled
-            for (int it = lane; it < nq; it += 32) {
-                FusedEntry q = read_entry(it);
-                run_entry(q);
-            }
-        } else if (lane < nq) {
-            mine = read_entry(lane);
-#ifdef WF_FUSED_PREFETCH
-            // (experiment, measured SLOWER on C4: 51.1 vs 47.5 us per step) the active path's inputs start their way from
-            // HBM now and are used after the observation block below
-            if (mine.B) prefetch_l2(e.FU + (size_t)mine.wi * kFuelRec);
-            prefetch_l2(e.hits + ((size_t)mine.x * H + 32 * mine.w));
-            prefetch_l2(e.hits + ((size_t)mine.x * H + 32 * mine.w) + 16);
-#endif
-        }
-        // ---- World.get_state of the previous step: bit streams of the group's 128 words
-        if (do_obs) {
-            const uint4 Fc = *reinterpret_cast<const uint4*>(in + 640 + 4 * lane);
-            const uint4 Ic = *reinterpret_cast<const uint4*>(in + 768 + 4 * lane);
-            const uint32_t Fw[4] = {Fc.x, Fc.y, Fc.z, Fc.w}, Iw[4] = {Ic.x, Ic.y, Ic.z, Ic.w};
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                const uint32_t F = Fw[j], freerow = ~Iw[j];
-                uint32_t p[4];
-#pragma unroll
-                for (int k = 0; k < 4; ++k)
-                    p[k] = (spread3[(F >> (8 * k)) & 255u] << 1) | (spread3[(freerow >> (8 * k)) & 255u] << 2);
-                if (i + j == aw) p[(ay & 31) >> 3] |= 1u << (3 * (ay & 7));
-                uint32_t* st = stage + (4 * lane + j) * 3;
-                st[0] = p[0] | (p[1] << 24);
-                st[1] = (p[1] >> 8) | (p[2] << 16);
-                st[2] = (p[2] >> 16) | (p[3] << 8);
-            }
-        }
-        __syncwarp();  // every lane is done with the staged inputs
-        if (gi + nwarps < n128) issue(gi + nwarps);
-#ifndef WF_FUSED_PREFETCH
-        if (mine.wi >= 0) run_entry(mine);
-#endif
-        if (do_obs) {
-            uint4* o = reinterpret_cast<uint4*>(obs_step + (((size_t)e.env * W) * H + (size_t)32 * g) * 3);
-#pragma unroll 8
-            for (int it = 0; it < 24; ++it) {
-                const int cidx = it * 32 + lane;  // 16-byte chunk of the warp's 12288 bytes = 16 stream bits
-                const uint32_t bits = stage16[cidx];
-#ifdef WF_OBS_ALU  // bits -> bytes with a multiply and a mask per 4 bytes instead of two 8-byte table look-ups
-                __stcs(&o[cidx], make_uint4(((bits & 15u) * 0x00204081u) & 0x01010101u, (((bits >> 4) & 15u) * 0x00204081u) & 0x01010101u,
-                                            (((bits >> 8) & 15u) * 0x00204081u) & 0x01010101u, ((bits >> 12) * 0x00204081u) & 0x01010101u));
-#else
-                const uint2 lo = tab8[bits & 255u], hi = tab8[bits >> 8];
-                __stcs(&o[cidx], make_uint4(lo.x, lo.y, hi.x, hi.y));  // streamed: not read again by this kernel
-#endif
-            }
-        }
-#ifdef WF_FUSED_PREFETCH
-        if (mine.wi >= 0) run_entry(mine);
-#endif
-        __syncwarp();
-    }
-    if (do_tick) {
-        my_nb = __reduce_add_sync(FULL, my_nb);
-        my_ng = __reduce_add_sync(FULL, my_ng);
-        my_edge = __any_sync(FULL, my_edge);
-        my_touch = __any_sync(FULL, my_touch);
-        my_bseed = __any_sync(FULL, my_bseed);
-        if (lane == 0) {
-            if (my_nb) atomicAdd(&red[0], my_nb);
-            if (my_ng) atomicAdd(&red[1], my_ng);
-            if (my_edge) atomicOr(&red[2], 1);
-            if (my_touch) atomicOr(&red[3], 1);
-            if (my_bseed) atomicOr(&red[4], 1);
-        }
-    }
-}
-
 // ---------------------------------------------------------------------------------------------
 // World.reset (environment.py:186-212) of this cluster's env: reset_map (:59-95), fire at the centre,
 // Agent.__init__ (:100-113), extra ignitions, reach plane, burning count.  Whole cluster.
@@ -1319,16 +1056,13 @@ __device__ void reset_env(const Env& e, const DevState& s, const StepCfg& c, con
     if ((tid & 31) == 0 && n) atomicAdd(&red[0], n);
     __syncthreads();
     exchange<CL>(e, red, xch, par, ss);
-    if (tid == 0) {
-        sc[WF_S_N_BURNING] = ss.tot[0];
-        ss.obs_vis = sc[WF_S_VISIBLE]; ss.obs_ax = sc[WF_S_AX]; ss.obs_ay = sc[WF_S_AY];
-    }
+    if (tid == 0) sc[WF_S_N_BURNING] = ss.tot[0];
     __syncthreads();
 }
 
 // ---------------------------------------------------------------------------------------------
 // K x ForestFire.step (forest_fire.py:30-49) or ForestFire.reset of one env per cluster.
-template <int FB, int VW, bool CL, bool FU>
+template <int FB, int VW, bool CL>
 #ifndef WF_TILE_MAXT
 #define WF_TILE_MAXT 512
 #define WF_TILE_MINB 2
@@ -1378,7 +1112,7 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
     unsigned long long t_last;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_last));
 #endif
-    if (!FU && io.reset_mode) {  // (the fused instantiations are never launched in reset mode)
+    if (io.reset_mode) {
         // ---------------- ForestFire.reset() ----------------
         if (io.mask == nullptr || io.mask[e.env] != 0) reset_env<FB, CL>(e, s, c, t, io.init, sc, ss, red, xch, par);
         if (io.obs != nullptr) emit_obs_slice(e, io.obs, io.obs_dtype, spread3, tab8, qmem, sc[WF_S_VISIBLE], sc[WF_S_AX], sc[WF_S_AY]);
@@ -1433,14 +1167,18 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
             }
             ss.reset_now = c.auto_reset && is_done;
         };
-        // Overlapped flow (two-phase path, TilePar::overlap).  Per step: barrier X -> tick -> CTA barrier -> the partial sums
-        // go to the peers and every thread ARRIVES at cluster barrier Y; warp 0 waits for it, adds the totals up, and thread
-        // 0 does finish + the agent phase of the next step, while the other warps already emit the observation (its agent
-        // layer was fixed by this step's agent phase; they wait for Y afterwards).  The observation is speculative in one
-        // respect: if the episode ends here and auto_reset is on, it is emitted again after the reset.  The rare step whose
-        // reward needs a whole-cluster pass (seed_cells_touch) finishes after the observation instead.
-        for (int k = 0; !FU && t.overlap && k < io.K; ++k) {
+        // Per step: barrier X -> tick -> CTA barrier -> the partial sums go to the peers and every thread ARRIVES at cluster
+        // barrier Y; warp 0 waits for it, adds the totals up, and thread 0 does finish + the agent phase of the next step,
+        // while the other warps already emit the observation (its agent layer was fixed by this step's agent phase; they
+        // wait for Y afterwards).  The observation is speculative in one respect: if the episode ends here and auto_reset
+        // is on, it is emitted again after the reset.  The rare step whose reward needs a whole-cluster pass
+        // (seed_cells_touch) finishes after the observation instead.
+        // WF_TSTAMP slots (thread 0 of the probe CTA, in warp 0): 0 barrier X, 1 re-flood + tick, 2 CTA barrier, 3 wait for
+        // Y + finish + next agent phase, 4 observation, 5 closing __syncthreads (the other warps' half of Y), 6 slow path +
+        // reset.
+        for (int k = 0; k < io.K; ++k) {
             sync_env<CL>();  // barrier X: agent phase k (and everything thread 0 wrote) is visible; no plane is written before
+            WF_TSTAMP(0);
             const bool act = ss.act != 0;
             int digw = ss.dig_word;
             const int ovis = ss.obs_agent[k & 1][0], oax = ss.obs_agent[k & 1][1], oay = ss.obs_agent[k & 1][2];
@@ -1456,8 +1194,10 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
             const int warp = tid >> 5;
             if (act) {
                 tick_slice<FB, VW>(e, s, c, t, sc, ss, dt != 0, digw, red, qmem);
+                WF_TSTAMP(1);
                 const int cur = sc[WF_S_RESERVED];  // (before thread 0 flips it)
                 __syncthreads();                    // red[] is complete, this CTA's planes are final
+                WF_TSTAMP(2);
                 if (CL) {
                     if (tid < kRed * e.CS) st_shared_cluster(&xch[par][e.rank][tid & (kRed - 1)], (uint32_t)(tid / kRed), red[tid & (kRed - 1)]);
                     cluster_arrive();  // barrier Y, first half
@@ -1485,10 +1225,13 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
                         }
                     }
                 }
+                WF_TSTAMP(3);
                 if (CL) par ^= 1;
                 if (obs_k != nullptr) emit_obs_slice(e, obs_k, io.obs_dtype, spread3, tab8, qmem, ovis, oax, oay, &ss.obs_ctr);
+                WF_TSTAMP(4);
                 if (CL && warp != 0) cluster_wait();  // barrier Y, second half
                 __syncthreads();  // what thread 0 decided is visible
+                WF_TSTAMP(5);
                 if (ss.slow) {
                     const int scratch = dt ? ((cur & 1) ? t.P_S1 : t.P_S0) : ((cur & 1) ? t.P_S0 : t.P_S1);  // not the current sources
                     const int touches = seed_cells_touch<CL>(e, t, scratch, red, xch, par, ss) ? 1 : 0;
@@ -1505,8 +1248,11 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
                     ss.slow = 0;
                     if (k + 1 < io.K) agent_phase(e, c, t, io, s, k + 1, do_tick, sc, ss, writer);
                 }
+                WF_TSTAMP(3);
                 if (obs_k != nullptr) emit_obs_slice(e, obs_k, io.obs_dtype, spread3, tab8, qmem, ovis, oax, oay, &ss.obs_ctr);
+                WF_TSTAMP(4);
                 __syncthreads();
+                WF_TSTAMP(5);
             }
             const bool late_agent = act && (ss.slow || ss.reset_now);
             if (ss.reset_now) {
@@ -1522,114 +1268,7 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
                 ss.obs_ctr = 0;
                 ss.slow = 0;
             }
-        }
-        for (int k = 0; (FU || !t.overlap) && k < io.K; ++k) {
-            WF_TSTAMP(0);
-            sync_env<CL>();  // barrier X
-            WF_TSTAMP(1);
-            const bool act = ss.act != 0;
-            int digw = ss.dig_word;
-            // FU: the observation of step k-1 is emitted by the pass that ticks step k (the planes it shows are the
-            // ones this tick reads); its agent_pos layer is what finish / reset of step k-1 left in ss.obs_*
-            uint8_t* obs_prev = (FU && io.obs != nullptr && k > 0) ? static_cast<uint8_t*>(io.obs) + (size_t)(k - 1) * step_bytes : nullptr;
-            if (ss.need_flood) {  // rare: the dig may cut the reach plane -> apply it now and re-flood R
-                if (FU && obs_prev != nullptr) {  // ... after the previous observation has been taken off the planes
-                    fused_slice<FB>(e, s, c, t, sc, ss, false, false, -1, red, qmem, spread3, tab8, obs_prev, ss.obs_vis, ss.obs_ax, ss.obs_ay);
-                    obs_prev = nullptr;
-                    __syncthreads();
-                }
-                if (tid == 0 && digw >= e.lo && digw < e.hi) apply_dig(e, t, digw, ss.dig_bit, ss.dig_clear_R);
-                digw = -1;
-                sync_env<CL>();
-                flood<CL>(e, t, red, xch, par, ss);
-            }
-            if (FU && (act || obs_prev != nullptr))
-                fused_slice<FB>(e, s, c, t, sc, ss, act, do_tick != 0, digw, red, qmem, spread3, tab8, obs_prev, ss.obs_vis, ss.obs_ax, ss.obs_ay);
-            if (act) {
-                const bool ticking = do_tick != 0;
-                if (!FU) tick_slice<FB, VW>(e, s, c, t, sc, ss, ticking, digw, red, qmem);
-                WF_TSTAMP(2);
-                __syncthreads();
-                WF_TSTAMP(3);
-                const int cur = sc[WF_S_RESERVED];
-                exchange<CL>(e, red, xch, par, ss);  // barrier Y
-                const int n_burning = ss.tot[0], n_grass = ss.tot[1], edge_ignition = ss.tot[2];
-                int touches = ss.tot[3];
-                const bool searching = !sc[WF_S_FIRE_AT_BORDER] && !sc[WF_S_LATCHED] && n_burning > 0 && !(do_tick && edge_ignition);
-                if (ss.tot[4] && searching && !touches) {  // rare (W > H maps): a burning cell is a border point itself
-                    __syncthreads();  // every thread has read ss.tot
-                    const int scratch = ticking ? ((cur & 1) ? t.P_S1 : t.P_S0) : ((cur & 1) ? t.P_S0 : t.P_S1);  // not the current sources
-                    touches = seed_cells_touch<CL>(e, t, scratch, red, xch, par, ss) ? 1 : 0;
-                }
-                WF_TSTAMP(4);
-                if (tid == 0) {
-                    // ---- RUNNING (forest_fire.py:105-106), World.get_reward (environment.py:342-390)
-                    if (ticking) sc[WF_S_RESERVED] = cur ^ 1;  // the source mask just written becomes current
-                    const bool anyB = n_burning > 0;
-                    sc[WF_S_N_BURNING] = n_burning;
-                    if (do_tick) {
-                        if (edge_ignition) sc[WF_S_FIRE_AT_BORDER] = 1;
-                        if (!sc[WF_S_ALIVE] || !anyB) sc[WF_S_RUNNING] = 0;
-                    }
-                    double rew;
-                    const bool check = !sc[WF_S_FIRE_AT_BORDER] && !sc[WF_S_LATCHED] && anyB;
-                    if (check && !touches) {
-                        sc[WF_S_LATCHED] = 1;  // bonus paid once (Q4), tested before the death test
-                        rew = c.contained_bonus;
-                        ss.stat[ST_CONTAINED] += 1u;
-                    } else if (!sc[WF_S_ALIVE]) {
-                        rew = c.death_penalty;
-                    } else if (!anyB) {
-                        rew = __dmul_rn(c.contained_bonus, __ddiv_rn((double)n_grass, (double)(s.W * s.H)));
-                    } else {
-                        rew = c.default_reward;
-                    }
-                    sc[WF_S_T] += 1;
-                    const bool is_done = !sc[WF_S_RUNNING];
-                    ss.stat[ST_STEPS] += 1u;
-                    if (do_tick) ss.stat[ST_TICKS] += 1u;
-                    if (is_done) {
-                        ss.stat[ST_EPISODES] += 1u;
-                        if (sc[WF_S_ALIVE]) ss.stat[ST_BURNOUTS] += 1u;
-                    }
-                    if (writer) {
-                        if (io.reward) io.reward[(size_t)k * s.N + e.env] = rew;
-                        if (io.done) io.done[(size_t)k * s.N + e.env] = is_done ? 1 : 0;
-                    }
-                    ss.reset_now = c.auto_reset && is_done;
-                    ss.obs_vis = sc[WF_S_VISIBLE]; ss.obs_ax = sc[WF_S_AX]; ss.obs_ay = sc[WF_S_AY];
-                    ss.obs_ctr = 0;
-                }
-            } else if (tid == 0) {  // frozen env: reward 0, done 1, nothing moves
-                if (writer) {
-                    if (io.reward) io.reward[(size_t)k * s.N + e.env] = 0.0;
-                    if (io.done) io.done[(size_t)k * s.N + e.env] = 1;
-                }
-                ss.reset_now = 0;
-                ss.obs_vis = sc[WF_S_VISIBLE]; ss.obs_ax = sc[WF_S_AX]; ss.obs_ay = sc[WF_S_AY];
-                ss.obs_ctr = 0;
-            }
-            WF_TSTAMP(5);
-            __syncthreads();
             WF_TSTAMP(6);
-            if (ss.reset_now) {
-                reset_env<FB, CL>(e, s, c, t, nullptr, sc, ss, red, xch, par);
-                if (tid == 0) ss.obs_ctr = 0;
-                __syncthreads();
-            }
-            WF_TSTAMP(7);
-            const int obs_vis = ss.obs_vis, obs_ax = ss.obs_ax, obs_ay = ss.obs_ay;
-            do_tick = tick_of(it);  // of step k+1
-            if (tid == 0 && k + 1 < io.K) agent_phase(e, c, t, io, s, k + 1, do_tick, sc, ss, writer);
-            if (!FU && io.obs != nullptr)
-                emit_obs_slice(e, static_cast<char*>(io.obs) + (size_t)k * step_bytes, io.obs_dtype, spread3, tab8, qmem,
-                               obs_vis, obs_ax, obs_ay, &ss.obs_ctr);
-            WF_TSTAMP(8);
-        }
-        if (FU && io.obs != nullptr && io.K > 0) {  // the last step's observation has no tick to ride on
-            __syncthreads();
-            fused_slice<FB>(e, s, c, t, sc, ss, false, false, -1, red, qmem, spread3, tab8,
-                            static_cast<uint8_t*>(io.obs) + (size_t)(io.K - 1) * step_bytes, ss.obs_vis, ss.obs_ax, ss.obs_ay);
         }
     }
     __syncthreads();
@@ -1704,14 +1343,13 @@ static void choose_geometry(const DevState& s, int& T, int& CS) {
     if (cs_env == 1 || cs_env == 2 || cs_env == 4 || cs_env == 8 || cs_env == 16) CS = cs_env;
 }
 
-template <int FB, int VW, bool CL, bool FU = false>
+template <int FB, int VW, bool CL>
 static cudaError_t set_smem_attr() {
     if (CL) {
-        cudaError_t e = cudaFuncSetAttribute(tile_rollout_kernel<FB, VW, CL, FU>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+        cudaError_t e = cudaFuncSetAttribute(tile_rollout_kernel<FB, VW, CL>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
         if (e != cudaSuccess) return e;
     }
-    return cudaFuncSetAttribute(tile_rollout_kernel<FB, VW, CL, FU>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                FU ? (512 / 32) * kFuWords * 4 : 512 * 4 * 28);
+    return cudaFuncSetAttribute(tile_rollout_kernel<FB, VW, CL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 512 * 4 * 28);
 }
 
 cudaError_t tile_create(TileState** out, const DevState& s, const StepCfg&) {
@@ -1720,8 +1358,6 @@ cudaError_t tile_create(TileState** out, const DevState& s, const StepCfg&) {
     t->P_S1 = P_FU0 + 1;
     t->P_R = P_FU0 + 2;
     choose_geometry(s, t->T, t->CS);
-    t->fused = env_int("WF_TILE_FUSED", 0) != 0;
-    t->overlap = env_int("WF_TILE_OVERLAP", 1) != 0;  // default on; 0: the strictly phased flow (A/B, tests)
     cudaError_t e = cudaSuccess;
     if (e == cudaSuccess) e = set_smem_attr<5, 1, false>();
     if (e == cudaSuccess) e = set_smem_attr<5, 4, false>();
@@ -1731,10 +1367,6 @@ cudaError_t tile_create(TileState** out, const DevState& s, const StepCfg&) {
     if (e == cudaSuccess) e = set_smem_attr<5, 4, true>();
     if (e == cudaSuccess) e = set_smem_attr<8, 1, true>();
     if (e == cudaSuccess) e = set_smem_attr<8, 4, true>();
-    if (e == cudaSuccess) e = set_smem_attr<5, 4, false, true>();
-    if (e == cudaSuccess) e = set_smem_attr<8, 4, false, true>();
-    if (e == cudaSuccess) e = set_smem_attr<5, 4, true, true>();
-    if (e == cudaSuccess) e = set_smem_attr<8, 4, true, true>();
     if (e != cudaSuccess) {
         delete t;
         return e;
@@ -1752,7 +1384,7 @@ cudaError_t tile_create(TileState** out, const DevState& s, const StepCfg&) {
         cfg.attrs = attr;
         cfg.numAttrs = 1;
         int nc = 0;
-        if (cudaOccupancyMaxActiveClusters(&nc, tile_rollout_kernel<5, 4, true, false>, &cfg) != cudaSuccess || nc < 1) {
+        if (cudaOccupancyMaxActiveClusters(&nc, tile_rollout_kernel<5, 4, true>, &cfg) != cudaSuccess || nc < 1) {
             cudaGetLastError();
             t->T = 256;
             t->CS = 8;
@@ -1784,17 +1416,15 @@ static TilePar make_par(const TileState* t, const DevState& s, int obs_dtype) {
     p.pstride = (size_t)s.N * s.RS * s.HW;
     p.env_words = (size_t)s.RS * s.HW;
     p.step_bytes = obs_step_bytes(s.N, s.W, s.H, obs_dtype);
-    p.overlap = t->overlap ? 1 : 0;
     return p;
 }
 
-template <int FB, int VW, bool FU = false>
+template <int FB, int VW>
 static cudaError_t launch(const TileState* t, const DevState& s, const StepCfg& c, const TileIO& io, cudaStream_t st) {
     const TilePar p = make_par(t, s, io.obs_dtype);
-    // per warp: 7 queue arrays of 32 * VW words (reused as observation staging), or the fused pass's staging
-    const size_t smem = FU ? (size_t)(t->T / 32) * kFuWords * 4 : (size_t)t->T * VW * 28;
+    const size_t smem = (size_t)t->T * VW * 28;  // per warp: 7 queue arrays of 32 * VW words (reused as observation staging)
     if (t->CS == 1) {
-        tile_rollout_kernel<FB, VW, false, FU><<<s.N, t->T, smem, st>>>(s, c, p, io);
+        tile_rollout_kernel<FB, VW, false><<<s.N, t->T, smem, st>>>(s, c, p, io);
         return cudaGetLastError();
     }
     cudaLaunchConfig_t cfg = {};
@@ -1812,25 +1442,17 @@ static cudaError_t launch(const TileState* t, const DevState& s, const StepCfg& 
     if (env_int("WF_TILE_DEBUG", 0)) {  // how many clusters of this shape the GPU holds at once (waves = grid / that)
         static bool said = false;
         int nc = 0;
-        if (!said && cudaOccupancyMaxActiveClusters(&nc, tile_rollout_kernel<FB, VW, true, FU>, &cfg) == cudaSuccess)
+        if (!said && cudaOccupancyMaxActiveClusters(&nc, tile_rollout_kernel<FB, VW, true>, &cfg) == cudaSuccess)
             fprintf(stderr, "wf_tile: %d clusters of %d x %d threads in the grid, %d resident at once\n", s.N, t->CS, t->T, nc);
         said = true;
     }
-    return cudaLaunchKernelEx(&cfg, tile_rollout_kernel<FB, VW, true, FU>, s, c, p, io);
+    return cudaLaunchKernelEx(&cfg, tile_rollout_kernel<FB, VW, true>, s, c, p, io);
 }
 
 cudaError_t launch_tile_family(TileState* t, const DevState& s, const StepCfg& c, const TileIO& io,
                                cudaStream_t stream, int64_t* launches) {
     *launches += 1;
     const bool v4 = (s.HW % 4 == 0);
-    // The fused pass (tick of step k + observation of step k-1 in one cp.async-staged sweep): rollouts on grids whose
-    // slices are whole 128-word groups of full-width words, uint8 observations.  Opt-in (WF_TILE_FUSED=1): bit-exact
-    // (tests/test_fullsize_gpu.py runs the production geometries both ways) but not faster than the two-phase path --
-    // A/B on one box, r02: C4 47.5-49.5 vs 47.2-48.7 us per step, C5 76/91/94 vs 76/90/94 -- see DESIGN.md section 8.
-    const int nwords = s.W * s.HW, per = (nwords + t->CS - 1) / t->CS, wpc = (per + 31) / 32 * 32;
-    const bool fused = v4 && !io.reset_mode && (s.H % 32) == 0 && (wpc % 128) == 0 && (nwords % wpc) == 0 &&
-                       (io.obs == nullptr || io.obs_dtype == WF_OBS_U8) && t->fused;
-    if (fused) return s.FB == 5 ? launch<5, 4, true>(t, s, c, io, stream) : launch<8, 4, true>(t, s, c, io, stream);
     if (s.FB == 5) return v4 ? launch<5, 4>(t, s, c, io, stream) : launch<5, 1>(t, s, c, io, stream);
     return v4 ? launch<8, 4>(t, s, c, io, stream) : launch<8, 1>(t, s, c, io, stream);
 }
