@@ -141,7 +141,9 @@ enum {
                              DQN.choose_randomwalk_action, DQN.py:353-389 (draws from the POLICY stream) */
     WF_POLICY_MLP = 2     /* the reference's Q-network evaluated inside the step kernel, eps-greedy
                              (DQN.choose_action DQN.py:188-196 on DQN.make_network DQN.py:209-233);
-                             weights from wf_set_policy_mlp; grids up to 32x32 only */
+                             weights from wf_set_policy_mlp(_dev) (or, up to 32x32, wf_set_policy_mlp_nets_dev);
+                             both kernel families.  The action depends only on the observation, the network and the
+                             EXPLORE stream: not on the launch geometry or how the steps are split into launches */
 };
 /* wf_rollout with the actions chosen on the device by a built-in policy (DQN.collect_memories' inner loop,
  * DQN.py:303-308: choose_randomwalk_action -> sim.step).  actions_out_dev: [K][N] int32 or NULL. */
@@ -153,7 +155,11 @@ int wf_rollout_policy(wf_env* env, int32_t k_steps, int32_t policy, int32_t* act
  * head (DQN_DUEL.py:18-48) pass the ADVANTAGE stream: argmax_a (V + A_a - mean A) = argmax_a A_a.
  * eps: probability of a uniformly random action instead of the greedy one (EXPLORE Philox stream:
  * step t uses words 2*(t&1), 2*(t&1)+1 of block t>>1: explore iff word < eps * 2^32, action = word' % n_actions).
- * hidden <= 64, n_actions <= 8. */
+ * hidden <= 64, n_actions <= 8.  Any grid: on grids larger than 32x32 (the tile family) the kernel sums the first layer
+ * exactly, in int64 fixed point (each weight rounded to a multiple of 2^-32), which needs the magnitudes summed into one
+ * hidden unit below 2^31: |kernel1| < 2^31 / (2*W*H + 1) suffices, and wf_set_policy_mlp refuses (WF_ERR_INVALID) a
+ * kernel1 entry that is not finite and below that bound there; sigmoid, second layer and argmax are float64 there.
+ * The warp family keeps float64 sums of float32 weights, updated incrementally. */
 int wf_set_policy_mlp(wf_env* env, const float* kernel1_host, const float* bias1_host, const float* kernel2_host,
                       const float* bias2_host, int32_t hidden, double eps);
 /* wf_set_policy_mlp from DEVICE tensors in nn.Linear orientation: weight1_dev [hidden][W*H*3], bias1_dev [hidden],
@@ -162,7 +168,9 @@ int wf_set_policy_mlp(wf_env* env, const float* kernel1_host, const float* bias1
  * weights that rollout's predecessors left and the next rollout on that stream sees the new ones.  The first call of a
  * handle allocates the packed buffer (as wf_set_policy_mlp does), later calls overwrite it in place: a rollout still
  * running on ANOTHER stream must be ordered by the caller.  The packed buffer is byte-identical to wf_set_policy_mlp's
- * for the same weights (the empty-map sum is accumulated in float64 in the same order), so rollouts are too. */
+ * for the same weights (the empty-map sum is accumulated in float64 in the same order), so rollouts are too.  Both kernel
+ * families, with wf_set_policy_mlp's precondition on the tile family (not checked here: the weights stay on the device).
+ * On the tile family every call re-sums the all-free map over W*H cells in float64, one thread per hidden unit. */
 int wf_set_policy_mlp_dev(wf_env* env, const float* weight1_dev, const float* bias1_dev, const float* weight2_dev,
                           const float* bias2_dev, int32_t hidden, double eps, void* stream);
 

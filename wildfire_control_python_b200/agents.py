@@ -554,7 +554,9 @@ class DQN:
 
         ``in_kernel`` (default: whenever the grid fits the warp kernel family, <= 32x32): the Q-network is
         evaluated INSIDE the step kernel (``wf_rollout_policy(WF_POLICY_MLP)``), 64 steps per launch;
-        otherwise torch evaluates it between two ``wf_step`` calls."""
+        otherwise torch evaluates it between two ``wf_step`` calls.  On grids larger than 32x32 ``in_kernel=True`` is
+        the fast path (the tile kernel's policy pass); the default stays the torch path there, whose exploration draws
+        come from another random stream, so its results are unchanged."""
         from .batched import BatchedForestFire
         from .constants import DQN_DEFAULTS as _D
         eps = self.min_eps if eps is None else eps
@@ -695,6 +697,25 @@ class DQN:
         self._until_sync = (phase - n_replays - 1) % te + 1
         return loss
 
+    def _fit_batches_torch(self, frames, s_row, sp_row, a, ap, r, d, n_replays):
+        """``fit_batches_fused`` as ``n_replays`` ``fit_batch`` calls, for grids ``wf_replay_fit`` does not take (larger
+        than 32x32): replay i unpacks its S and S' rows of ``frames`` to float32, and the target network is refreshed
+        every ``target_update`` replays from the phase the previous call left (``_until_sync``)."""
+        from .batched import unpack_obs
+        W, H = self.obs_shape[0], self.obs_shape[1]
+        batch = len(s_row) // n_replays
+        te = int(self.target_update_freq)
+        until_sync = int(getattr(self, "_until_sync", te))
+        for i in range(n_replays):
+            sl = slice(i * batch, (i + 1) * batch)
+            self.fit_batch((unpack_obs(frames, W, H, index=s_row[sl]), a[sl].long(), r[sl].float(),
+                            unpack_obs(frames, W, H, index=sp_row[sl]), ap[sl].long(), d[sl].bool()))
+            until_sync -= 1
+            if until_sync == 0:
+                until_sync = te
+                self.target.load_state_dict(self.model.state_dict())
+        self._until_sync = until_sync
+
     def learn_batched(self, n_episodes, n_envs=1024, k_steps=16, replays_per_launch=None, batch_size=None, seed=0,
                       replay_seed=None):
         """``learn`` over ``n_envs`` CUDA environments at once: the envs act with the eps-greedy Q-network evaluated inside
@@ -715,14 +736,14 @@ class DQN:
         in the reference's format (``total_rewards``, ``agent_deaths``, ``n_episodes``, ``init_memories``,
         ``total_time``; ``write_data``).  Per-episode ``maps`` and ``agent_pos`` are not recorded: the envs run on the
         device and are not rendered.  One small device-to-host read per launch (rewards and done flags).
-        ``eps_per_launch`` / ``episodes_before_launch`` record the schedule.  Grids up to 32x32 only (the in-kernel
-        policy).  Returns the number of environment steps simulated."""
+        ``eps_per_launch`` / ``episodes_before_launch`` record the schedule.  Any grid: on grids larger than 32x32, which
+        ``wf_replay_fit`` does not take, each launch's replays run as ``fit_batch`` calls on the same batches (unpacked
+        to float32), with the same target refresh.  Returns the number of environment steps simulated."""
         from .batched import BatchedForestFire
         from .constants import DQN_DEFAULTS as _D
         t_run = time.time()
         W, H = self.obs_shape[0], self.obs_shape[1]
-        if W > 32 or H > 32:
-            raise ValueError("learn_batched runs the in-kernel policy: grids up to 32x32 only")
+        fused = W <= 32 and H <= 32
         N, K = int(n_envs), int(k_steps)
         R = K if replays_per_launch is None else int(replays_per_launch)
         B = int(self.METADATA["batch_size"] if batch_size is None else batch_size)
@@ -746,7 +767,11 @@ class DQN:
                 env.set_policy_mlp_dev(net.dense_1.weight, net.dense_1.bias, net.dense_2.weight, net.dense_2.bias, eps=self.eps)
                 rew, done = ring.launch()
                 if R > 0 and ring.n_sampleable > B:
-                    self.fit_batches_fused(ring.frames, *ring.gather(ring.sample(R, B, gen)), R)
+                    batches = ring.gather(ring.sample(R, B, gen))
+                    if fused:
+                        self.fit_batches_fused(ring.frames, *batches, R)
+                    else:
+                        self._fit_batches_torch(ring.frames, *batches, R)
                 rd = torch.stack((rew, done.double())).cpu().numpy()
                 e_idx, k_idx, ret, carry = _episode_ends(carry, rd[0], rd[1] != 0)
                 order = np.lexsort((e_idx, k_idx))

@@ -231,7 +231,8 @@ class BatchedForestFire:
         ``actions``: ``[K, N]`` ints, or ``None`` = chosen on the device by ``policy``:
         ``"stream"`` (uniform random, ACTION stream), ``"walk"`` (the reference's heuristic
         demonstration / Baseline policy ``DQN.choose_randomwalk_action``, DQN.py:353-389) or ``"mlp"``
-        (the Q-network given to ``set_policy_mlp``, eps-greedy, evaluated inside the step kernel).
+        (the Q-network given to ``set_policy_mlp``, eps-greedy, evaluated inside the step kernel of either family: on
+        grids larger than 32x32 the tile kernel runs a policy pass after every step, with an exact fixed-point first layer).
         ``out``: optional ``(obs_or_None, reward, done_u8)`` buffers to write into.
         Returns ``(obs [K,N,W,H,3] or None, reward [K,N], done [K,N])`` (+ ``actions [K,N]`` if asked);
         with ``obs_dtype="bits"`` obs is ``[K, N, words]`` int32.
@@ -264,7 +265,9 @@ class BatchedForestFire:
     def set_policy_mlp(self, kernel1, bias1, kernel2, bias2, eps: float = 0.0):
         """Weights of the in-kernel Q-network (``rollout(policy="mlp")``): Keras orientation, ``kernel1``
         ``[W*H*3, hidden]``, ``kernel2`` ``[hidden, n_actions]`` (DQN.make_network, DQN.py:209-233; for a
-        dueling head pass the advantage stream).  ``eps``: exploration rate (DQN.choose_action :188-196)."""
+        dueling head pass the advantage stream).  ``eps``: exploration rate (DQN.choose_action :188-196).
+        Both kernel families; on grids larger than 32x32 ``|kernel1|`` must stay below ``2**31 / (2*W*H + 1)``
+        (the exact fixed-point sum, include/wildfire.h)."""
         arrs = [np.ascontiguousarray(torch.as_tensor(a).detach().cpu().numpy() if torch.is_tensor(a) else a, dtype=np.float32)
                 for a in (kernel1, bias1, kernel2, bias2)]
         k1, b1, k2, b2 = arrs
@@ -279,7 +282,8 @@ class BatchedForestFire:
         """``set_policy_mlp`` from float32 CUDA tensors in ``nn.Linear`` orientation (``weight1`` ``[hidden, W*H*3]``,
         ``weight2`` ``[n_actions, hidden]``), repacked by a kernel on the current stream: no host copy, no synchronisation
         (``wf_set_policy_mlp_dev``).  Rollouts queued after it on the same stream use the new weights, and they act
-        exactly as after ``set_policy_mlp`` with the same weights.  For a dueling head pass the advantage stream."""
+        exactly as after ``set_policy_mlp`` with the same weights.  For a dueling head pass the advantage stream.
+        Both kernel families, as ``set_policy_mlp``."""
         ts = []
         for t in (weight1, bias1, weight2, bias2):
             if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float32 and t.device == self.device):

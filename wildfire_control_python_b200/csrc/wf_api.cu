@@ -703,10 +703,8 @@ static int rollout_impl(wf_env* e, int32_t k_steps, const int32_t* actions_dev, 
     if (k_steps < 1) return fail(WF_ERR_INVALID, "k_steps must be >= 1");
     if (policy != WF_POLICY_STREAM && policy != WF_POLICY_WALK && policy != WF_POLICY_MLP)
         return fail(WF_ERR_INVALID, "unknown policy");
-    if (policy == WF_POLICY_MLP && !actions_dev) {
-        if (e->tile) return fail(WF_ERR_INVALID, "WF_POLICY_MLP is implemented for grids up to 32x32 (warp family) only");
-        if (e->mlp.hid == 0) return fail(WF_ERR_STATE, "WF_POLICY_MLP: call wf_set_policy_mlp first");
-    }
+    if (policy == WF_POLICY_MLP && !actions_dev && e->mlp.hid == 0)
+        return fail(WF_ERR_STATE, "WF_POLICY_MLP: call wf_set_policy_mlp first");
     if (int rc = check_obs(obs_dev, obs_dtype)) return rc;
     WF_ON_DEVICE(e);
     WF_QUIESCE(e);
@@ -714,7 +712,7 @@ static int rollout_impl(wf_env* e, int32_t k_steps, const int32_t* actions_dev, 
     note_dev_call(e, st);
     if (e->tile) {  // one thread-block cluster per env runs all K steps in one launch
         TileIO io{actions_dev, obs_dev, reward_dev, done_dev, nullptr, nullptr, obs_dtype, k_steps, e->a_iter, 0, policy,
-                  actions_out};
+                  actions_out, e->mlp};
         WF_CUDA(launch_tile_family(e->tstate, e->st, e->sc, io, st, &e->launches));
         e->a_iter = advance_a_iter(e, k_steps);
         return WF_OK;
@@ -739,6 +737,9 @@ int wf_rollout_policy(wf_env* e, int32_t k_steps, int32_t policy, int32_t* actio
 
 // Explore threshold of eps: a 32-bit draw below it explores.
 static uint32_t mlp_eps_threshold(double eps) { return eps >= 1.0 ? 0xffffffffu : (uint32_t)(eps * 4294967296.0); }
+
+// Lanes of MlpPolicy::w1's layout: the warp family's lanes per env; the tile family's policy pass adds rows with 32 lanes.
+static int mlp_lanes(const wf_env* e) { return e->tile ? 32 : e->st.RS; }
 
 // The handle's packed buffer holds at least n_nets network blocks; network 0's pointers, one group covering every env.
 static int mlp_reserve(wf_env* e, int n_nets, int hidden) {
@@ -769,12 +770,19 @@ int wf_set_policy_mlp(wf_env* e, const float* k1, const float* b1, const float* 
     if (hidden < 1 || hidden > 64) return fail(WF_ERR_INVALID, "hidden must be in 1..64");
     if (e->cfg.n_actions > 8) return fail(WF_ERR_INVALID, "WF_POLICY_MLP supports at most 8 actions");
     if (!(eps >= 0.0 && eps <= 1.0)) return fail(WF_ERR_INVALID, "eps must be in [0, 1]");
+    if (e->tile) {  // the tile kernel's exact fixed-point first layer (include/wildfire.h)
+        const double bound = 2147483648.0 / (2.0 * e->st.W * e->st.H + 1.0);
+        for (size_t i = 0, n = (size_t)e->st.W * e->st.H * 3 * hidden; i < n; ++i)
+            if (!(std::fabs((double)k1[i]) < bound))
+                return fail(WF_ERR_INVALID, "wf_set_policy_mlp: on this grid every kernel1 entry must be finite and below "
+                                            "2^31 / (2*W*H + 1) in magnitude");
+    }
     WF_ON_DEVICE(e);
     WF_QUIESCE(e);
     const DevState& s = e->st;
     const int n_in = s.W * s.H * 3, A = e->cfg.n_actions;
     // device layout (MlpPolicy): w1 [n_in][64] permuted for the lanes | base [64] | w2 [2][64][4] | b2 [8] | threshold [8]
-    const int L = s.RS, hpl = 64 / L;
+    const int L = mlp_lanes(e), hpl = 64 / L;
     const size_t n_w1 = (size_t)n_in * 64, total = mlp_net_floats(n_in);
     std::vector<float> hbuf(total, 0.0f);
     float* h = hbuf.data();
@@ -812,7 +820,7 @@ static int pack_policy_nets(wf_env* e, int n_nets, const float* w1, const float*
     const size_t total = mlp_net_floats(n_in);
     const dim3 grid((unsigned)std::min<size_t>((total + 255) / 256, 148 * 16), (unsigned)n_nets);
     pack_policy_mlp_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(e->mlp_dev, w1, b1, w2, b2, in_stride, n_in,
-                                                                                  s.W * s.H, hidden, e->cfg.n_actions, s.RS, thr);
+                                                                                  s.W * s.H, hidden, e->cfg.n_actions, mlp_lanes(e), thr);
     WF_CUDA(cudaGetLastError());
     return WF_OK;
 }

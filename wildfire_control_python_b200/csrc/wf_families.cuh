@@ -72,8 +72,9 @@ struct TileIO {
     const uint8_t* mask;     // reset mode: [N] or nullptr
     const wf_init* init;     // reset mode: [N] or nullptr
     int32_t obs_dtype, K, a_iter0, reset_mode;
-    int32_t policy;          // actions == nullptr: WF_POLICY_STREAM or WF_POLICY_WALK
+    int32_t policy;          // actions == nullptr: WF_POLICY_STREAM, WF_POLICY_WALK or WF_POLICY_MLP
     int32_t* actions_out;    // [K][N] or nullptr
+    MlpPolicy mlp;           // WF_POLICY_MLP only (packed with 32 lanes: unit j at (j % 32) * 2 + j / 32 of a w1 row)
 };
 struct TileState;
 int tile_extra_planes();

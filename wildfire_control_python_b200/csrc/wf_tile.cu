@@ -22,6 +22,10 @@
 //                 to the border-connected reach plane R), done, statistics; auto-reset
 //   observation   World.get_state (environment.py:399-402): 2 plane words in, 96 bytes out per word
 //
+// WF_POLICY_MLP (the MLP instantiations) adds a policy pass after every step and before step 0: the Q-network's first
+// layer over the observation the step left (mlp_action), summed exactly in int64 fixed point, exchanged through DSMEM;
+// the agent phase of the next step then runs after it instead of during the observation.
+//
 // The A* containment search (pyastar/astar.cpp) is the persistent reach plane R (cells with a finite
 // 4-connected path to a finite border point), re-flooded by the cluster only when a dig may disconnect
 // it; burning cells that are border points themselves (W > H maps) get a scratch flood (seed_cells_touch).
@@ -116,6 +120,12 @@ __device__ __forceinline__ void st_shared_cluster(int* local_ptr, uint32_t peer,
     uint32_t ra;
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(a), "r"(peer));
     asm volatile("st.shared::cluster.s32 [%0], %1;" ::"r"(ra), "r"(v) : "memory");
+}
+__device__ __forceinline__ void st_shared_cluster(long long* local_ptr, uint32_t peer, long long v) {
+    const uint32_t a = (uint32_t)__cvta_generic_to_shared(local_ptr);
+    uint32_t ra;
+    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(a), "r"(peer));
+    asm volatile("st.shared::cluster.s64 [%0], %1;" ::"r"(ra), "l"(v) : "memory");
 }
 template <bool CL>
 __device__ __forceinline__ void sync_env() {
@@ -311,17 +321,20 @@ __device__ __forceinline__ void apply_dig(const Env& e, const TilePar& t, int wi
 
 // ForestFire.step part 1: the action (Agent.move :141-155, toggle_digging :136-138) and, on tick
 // steps, Agent.is_dead (:116-120).  Thread 0 of every CTA computes the same thing; only `writer`
-// (cluster rank 0) touches global memory.
+// (cluster rank 0) touches global memory.  MLP: the action is `mlp_act`, what mlp_action chose.
+template <bool MLP>
 __device__ void agent_phase_impl(const Env& e, const StepCfg& c, const TilePar& t, const TileIO& io, const DevState& s, int k,
-                                 int do_tick, int32_t* sc, StepShared& ss, bool writer);
+                                 int do_tick, int32_t* sc, StepShared& ss, bool writer, int mlp_act);
+template <bool MLP>
 __device__ __forceinline__ void agent_phase(const Env& e, const StepCfg& c, const TilePar& t, const TileIO& io, const DevState& s,
-                                            int k, int do_tick, int32_t* sc, StepShared& ss, bool writer) {
-    agent_phase_impl(e, c, t, io, s, k, do_tick, sc, ss, writer);
+                                            int k, int do_tick, int32_t* sc, StepShared& ss, bool writer, int mlp_act = 0) {
+    agent_phase_impl<MLP>(e, c, t, io, s, k, do_tick, sc, ss, writer, mlp_act);
     // the agent_pos layer of step k's observation (nothing after the action moves the agent; a reset re-reads the scalars)
     ss.obs_agent[k & 1][0] = sc[WF_S_VISIBLE]; ss.obs_agent[k & 1][1] = sc[WF_S_AX]; ss.obs_agent[k & 1][2] = sc[WF_S_AY];
 }
+template <bool MLP>
 __device__ void agent_phase_impl(const Env& e, const StepCfg& c, const TilePar& t, const TileIO& io, const DevState& s, int k,
-                                 int do_tick, int32_t* sc, StepShared& ss, bool writer) {
+                                 int do_tick, int32_t* sc, StepShared& ss, bool writer, int mlp_act) {
     ss.act = sc[WF_S_RUNNING];
     ss.dig_word = -1;
     ss.dig_bit = 0u;
@@ -330,7 +343,9 @@ __device__ void agent_phase_impl(const Env& e, const StepCfg& c, const TilePar& 
     if (!sc[WF_S_RUNNING]) return;
     const int W = e.W, H = e.H;
     int action;
-    if (io.actions != nullptr) {
+    if (MLP) {
+        action = mlp_act;
+    } else if (io.actions != nullptr) {
         action = io.actions[(size_t)k * s.N + e.env];
     } else if (io.policy == WF_POLICY_WALK) {  // DQN.choose_randomwalk_action, DQN.py:353-389
         action = 0;
@@ -709,6 +724,122 @@ __device__ bool seed_cells_touch(const Env& e, const TilePar& t, int scratch_pla
 }
 
 // ---------------------------------------------------------------------------------------------
+// WF_POLICY_MLP: DQN.choose_action (DQN.py:188-196) on the observation of the state the planes and scalars hold now, i.e.
+// what the last step emitted (after an auto-reset: the new episode's first frame).  Whole cluster; the action is returned
+// in thread 0.  Hidden unit j = base_j + [visible] w1[agent, 0] + sum_F w1[cell, 1] - sum_I w1[cell, 2] (base: the
+// all-free map, MlpPolicy::base).  The sums are exact: every weight is rounded to int64 fixed point (w * 2^32: exact
+// scaling, then round to nearest), so any order -- warps, shared atomics, the CTAs of any cluster size -- gives the same
+// totals, and the action does not depend on the geometry or on how the steps are split into launches.  Precondition: the
+// magnitudes summed into one unit stay below 2^31 (at most 2 W H + 1 rows: |w1| < 2^31 / (2 W H + 1) suffices).
+// Each warp sweeps 32 words of its CTA's slice at a time; every lane with a set bit left announces its lowest one and all
+// lanes add that row (lane l: packed positions 2l, 2l + 1 = units l, l + 32), four rows per round so their loads overlap.
+// Then sigmoid, the second layer and the first-max argmax in float64 (warp 0), eps-greedy from the EXPLORE stream as
+// in the warp family (wf_warp.cu).
+template <bool CL>
+__device__ int mlp_action(const Env& e, const StepCfg& c, const MlpPolicy& m, const int32_t* sc) {
+    __shared__ long long part[64];                          // this CTA's sums of the 64 packed positions
+    __shared__ long long xmlp[CL ? kMaxCluster : 1][64];    // every CTA's sums (written by the peers)
+    constexpr unsigned FULL = 0xffffffffu;
+    const int H = e.H, HW = e.HW, tid = e.tid, lane = tid & 31, warp = tid >> 5, nwarps = e.T >> 5;
+    const size_t off = (size_t)(e.env / m.group_envs) * m.net_stride;
+    const float2* w1 = reinterpret_cast<const float2*>(m.w1 + off);
+    if (tid < 64) part[tid] = 0;
+    __syncthreads();  // (also: this CTA's words of the planes are final)
+    const int aw = sc[WF_S_VISIBLE] ? sc[WF_S_AX] * HW + (sc[WF_S_AY] >> 5) : -1;
+    const uint32_t abit = 1u << (sc[WF_S_AY] & 31);
+    const uint32_t* PF = e.plane(P_F);
+    const uint32_t* PI = e.plane(P_I);
+    long long acc0 = 0, acc1 = 0;
+    for (int g = e.lo + warp * 32; g < e.hi; g += nwarps * 32) {  // warp-uniform
+        const int i = g + lane;
+        uint32_t dA = 0u, dF = 0u, dI = 0u;
+        int cell0 = 0;
+        if (i < e.hi) {
+            const int x = e.row_of(i), w = i - x * HW;
+            const uint32_t v = valid_word(H, w);
+            dF = PF[i] & v;
+            dI = PI[i] & v;
+            dA = i == aw ? abit : 0u;
+            cell0 = x * H + 32 * w;
+        }
+        for (;;) {
+            const bool has = (dA | dF | dI) != 0u;
+            int code = 0;  // (input row << 1) | subtract
+            if (has) {
+                const int ch = dA ? 0 : dF ? 1 : 2;
+                uint32_t& d = dA ? dA : dF ? dF : dI;
+                const int y = __ffs(d) - 1;
+                d &= d - 1u;
+                code = (((cell0 + y) * 3 + ch) << 1) | (ch == 2 ? 1 : 0);
+            }
+            uint32_t todo = __ballot_sync(FULL, has);
+            if (todo == 0u) break;
+            while (todo) {
+                int cd[4];
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    const int src = todo ? __ffs(todo) - 1 : -1;
+                    todo &= todo - 1u;
+                    cd[j] = __shfl_sync(FULL, code, src < 0 ? 0 : src);
+                    if (src < 0) cd[j] = -1;
+                }
+                float2 wv[4];
+#pragma unroll
+                for (int j = 0; j < 4; ++j) wv[j] = cd[j] >= 0 ? __ldg(&w1[(size_t)(cd[j] >> 1) * 32 + lane]) : make_float2(0.0f, 0.0f);
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    const long long a = __float2ll_rn(wv[j].x * 0x1p32f), b = __float2ll_rn(wv[j].y * 0x1p32f);
+                    if (cd[j] & 1) { acc0 -= a; acc1 -= b; }
+                    else { acc0 += a; acc1 += b; }
+                }
+            }
+        }
+    }
+    if (acc0) atomicAdd(reinterpret_cast<unsigned long long*>(&part[2 * lane]), (unsigned long long)acc0);
+    if (acc1) atomicAdd(reinterpret_cast<unsigned long long*>(&part[2 * lane + 1]), (unsigned long long)acc1);
+    __syncthreads();
+    long long h0 = 0, h1 = 0;
+    if (CL) {
+        for (int v = tid; v < 64 * e.CS; v += e.T) st_shared_cluster(&xmlp[e.rank][v & 63], (uint32_t)(v >> 6), part[v & 63]);
+        cluster_barrier();
+        if (warp == 0)
+            for (int r = 0; r < e.CS; ++r) { h0 += xmlp[r][2 * lane]; h1 += xmlp[r][2 * lane + 1]; }
+    } else if (warp == 0) {
+        h0 = part[2 * lane]; h1 = part[2 * lane + 1];
+    }
+    int action = 0;
+    if (warp == 0) {
+        const float* base = m.base + off;
+        const float4* w2 = reinterpret_cast<const float4*>(m.w2 + off);  // [2][64]: actions 0..3, 4..7 of unit j
+        const float* b2 = m.b2 + off;                                   // [8] (-inf: no such action), then the threshold
+        const double s0 = 1.0 / (1.0 + exp(-((double)base[lane] + (double)h0 * 0x1p-32)));
+        const double s1 = 1.0 / (1.0 + exp(-((double)base[lane + 32] + (double)h1 * 0x1p-32)));
+        const float4 a0 = w2[lane], b0 = w2[64 + lane], a1 = w2[lane + 32], b1 = w2[96 + lane];
+        double q[8] = {s0 * a0.x + s1 * a1.x, s0 * a0.y + s1 * a1.y, s0 * a0.z + s1 * a1.z, s0 * a0.w + s1 * a1.w,
+                       s0 * b0.x + s1 * b1.x, s0 * b0.y + s1 * b1.y, s0 * b0.z + s1 * b1.z, s0 * b0.w + s1 * b1.w};
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1)
+#pragma unroll
+            for (int b = 0; b < 8; ++b) q[b] += __shfl_xor_sync(FULL, q[b], o);
+        if (lane == 0) {
+            int greedy = 0;
+            double best = q[0] + (double)b2[0];
+#pragma unroll
+            for (int b = 1; b < 8; ++b) {
+                const double v = q[b] + (double)b2[b];
+                if (v > best) { best = v; greedy = b; }
+            }
+            uint32_t w[4];
+            const uint32_t tt = (uint32_t)sc[WF_S_T];
+            philox4x32_10((uint32_t)(c.env_id_base + e.env), (uint32_t)sc[WF_S_EPISODE], tt >> 1, kStreamExplore, c.key0, c.key1, w);
+            const uint32_t u0 = (tt & 1u) ? w[2] : w[0], u1 = (tt & 1u) ? w[3] : w[1];
+            action = (u0 < __float_as_uint(b2[8])) ? (int)(u1 % (uint32_t)c.n_actions) : greedy;
+        }
+    }
+    return action;
+}
+
+// ---------------------------------------------------------------------------------------------
 // Float observations (WF_OBS_BF16 / WF_OBS_F32) of a staged bit stream: `nelem` (a multiple of 512) stream bits
 // become `nelem` elements starting at element `elem0` of the step's block, 16 bytes per lane and store.
 __device__ __forceinline__ uint32_t bf16_pair(uint32_t bytes01, uint32_t sel) {  // two 0/1 bytes -> two bfloat16
@@ -1062,7 +1193,8 @@ __device__ void reset_env(const Env& e, const DevState& s, const StepCfg& c, con
 
 // ---------------------------------------------------------------------------------------------
 // K x ForestFire.step (forest_fire.py:30-49) or ForestFire.reset of one env per cluster.
-template <int FB, int VW, bool CL>
+// MLP: WF_POLICY_MLP steps (no reset mode, no action array).
+template <int FB, int VW, bool CL, bool MLP>
 #ifndef WF_TILE_MAXT
 #define WF_TILE_MAXT 512
 #define WF_TILE_MINB 2
@@ -1129,7 +1261,15 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
         };
         int do_tick = tick_of(it);
         if (tid == 0) { ss.obs_ctr = 0; ss.slow = 0; }
-        if (tid == 0 && io.K > 0) agent_phase(e, c, t, io, s, 0, do_tick, sc, ss, writer);
+        if (MLP) {
+            // the policy pass: every CTA of the cluster, or none (a frozen env's action is not used).  Its DSMEM stores need
+            // every CTA of the cluster to have started: one cluster barrier first (later passes follow barrier X).
+            if (CL) cluster_barrier();
+            const int a = sc[WF_S_RUNNING] ? mlp_action<CL>(e, c, io.mlp, sc) : 0;
+            if (tid == 0) agent_phase<true>(e, c, t, io, s, 0, do_tick, sc, ss, writer, a);
+        } else if (tid == 0 && io.K > 0) {
+            agent_phase<false>(e, c, t, io, s, 0, do_tick, sc, ss, writer);
+        }
         // ---- RUNNING (forest_fire.py:105-106), World.get_reward (environment.py:342-390), done; thread 0 only
         auto finish_step = [&](int k, int dt, int touches, int n_burning, int n_grass, int edge_ignition) {
             const int cur = sc[WF_S_RESERVED];
@@ -1221,7 +1361,7 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
                         } else {
                             ss.slow = 0;
                             finish_step(k, dt, ss.tot[3], ss.tot[0], ss.tot[1], ss.tot[2]);
-                            if (!ss.reset_now && k + 1 < io.K) agent_phase(e, c, t, io, s, k + 1, do_tick, sc, ss, writer);
+                            if (!MLP && !ss.reset_now && k + 1 < io.K) agent_phase<false>(e, c, t, io, s, k + 1, do_tick, sc, ss, writer);
                         }
                     }
                 }
@@ -1246,7 +1386,7 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
                     }
                     ss.reset_now = 0;
                     ss.slow = 0;
-                    if (k + 1 < io.K) agent_phase(e, c, t, io, s, k + 1, do_tick, sc, ss, writer);
+                    if (!MLP && k + 1 < io.K) agent_phase<false>(e, c, t, io, s, k + 1, do_tick, sc, ss, writer);
                 }
                 WF_TSTAMP(3);
                 if (obs_k != nullptr) emit_obs_slice(e, obs_k, io.obs_dtype, spread3, tab8, qmem, ovis, oax, oay, &ss.obs_ctr);
@@ -1264,9 +1404,13 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
                 __syncthreads();
             }
             if (tid == 0) {
-                if (late_agent && k + 1 < io.K) agent_phase(e, c, t, io, s, k + 1, do_tick, sc, ss, writer);
+                if (!MLP && late_agent && k + 1 < io.K) agent_phase<false>(e, c, t, io, s, k + 1, do_tick, sc, ss, writer);
                 ss.obs_ctr = 0;
                 ss.slow = 0;
+            }
+            if (MLP && k + 1 < io.K) {  // the policy pass on the state this step left, then the next step's agent phase
+                const int a = sc[WF_S_RUNNING] ? mlp_action<CL>(e, c, io.mlp, sc) : 0;
+                if (tid == 0) agent_phase<true>(e, c, t, io, s, k + 1, do_tick, sc, ss, writer, a);
             }
             WF_TSTAMP(6);
         }
@@ -1343,13 +1487,26 @@ static void choose_geometry(const DevState& s, int& T, int& CS) {
     if (cs_env == 1 || cs_env == 2 || cs_env == 4 || cs_env == 8 || cs_env == 16) CS = cs_env;
 }
 
-template <int FB, int VW, bool CL>
+template <int FB, int VW, bool CL, bool MLP>
 static cudaError_t set_smem_attr() {
     if (CL) {
-        cudaError_t e = cudaFuncSetAttribute(tile_rollout_kernel<FB, VW, CL>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+        cudaError_t e = cudaFuncSetAttribute(tile_rollout_kernel<FB, VW, CL, MLP>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
         if (e != cudaSuccess) return e;
     }
-    return cudaFuncSetAttribute(tile_rollout_kernel<FB, VW, CL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 512 * 4 * 28);
+    return cudaFuncSetAttribute(tile_rollout_kernel<FB, VW, CL, MLP>, cudaFuncAttributeMaxDynamicSharedMemorySize, 512 * 4 * 28);
+}
+template <bool MLP>
+static cudaError_t set_smem_attrs() {
+    cudaError_t e = cudaSuccess;
+    if (e == cudaSuccess) e = set_smem_attr<5, 1, false, MLP>();
+    if (e == cudaSuccess) e = set_smem_attr<5, 4, false, MLP>();
+    if (e == cudaSuccess) e = set_smem_attr<8, 1, false, MLP>();
+    if (e == cudaSuccess) e = set_smem_attr<8, 4, false, MLP>();
+    if (e == cudaSuccess) e = set_smem_attr<5, 1, true, MLP>();
+    if (e == cudaSuccess) e = set_smem_attr<5, 4, true, MLP>();
+    if (e == cudaSuccess) e = set_smem_attr<8, 1, true, MLP>();
+    if (e == cudaSuccess) e = set_smem_attr<8, 4, true, MLP>();
+    return e;
 }
 
 cudaError_t tile_create(TileState** out, const DevState& s, const StepCfg&) {
@@ -1358,15 +1515,8 @@ cudaError_t tile_create(TileState** out, const DevState& s, const StepCfg&) {
     t->P_S1 = P_FU0 + 1;
     t->P_R = P_FU0 + 2;
     choose_geometry(s, t->T, t->CS);
-    cudaError_t e = cudaSuccess;
-    if (e == cudaSuccess) e = set_smem_attr<5, 1, false>();
-    if (e == cudaSuccess) e = set_smem_attr<5, 4, false>();
-    if (e == cudaSuccess) e = set_smem_attr<8, 1, false>();
-    if (e == cudaSuccess) e = set_smem_attr<8, 4, false>();
-    if (e == cudaSuccess) e = set_smem_attr<5, 1, true>();
-    if (e == cudaSuccess) e = set_smem_attr<5, 4, true>();
-    if (e == cudaSuccess) e = set_smem_attr<8, 1, true>();
-    if (e == cudaSuccess) e = set_smem_attr<8, 4, true>();
+    cudaError_t e = set_smem_attrs<false>();
+    if (e == cudaSuccess) e = set_smem_attrs<true>();
     if (e != cudaSuccess) {
         delete t;
         return e;
@@ -1384,7 +1534,7 @@ cudaError_t tile_create(TileState** out, const DevState& s, const StepCfg&) {
         cfg.attrs = attr;
         cfg.numAttrs = 1;
         int nc = 0;
-        if (cudaOccupancyMaxActiveClusters(&nc, tile_rollout_kernel<5, 4, true>, &cfg) != cudaSuccess || nc < 1) {
+        if (cudaOccupancyMaxActiveClusters(&nc, tile_rollout_kernel<5, 4, true, false>, &cfg) != cudaSuccess || nc < 1) {
             cudaGetLastError();
             t->T = 256;
             t->CS = 8;
@@ -1419,12 +1569,12 @@ static TilePar make_par(const TileState* t, const DevState& s, int obs_dtype) {
     return p;
 }
 
-template <int FB, int VW>
+template <int FB, int VW, bool MLP>
 static cudaError_t launch(const TileState* t, const DevState& s, const StepCfg& c, const TileIO& io, cudaStream_t st) {
     const TilePar p = make_par(t, s, io.obs_dtype);
     const size_t smem = (size_t)t->T * VW * 28;  // per warp: 7 queue arrays of 32 * VW words (reused as observation staging)
     if (t->CS == 1) {
-        tile_rollout_kernel<FB, VW, false><<<s.N, t->T, smem, st>>>(s, c, p, io);
+        tile_rollout_kernel<FB, VW, false, MLP><<<s.N, t->T, smem, st>>>(s, c, p, io);
         return cudaGetLastError();
     }
     cudaLaunchConfig_t cfg = {};
@@ -1442,19 +1592,25 @@ static cudaError_t launch(const TileState* t, const DevState& s, const StepCfg& 
     if (env_int("WF_TILE_DEBUG", 0)) {  // how many clusters of this shape the GPU holds at once (waves = grid / that)
         static bool said = false;
         int nc = 0;
-        if (!said && cudaOccupancyMaxActiveClusters(&nc, tile_rollout_kernel<FB, VW, true>, &cfg) == cudaSuccess)
+        if (!said && cudaOccupancyMaxActiveClusters(&nc, tile_rollout_kernel<FB, VW, true, MLP>, &cfg) == cudaSuccess)
             fprintf(stderr, "wf_tile: %d clusters of %d x %d threads in the grid, %d resident at once\n", s.N, t->CS, t->T, nc);
         said = true;
     }
-    return cudaLaunchKernelEx(&cfg, tile_rollout_kernel<FB, VW, true>, s, c, p, io);
+    return cudaLaunchKernelEx(&cfg, tile_rollout_kernel<FB, VW, true, MLP>, s, c, p, io);
+}
+
+template <bool MLP>
+static cudaError_t launch_fb_vw(const TileState* t, const DevState& s, const StepCfg& c, const TileIO& io, cudaStream_t st) {
+    const bool v4 = (s.HW % 4 == 0);
+    if (s.FB == 5) return v4 ? launch<5, 4, MLP>(t, s, c, io, st) : launch<5, 1, MLP>(t, s, c, io, st);
+    return v4 ? launch<8, 4, MLP>(t, s, c, io, st) : launch<8, 1, MLP>(t, s, c, io, st);
 }
 
 cudaError_t launch_tile_family(TileState* t, const DevState& s, const StepCfg& c, const TileIO& io,
                                cudaStream_t stream, int64_t* launches) {
     *launches += 1;
-    const bool v4 = (s.HW % 4 == 0);
-    if (s.FB == 5) return v4 ? launch<5, 4>(t, s, c, io, stream) : launch<5, 1>(t, s, c, io, stream);
-    return v4 ? launch<8, 4>(t, s, c, io, stream) : launch<8, 1>(t, s, c, io, stream);
+    if (io.policy == WF_POLICY_MLP && io.actions == nullptr && !io.reset_mode) return launch_fb_vw<true>(t, s, c, io, stream);
+    return launch_fb_vw<false>(t, s, c, io, stream);
 }
 
 #ifdef WF_TILE_TIMING
