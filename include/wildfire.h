@@ -318,6 +318,21 @@ int wf_replay_fit(const wf_mlp_shape* shape, const wf_fit_params* params, int32_
                   const int32_t* next_action_dev, const float* reward_dev, const uint8_t* done_dev, float* loss_dev,
                   void* stream);
 
+/* wf_replay_fit for any grid wf_create takes: 10 <= height <= width, no upper bound (hidden, n_actions, dueling and batch
+ * as above; the flat parameter buffer must hold at most 2^31 - 1 floats).  Same arguments, update rule, target sync,
+ * losses and out-of-range rules as wf_replay_fit.  Runs as ONE cooperative launch of as many CTAs as the device holds at
+ * once: each CTA owns a fixed set of chunks of the first layer's input columns (the chunking is a function of the shape)
+ * and every sum runs in an order fixed by the shape, so the result is deterministic (no floating-point atomics) and does
+ * not depend on the number of CTAs (environment variable WF_FIT_CTAS, read on every call: at most that many).  Allocates
+ * and frees its scratch (at most 32 MB + 8 * batch * (2 * hidden + 10) bytes) stream-ordered on `stream`.  Grids up to
+ * 32x32 are taken too; its sums are ordered differently from wf_replay_fit's, so the two agree to rounding, not bit for
+ * bit.  Needs no handle; without a CUDA device it fails with WF_ERR_CUDA (no CPU fallback). */
+int wf_replay_fit_large(const wf_mlp_shape* shape, const wf_fit_params* params, int32_t n_replays, float* params_dev,
+                        float* target_dev, float* adam_m_dev, float* adam_v_dev, const uint32_t* frames_dev,
+                        int64_t n_frames, const int64_t* s_row_dev, const int64_t* sp_row_dev, const int32_t* action_dev,
+                        const int32_t* next_action_dev, const float* reward_dev, const uint8_t* done_dev, float* loss_dev,
+                        void* stream);
+
 /* ---- populations: up to 64 independent learners in one launch -------------------------------------------------------
  * One learner of wf_replay_fit_many: its own flat model, target and Adam moments (the layout above), its own transitions
  * ([n_replays * batch] each, as for wf_replay_fit; next_action NULL = the DQN target, max_a Q_target(s', a)), its own loss

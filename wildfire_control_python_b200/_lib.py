@@ -121,6 +121,8 @@ def lib():
     L.wf_replay_fit.argtypes = [C.POINTER(WfMlpShape), C.POINTER(WfFitParams), C.c_int32, vp, vp, vp, vp, vp, C.c_int64,
                                 vp, vp, vp, vp, vp, vp, vp, vp]
     L.wf_replay_fit.restype = C.c_int
+    L.wf_replay_fit_large.argtypes = L.wf_replay_fit.argtypes
+    L.wf_replay_fit_large.restype = C.c_int
     L.wf_replay_fit_many.argtypes = [C.POINTER(WfMlpShape), C.c_int32, C.POINTER(WfFitLearner), C.c_int32, vp, C.c_int64, vp]
     L.wf_replay_fit_many.restype = C.c_int
     L.wf_set_policy_mlp_nets_dev.argtypes = [vp, C.POINTER(WfMlpShape), C.c_int32, vp, C.POINTER(C.c_double), vp]
@@ -174,4 +176,5 @@ EXPORTED_SYMBOLS = [
     "wf_get_obs", "wf_get_wind_table", "wf_stats", "wf_stats_reset", "wf_philox_kat", "wf_launch_count",
     "wf_state_bytes_per_env", "wf_host_threads", "wf_expand_packed_obs", "wf_apply_change_blocks", "wf_get_a_iter", "wf_set_a_iter", "wf_reset_host", "wf_tile_geometry", "wf_host_session", "wf_host_session_active",
     "wf_unpack_obs_bits", "wf_set_policy_mlp_dev", "wf_replay_fit", "wf_replay_fit_many", "wf_set_policy_mlp_nets_dev",
+    "wf_replay_fit_large",
 ]

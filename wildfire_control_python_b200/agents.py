@@ -633,8 +633,9 @@ class DQN:
                                dueling=int(hasattr(self.model, "dense_3")), batch=int(batch))
 
     def fit_batches_fused(self, frames, s_row, sp_row, a, ap, r, d, n_replays, phase=None):
-        """``n_replays`` consecutive ``fit_batch`` updates in ONE launch of ``wf_replay_fit`` (include/wildfire.h), the
-        same rule (targets from the target network, MSE, clipped Keras Adam) on packed observations.
+        """``n_replays`` consecutive ``fit_batch`` updates in ONE kernel launch (include/wildfire.h), the same rule (targets
+        from the target network, MSE, clipped Keras Adam) on packed observations: ``wf_replay_fit`` on grids up to 32x32,
+        ``wf_replay_fit_large`` (the whole GPU, first layer cut into column chunks) on larger grids.
 
         ``frames``: ``[n_frames, words]`` int32 CUDA tensor of ``WF_OBS_BITS`` rows (``pack_obs`` / ``obs_dtype="bits"``);
         ``s_row`` / ``sp_row``: int64 row numbers of S and S'; ``a`` / ``ap``: actions and next actions (``ap`` is used by
@@ -679,8 +680,10 @@ class DQN:
                               epsilon=group["epsilon"], clipvalue=math.inf if group["clipvalue"] is None else group["clipvalue"],
                               adam_t=t0, target_every=te, phase=phase)
         loss = torch.empty(n_replays, dtype=torch.float32, device=dev)
+        W, H = self.obs_shape[0], self.obs_shape[1]
+        fit = _lib.lib().wf_replay_fit if W <= 32 and H <= 32 else _lib.lib().wf_replay_fit_large
         with torch.cuda.device(dev):
-            _lib.check(_lib.lib().wf_replay_fit(
+            _lib.check(fit(
                 ctypes.byref(self._flat_shape(batch)), ctypes.byref(hp), n_replays, _ptr(flat), _ptr(tgt), _ptr(m), _ptr(v),
                 _ptr(frames), frames.shape[0], _ptr(s_row), _ptr(sp_row), _ptr(a), _ptr(ap) if self._SARSA else None,
                 _ptr(r), _ptr(d), _ptr(loss), ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
@@ -696,25 +699,6 @@ class DQN:
                 off += n
         self._until_sync = (phase - n_replays - 1) % te + 1
         return loss
-
-    def _fit_batches_torch(self, frames, s_row, sp_row, a, ap, r, d, n_replays):
-        """``fit_batches_fused`` as ``n_replays`` ``fit_batch`` calls, for grids ``wf_replay_fit`` does not take (larger
-        than 32x32): replay i unpacks its S and S' rows of ``frames`` to float32, and the target network is refreshed
-        every ``target_update`` replays from the phase the previous call left (``_until_sync``)."""
-        from .batched import unpack_obs
-        W, H = self.obs_shape[0], self.obs_shape[1]
-        batch = len(s_row) // n_replays
-        te = int(self.target_update_freq)
-        until_sync = int(getattr(self, "_until_sync", te))
-        for i in range(n_replays):
-            sl = slice(i * batch, (i + 1) * batch)
-            self.fit_batch((unpack_obs(frames, W, H, index=s_row[sl]), a[sl].long(), r[sl].float(),
-                            unpack_obs(frames, W, H, index=sp_row[sl]), ap[sl].long(), d[sl].bool()))
-            until_sync -= 1
-            if until_sync == 0:
-                until_sync = te
-                self.target.load_state_dict(self.model.state_dict())
-        self._until_sync = until_sync
 
     def learn_batched(self, n_episodes, n_envs=1024, k_steps=16, replays_per_launch=None, batch_size=None, seed=0,
                       replay_seed=None):
@@ -736,14 +720,12 @@ class DQN:
         in the reference's format (``total_rewards``, ``agent_deaths``, ``n_episodes``, ``init_memories``,
         ``total_time``; ``write_data``).  Per-episode ``maps`` and ``agent_pos`` are not recorded: the envs run on the
         device and are not rendered.  One small device-to-host read per launch (rewards and done flags).
-        ``eps_per_launch`` / ``episodes_before_launch`` record the schedule.  Any grid: on grids larger than 32x32, which
-        ``wf_replay_fit`` does not take, each launch's replays run as ``fit_batch`` calls on the same batches (unpacked
-        to float32), with the same target refresh.  Returns the number of environment steps simulated."""
+        ``eps_per_launch`` / ``episodes_before_launch`` record the schedule.  Any grid: ``fit_batches_fused`` runs the
+        replays in ``wf_replay_fit`` up to 32x32 and in ``wf_replay_fit_large`` on larger grids.  Returns the number of
+        environment steps simulated."""
         from .batched import BatchedForestFire
         from .constants import DQN_DEFAULTS as _D
         t_run = time.time()
-        W, H = self.obs_shape[0], self.obs_shape[1]
-        fused = W <= 32 and H <= 32
         N, K = int(n_envs), int(k_steps)
         R = K if replays_per_launch is None else int(replays_per_launch)
         B = int(self.METADATA["batch_size"] if batch_size is None else batch_size)
@@ -767,11 +749,7 @@ class DQN:
                 env.set_policy_mlp_dev(net.dense_1.weight, net.dense_1.bias, net.dense_2.weight, net.dense_2.bias, eps=self.eps)
                 rew, done = ring.launch()
                 if R > 0 and ring.n_sampleable > B:
-                    batches = ring.gather(ring.sample(R, B, gen))
-                    if fused:
-                        self.fit_batches_fused(ring.frames, *batches, R)
-                    else:
-                        self._fit_batches_torch(ring.frames, *batches, R)
+                    self.fit_batches_fused(ring.frames, *ring.gather(ring.sample(R, B, gen)), R)
                 rd = torch.stack((rew, done.double())).cpu().numpy()
                 e_idx, k_idx, ret, carry = _episode_ends(carry, rd[0], rd[1] != 0)
                 order = np.lexsort((e_idx, k_idx))

@@ -17,8 +17,11 @@
 //
 // The first layer reads the observation bits directly: a sum of weight-row entries over the set bits.
 #include <cooperative_groups.h>
+#include <algorithm>
 #include <atomic>
+#include <climits>
 #include <cmath>
+#include <cstdlib>
 #include <string>
 
 #include "wf_common.cuh"
@@ -334,6 +337,335 @@ int cluster_size_for(int device, size_t smem, cudaError_t* err) {
     return 0;
 }
 
+// ---- wf_replay_fit_large: the same replays for any grid, spread over the whole GPU ----------------------------------
+// One cooperatively launched grid of as many CTAs as are co-resident.  The first layer's input columns are cut into
+// `nc` chunks of `cw` whole observation words (a function of the shape only); CTA k owns chunks k, k + grid, ... for the
+// whole launch.  Per replay:
+//   forward  each CTA sums, for its chunks, the first-layer rows of the set bits of s (model and target) and s'
+//            (target) in feature order, staging `sub` words of both weight matrices at a time in shared memory, and
+//            writes one partial [3][B][units] per chunk to scratch;
+//   -- grid barrier --
+//   reduce   one CTA per sample adds the partials over chunks in a fixed tree (kSegs segments of consecutive chunks,
+//            each summed in chunk order, then the segments in order), then computes the sigmoid, the second layer, the
+//            target, the output gradient dout and the first-layer gradient dz of that sample;
+//   -- grid barrier --
+//   update   each CTA runs Adam on the first-layer entries of its chunks, g = sum over b of dz[b][u] * x[b][f] in b
+//            order (the sum wf_replay_fit forms); every small parameter (first-layer biases, second layer, output
+//            biases) has one owner thread of the grid; global thread 0 writes the loss.
+// A CTA reads and writes only its own chunks' first-layer weights, so no barrier is needed between one replay's update
+// and the next replay's forward; and the reduce of replay r + 1 starts only after every CTA has left update r, so the
+// scratch needs no second buffer.  Every sum runs in an order fixed by the shape and no floating-point atomic is used:
+// the result is bit-identical from run to run and whatever the number of CTAs (WF_FIT_CTAS forces it).
+constexpr int kLThreads = 512;
+constexpr int kMaxChunks = 128;                 // chunks of the first layer's columns
+constexpr int64_t kPartBudget = int64_t(1) << 23;  // floats of the chunk partials: at most 32 MB of scratch
+constexpr int kSegs = 8;                        // chunk segments of the reduction tree
+constexpr int kWsFloats = 24576;                // staged first-layer weights per sub-tile: 96 KB
+constexpr int kMaxSub = 8;                      // words per sub-tile
+constexpr int kSlots = 4;                       // units per lane in the forward: 128 = 2 * kMaxHidden units
+constexpr int kBatch = 4;                       // first-layer entries a thread loads before it uses them
+
+struct LargeArgs {
+    FitLearner l;
+    const uint32_t* frames;
+    int64_t n_frames;
+    int n_replays;
+    int n_in, words, hid, A, duel, B;
+    int off_b1, off_w2, off_b2, off_w3, off_b3, off_w4, off_b4;
+    int units, cw, nc, sub;
+    float* part;  // [nc][3][B][units]: model(s), target(s), target(s') pre-activations of each chunk
+    float* h;     // [B][units]: model hidden activations on s
+    float* dz;    // [B][units]: dLoss / d(first-layer pre-activation)
+    float* dout;  // [B][kOut]: dLoss / d(second-layer output)
+    float* sq;    // [B]: squared error of each sample
+};
+
+// Word w of row `row` of the frames table: 0 for a row outside [0, n_frames), and bits past n_in cleared.
+__device__ __forceinline__ uint32_t frame_word(const LargeArgs& a, int64_t row, int w) {
+    if (row < 0 || row >= a.n_frames) return 0u;
+    const uint32_t x = __ldg(a.frames + row * a.words + w);
+    const int tail = a.n_in - w * 32;
+    return tail >= 32 ? x : x & ((1u << tail) - 1u);
+}
+
+__global__ void __launch_bounds__(kLThreads) replay_fit_large_kernel(const __grid_constant__ LargeArgs a) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    float* fs = reinterpret_cast<float*>(smem_raw);
+    cg::grid_group grid = cg::this_grid();
+    const FitLearner& l = a.l;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = kLThreads / 32;
+    const int A = a.A, A1 = A + 1, B = a.B, hid = a.hid, U = a.units, n_in = a.n_in, sub = a.sub;
+    const int blk = blockIdx.x, nblk = gridDim.x;
+    const float inv_n = 1.0f / (float)(B * A);
+
+    auto w1_off = [&](int g) { return g < hid ? (int64_t)g * n_in : a.off_w3 + (int64_t)(g - hid) * n_in; };
+    auto b1_off = [&](int g) { return g < hid ? a.off_b1 + g : a.off_b3 + (g - hid); };
+    auto w2_off = [&](int g, int o) { return g < hid ? a.off_w2 + o * hid + g : a.off_w4 + (g - hid); };
+
+    int until_sync = l.phase;
+    for (int r = 0; r < a.n_replays; ++r) {
+        const int64_t i0 = (int64_t)r * B;
+
+        // ---- forward: partial pre-activations of this CTA's chunks; warp job (j, b): j 0 = model and target on s,
+        //      j 1 = target on s'; lane owns units lane + 32 * s
+        float* Ws = fs;                                                      // [2][sub * 32][U]: model, target
+        uint32_t* sb = reinterpret_cast<uint32_t*>(fs + 2 * sub * 32 * U);  // [2][B][sub]
+        for (int c = blk; c < a.nc; c += nblk) {
+            const int cw0 = c * a.cw, cw1 = min(a.words, cw0 + a.cw);
+            for (int w0 = cw0; w0 < cw1; w0 += sub) {
+                const int nw = min(sub, cw1 - w0), nf = nw * 32, f0 = w0 * 32;
+                __syncthreads();
+                for (int k0 = 0; k0 < 2 * U * nf; k0 += kBatch * kLThreads) {
+                    float x[kBatch];
+                    int at[kBatch];
+#pragma unroll
+                    for (int i = 0; i < kBatch; ++i) {
+                        const int k = k0 + i * kLThreads + tid;
+                        const int net = k / (U * nf), rem = k - net * U * nf, u = rem / nf, f = rem - u * nf;
+                        at[i] = k < 2 * U * nf ? (net * nf + f) * U + u : -1;
+                        x[i] = at[i] >= 0 && f0 + f < n_in ? (net ? l.T : l.P)[w1_off(u) + f0 + f] : 0.0f;
+                    }
+#pragma unroll
+                    for (int i = 0; i < kBatch; ++i)
+                        if (at[i] >= 0) Ws[at[i]] = x[i];
+                }
+                for (int k = tid; k < 2 * B * nw; k += kLThreads) {
+                    const int j = k / (B * nw), rem = k - j * B * nw, b = rem / nw, w = rem - b * nw;
+                    sb[(j * B + b) * sub + w] = frame_word(a, (j ? l.sp_row : l.s_row)[i0 + b], w0 + w);
+                }
+                __syncthreads();
+                for (int job = warp; job < 2 * B; job += nwarps) {
+                    const int j = job / B, b = job - j * B;
+                    float* pm = a.part + ((int64_t)c * 3 * B + b) * U + lane;  // + q * B * U: pass q
+                    float* p1 = pm + (j ? 2 : 1) * B * U;                        // target on s (j 0) or s' (j 1)
+                    float acc0[kSlots], acc1[kSlots];
+#pragma unroll
+                    for (int s = 0; s < kSlots; ++s) {
+                        const bool on = lane + 32 * s < U && w0 > cw0;
+                        acc0[s] = on && !j ? pm[32 * s] : 0.0f;
+                        acc1[s] = on ? p1[32 * s] : 0.0f;
+                    }
+                    for (int w = 0; w < nw; ++w) {
+                        uint32_t bits = sb[(j * B + b) * sub + w];
+                        while (bits) {
+                            const int f = w * 32 + __ffs(bits) - 1;
+                            bits &= bits - 1u;
+                            const float* wm = Ws + f * U + lane;
+                            const float* wt = wm + nf * U;
+#pragma unroll
+                            for (int s = 0; s < kSlots; ++s) {
+                                if (lane + 32 * s < U) {
+                                    if (!j) acc0[s] += wm[32 * s];
+                                    acc1[s] += wt[32 * s];
+                                }
+                            }
+                        }
+                    }
+#pragma unroll
+                    for (int s = 0; s < kSlots; ++s) {
+                        if (lane + 32 * s < U) {
+                            if (!j) pm[32 * s] = acc0[s];
+                            p1[32 * s] = acc1[s];
+                        }
+                    }
+                }
+            }
+        }
+        grid.sync();
+
+        // ---- reduce and head, one CTA per sample
+        for (int b = blk; b < B; b += nblk) {
+            float* seg = fs;                  // [kSegs][3][U]
+            float* hq = seg + kSegs * 3 * U;  // [3][U]: hidden activations of model(s), target(s), target(s')
+            float* q = hq + 3 * U;            // [3][kOut]
+            float* dout = q + 3 * kOut;       // [kOut]
+            const int per = (a.nc + kSegs - 1) / kSegs;
+            for (int k = tid; k < kSegs * 3 * U; k += kLThreads) {
+                const int s = k / (3 * U), pu = k - s * 3 * U, p = pu / U, u = pu - p * U;
+                const int c1 = min(a.nc, (s + 1) * per);
+                float z = 0.0f;
+#pragma unroll 8
+                for (int c = s * per; c < c1; ++c) z += __ldcg(a.part + (((int64_t)c * 3 + p) * B + b) * U + u);
+                seg[k] = z;
+            }
+            __syncthreads();
+            for (int k = tid; k < 3 * U; k += kLThreads) {
+                const int p = k / U, u = k - p * U;
+                float z = 0.0f;
+                for (int s = 0; s < kSegs; ++s) z += seg[s * 3 * U + k];
+                hq[k] = sigmoidf(z + __ldcg((p ? l.T : l.P) + b1_off(u)));
+            }
+            __syncthreads();
+            if (tid < 3 * A1) {
+                const int p = tid / A1, o = tid - p * A1;
+                const float* W = p ? l.T : l.P;
+                float s = 0.0f;
+                if (o < A) {
+                    for (int u = 0; u < hid; ++u) s += hq[p * U + u] * __ldcg(W + a.off_w2 + o * hid + u);
+                    s += __ldcg(W + a.off_b2 + o);
+                } else if (a.duel) {
+                    for (int u = 0; u < hid; ++u) s += hq[p * U + hid + u] * __ldcg(W + a.off_w4 + u);
+                    s += __ldcg(W + a.off_b4);
+                }
+                q[p * kOut + o] = s;
+            }
+            __syncthreads();
+            if (tid == 0) {  // target, squared error and output gradient (as replay_fit_kernel)
+                float qv[3][kMaxActions];
+                for (int p = 0; p < 3; ++p) {
+                    float mean = 0.0f;
+                    if (a.duel) {
+                        for (int o = 0; o < A; ++o) mean += q[p * kOut + o];
+                        mean /= (float)A;
+                    }
+                    for (int o = 0; o < A; ++o) qv[p][o] = a.duel ? q[p * kOut + A] + (q[p * kOut + o] - mean) : q[p * kOut + o];
+                }
+                const int act = l.action[i0 + b], nact = l.next_action ? l.next_action[i0 + b] : 0;
+                const float rew = l.reward[i0 + b];
+                float upd = rew;
+                if (!l.done[i0 + b]) {
+                    if (l.next_action) {
+                        if (nact >= 0 && nact < A) upd = rew + l.gamma * qv[2][nact];
+                    } else {
+                        float best = qv[2][0];
+                        for (int o = 1; o < A; ++o) best = fmaxf(best, qv[2][o]);
+                        upd = rew + l.gamma * best;
+                    }
+                }
+                float se = 0.0f, dsum = 0.0f, dq[kMaxActions];
+                for (int o = 0; o < A; ++o) {
+                    const float e = qv[0][o] - ((o == act) ? upd : qv[1][o]);
+                    se += e * e;
+                    dq[o] = 2.0f * e * inv_n;
+                    dsum += dq[o];
+                }
+                const float dmean = dsum / (float)A;
+                for (int o = 0; o < A; ++o) dout[o] = a.duel ? dq[o] - dmean : dq[o];
+                dout[A] = a.duel ? dsum : 0.0f;
+                a.sq[b] = se;
+                for (int o = 0; o < A1; ++o) a.dout[b * kOut + o] = dout[o];
+            }
+            __syncthreads();
+            for (int u = tid; u < U; u += kLThreads) {  // back through the second layer (before it is updated)
+                float dh = 0.0f;
+                if (u < hid) {
+                    for (int o = 0; o < A; ++o) dh += dout[o] * __ldcg(l.P + w2_off(u, o));
+                } else {
+                    dh = dout[A] * __ldcg(l.P + w2_off(u, A));
+                }
+                const float hv = hq[u];
+                a.h[b * U + u] = hv;
+                a.dz[b * U + u] = dh * hv * (1.0f - hv);
+            }
+            __syncthreads();
+        }
+        grid.sync();
+
+        // ---- Adam
+        const int64_t t = l.adam_t + r + 1;
+        const float lr_t = (float)(l.lr * sqrt(1.0 - pow(l.beta_2, (double)t)) / (1.0 - pow(l.beta_1, (double)t)));
+        const bool sync = --until_sync == 0;
+        if (sync) until_sync = l.target_every;
+        const int n_small = U * (1 + A1) + A1;  // per unit: bias, second-layer column; then the output biases
+        for (int k = blk * kLThreads + tid; k < n_small; k += nblk * kLThreads) {
+            int off;
+            float gr = 0.0f;
+            if (k < U * (1 + A1)) {
+                const int g = k / (1 + A1), c = k - g * (1 + A1);
+                if (c == 0) {
+                    off = b1_off(g);
+                    for (int b = 0; b < B; ++b) gr += __ldcg(a.dz + b * U + g);
+                } else {
+                    const int o = c - 1;
+                    if (g < hid ? o >= A : o != A) continue;
+                    off = w2_off(g, o);
+                    for (int b = 0; b < B; ++b) gr += __ldcg(a.dout + b * kOut + o) * __ldcg(a.h + b * U + g);
+                }
+            } else {
+                const int o = k - U * (1 + A1);
+                if (o == A && !a.duel) continue;
+                off = o < A ? a.off_b2 + o : a.off_b4;
+                for (int b = 0; b < B; ++b) gr += __ldcg(a.dout + b * kOut + o);
+            }
+            float m = l.M[off], v = l.V[off];
+            const float p = adam(l, lr_t, l.P[off], gr, m, v);
+            l.P[off] = p;
+            l.M[off] = m;
+            l.V[off] = v;
+            if (sync) l.T[off] = p;
+        }
+        if (blk == 0 && tid == 0 && l.loss) {
+            float s = 0.0f;
+            for (int b = 0; b < B; ++b) s += __ldcg(a.sq + b);
+            l.loss[r] = s * inv_n;
+        }
+        // first layer of this CTA's chunks; mk[bb][f]: which samples 32 * bb .. 32 * bb + 31 have bit f set
+        const int nbb = (B + 31) / 32;
+        float* dzs = fs;                                                // [B][U]
+        uint32_t* ub = reinterpret_cast<uint32_t*>(fs + B * U);        // [B][sub]
+        uint32_t* mk = ub + B * sub;                                    // [nbb][sub * 32]
+        if (blk < a.nc) {
+            __syncthreads();
+            for (int k = tid; k < B * U; k += kLThreads) dzs[k] = __ldcg(a.dz + k);
+        }
+        for (int c = blk; c < a.nc; c += nblk) {
+            const int cw0 = c * a.cw, cw1 = min(a.words, cw0 + a.cw);
+            for (int w0 = cw0; w0 < cw1; w0 += sub) {
+                const int nw = min(sub, cw1 - w0), nf = nw * 32, f0 = w0 * 32;
+                __syncthreads();
+                for (int k = tid; k < B * nw; k += kLThreads) {
+                    const int b = k / nw, w = k - b * nw;
+                    ub[b * sub + w] = frame_word(a, l.s_row[i0 + b], w0 + w);
+                }
+                __syncthreads();
+                for (int k = tid; k < nbb * nf; k += kLThreads) {
+                    const int bb = k / nf, f = k - bb * nf;
+                    uint32_t m = 0u;
+                    for (int i = 0; i < 32 && bb * 32 + i < B; ++i) m |= ((ub[(bb * 32 + i) * sub + (f >> 5)] >> (f & 31)) & 1u) << i;
+                    mk[bb * sub * 32 + f] = m;
+                }
+                __syncthreads();
+                for (int k0 = 0; k0 < U * nf; k0 += kBatch * kLThreads) {  // kBatch entries per thread: loads in flight
+                    float g[kBatch], p[kBatch], m[kBatch], v[kBatch];
+                    int64_t off[kBatch];
+                    bool ok[kBatch];
+#pragma unroll
+                    for (int i = 0; i < kBatch; ++i) {
+                        const int k = k0 + i * kLThreads + tid, u = k / nf, f = k - u * nf;
+                        ok[i] = k < U * nf && f0 + f < n_in;
+                        g[i] = 0.0f;
+                        off[i] = ok[i] ? w1_off(u) + f0 + f : 0;
+                        if (ok[i]) {
+                            for (int bb = 0; bb < nbb; ++bb) {
+                                const float* d = dzs + bb * 32 * U + u;
+                                for (uint32_t mb = mk[bb * sub * 32 + f]; mb; mb &= mb - 1u) g[i] += d[(__ffs(mb) - 1) * U];
+                            }
+                        }
+                    }
+#pragma unroll
+                    for (int i = 0; i < kBatch; ++i) {
+                        if (ok[i]) {
+                            p[i] = l.P[off[i]];
+                            m[i] = l.M[off[i]];
+                            v[i] = l.V[off[i]];
+                        }
+                    }
+#pragma unroll
+                    for (int i = 0; i < kBatch; ++i) {
+                        if (ok[i]) {
+                            p[i] = adam(l, lr_t, p[i], g[i], m[i], v[i]);
+                            l.P[off[i]] = p[i];
+                            l.M[off[i]] = m[i];
+                            l.V[off[i]] = v[i];
+                            if (sync) l.T[off[i]] = p[i];
+                        }
+                    }
+                }
+            }
+        }
+    }
+}
+
 // Refuses a learner whose pointers or hyper-parameters wf_replay_fit would refuse; `who` prefixes the message.
 int check_learner(const std::string& who, const wf_fit_learner& l) {
     if (!l.params || !l.target || !l.adam_m || !l.adam_v || !l.s_row || !l.sp_row || !l.action || !l.reward || !l.done)
@@ -353,13 +685,9 @@ int check_learner(const std::string& who, const wf_fit_learner& l) {
     return WF_OK;
 }
 
-// wf_replay_fit_many after the caller's null checks; `name` is the entry point the messages name.
-int replay_fit_impl(const char* name, const wf_mlp_shape& sh, int32_t n_learners, const wf_fit_learner* learners,
-                    int32_t n_replays, const uint32_t* frames_dev, int64_t n_frames, void* stream) {
-    const std::string fn(name);
-    if (n_learners < 1 || n_learners > kMaxLearners) return api_fail(WF_ERR_INVALID, fn + ": n_learners must be in 1..64");
-    if (sh.height < 10 || sh.width < sh.height || sh.width > 32)
-        return api_fail(WF_ERR_INVALID, fn + ": the grid must satisfy 10 <= height <= width <= 32");
+// The shape and call checks wf_replay_fit and wf_replay_fit_large share (the grid is checked by the caller).
+int check_fit_args(const std::string& fn, const wf_mlp_shape& sh, int32_t n_replays, const uint32_t* frames_dev,
+                   int64_t n_frames) {
     if (sh.hidden < 1 || sh.hidden > kMaxHidden) return api_fail(WF_ERR_INVALID, fn + ": hidden must be in 1..64");
     if (sh.n_actions < 1 || sh.n_actions > kMaxActions) return api_fail(WF_ERR_INVALID, fn + ": n_actions must be in 1..8");
     if (sh.dueling != 0 && sh.dueling != 1) return api_fail(WF_ERR_INVALID, fn + ": dueling must be 0 or 1");
@@ -367,14 +695,12 @@ int replay_fit_impl(const char* name, const wf_mlp_shape& sh, int32_t n_learners
     if (n_replays < 1) return api_fail(WF_ERR_INVALID, fn + ": n_replays must be >= 1");
     if (n_frames < 0) return api_fail(WF_ERR_INVALID, fn + ": n_frames must be >= 0");
     if (reinterpret_cast<uintptr_t>(frames_dev) & 3u) return api_fail(WF_ERR_INVALID, fn + ": buffers must be 4-byte aligned");
-    for (int j = 0; j < n_learners; ++j)
-        if (int rc = check_learner(n_learners == 1 ? fn : fn + ": learner " + std::to_string(j), learners[j])) return rc;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        return api_fail(WF_ERR_CUDA, "no CUDA device: libwildfire_b200 has no CPU fallback");
+    return WF_OK;
+}
 
-    FitArgs a{};
-    a.frames = frames_dev, a.n_frames = n_frames, a.n_replays = n_replays;
+// The flat layout of include/wildfire.h in a kernel's arguments (FitArgs, LargeArgs).
+template <class Args>
+void set_layout(Args& a, const wf_mlp_shape& sh) {
     a.n_in = sh.width * sh.height * 3;
     a.words = (int)wf::obs_bits_words(sh.width, sh.height);
     a.hid = sh.hidden, a.A = sh.n_actions, a.duel = sh.dueling, a.B = sh.batch;
@@ -385,21 +711,42 @@ int replay_fit_impl(const char* name, const wf_mlp_shape& sh, int32_t n_learners
     a.off_b3 = a.off_w3 + a.hid * a.n_in;
     a.off_w4 = a.off_b3 + a.hid;
     a.off_b4 = a.off_w4 + a.hid;
-    for (int j = 0; j < n_learners; ++j) {
-        const wf_fit_learner& in = learners[j];
-        const wf_fit_params* hp = &in.hp;
-        FitLearner& l = a.learner[j];
-        l.P = in.params, l.T = in.target, l.M = in.adam_m, l.V = in.adam_v;
-        l.s_row = in.s_row, l.sp_row = in.sp_row, l.action = in.action, l.next_action = in.next_action;
-        l.reward = in.reward, l.done = in.done, l.loss = in.loss;
-        // scalars as torch applies them to float32 tensors (KerasAdam.step): cast once to float
-        l.gamma = (float)hp->gamma;
-        l.b1 = (float)hp->beta_1, l.omb1 = (float)(1.0 - hp->beta_1);
-        l.b2 = (float)hp->beta_2, l.omb2 = (float)(1.0 - hp->beta_2);
-        l.eps = (float)hp->epsilon, l.clip = (float)hp->clipvalue;
-        l.lr = hp->lr, l.beta_1 = hp->beta_1, l.beta_2 = hp->beta_2;
-        l.adam_t = hp->adam_t, l.target_every = hp->target_every, l.phase = hp->phase;
-    }
+}
+
+FitLearner prepare_learner(const wf_fit_learner& in) {
+    const wf_fit_params* hp = &in.hp;
+    FitLearner l;
+    l.P = in.params, l.T = in.target, l.M = in.adam_m, l.V = in.adam_v;
+    l.s_row = in.s_row, l.sp_row = in.sp_row, l.action = in.action, l.next_action = in.next_action;
+    l.reward = in.reward, l.done = in.done, l.loss = in.loss;
+    // scalars as torch applies them to float32 tensors (KerasAdam.step): cast once to float
+    l.gamma = (float)hp->gamma;
+    l.b1 = (float)hp->beta_1, l.omb1 = (float)(1.0 - hp->beta_1);
+    l.b2 = (float)hp->beta_2, l.omb2 = (float)(1.0 - hp->beta_2);
+    l.eps = (float)hp->epsilon, l.clip = (float)hp->clipvalue;
+    l.lr = hp->lr, l.beta_1 = hp->beta_1, l.beta_2 = hp->beta_2;
+    l.adam_t = hp->adam_t, l.target_every = hp->target_every, l.phase = hp->phase;
+    return l;
+}
+
+// wf_replay_fit_many after the caller's null checks; `name` is the entry point the messages name.
+int replay_fit_impl(const char* name, const wf_mlp_shape& sh, int32_t n_learners, const wf_fit_learner* learners,
+                    int32_t n_replays, const uint32_t* frames_dev, int64_t n_frames, void* stream) {
+    const std::string fn(name);
+    if (n_learners < 1 || n_learners > kMaxLearners) return api_fail(WF_ERR_INVALID, fn + ": n_learners must be in 1..64");
+    if (sh.height < 10 || sh.width < sh.height || sh.width > 32)
+        return api_fail(WF_ERR_INVALID, fn + ": the grid must satisfy 10 <= height <= width <= 32");
+    if (int rc = check_fit_args(fn, sh, n_replays, frames_dev, n_frames)) return rc;
+    for (int j = 0; j < n_learners; ++j)
+        if (int rc = check_learner(n_learners == 1 ? fn : fn + ": learner " + std::to_string(j), learners[j])) return rc;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+        return api_fail(WF_ERR_CUDA, "no CUDA device: libwildfire_b200 has no CPU fallback");
+
+    FitArgs a{};
+    a.frames = frames_dev, a.n_frames = n_frames, a.n_replays = n_replays;
+    set_layout(a, sh);
+    for (int j = 0; j < n_learners; ++j) a.learner[j] = prepare_learner(learners[j]);
 
     const size_t smem = sizeof(Smem);
     int device = 0;
@@ -424,6 +771,69 @@ int replay_fit_impl(const char* name, const wf_mlp_shape& sh, int32_t n_learners
     return WF_OK;
 }
 
+// wf_replay_fit_large after the null checks.
+int replay_fit_large_impl(const wf_mlp_shape& sh, const wf_fit_learner& learner, int32_t n_replays,
+                          const uint32_t* frames_dev, int64_t n_frames, void* stream) {
+    const std::string fn("wf_replay_fit_large");
+    if (sh.height < 10 || sh.width < sh.height)
+        return api_fail(WF_ERR_INVALID, fn + ": the grid must satisfy 10 <= height <= width");
+    if (int rc = check_fit_args(fn, sh, n_replays, frames_dev, n_frames)) return rc;
+    const int64_t n_in = (int64_t)sh.width * sh.height * 3;
+    const int64_t n_flat = sh.hidden * (n_in + 1 + sh.n_actions) + sh.n_actions + (sh.dueling ? sh.hidden * (n_in + 2) + 1 : 0);
+    if (n_flat > INT32_MAX)
+        return api_fail(WF_ERR_INVALID, fn + ": the flat parameter buffer would exceed 2^31 - 1 floats");
+    if (int rc = check_learner(fn, learner)) return rc;
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+        return api_fail(WF_ERR_CUDA, "no CUDA device: libwildfire_b200 has no CPU fallback");
+
+    LargeArgs a{};
+    a.l = prepare_learner(learner);
+    a.frames = frames_dev, a.n_frames = n_frames, a.n_replays = n_replays;
+    set_layout(a, sh);
+    a.units = a.hid * (a.duel ? 2 : 1);
+    // chunks: at most kMaxChunks, and at most kPartBudget floats of partials; sub-tiles: kWsFloats staged weights
+    const int64_t per_chunk = 3LL * a.B * a.units;
+    const int64_t nc_max = std::max<int64_t>(1, std::min<int64_t>(kMaxChunks, kPartBudget / per_chunk));
+    a.cw = (int)((a.words + nc_max - 1) / nc_max);
+    a.nc = (a.words + a.cw - 1) / a.cw;
+    a.sub = std::max(1, std::min(kMaxSub, kWsFloats / (64 * a.units)));
+    const int nbb = (a.B + 31) / 32;
+    const size_t smem = 4 * std::max({(size_t)2 * a.sub * 32 * a.units + 2 * a.B * a.sub,                  // forward
+                                      (size_t)(kSegs + 1) * 3 * a.units + 4 * kOut,                       // reduce
+                                      (size_t)a.B * a.units + a.B * a.sub + nbb * a.sub * 32});           // update
+    const size_t scratch = 4 * ((size_t)a.nc * per_chunk + 2 * a.B * a.units + a.B * kOut + a.B);
+
+    int device = 0, n_sm = 0, per_sm = 0;
+    cudaError_t err = cudaGetDevice(&device);
+    if (err == cudaSuccess) err = cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device);
+    if (err == cudaSuccess) err = cudaFuncSetAttribute(replay_fit_large_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (err == cudaSuccess) err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, replay_fit_large_kernel, kLThreads, smem);
+    if (err != cudaSuccess) return api_fail(WF_ERR_CUDA, fn + ": " + cudaGetErrorString(err));
+    int ctas = n_sm * per_sm;
+    if (ctas < 1) return api_fail(WF_ERR_CUDA, fn + ": the kernel does not fit this device");
+    if (const char* env = std::getenv("WF_FIT_CTAS")) {  // experiments and tests: the result does not depend on it
+        const int want = std::atoi(env);
+        if (want > 0) ctas = std::min(ctas, want);
+    }
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    void* buf = nullptr;
+    err = cudaMallocAsync(&buf, scratch, st);
+    if (err != cudaSuccess) return api_fail(WF_ERR_CUDA, fn + ": scratch: " + cudaGetErrorString(err));
+    float* f = static_cast<float*>(buf);
+    a.part = f;
+    a.h = a.part + (size_t)a.nc * per_chunk;
+    a.dz = a.h + a.B * a.units;
+    a.dout = a.dz + a.B * a.units;
+    a.sq = a.dout + a.B * kOut;
+    void* args[] = {&a};
+    err = cudaLaunchCooperativeKernel((const void*)replay_fit_large_kernel, dim3(ctas), dim3(kLThreads), args, smem, st);
+    const cudaError_t err_free = cudaFreeAsync(buf, st);
+    if (err == cudaSuccess) err = err_free;
+    if (err != cudaSuccess) return api_fail(WF_ERR_CUDA, fn + ": " + cudaGetErrorString(err));
+    return WF_OK;
+}
+
 }  // namespace
 
 extern "C" int wf_replay_fit_many(const wf_mlp_shape* shape, int32_t n_learners, const wf_fit_learner* learners_host,
@@ -441,4 +851,15 @@ extern "C" int wf_replay_fit(const wf_mlp_shape* shape, const wf_fit_params* hp,
     const wf_fit_learner l{params_dev, target_dev, adam_m_dev, adam_v_dev, s_row_dev, sp_row_dev, action_dev, next_action_dev,
                            reward_dev, done_dev, loss_dev, *hp};
     return replay_fit_impl("wf_replay_fit", *shape, 1, &l, n_replays, frames_dev, n_frames, stream);
+}
+
+extern "C" int wf_replay_fit_large(const wf_mlp_shape* shape, const wf_fit_params* hp, int32_t n_replays, float* params_dev,
+                                   float* target_dev, float* adam_m_dev, float* adam_v_dev, const uint32_t* frames_dev,
+                                   int64_t n_frames, const int64_t* s_row_dev, const int64_t* sp_row_dev,
+                                   const int32_t* action_dev, const int32_t* next_action_dev, const float* reward_dev,
+                                   const uint8_t* done_dev, float* loss_dev, void* stream) {
+    if (!shape || !hp || !frames_dev) return api_fail(WF_ERR_INVALID, "wf_replay_fit_large: null argument");
+    const wf_fit_learner l{params_dev, target_dev, adam_m_dev, adam_v_dev, s_row_dev, sp_row_dev, action_dev, next_action_dev,
+                           reward_dev, done_dev, loss_dev, *hp};
+    return replay_fit_large_impl(*shape, l, n_replays, frames_dev, n_frames, stream);
 }
