@@ -701,7 +701,7 @@ class DQN:
         return loss
 
     def learn_batched(self, n_episodes, n_envs=1024, k_steps=16, replays_per_launch=None, batch_size=None, seed=0,
-                      replay_seed=None):
+                      replay_seed=None, checkpoint=None, time_limit=None):
         """``learn`` over ``n_envs`` CUDA environments at once: the envs act with the eps-greedy Q-network evaluated inside
         the step kernel (``rollout(policy="mlp")``, ``k_steps`` steps per launch), each rollout writes its packed
         observations straight into a device replay ring, and after every launch ``replays_per_launch`` (default
@@ -722,25 +722,47 @@ class DQN:
         device and are not rendered.  One small device-to-host read per launch (rewards and done flags).
         ``eps_per_launch`` / ``episodes_before_launch`` record the schedule.  Any grid: ``fit_batches_fused`` runs the
         replays in ``wf_replay_fit`` up to 32x32 and in ``wf_replay_fit_large`` on larger grids.  Returns the number of
-        environment steps simulated."""
+        environment steps simulated.
+
+        ``checkpoint=PATH``: resume the run from that file if it exists (``ValueError`` if it was written by a run with
+        another class, network shape, METADATA, demonstration count or other arguments); remove it once the logs are
+        written.  ``time_limit=SECONDS`` (needs ``checkpoint``): checked after each launch's replays and episode
+        accounting; once this call has run that long and the run is not finished, write the run's whole state to the
+        checkpoint (atomically) and return None without writing logs.  Calling again with the same arguments continues
+        exactly where the run stopped, with byte-identical results, from a freshly built agent too: the model, target,
+        optimiser state, ``_until_sync``, logs and eps schedule are overwritten from the file.  ``logs['total_time']`` is
+        the sum of the calls' times."""
         from .batched import BatchedForestFire
         from .constants import DQN_DEFAULTS as _D
+        if time_limit is not None and checkpoint is None:
+            raise ValueError("time_limit needs a checkpoint file to save the run to")
         t_run = time.time()
         N, K = int(n_envs), int(k_steps)
         R = K if replays_per_launch is None else int(replays_per_launch)
         B = int(self.METADATA["batch_size"] if batch_size is None else batch_size)
+        rseed = int(seed if replay_seed is None else replay_seed)
+        ckpt = _RunCheckpoint(checkpoint, _run_fingerprint("learn_batched", [self], n_episodes=n_episodes, n_envs=N, k_steps=K,
+                                                           replays_per_launch=R, batch_size=B, seed=seed, replay_seed=rseed))
+        saved = ckpt.load()
         keys = {k: v for k, v in self.METADATA.items() if k not in _D and k not in ("debug", "a_speed_iter", "seed", "auto_reset")}
         env = BatchedForestFire(N, device=self.device, obs_dtype="bits", auto_reset=True, seed=seed, **keys)
         death_penalty = float(self.METADATA["death_penalty"])
-        gen = torch.Generator(device=env.device).manual_seed(int(seed if replay_seed is None else replay_seed))
+        gen = torch.Generator(device=env.device).manual_seed(rseed)
         self._until_sync = self.target_update_freq
         self.logs["n_episodes"] = n_episodes
         self.eps_per_launch, self.episodes_before_launch = [], []
         rewards, deaths = [], []
         carry = np.zeros(N)
-        done_eps = 0
+        done_eps, elapsed = 0, 0.0
         try:
             ring = _PackedReplayRing(env, K, int(self.METADATA["memory_size"]), self.memory, self._SARSA)
+            if saved is not None:
+                env.set_state(**saved["env"])
+                ring.load_state_dict(saved["ring"])
+                gen.set_state(saved["replay_generator"])
+                self._load_learner_state(saved["agent"])
+                carry, done_eps, elapsed = saved["carry"].numpy(), saved["done_eps"], saved["elapsed"]
+                rewards, deaths = saved["rewards"], saved["deaths"]
             while len(rewards) < n_episodes:
                 self.eps = self.min_eps + (self.max_eps - self.min_eps) * np.exp(-self.eps_decay_rate * done_eps)
                 self.eps_per_launch.append(float(self.eps))
@@ -757,14 +779,40 @@ class DQN:
                     rewards.append(float(ret[i]))
                     deaths.append(bool(rd[0][k_idx[i], e_idx[i]] == death_penalty))
                 done_eps += len(e_idx)
+                if len(rewards) < n_episodes and time_limit is not None and time.time() - t_run >= time_limit:
+                    ckpt.save(dict(env=_env_state(env), ring=ring.state_dict(), replay_generator=gen.get_state(),
+                                   agent=self._learner_state(), carry=torch.from_numpy(carry), done_eps=done_eps,
+                                   rewards=rewards, deaths=deaths, elapsed=elapsed + time.time() - t_run))
+                    return None
             steps = ring.steps
         finally:
             env.close()
         self.logs["total_rewards"] = rewards
         self.logs["agent_deaths"] = deaths
-        self.logs["total_time"] = round(time.time() - t_run, 3)
+        self.logs["total_time"] = round(elapsed + time.time() - t_run, 3)
         self.write_data()
+        ckpt.remove()
         return steps * N
+
+    def _learner_state(self):
+        """What ``learn_batched`` checkpoints of this agent, on the CPU: model, target, ``KerasAdam`` step and moments,
+        ``_until_sync``, logs and eps schedule."""
+        params = list(self.model.parameters())
+        opt = [self.optimizer.state[p] for p in params]
+        t = opt[0]["t"] if opt[0] else 0
+        cpu = lambda sd: {k: v.cpu() for k, v in sd.items()}  # noqa: E731
+        return dict(model=cpu(self.model.state_dict()), target=cpu(self.target.state_dict()), adam_t=t,
+                    adam_m=[st["m"].cpu() for st in opt] if t else [], adam_v=[st["v"].cpu() for st in opt] if t else [],
+                    until_sync=self._until_sync, **_schedule_state(self))
+
+    def _load_learner_state(self, st):
+        self.model.load_state_dict(st["model"])  # copies into the existing parameters: the optimiser keeps them
+        self.target.load_state_dict(st["target"])
+        self.optimizer.state.clear()
+        for p, m, v in zip(self.model.parameters(), st["adam_m"], st["adam_v"]):
+            self.optimizer.state[p] = dict(t=st["adam_t"], m=m.to(p.device), v=v.to(p.device))
+        self._until_sync = st["until_sync"]
+        _load_schedule_state(self, st)
 
     def save_model(self, name):  # DQN.py:441-443
         path = os.path.join(self.out_dir, "Models", name)
@@ -841,6 +889,23 @@ class _PackedReplayRing:
         self.steps += self.K
         return self.rews[sl], self.dones[sl]
 
+    def state_dict(self):
+        """The ring's contents and step count on the CPU (``frames`` includes the reset frames and the packed
+        demonstrations)."""
+        return dict(frames=self.frames.cpu(), acts=self.acts.cpu(), rews=self.rews.cpu(), dones=self.dones.cpu(),
+                    steps=self.steps)
+
+    def load_state_dict(self, state):
+        """Overwrite the ring with a ``state_dict()`` of a ring of the same layout (same env batch, K, memory_size and
+        demonstration counts)."""
+        for k in ("frames", "acts", "rews", "dones"):
+            t = getattr(self, k)
+            if tuple(state[k].shape) != tuple(t.shape) or state[k].dtype != t.dtype:
+                raise ValueError(f"replay ring {k}: the state holds {state[k].dtype} {tuple(state[k].shape)}, this ring "
+                                 f"{t.dtype} {tuple(t.shape)}")
+            t.copy_(state[k])  # in place: self.ring is a view of frames
+        self.steps = int(state["steps"])
+
     @property
     def window(self):
         """Global steps [lo, hi) whose transitions are held."""
@@ -882,12 +947,100 @@ class _PackedReplayRing:
         return s_row, sp_row, a, ap, r, d
 
 
+def _run_fingerprint(entry, agents, **args):
+    """What a checkpoint must agree on to continue a run: the entry point, the agents' class and network shape, every
+    agent's METADATA and demonstration count, and the call's arguments (as JSON values)."""
+    a0 = agents[0]
+    fp = dict(entry=entry, agent_class=type(a0).__name__, network=[list(p.shape) for p in a0.model.parameters()],
+              agents=len(agents), METADATA=[a.METADATA for a in agents], demonstrations=[len(a.memory) for a in agents],
+              **args)
+    return json.loads(json.dumps(fp, default=_jsonable))
+
+
+def _first_difference(x, y, where):
+    """(path, x value, y value) of the first entry in which two JSON values differ, e.g. ``METADATA[1]['alpha']``."""
+    if isinstance(x, dict) and isinstance(y, dict):
+        for k in sorted(set(x) | set(y)):
+            if x.get(k) != y.get(k):
+                return _first_difference(x.get(k), y.get(k), f"{where}[{k!r}]")
+    elif isinstance(x, list) and isinstance(y, list) and len(x) == len(y):
+        for i, (a, b) in enumerate(zip(x, y)):
+            if a != b:
+                return _first_difference(a, b, f"{where}[{i}]")
+    return where, x, y
+
+
+class _RunCheckpoint:
+    """The file behind ``checkpoint=PATH`` of ``DQN.learn_batched`` and ``learn_population``: one ``torch.save`` dict of a
+    run's fingerprint (``_run_fingerprint``) and its state (CPU tensors and plain Python values, so that
+    ``torch.load(weights_only=True)`` reads it).  ``path=None``: no file; ``load`` returns None."""
+
+    def __init__(self, path, fingerprint):
+        self.path = None if path is None else os.fspath(path)
+        self.fingerprint = fingerprint
+
+    def load(self):
+        """The state stored in the file, or None if there is no file.  ValueError naming the first field that differs if the
+        file was written by another run."""
+        if self.path is None or not os.path.exists(self.path):
+            return None
+        ck = torch.load(self.path, map_location="cpu", weights_only=True)
+        saved = json.loads(ck["fingerprint"])
+        for k, v in self.fingerprint.items():
+            if saved.get(k) != v:
+                where, was, now = _first_difference(saved.get(k), v, k)
+                raise ValueError(f"checkpoint {self.path} was written by another run: {where} is {was!r} there and {now!r} "
+                                 f"in this call")
+        return ck["state"]
+
+    def save(self, state):
+        """Replace the file atomically: write a temporary file next to it, flush and fsync it, then rename it over the old
+        one.  A kill at any point leaves the previous checkpoint or the new one, never a partial file."""
+        tmp = self.path + ".tmp"
+        try:
+            with open(tmp, "wb") as f:
+                torch.save(dict(fingerprint=json.dumps(self.fingerprint), state=state), f)
+                f.flush()
+                os.fsync(f.fileno())
+            os.replace(tmp, self.path)
+        finally:
+            if os.path.exists(tmp):
+                os.remove(tmp)
+        fd = os.open(os.path.dirname(os.path.abspath(self.path)), os.O_RDONLY)  # makes the rename itself durable
+        try:
+            os.fsync(fd)
+        finally:
+            os.close(fd)
+
+    def remove(self):
+        if self.path is not None and os.path.exists(self.path):
+            os.remove(self.path)
+
+
+def _env_state(env):
+    """The env batch's state as ``BatchedForestFire.set_state`` takes it (``a_iter`` included; the derived ``temp`` and
+    ``apos`` left out), on the CPU."""
+    return {k: v.cpu() for k, v in env.get_state().items() if k not in ("temp", "apos")}
+
+
+def _schedule_state(ag):
+    """An agent's logs and eps schedule, as a checkpoint stores them (the logs as the JSON ``write_data`` writes)."""
+    return dict(logs=json.dumps(ag.logs, default=_jsonable), eps=float(ag.eps), eps_per_launch=list(ag.eps_per_launch),
+                episodes_before_launch=list(ag.episodes_before_launch))
+
+
+def _load_schedule_state(ag, st):
+    ag.logs = json.loads(st["logs"])
+    ag.eps, ag.eps_per_launch, ag.episodes_before_launch = st["eps"], list(st["eps_per_launch"]), list(st["episodes_before_launch"])
+
+
 # METADATA keys the learners of one learn_population may set differently: the learning rate, the discount, the target
 # refresh interval and the eps schedule.  Everything else (the environment, memory_size, batch_size) must agree.
 _POPULATION_FREE_KEYS = ("alpha", "gamma", "target_update", "max_eps", "min_eps", "eps_decay_rate")
 
 
-def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replays_per_launch=None, batch_size=None, seed=0):
+def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replays_per_launch=None, batch_size=None, seed=0,
+                     checkpoint=None, time_limit=None):
     """``DQN.learn_batched`` for M = len(agents) independent learners (1 to 64) at once on one GPU, with one rollout launch
     and one ``wf_replay_fit_many`` launch per iteration for all of them.
 
@@ -905,11 +1058,18 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
     stepping, ignored, until every learner has finished.  Then each agent calls ``write_data()``.  Agent j's result is
     that of ``agent.learn_batched(n_episodes, envs_per_learner, k_steps, replays_per_launch, batch_size, seed=seed,
     replay_seed=seed + j)`` with METADATA ``env_id_base = j * envs_per_learner``, byte for byte.
-    Returns the env-step count of each learner (what ``learn_batched`` returns)."""
+    Returns the env-step count of each learner (what ``learn_batched`` returns).
+
+    ``checkpoint`` and ``time_limit`` work as in ``learn_batched``: the file holds the stacked model, target and Adam
+    state, each learner's Adam step, sync phase, generator, episode accounting, logs and eps schedule, the env batch and
+    the replay ring, and its fingerprint covers the number of agents and each agent's METADATA and demonstration count.
+    A stopped call returns None and writes no logs."""
     from torch.nn.utils import parameters_to_vector
     from . import _lib
     from .batched import BatchedForestFire, _ptr
     from .constants import DQN_DEFAULTS as _D
+    if time_limit is not None and checkpoint is None:
+        raise ValueError("time_limit needs a checkpoint file to save the run to")
     agents = list(agents)
     M = len(agents)
     if not 1 <= M <= _lib.MAX_LEARNERS:
@@ -931,12 +1091,15 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
         raise ValueError("envs_per_learner must be a positive multiple of 8")
     if any(a.device != a0.device for a in agents):
         raise ValueError("learn_population: every agent must be on the same device")
-    if a0.device.type != "cuda":
-        raise _lib.WildfireError("learn_population needs a CUDA device (no CPU fallback)")
     t_run = time.time()
-    N = M * G
     R = K if replays_per_launch is None else int(replays_per_launch)
     B = int(a0.METADATA["batch_size"] if batch_size is None else batch_size)
+    ckpt = _RunCheckpoint(checkpoint, _run_fingerprint("learn_population", agents, n_episodes=n_episodes, envs_per_learner=G,
+                                                       k_steps=K, replays_per_launch=R, batch_size=B, seed=seed))
+    saved = ckpt.load()
+    if a0.device.type != "cuda":
+        raise _lib.WildfireError("learn_population needs a CUDA device (no CPU fallback)")
+    N = M * G
     sarsa, dueling = a0._SARSA, hasattr(a0.model, "dense_3")
     hidden = a0.model.dense_1.out_features
     keys = {k: v for k, v in a0.METADATA.items() if k not in _D and k not in ("debug", "a_speed_iter", "seed", "auto_reset")}
@@ -957,6 +1120,7 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
     rewards, deaths = [[] for _ in agents], [[] for _ in agents]
     carry = [np.zeros(G) for _ in agents]
     done_eps, steps, finished = [0] * M, [0] * M, [False] * M
+    elapsed = 0.0
     for a in agents:
         a.logs["n_episodes"] = n_episodes
         a.eps_per_launch, a.episodes_before_launch = [], []
@@ -964,6 +1128,19 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
     stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
     try:
         ring = _PackedReplayRing(env, K, int(a0.METADATA["memory_size"]), [a.memory for a in agents], sarsa, groups=M)
+        if saved is not None:
+            env.set_state(**saved["env"])
+            ring.load_state_dict(saved["ring"])
+            for g, st in zip(gens, saved["replay_generators"]):
+                g.set_state(st)
+            for x, k in ((P, "params"), (Tg, "target"), (Mm, "adam_m"), (Vv, "adam_v")):
+                x.copy_(saved[k])
+            adam_t, until_sync = list(saved["adam_t"]), list(saved["until_sync"])
+            carry = [c.numpy() for c in saved["carry"]]
+            done_eps, steps, finished = list(saved["done_eps"]), list(saved["steps"]), list(saved["finished"])
+            rewards, deaths, elapsed = saved["rewards"], saved["deaths"], saved["elapsed"]
+            for a, st in zip(agents, saved["agents"]):
+                _load_schedule_state(a, st)
         while not all(finished):
             for j, a in enumerate(agents):
                 if not finished[j]:
@@ -1011,9 +1188,16 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
                 done_eps[j] += len(e_idx)
                 if len(rewards[j]) >= n_episodes:
                     finished[j], steps[j] = True, ring.steps * G
+            if not all(finished) and time_limit is not None and time.time() - t_run >= time_limit:
+                ckpt.save(dict(env=_env_state(env), ring=ring.state_dict(), replay_generators=[g.get_state() for g in gens],
+                               params=P.cpu(), target=Tg.cpu(), adam_m=Mm.cpu(), adam_v=Vv.cpu(), adam_t=adam_t,
+                               until_sync=until_sync, carry=[torch.from_numpy(c) for c in carry], done_eps=done_eps,
+                               steps=steps, finished=finished, rewards=rewards, deaths=deaths,
+                               agents=[_schedule_state(a) for a in agents], elapsed=elapsed + time.time() - t_run))
+                return None
     finally:
         env.close()
-    total_time = round(time.time() - t_run, 3)
+    total_time = round(elapsed + time.time() - t_run, 3)
     with torch.no_grad():
         for j, a in enumerate(agents):
             params = list(a.model.parameters())
@@ -1033,6 +1217,7 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
             a.logs["agent_deaths"] = deaths[j]
             a.logs["total_time"] = total_time
             a.write_data()
+    ckpt.remove()
     return steps
 
 
