@@ -35,7 +35,8 @@ extern "C" {
 
 #define WF_ABI_VERSION 2 /* 2: + wf_reset_host, wf_host_session(_active), wf_get/set_a_iter, wf_tile_geometry, wf_apply_change_blocks;
                             later, still 2: + WF_OBS_BITS, wf_unpack_obs_bits; + wf_set_policy_mlp_dev, wf_replay_fit;
-                            + wf_set_policy_mlp_nets_dev, wf_replay_fit_many (additions only) */
+                            + wf_set_policy_mlp_nets_dev, wf_replay_fit_many; + wf_set_final_capture,
+                            wf_final_record_words (additions only) */
 
 enum {
     WF_OK = 0,
@@ -173,6 +174,39 @@ int wf_set_policy_mlp(wf_env* env, const float* kernel1_host, const float* bias1
  * On the tile family every call re-sums the all-free map over W*H cells in float64, one thread per hidden unit. */
 int wf_set_policy_mlp_dev(wf_env* env, const float* weight1_dev, const float* bias1_dev, const float* weight2_dev,
                           const float* bias2_dev, int32_t hidden, double eps, void* stream);
+
+/* ---- final states of finished episodes ----------------------------------------------------------------------------
+ * With an auto-reset the state an episode ends in is overwritten inside the step that ends it.  While final-state capture
+ * is on (wf_set_final_capture), the step kernels of both families write ONE RECORD for every env that returns done at
+ * step k of a wf_step / wf_rollout / wf_rollout_policy launch: before the auto-reset, or at the done step itself without
+ * auto_reset (a frozen env, already done, never records again).  A record is wf_final_record_words(W, H) uint32 words:
+ *   header, WF_FINAL_HEADER_WORDS words of int32, indexed by WF_F_*: k (the step of the launch), env, the finished
+ *     episode's WF_S_EPISODE and WF_S_T (its length), the final WF_S_AX / WF_S_AY, a flag word (WF_FINAL_ALIVE,
+ *     WF_FINAL_VISIBLE, WF_FINAL_DEAD, WF_FINAL_DIGGING), and the start cell of the next episode (-1, -1 without
+ *     auto_reset); the remaining header words are zero;
+ *   from word WF_FINAL_OBS: the terminal observation as one WF_OBS_BITS row (ceil(W*H*3 / 32) words), what the step
+ *     would have returned without the reset;
+ *   from word WF_FINAL_OBS + ceil(ceil(W*H*3 / 32) / 4) * 4: four bit planes of ceil(W*H / 32) words each, in the order
+ *     fire, burnt, dirt, water (WF_FINAL_PLANE_*; a cell in none of them is grass): cell (x, y) is bit (x*H + y) % 32 of
+ *     word (x*H + y) / 32 of its plane, padding bits zero.
+ * The record length is a multiple of 4 words.  The slot of a record is an atomicAdd on *count_dev, so the order of records
+ * is unspecified while every record's content is deterministic; a record whose slot is >= capacity is counted but not
+ * written, so *count_dev > capacity shows an overflow.  The counter is never reset by the library: the caller zeroes it
+ * (and reads it) between calls as it likes. */
+enum {
+    WF_F_K = 0, WF_F_ENV, WF_F_EPISODE, WF_F_T, WF_F_AX, WF_F_AY, WF_F_FLAGS, WF_F_NEXT_AX, WF_F_NEXT_AY,
+    WF_FINAL_HEADER_WORDS = 16,
+    WF_FINAL_OBS = WF_FINAL_HEADER_WORDS
+};
+enum { WF_FINAL_ALIVE = 1, WF_FINAL_VISIBLE = 2, WF_FINAL_DEAD = 4, WF_FINAL_DIGGING = 8 };
+enum { WF_FINAL_PLANE_FIRE = 0, WF_FINAL_PLANE_BURNT = 1, WF_FINAL_PLANE_DIRT = 2, WF_FINAL_PLANE_WATER = 3 };
+/* uint32 words of one record for a W x H grid. */
+int64_t wf_final_record_words(int32_t width, int32_t height);
+/* Turn final-state capture on (records_dev: capacity records of wf_final_record_words words, device memory; count_dev:
+ * one device uint32) or off (records_dev NULL).  Handle state, like the policy weights: it applies to every later
+ * wf_step, wf_rollout and wf_rollout_policy until it is turned off, and the buffers must stay valid meanwhile.  While it is
+ * on, wf_step_host and wf_host_session return WF_ERR_STATE (no capture there). */
+int wf_set_final_capture(wf_env* env, uint32_t* records_dev, int64_t capacity, uint32_t* count_dev);
 
 /* Host-buffer variant of wf_step (what a CPU-side caller of the reference would bind):
  * copies actions H2D, steps, copies obs/reward/done D2H and synchronises.  Buffers should

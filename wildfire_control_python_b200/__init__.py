@@ -10,7 +10,8 @@ from ._lib import obs_bits_words
 from .constants import METADATA, grass, layer, make_metadata, types
 
 __all__ = ["BatchedForestFire", "ForestFire", "METADATA", "grass", "layer", "types", "make_metadata", "build",
-           "DQN", "DQN_SARSA", "DQN_DUEL", "DQN_BOTH", "learn_population", "obs_bits_words", "unpack_obs", "pack_obs"]
+           "DQN", "DQN_SARSA", "DQN_DUEL", "DQN_BOTH", "learn_population", "obs_bits_words", "unpack_obs", "pack_obs",
+           "FinalStates"]
 
 
 def build(force: bool = False, verbose: bool = False) -> str:
@@ -21,7 +22,7 @@ def __getattr__(name):  # torch is imported lazily so that `import wildfire_cont
     if name == "BatchedForestFire":
         from .batched import BatchedForestFire
         return BatchedForestFire
-    if name in ("unpack_obs", "pack_obs"):
+    if name in ("unpack_obs", "pack_obs", "FinalStates"):
         from . import batched
         return getattr(batched, name)
     if name == "ForestFire":

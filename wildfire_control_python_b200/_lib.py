@@ -28,6 +28,29 @@ def obs_bits_words(width: int, height: int) -> int:
     return (int(width) * int(height) * 3 + 31) // 32
 
 
+# Final-state records (wf_set_final_capture, include/wildfire.h): header words, flag bits, type planes.
+(F_K, F_ENV, F_EPISODE, F_T, F_AX, F_AY, F_FLAGS, F_NEXT_AX, F_NEXT_AY) = range(9)
+FINAL_HEADER_WORDS = 16
+FINAL_OBS = FINAL_HEADER_WORDS
+FINAL_ALIVE, FINAL_VISIBLE, FINAL_DEAD, FINAL_DIGGING = 1, 2, 4, 8
+FINAL_PLANE_FIRE, FINAL_PLANE_BURNT, FINAL_PLANE_DIRT, FINAL_PLANE_WATER = range(4)
+
+
+def final_plane_words(width: int, height: int) -> int:
+    """uint32 words of one type plane of a final-state record: ceil(W*H / 32)."""
+    return (int(width) * int(height) + 31) // 32
+
+
+def final_plane_offset(width: int, height: int) -> int:
+    """First word of the fire plane within a record: after the header and the observation row, rounded up to 4 words."""
+    return FINAL_OBS + (obs_bits_words(width, height) + 3) // 4 * 4
+
+
+def final_record_words(width: int, height: int) -> int:
+    """uint32 words of one final-state record (``wf_final_record_words``), a multiple of 4."""
+    return (final_plane_offset(width, height) + 4 * final_plane_words(width, height) + 3) // 4 * 4
+
+
 class WfConfig(C.Structure):
     _fields_ = [
         ("width", C.c_int32), ("height", C.c_int32), ("n_actions", C.c_int32), ("a_speed", C.c_int32),
@@ -156,6 +179,10 @@ def lib():
     L.wf_apply_change_blocks.restype = C.c_int
     L.wf_unpack_obs_bits.argtypes = [vp, C.c_int64, vp, C.c_int64, C.c_int32, C.c_int32, vp, C.c_int32, vp]
     L.wf_unpack_obs_bits.restype = C.c_int
+    L.wf_set_final_capture.argtypes = [vp, vp, C.c_int64, vp]
+    L.wf_set_final_capture.restype = C.c_int
+    L.wf_final_record_words.argtypes = [C.c_int32, C.c_int32]
+    L.wf_final_record_words.restype = C.c_int64
     L.wf_state_bytes_per_env.argtypes = [vp]
     L.wf_state_bytes_per_env.restype = C.c_int64
     for name in ("wf_create", "wf_reset", "wf_step", "wf_rollout", "wf_rollout_policy", "wf_set_policy_mlp", "wf_step_host", "wf_get_state", "wf_set_state",
@@ -176,5 +203,5 @@ EXPORTED_SYMBOLS = [
     "wf_get_obs", "wf_get_wind_table", "wf_stats", "wf_stats_reset", "wf_philox_kat", "wf_launch_count",
     "wf_state_bytes_per_env", "wf_host_threads", "wf_expand_packed_obs", "wf_apply_change_blocks", "wf_get_a_iter", "wf_set_a_iter", "wf_reset_host", "wf_tile_geometry", "wf_host_session", "wf_host_session_active",
     "wf_unpack_obs_bits", "wf_set_policy_mlp_dev", "wf_replay_fit", "wf_replay_fit_many", "wf_set_policy_mlp_nets_dev",
-    "wf_replay_fit_large",
+    "wf_replay_fit_large", "wf_set_final_capture", "wf_final_record_words",
 ]

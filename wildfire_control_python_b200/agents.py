@@ -282,12 +282,8 @@ class DQN:
         dead = len(self.sim.W.agents) == 0
         if self.DEBUG > 0:
             self.logs["agent_deaths"].append(dead)
-        if total_reward >= 0.9 * self.logs["best_reward"] or total_reward > 300:
-            map_string = self._render_string()
-            if total_reward > self.logs["best_reward"]:
-                self.logs["best_reward"] = total_reward
-            if self.DEBUG > 0:
-                self.logs["maps"].append([episode, map_string])
+        self.logs["best_reward"] = _map_rule(self.logs["maps"] if self.DEBUG > 0 else None, self.logs["best_reward"],
+                                             episode, total_reward, self._render_string)
         if self.verbose:
             print(f"[Episode {episode + 1}]\tTime: {round(time.time() - t0, 3)}")
             print(f"\t\tEpsilon: {round(self.eps, 3)}")
@@ -547,7 +543,8 @@ class DQN:
         from .keras_h5 import canonical_dense_names, read_keras_weights
         self.set_weights(canonical_dense_names(read_keras_weights(path)))
 
-    def evaluate_batched(self, n_envs=4096, episodes_per_env=1, eps=None, seed=0, max_steps=100000, in_kernel=None):
+    def evaluate_batched(self, n_envs=4096, episodes_per_env=1, eps=None, seed=0, max_steps=100000, in_kernel=None,
+                         record_maps=False):
         """Roll the current policy out on ``n_envs`` CUDA environments at once (eps-greedy, DQN.py:188-196) and
         return (total reward, agent died) of the first ``episodes_per_env`` episodes of every env -- the
         quantity ``logs['total_rewards']`` / ``logs['agent_deaths']`` hold per training episode.
@@ -556,7 +553,10 @@ class DQN:
         evaluated INSIDE the step kernel (``wf_rollout_policy(WF_POLICY_MLP)``), 64 steps per launch;
         otherwise torch evaluates it between two ``wf_step`` calls.  On grids larger than 32x32 ``in_kernel=True`` is
         the fast path (the tile kernel's policy pass); the default stays the torch path there, whose exploration draws
-        come from another random stream, so its results are unchanged."""
+        come from another random stream, so its results are unchanged.
+
+        ``record_maps=True`` (needs the in-kernel path): also return the final map of every evaluated episode, the string
+        ``ForestFire.render(print_map=False)`` gives for its last state, in the order of the returns."""
         from .batched import BatchedForestFire
         from .constants import DQN_DEFAULTS as _D
         eps = self.min_eps if eps is None else eps
@@ -564,9 +564,12 @@ class DQN:
         env = BatchedForestFire(n_envs, device=self.device, auto_reset=True, seed=seed, **keys)
         if in_kernel is None:
             in_kernel = env.kernel_family == "warp"
+        if record_maps and not in_kernel:
+            env.close()
+            raise ValueError("evaluate_batched(record_maps=True) needs the in-kernel path (in_kernel=True)")
         if in_kernel:
             try:
-                return self._evaluate_in_kernel(env, n_envs, episodes_per_env, eps, max_steps)
+                return self._evaluate_in_kernel(env, n_envs, episodes_per_env, eps, max_steps, record_maps=record_maps)
             finally:
                 env.close()
         dev = self.device
@@ -600,7 +603,7 @@ class DQN:
             env.close()
         return returns.flatten().cpu().numpy(), died.flatten().cpu().numpy()
 
-    def _evaluate_in_kernel(self, env, n_envs, episodes_per_env, eps, max_steps, chunk=64):
+    def _evaluate_in_kernel(self, env, n_envs, episodes_per_env, eps, max_steps, chunk=64, record_maps=False):
         w = self.get_weights()  # dense_1 / dense_2 are the advantage stream of a dueling head: argmax Q = argmax A
         env.set_policy_mlp(w["dense_1/kernel:0"], w["dense_1/bias:0"], w["dense_2/kernel:0"], w["dense_2/bias:0"], eps=eps)
         env.reset()
@@ -609,9 +612,10 @@ class DQN:
         died = np.zeros((n_envs, episodes_per_env), dtype=bool)
         n_done = np.zeros(n_envs, dtype=np.int64)
         carry = np.zeros(n_envs)  # reward of the running episode before this chunk
+        maps = np.empty((n_envs, episodes_per_env), dtype=object) if record_maps else None
         for _ in range(0, max_steps, chunk):
-            _, rew, done = env.rollout(chunk, policy="mlp", obs=False)
-            rew, done = rew.cpu().numpy(), done.cpu().numpy()
+            res = env.rollout(chunk, policy="mlp", obs=False, finals=record_maps)
+            rew, done = res[1].cpu().numpy(), res[2].cpu().numpy()
             e_idx, k_idx, ret, carry = _episode_ends(carry, rew, done)
             same = np.r_[False, e_idx[1:] == e_idx[:-1]]
             first = np.r_[True, ~same[1:]] if len(e_idx) else np.zeros(0, bool)
@@ -620,8 +624,15 @@ class DQN:
             keep = slot < episodes_per_env
             returns[e_idx[keep], slot[keep]] = ret[keep]
             died[e_idx[keep], slot[keep]] = rew[k_idx[keep], e_idx[keep]] == death_penalty
+            if record_maps:
+                fin = res[3]
+                at = _final_index(fin)[0]
+                for e, k, sl in zip(e_idx[keep], k_idx[keep], slot[keep]):
+                    maps[e, sl] = fin.render(at[(int(k), int(e))])
             n_done += np.bincount(e_idx, minlength=n_envs)
             if (n_done >= episodes_per_env).all():
+                if record_maps:
+                    return returns.flatten(), died.flatten(), list(maps.flatten())
                 return returns.flatten(), died.flatten()
         raise RuntimeError("evaluate_batched: some episodes did not finish")
 
@@ -701,7 +712,7 @@ class DQN:
         return loss
 
     def learn_batched(self, n_episodes, n_envs=1024, k_steps=16, replays_per_launch=None, batch_size=None, seed=0,
-                      replay_seed=None, checkpoint=None, time_limit=None):
+                      replay_seed=None, checkpoint=None, time_limit=None, record_maps=False):
         """``learn`` over ``n_envs`` CUDA environments at once: the envs act with the eps-greedy Q-network evaluated inside
         the step kernel (``rollout(policy="mlp")``, ``k_steps`` steps per launch), each rollout writes its packed
         observations straight into a device replay ring, and after every launch ``replays_per_launch`` (default
@@ -718,8 +729,12 @@ class DQN:
 
         Runs until ``n_episodes`` episodes have ended (over all envs, in order of their last step, then env) and logs those
         in the reference's format (``total_rewards``, ``agent_deaths``, ``n_episodes``, ``init_memories``,
-        ``total_time``; ``write_data``).  Per-episode ``maps`` and ``agent_pos`` are not recorded: the envs run on the
-        device and are not rendered.  One small device-to-host read per launch (rewards and done flags).
+        ``total_time``; ``write_data``).  One small device-to-host read per launch (rewards and done flags).
+        ``record_maps=True`` also keeps the reference's ``maps``, ``best_reward`` and ``agent_pos`` logs: every launch
+        captures the final state of each episode that ends (``rollout(finals=True)``), every logged episode goes through
+        ``_end_of_episode``'s map rule in the order it is logged, with the map string rendered from its final state, and
+        DQN / DQN_DUEL log each episode's start cell (the SARSA classes do not, as in ``learn``).  Capture is an output
+        only: trajectories, weights and the other logs are byte-identical to ``record_maps=False``.
         ``eps_per_launch`` / ``episodes_before_launch`` record the schedule.  Any grid: ``fit_batches_fused`` runs the
         replays in ``wf_replay_fit`` up to 32x32 and in ``wf_replay_fit_large`` on larger grids.  Returns the number of
         environment steps simulated.
@@ -732,6 +747,7 @@ class DQN:
         exactly where the run stopped, with byte-identical results, from a freshly built agent too: the model, target,
         optimiser state, ``_until_sync``, logs and eps schedule are overwritten from the file.  ``logs['total_time']`` is
         the sum of the calls' times."""
+        from . import _lib
         from .batched import BatchedForestFire
         from .constants import DQN_DEFAULTS as _D
         if time_limit is not None and checkpoint is None:
@@ -742,7 +758,8 @@ class DQN:
         B = int(self.METADATA["batch_size"] if batch_size is None else batch_size)
         rseed = int(seed if replay_seed is None else replay_seed)
         ckpt = _RunCheckpoint(checkpoint, _run_fingerprint("learn_batched", [self], n_episodes=n_episodes, n_envs=N, k_steps=K,
-                                                           replays_per_launch=R, batch_size=B, seed=seed, replay_seed=rseed))
+                                                           replays_per_launch=R, batch_size=B, seed=seed, replay_seed=rseed,
+                                                           **({"record_maps": True} if record_maps else {})))
         saved = ckpt.load()
         keys = {k: v for k, v in self.METADATA.items() if k not in _D and k not in ("debug", "a_speed_iter", "seed", "auto_reset")}
         env = BatchedForestFire(N, device=self.device, obs_dtype="bits", auto_reset=True, seed=seed, **keys)
@@ -756,6 +773,9 @@ class DQN:
         done_eps, elapsed = 0, 0.0
         try:
             ring = _PackedReplayRing(env, K, int(self.METADATA["memory_size"]), self.memory, self._SARSA)
+            if record_maps:
+                sc = env.get_state()["scalars"]
+                maplog = _MapLog(self, sc[:, _lib.S_AX:_lib.S_AY + 1].cpu().numpy())
             if saved is not None:
                 env.set_state(**saved["env"])
                 ring.load_state_dict(saved["ring"])
@@ -763,32 +783,40 @@ class DQN:
                 self._load_learner_state(saved["agent"])
                 carry, done_eps, elapsed = saved["carry"].numpy(), saved["done_eps"], saved["elapsed"]
                 rewards, deaths = saved["rewards"], saved["deaths"]
+                if record_maps:
+                    maplog.load(saved["maps"])
             while len(rewards) < n_episodes:
                 self.eps = self.min_eps + (self.max_eps - self.min_eps) * np.exp(-self.eps_decay_rate * done_eps)
                 self.eps_per_launch.append(float(self.eps))
                 self.episodes_before_launch.append(done_eps)
                 net = self.model
                 env.set_policy_mlp_dev(net.dense_1.weight, net.dense_1.bias, net.dense_2.weight, net.dense_2.bias, eps=self.eps)
-                rew, done = ring.launch()
+                rew, done = ring.launch(finals=record_maps)
                 if R > 0 and ring.n_sampleable > B:
                     self.fit_batches_fused(ring.frames, *ring.gather(ring.sample(R, B, gen)), R)
                 rd = torch.stack((rew, done.double())).cpu().numpy()
                 e_idx, k_idx, ret, carry = _episode_ends(carry, rd[0], rd[1] != 0)
                 order = np.lexsort((e_idx, k_idx))
+                at = _final_index(ring.finals) if record_maps else None
                 for i in order[: n_episodes - len(rewards)]:
+                    if record_maps:
+                        maplog.episode(len(rewards), float(ret[i]), e_idx[i], ring.finals, at, (int(k_idx[i]), int(e_idx[i])))
                     rewards.append(float(ret[i]))
                     deaths.append(bool(rd[0][k_idx[i], e_idx[i]] == death_penalty))
                 done_eps += len(e_idx)
                 if len(rewards) < n_episodes and time_limit is not None and time.time() - t_run >= time_limit:
                     ckpt.save(dict(env=_env_state(env), ring=ring.state_dict(), replay_generator=gen.get_state(),
                                    agent=self._learner_state(), carry=torch.from_numpy(carry), done_eps=done_eps,
-                                   rewards=rewards, deaths=deaths, elapsed=elapsed + time.time() - t_run))
+                                   rewards=rewards, deaths=deaths, elapsed=elapsed + time.time() - t_run,
+                                   **({"maps": maplog.state()} if record_maps else {})))
                     return None
             steps = ring.steps
         finally:
             env.close()
         self.logs["total_rewards"] = rewards
         self.logs["agent_deaths"] = deaths
+        if record_maps:
+            maplog.write(self)
         self.logs["total_time"] = round(elapsed + time.time() - t_run, 3)
         self.write_data()
         ckpt.remove()
@@ -880,11 +908,14 @@ class _PackedReplayRing:
         self.steps = 0
         self.frames[T * N:T * N + N] = env.reset()
 
-    def launch(self):
-        """One ``rollout(K, policy="mlp")`` into the next K slots; returns its rewards [K, N] and done flags [K, N]."""
+    def launch(self, finals=False):
+        """One ``rollout(K, policy="mlp")`` into the next K slots; returns its rewards [K, N] and done flags [K, N].
+        ``finals``: the launch also captures the final state of every episode that ends (``self.finals``)."""
         sl = slice(self.steps % self.T, self.steps % self.T + self.K)
-        _, _, _, chosen = self.env.rollout(self.K, policy="mlp", return_actions=True,
-                                           out=(self.ring[sl], self.rews[sl], self.dones[sl]))
+        res = self.env.rollout(self.K, policy="mlp", return_actions=True, out=(self.ring[sl], self.rews[sl], self.dones[sl]),
+                               finals=finals)
+        chosen = res[3]
+        self.finals = res[4] if finals else None
         self.acts[sl] = chosen
         self.steps += self.K
         return self.rews[sl], self.dones[sl]
@@ -1040,7 +1071,7 @@ _POPULATION_FREE_KEYS = ("alpha", "gamma", "target_update", "max_eps", "min_eps"
 
 
 def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replays_per_launch=None, batch_size=None, seed=0,
-                     checkpoint=None, time_limit=None):
+                     checkpoint=None, time_limit=None, record_maps=False):
     """``DQN.learn_batched`` for M = len(agents) independent learners (1 to 64) at once on one GPU, with one rollout launch
     and one ``wf_replay_fit_many`` launch per iteration for all of them.
 
@@ -1063,7 +1094,11 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
     ``checkpoint`` and ``time_limit`` work as in ``learn_batched``: the file holds the stacked model, target and Adam
     state, each learner's Adam step, sync phase, generator, episode accounting, logs and eps schedule, the env batch and
     the replay ring, and its fingerprint covers the number of agents and each agent's METADATA and demonstration count.
-    A stopped call returns None and writes no logs."""
+    A stopped call returns None and writes no logs.
+
+    ``record_maps=True``: every learner also keeps ``maps``, ``best_reward`` and ``agent_pos`` as ``learn_batched(...,
+    record_maps=True)`` does, equal to that run's byte for byte; the episodes of a learner that has finished are not
+    rendered."""
     from torch.nn.utils import parameters_to_vector
     from . import _lib
     from .batched import BatchedForestFire, _ptr
@@ -1095,7 +1130,8 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
     R = K if replays_per_launch is None else int(replays_per_launch)
     B = int(a0.METADATA["batch_size"] if batch_size is None else batch_size)
     ckpt = _RunCheckpoint(checkpoint, _run_fingerprint("learn_population", agents, n_episodes=n_episodes, envs_per_learner=G,
-                                                       k_steps=K, replays_per_launch=R, batch_size=B, seed=seed))
+                                                       k_steps=K, replays_per_launch=R, batch_size=B, seed=seed,
+                                                       **({"record_maps": True} if record_maps else {})))
     saved = ckpt.load()
     if a0.device.type != "cuda":
         raise _lib.WildfireError("learn_population needs a CUDA device (no CPU fallback)")
@@ -1128,6 +1164,9 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
     stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
     try:
         ring = _PackedReplayRing(env, K, int(a0.METADATA["memory_size"]), [a.memory for a in agents], sarsa, groups=M)
+        if record_maps:
+            starts = env.get_state()["scalars"][:, _lib.S_AX:_lib.S_AY + 1].cpu().numpy()
+            maplogs = [_MapLog(a, starts[j * G:(j + 1) * G]) for j, a in enumerate(agents)]
         if saved is not None:
             env.set_state(**saved["env"])
             ring.load_state_dict(saved["ring"])
@@ -1141,6 +1180,9 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
             rewards, deaths, elapsed = saved["rewards"], saved["deaths"], saved["elapsed"]
             for a, st in zip(agents, saved["agents"]):
                 _load_schedule_state(a, st)
+            if record_maps:
+                for ml, st in zip(maplogs, saved["maps"]):
+                    ml.load(st)
         while not all(finished):
             for j, a in enumerate(agents):
                 if not finished[j]:
@@ -1148,7 +1190,7 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
                     a.eps_per_launch.append(float(a.eps))
                     a.episodes_before_launch.append(done_eps[j])
             env.set_policy_mlp_flat_dev(P, hidden, dueling, [float(a.eps) for a in agents])
-            rew, done = ring.launch()
+            rew, done = ring.launch(finals=record_maps)
             fit = [j for j in range(M) if not finished[j] and R > 0 and ring.sampleable(j) > B]
             if fit:
                 keep, desc = [], (_lib.WfFitLearner * len(fit))()
@@ -1176,6 +1218,7 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
                     te = int(agents[j].target_update_freq)
                     until_sync[j] = (until_sync[j] - R - 1) % te + 1
             rd = torch.stack((rew, done.double())).cpu().numpy()
+            at = _final_index(ring.finals) if record_maps else None
             for j in range(M):
                 if finished[j]:
                     continue
@@ -1183,6 +1226,9 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
                 e_idx, k_idx, ret, carry[j] = _episode_ends(carry[j], rd[0][:, cols], rd[1][:, cols] != 0)
                 order = np.lexsort((e_idx, k_idx))
                 for i in order[: n_episodes - len(rewards[j])]:
+                    if record_maps:
+                        maplogs[j].episode(len(rewards[j]), float(ret[i]), e_idx[i], ring.finals, at,
+                                           (int(k_idx[i]), j * G + int(e_idx[i])))
                     rewards[j].append(float(ret[i]))
                     deaths[j].append(bool(rd[0][k_idx[i], j * G + e_idx[i]] == death_penalty))
                 done_eps[j] += len(e_idx)
@@ -1193,7 +1239,8 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
                                params=P.cpu(), target=Tg.cpu(), adam_m=Mm.cpu(), adam_v=Vv.cpu(), adam_t=adam_t,
                                until_sync=until_sync, carry=[torch.from_numpy(c) for c in carry], done_eps=done_eps,
                                steps=steps, finished=finished, rewards=rewards, deaths=deaths,
-                               agents=[_schedule_state(a) for a in agents], elapsed=elapsed + time.time() - t_run))
+                               agents=[_schedule_state(a) for a in agents], elapsed=elapsed + time.time() - t_run,
+                               **({"maps": [ml.state() for ml in maplogs]} if record_maps else {})))
                 return None
     finally:
         env.close()
@@ -1215,10 +1262,68 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
             a._until_sync = until_sync[j]
             a.logs["total_rewards"] = rewards[j]
             a.logs["agent_deaths"] = deaths[j]
+            if record_maps:
+                maplogs[j].write(a)
             a.logs["total_time"] = total_time
             a.write_data()
     ckpt.remove()
     return steps
+
+
+def _map_rule(maps, best_reward, episode, total_reward, render):
+    """The map log of DQN._end_of_episode (DQN.py:120-148): an episode whose return is at least 0.9 times the best so far,
+    or above 300, is rendered (``render()``) and appended to ``maps`` as [episode, map] (``maps`` None: not kept), and
+    raises the best return.  Returns the new best return."""
+    if total_reward >= 0.9 * best_reward or total_reward > 300:
+        map_string = render()
+        if total_reward > best_reward:
+            best_reward = total_reward
+        if maps is not None:
+            maps.append([episode, map_string])
+    return best_reward
+
+
+class _MapLog:
+    """``maps`` and ``agent_pos`` of one learner whose episodes run on the device (``record_maps=True``): the map rule of
+    ``_end_of_episode`` over the logged episodes, in the order they are logged, with the map strings rendered from the
+    step kernels' final-state records, and each logged episode's start cell (``agent_pos`` is kept only by the classes
+    whose ``learn`` keeps it, DQN and DQN_DUEL, and only with DEBUG > 0, as there).  ``starts``: [envs, 2] start cells of
+    the envs' running episodes."""
+
+    def __init__(self, agent, starts):
+        self.keep = agent.DEBUG > 0
+        self.with_pos = self.keep and not agent._SARSA
+        self.best = agent.logs["best_reward"]
+        self.maps, self.pos = [], []
+        self.starts = np.array(starts, dtype=np.int64).reshape(-1, 2)
+
+    def episode(self, index, ret, env, fin, at, key):
+        """Log episode number ``index`` (return ``ret``) of env ``env`` (local index), whose final state is the record of
+        ``fin`` that ``at = _final_index(fin)`` finds under ``key`` = (k, env)."""
+        i = at[0][key]
+        if self.with_pos:
+            self.pos.append((int(self.starts[env, 0]), int(self.starts[env, 1])))
+        self.starts[env] = at[1][i]
+        self.best = _map_rule(self.maps if self.keep else None, self.best, index, ret, lambda: fin.render(i))
+
+    def state(self):
+        return dict(best=self.best, maps=[list(m) for m in self.maps], pos=[list(p) for p in self.pos],
+                    starts=torch.from_numpy(self.starts.copy()))
+
+    def load(self, st):
+        self.best, self.maps = st["best"], [list(m) for m in st["maps"]]
+        self.pos = [tuple(p) for p in st["pos"]]
+        self.starts = st["starts"].numpy().copy()
+
+    def write(self, agent):
+        agent.logs["best_reward"] = self.best
+        agent.logs["maps"] = self.maps
+        agent.logs["agent_pos"] = self.pos
+
+
+def _final_index(fin):
+    """(k, env) -> record index of a ``FinalStates``, and its ``next_start`` on the host."""
+    return {key: i for i, key in enumerate(zip(fin.k.tolist(), fin.env.tolist()))}, fin.next_start.cpu().numpy()
 
 
 def _episode_ends(carry, rew, done):

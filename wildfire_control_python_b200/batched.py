@@ -16,7 +16,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .constants import make_metadata
+from .constants import ascii_of_type, make_metadata
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -95,6 +95,80 @@ def pack_obs(obs: torch.Tensor) -> torch.Tensor:
     shifts = torch.arange(32, device=obs.device, dtype=torch.int64)
     packed = (flat << shifts).sum(-1)  # < 2**32: the uint32 pattern; as int32 with the same bits
     return torch.where(packed >= 2**31, packed - 2**32, packed).to(torch.int32)
+
+
+class FinalStates:
+    """The final states of the episodes that ended in one ``step`` / ``rollout`` call (``finals=True``), one entry per
+    finished episode, sorted by ``(k, env)``: the state each env was in when it returned ``done`` at step ``k`` of the call,
+    before the auto-reset replaced it (the ``final_observation`` of an auto-reset vector env).
+
+    Written by the step kernels (``wf_set_final_capture``, include/wildfire.h) as one fixed-size record per episode.
+    Tensors on the env's device: ``k``, ``env``, ``episode`` (the finished episode's number) and ``t`` (its length in
+    steps) ``[F]`` int32; ``agent`` ``[F, 2]`` (final cell); ``alive``, ``visible``, ``dead``, ``digging`` ``[F]`` bool;
+    ``next_start`` ``[F, 2]``, the next episode's start cell (-1, -1 without auto_reset); ``obs``, the terminal observation
+    (``[F, words]`` bits rows for ``obs_dtype="bits"``, else ``[F, W, H, 3]`` of the env's dtype); ``records``, the raw
+    ``[F, words]`` int32 records."""
+
+    def __init__(self, records: torch.Tensor, width: int, height: int, obs_dtype=torch.uint8, n_envs: Optional[int] = None):
+        W, H = int(width), int(height)
+        self.width, self.height = W, H
+        hdr = records[:, :_lib.FINAL_HEADER_WORDS]
+        if records.shape[0] > 1:  # (k, env) order: the kernels' slot order is unspecified
+            n = int(n_envs) if n_envs is not None else int(hdr[:, _lib.F_ENV].max()) + 1
+            order = torch.argsort(hdr[:, _lib.F_K].long() * n + hdr[:, _lib.F_ENV].long())
+            records, hdr = records[order], hdr[order]
+        self.records = records
+        self.k, self.env = hdr[:, _lib.F_K], hdr[:, _lib.F_ENV]
+        self.episode, self.t = hdr[:, _lib.F_EPISODE], hdr[:, _lib.F_T]
+        self.agent = hdr[:, _lib.F_AX:_lib.F_AY + 1]
+        flags = hdr[:, _lib.F_FLAGS]
+        self.alive = (flags & _lib.FINAL_ALIVE) != 0
+        self.visible = (flags & _lib.FINAL_VISIBLE) != 0
+        self.dead = (flags & _lib.FINAL_DEAD) != 0
+        self.digging = (flags & _lib.FINAL_DIGGING) != 0
+        self.next_start = hdr[:, _lib.F_NEXT_AX:_lib.F_NEXT_AY + 1]
+        ow = _lib.obs_bits_words(W, H)
+        bits = records[:, _lib.FINAL_OBS:_lib.FINAL_OBS + ow]
+        if obs_dtype == "bits":
+            self.obs = bits
+        elif records.shape[0] == 0:
+            self.obs = torch.empty((0, W, H, 3), dtype=obs_dtype, device=records.device)
+        else:
+            self.obs = unpack_obs(bits.contiguous(), W, H, dtype=obs_dtype)
+        self._types = None
+        self._host = None
+
+    def __len__(self) -> int:
+        return int(self.records.shape[0])
+
+    def planes(self) -> torch.Tensor:
+        """``[F, 4, W, H]`` bool: the fire, burnt, dirt and water planes of every record (grass is none of them)."""
+        W, H = self.width, self.height
+        pw, po = _lib.final_plane_words(W, H), _lib.final_plane_offset(W, H)
+        words = self.records[:, po:po + 4 * pw].reshape(-1, 4, pw)
+        shifts = torch.arange(32, device=words.device, dtype=torch.int32)
+        bits = (words.unsqueeze(-1) >> shifts) & 1  # (an arithmetic shift of the sign bit is masked away)
+        return bits.reshape(-1, 4, pw * 32)[:, :, :W * H].reshape(-1, 4, W, H).bool()
+
+    def types(self) -> torch.Tensor:
+        """``[F, W, H]`` uint8 cell types (``WF_GRASS`` 0, fire 1, burnt 2, dirt 3, water 4), computed on the device."""
+        if self._types is None:
+            p = self.planes().to(torch.uint8)
+            code = torch.tensor([1, 2, 3, 4], dtype=torch.uint8, device=p.device).view(1, 4, 1, 1)
+            self._types = (p * code).sum(1, dtype=torch.uint8)
+        return self._types
+
+    def render(self, i: int) -> str:
+        """Record ``i`` as the string ``ForestFire.render(print_map=False)`` returns for that state (forest_fire.py:57-82):
+        '+' grass, '@' fire, '#' burnt, '0' dirt, 'x' water, 'A' the agent while it is alive."""
+        if self._host is None:  # one device-to-host copy for all the records
+            self._host = (self.types().cpu().numpy(), self.agent.cpu().numpy(), self.alive.cpu().numpy())
+        types, agent, alive = self._host
+        t, (ax, ay), alive = types[i], (int(v) for v in agent[i]), bool(alive[i])
+        rows = []
+        for y in range(self.height):
+            rows.append("".join("A" if alive and (x, y) == (ax, ay) else ascii_of_type[int(t[x, y])] for x in range(self.width)))
+        return "\n" + "\n".join(rows) + "\n"
 
 
 class BatchedForestFire:
@@ -210,13 +284,20 @@ class BatchedForestFire:
             _lib.check(_lib.lib().wf_reset(self._h, _ptr(m), _ptr(s), _ptr(self._obs), self._obs_code, self._stream()))
         return self._obs
 
-    def step(self, actions):
+    def step(self, actions, finals: bool = False, finals_capacity: Optional[int] = None):
         """``ForestFire.step(action)`` (forest_fire.py:30-49) for the whole batch.
 
         ``actions``: ``[N]`` ints, 0..3 = N,S,E,W; 4 = dig toggle iff ``allow_dig_toggle``; other = no-op.
         Returns ``(obs [N,W,H,3], reward float64 [N], done bool [N], {})``.  The returned tensors are
         the handle's persistent buffers (overwritten by the next call).
+        ``finals=True``: the info dict holds ``"final"``, the ``FinalStates`` of the envs that returned done (as ``rollout``).
         """
+        if finals:
+            a = self._as_i32(actions, (self.n_envs,))
+            with torch.cuda.device(self.device), self._capture(1, finals_capacity) as cap:
+                _lib.check(self._wf_step(self._h, a.data_ptr(), self._obs_ptr, self._obs_code, self._reward_ptr, self._done_ptr,
+                                         torch.cuda.current_stream(self.device).cuda_stream))
+            return self._obs, self._reward, self._done_bool, {"final": cap.result}
         a = self._as_i32(actions, (self.n_envs,))
         rc = self._wf_step(self._h, a.data_ptr(), self._obs_ptr, self._obs_code, self._reward_ptr, self._done_ptr,
                            torch.cuda.current_stream(self.device).cuda_stream)
@@ -225,7 +306,7 @@ class BatchedForestFire:
         return self._obs, self._reward, self._done_bool, {}
 
     def rollout(self, k_steps: int, actions=None, obs: bool = True, out=None, policy: str = "stream",
-                return_actions: bool = False):
+                return_actions: bool = False, finals: bool = False, finals_capacity: Optional[int] = None):
         """``k_steps`` consecutive ``step`` calls in one launch (state stays on chip in between).
 
         ``actions``: ``[K, N]`` ints, or ``None`` = chosen on the device by ``policy``:
@@ -236,7 +317,18 @@ class BatchedForestFire:
         ``out``: optional ``(obs_or_None, reward, done_u8)`` buffers to write into.
         Returns ``(obs [K,N,W,H,3] or None, reward [K,N], done [K,N])`` (+ ``actions [K,N]`` if asked);
         with ``obs_dtype="bits"`` obs is ``[K, N, words]`` int32.
+        ``finals=True``: a ``FinalStates`` of every episode that ended during the call is appended to the tuple.  The step
+        kernels write one record per finished episode before the auto-reset; ``finals_capacity`` records fit (default
+        ``N * K``, enough for every env ending at every step) and a call in which more episodes ended raises
+        ``WildfireError``.  Without ``finals`` the same kernels as ever run.  Memory: the call allocates ``finals_capacity``
+        records of ``final_record_words(W, H) * 4`` bytes (about W*H*2 bytes each: 256 B at 14x14, 57 KB at 256x256, so the
+        default is 3.7 GB for 1024 envs of 256x256 and K = 64; pass a smaller ``finals_capacity`` where few episodes end),
+        and reading the record count synchronises the stream.
         """
+        if finals:
+            with self._capture(k_steps, finals_capacity) as cap:
+                res = self.rollout(k_steps, actions, obs, out, policy, return_actions)
+            return (*res, cap.result)
         K, N = int(k_steps), self.n_envs
         a = None if actions is None else self._as_i32(actions, (K, N))
         pol = {"stream": _lib.WF_POLICY_STREAM, "walk": _lib.WF_POLICY_WALK, "mlp": _lib.WF_POLICY_MLP}[policy]
@@ -261,6 +353,34 @@ class BatchedForestFire:
         if return_actions:
             return o, r, d.view(torch.bool), chosen
         return o, r, d.view(torch.bool)
+
+    def _capture(self, k_steps: int, capacity: Optional[int]):
+        """Context of one call with final-state capture on (``wf_set_final_capture``); ``.result`` afterwards."""
+        env = self
+        cap_n = env.n_envs * int(k_steps) if capacity is None else int(capacity)
+        if cap_n < 0:
+            raise ValueError("finals_capacity must be >= 0")
+
+        class _Cap:
+            def __enter__(self):
+                words = _lib.final_record_words(env.width, env.height)
+                with torch.cuda.device(env.device):
+                    self.buf = torch.empty((max(cap_n, 1), words), dtype=torch.int32, device=env.device)
+                    self.count = torch.zeros((1,), dtype=torch.int32, device=env.device)
+                _lib.check(_lib.lib().wf_set_final_capture(env._h, _ptr(self.buf), cap_n, _ptr(self.count)))
+                return self
+
+            def __exit__(self, exc_type, exc, tb):
+                _lib.check(_lib.lib().wf_set_final_capture(env._h, None, 0, None))
+                if exc_type is not None:
+                    return False
+                n = int(self.count.item()) & 0xFFFFFFFF
+                if n > cap_n:
+                    raise _lib.WildfireError(f"{n} episodes ended in this call but finals_capacity is {cap_n}")
+                self.result = FinalStates(self.buf[:n], env.width, env.height, env.obs_dtype, env.n_envs)
+                return False
+
+        return _Cap()
 
     def set_policy_mlp(self, kernel1, bias1, kernel2, bias2, eps: float = 0.0):
         """Weights of the in-kernel Q-network (``rollout(policy="mlp")``): Keras orientation, ``kernel1``

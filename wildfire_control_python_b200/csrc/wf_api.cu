@@ -81,6 +81,7 @@ struct wf_env {
     float* mlp_dev;      // WF_POLICY_MLP weights: per network w1 | base | w2 | b2 | threshold
     int32_t mlp_cap;     // network blocks mlp_dev holds
     MlpPolicy mlp;       // device pointers into mlp_dev (hid == 0: not set)
+    FinalCapture fin;    // wf_set_final_capture (records == nullptr: off)
     // wf_step_host staging
     cudaStream_t hstream;
     // wf_step_host runs on its own stream: it is ordered behind everything the caller queued through the *_dev entry
@@ -713,13 +714,13 @@ static int rollout_impl(wf_env* e, int32_t k_steps, const int32_t* actions_dev, 
     if (e->tile) {  // one thread-block cluster per env runs all K steps in one launch
         TileIO io{actions_dev, obs_dev, reward_dev, done_dev, nullptr, nullptr, obs_dtype, k_steps, e->a_iter, 0, policy,
                   actions_out, e->mlp};
-        WF_CUDA(launch_tile_family(e->tstate, e->st, e->sc, io, st, &e->launches));
+        WF_CUDA(launch_tile_family(e->tstate, e->st, e->sc, io, st, &e->launches, &e->fin));
         e->a_iter = advance_a_iter(e, k_steps);
         return WF_OK;
     }
     WarpIO io{actions_dev, obs_dev, reward_dev, done_dev, nullptr, nullptr, obs_dtype, k_steps, e->a_iter, 0,
               magic_for(e->st.H), policy, actions_out, e->mlp};
-    WF_CUDA(launch_warp_family(e->st, e->sc, io, st));
+    WF_CUDA(launch_warp_family(e->st, e->sc, io, st, &e->fin));
     e->launches += 1;
     e->a_iter = advance_a_iter(e, k_steps);
     return WF_OK;
@@ -868,6 +869,31 @@ int wf_set_policy_mlp_nets_dev(wf_env* e, const wf_mlp_shape* shape, int32_t n_n
     const float* b2 = w2 + (size_t)A * hid;
     if (int rc = pack_policy_nets(e, n_nets, w1, b1, w2, b2, P, hid, eps_host, stream)) return rc;
     e->mlp.group_envs = group;
+    return WF_OK;
+}
+
+int64_t wf_final_record_words(int32_t width, int32_t height) {
+    if (width < 1 || height < 1) return 0;
+    return final_record_words(width, height);
+}
+
+int wf_set_final_capture(wf_env* e, uint32_t* records_dev, int64_t capacity, uint32_t* count_dev) {
+    if (!e) return fail(WF_ERR_INVALID, "null handle");
+    if (!records_dev) {
+        e->fin = FinalCapture{};
+        return WF_OK;
+    }
+    if (!count_dev) return fail(WF_ERR_INVALID, "wf_set_final_capture: count_dev is null");
+    if (capacity < 0) return fail(WF_ERR_INVALID, "wf_set_final_capture: capacity must be >= 0");
+    if (reinterpret_cast<uintptr_t>(records_dev) & 15u) return fail(WF_ERR_INVALID, "wf_set_final_capture: records must be 16-byte aligned");
+    if (reinterpret_cast<uintptr_t>(count_dev) & 3u) return fail(WF_ERR_INVALID, "wf_set_final_capture: count must be 4-byte aligned");
+    WF_ON_DEVICE(e);
+    WF_QUIESCE(e);  // a resident step server is parked first: it has no capture
+    e->fin.records = records_dev;
+    e->fin.count = count_dev;
+    e->fin.capacity = capacity;
+    e->fin.words = final_record_words(e->cfg.width, e->cfg.height);
+    e->fin.plane_off = final_plane_offset(e->cfg.width, e->cfg.height);
     return WF_OK;
 }
 
@@ -1135,6 +1161,7 @@ int wf_host_session(wf_env* e, int32_t on) {
     WF_ON_DEVICE(e);
     if (on) {
         if (e->tile) return fail(WF_ERR_INVALID, "wf_host_session: grids up to 32x32 (warp family) only");
+        if (e->fin.records) return fail(WF_ERR_STATE, "wf_host_session: final-state capture is on (wf_set_final_capture)");
         int coop = 0;
         WF_CUDA(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, e->device));
         if (!coop) return fail(WF_ERR_INVALID, "wf_host_session: the device has no cooperative launch");
@@ -1156,6 +1183,7 @@ int wf_step_host(wf_env* e, const int32_t* actions_host, void* obs_host, int32_t
                  uint8_t* done_host) {
     if (!e || !actions_host) return fail(WF_ERR_INVALID, "null argument");
     if (!public_obs_dtype(obs_dtype)) return fail(WF_ERR_INVALID, "bad obs_dtype");
+    if (e->fin.records) return fail(WF_ERR_STATE, "wf_step_host: final-state capture is on (wf_set_final_capture)");
     WF_ON_DEVICE(e);
     const DevState& s = e->st;
     const size_t obs_bytes = obs_step_bytes(s.N, s.W, s.H, obs_dtype);

@@ -46,6 +46,20 @@ struct SrvCtl {
                                   // barrier (the slowest warp), 3 steps, 4 fence + arrival
 };
 
+// Final-state capture (wf_set_final_capture): one record per finished episode, layout in include/wildfire.h.
+struct FinalCapture {
+    uint32_t* records;   // [capacity][words], or nullptr: capture off
+    uint32_t* count;     // slots taken (records past capacity are counted, not written)
+    int64_t capacity;
+    int32_t words;       // wf_final_record_words(W, H)
+    int32_t plane_off;   // first word of the fire plane within a record
+};
+__host__ __device__ inline int32_t final_plane_words(int W, int H) { return (W * H + 31) / 32; }
+__host__ __device__ inline int32_t final_plane_offset(int W, int H) { return WF_FINAL_OBS + ((W * H * 3 + 31) / 32 + 3) / 4 * 4; }
+__host__ __device__ inline int32_t final_record_words(int W, int H) {
+    return (final_plane_offset(W, H) + 4 * final_plane_words(W, H) + 3) / 4 * 4;
+}
+
 struct WarpIO {
     const int32_t* actions;  // [K][N] or nullptr (ACTION stream)
     void* obs;               // [K][N][W][H][3] or nullptr
@@ -59,7 +73,13 @@ struct WarpIO {
     int32_t* actions_out;    // [K][N] or nullptr: the actions the policy chose
     MlpPolicy mlp;           // WF_POLICY_MLP only
 };
-cudaError_t launch_warp_family(const DevState& s, const StepCfg& c, const WarpIO& io, cudaStream_t stream);
+// fin: final-state capture (nullptr or records == nullptr: off); a separate kernel argument, so that the kernels without
+// capture keep their parameters and code.
+struct WarpFinIO : WarpIO {  // the kernel argument of the warp family's capture kernels
+    FinalCapture fin;
+};
+cudaError_t launch_warp_family(const DevState& s, const StepCfg& c, const WarpIO& io, cudaStream_t stream,
+                               const FinalCapture* fin = nullptr);
 // The same kernel as a cooperative launch (every CTA resident) that serves steps until told to park; io.actions / io.obs
 // are mapped host buffers (obs_dtype kObsPackedStatus).  cudaErrorCooperativeLaunchTooLarge if the batch does not fit.
 cudaError_t launch_warp_server(const DevState& s, const StepCfg& c, const WarpIO& io, const SrvCtl& srv, cudaStream_t stream);
@@ -82,7 +102,7 @@ cudaError_t tile_create(TileState** out, const DevState& s, const StepCfg& c);
 void tile_destroy(TileState* t);
 void tile_geometry(const TileState* t, int32_t* threads, int32_t* cluster);
 cudaError_t launch_tile_family(TileState* t, const DevState& s, const StepCfg& c, const TileIO& io,
-                               cudaStream_t stream, int64_t* launches);
+                               cudaStream_t stream, int64_t* launches, const FinalCapture* fin = nullptr);
 cudaError_t tile_after_set_state(TileState* t, const DevState& s, const StepCfg& c, cudaStream_t stream,
                                  int64_t* launches);
 

@@ -875,6 +875,8 @@ __device__ __forceinline__ void expand_stream_float(void* obs_step, int obs_dtyp
 // 512 contiguous bytes.  2 plane words in, 96 bytes out per word.
 // ctr (optional, shared, zeroed by the caller): the warps take their 128-word groups from this counter instead of
 // a fixed stride, so that a warp that starts late (warp 0 runs the next step's agent phase first) does less.
+// ROW (WF_OBS_BITS only): obs_step is the env's own row (a final-state record's observation), not an [N][words] block.
+template <bool ROW = false>
 __device__ __forceinline__ void emit_obs_slice(const Env& e, void* obs_step, int obs_dtype, const uint32_t* spread3,
                                                const uint2* tab8, uint32_t* stage_all, int vis, int ax, int ay, int* ctr = nullptr) {
     const int W = e.W, H = e.H, HW = e.HW;
@@ -888,7 +890,7 @@ __device__ __forceinline__ void emit_obs_slice(const Env& e, void* obs_step, int
     uint32_t* stage = stage_all + warp * ((HW & 3) == 0 ? 384 : 96);  // 32 words x 96 bits
     const uint16_t* stage16 = reinterpret_cast<const uint16_t*>(stage);
     // WF_OBS_BITS: the env's words.  With H % 32 == 0 word i's 96-bit stream is exactly output words 3i .. 3i+2.
-    uint32_t* const obits = static_cast<uint32_t*>(obs_step) + (size_t)e.env * obs_bits_words(W, H);
+    uint32_t* const obits = static_cast<uint32_t*>(obs_step) + (ROW ? (size_t)0 : (size_t)e.env * obs_bits_words(W, H));
     int g_first = e.lo;
     if ((H & 31) == 0 && (HW & 3) == 0) {
         // One instantiation per element type, so that the loop carries no per-iteration test of it.
@@ -1192,14 +1194,80 @@ __device__ void reset_env(const Env& e, const DevState& s, const StepCfg& c, con
 }
 
 // ---------------------------------------------------------------------------------------------
+// Final-state capture (`fin`, wf_set_final_capture): the record of this cluster's env, whose episode ended at step k, taken before the
+// auto-reset.  Whole cluster: rank 0 takes the slot and hands it to every CTA; each CTA writes the terminal observation of
+// its slice and its share of the type planes' words (gathered from any row: nothing writes a plane until the closing
+// barrier).  fin_sh[1] receives the slot.
+template <bool CL>
+__device__ void capture_final(const Env& e, const FinalCapture& fin, int k, const int32_t* sc, int32_t* fin_sh, const uint32_t* spread3,
+                              const uint2* tab8, uint32_t* qmem, int ovis, int oax, int oay) {
+    if (e.rank == 0 && e.tid == 0) {
+        const int slot = (int)atomicAdd(fin.count, 1u);
+        if (CL) {
+            for (int r = 0; r < e.CS; ++r) st_shared_cluster(&fin_sh[1], (uint32_t)r, slot);
+        } else {
+            fin_sh[1] = slot;
+        }
+    }
+    sync_env<CL>();
+    const uint32_t slot = (uint32_t)fin_sh[1];
+    if ((int64_t)slot < fin.capacity) {
+        uint32_t* const rec = fin.records + (size_t)slot * fin.words;
+        const int W = e.W, H = e.H, HW = e.HW;
+        if (e.rank == 0 && e.tid < WF_FINAL_HEADER_WORDS) {
+            const int i = e.tid;
+            const int flags = (sc[WF_S_ALIVE] ? WF_FINAL_ALIVE : 0) | (sc[WF_S_VISIBLE] ? WF_FINAL_VISIBLE : 0) |
+                              (sc[WF_S_DEAD] ? WF_FINAL_DEAD : 0) | (sc[WF_S_DIGGING] ? WF_FINAL_DIGGING : 0);
+            const int v = i == WF_F_K ? k : i == WF_F_ENV ? e.env : i == WF_F_EPISODE ? sc[WF_S_EPISODE] : i == WF_F_T ? sc[WF_S_T]
+                        : i == WF_F_AX ? sc[WF_S_AX] : i == WF_F_AY ? sc[WF_S_AY] : i == WF_F_FLAGS ? flags
+                        : (i == WF_F_NEXT_AX || i == WF_F_NEXT_AY) ? -1 : 0;
+            rec[i] = (uint32_t)v;
+        }
+        if (e.rank == 0) {  // the padding words after the observation and after the planes
+            const int pad0 = WF_FINAL_OBS + obs_bits_words(W, H), pad1 = fin.plane_off + 4 * final_plane_words(W, H);
+            for (int i = e.tid; i < (fin.plane_off - pad0) + (fin.words - pad1); i += e.T)
+                rec[i < fin.plane_off - pad0 ? pad0 + i : pad1 + i - (fin.plane_off - pad0)] = 0u;
+        }
+        // the terminal observation, straight into the record's row
+        emit_obs_slice<true>(e, rec + WF_FINAL_OBS, WF_OBS_BITS, spread3, tab8, qmem, ovis, oax, oay);
+        // the type planes: word j of a plane holds cells 32j .. 32j + 31 in x*H + y order
+        const int pw = final_plane_words(W, H), per = (pw + e.CS - 1) / e.CS;
+        const int j0 = min(pw, e.rank * per), nj = min(pw, j0 + per) - j0;
+        const int src[4] = {P_F, P_BT, P_D, P_WT};
+        for (int q = e.tid; q < 4 * nj; q += e.T) {
+            const int p = q / nj, j = j0 + q - p * nj;
+            const uint32_t* P = e.plane(src[p]);
+            const int cend = min(32 * j + 32, W * H);
+            uint32_t v = 0u;
+            for (int cell = 32 * j; cell < cend;) {
+                const int x = cell / H, y = cell - x * H;
+                const int n = min(min(cend - cell, H - y), 32);
+                const int wi = x * HW + (y >> 5), sh = y & 31;
+                const uint32_t hi = (sh != 0 && (y >> 5) + 1 < HW) ? P[wi + 1] : 0u;
+                uint32_t bits = __funnelshift_r(P[wi], hi, sh);
+                if (n < 32) bits &= (1u << n) - 1u;
+                v |= bits << (cell - 32 * j);
+                cell += n;
+            }
+            rec[fin.plane_off + p * pw + j] = v;
+        }
+    }
+    sync_env<CL>();
+}
+
+// Shared words of the capture kernels only (a kernel that never calls this has none).
+__device__ __forceinline__ int32_t* fin_shared() {
+    __shared__ int32_t v[2];
+    return v;
+}
+
+// ---------------------------------------------------------------------------------------------
 // K x ForestFire.step (forest_fire.py:30-49) or ForestFire.reset of one env per cluster.
-// MLP: WF_POLICY_MLP steps (no reset mode, no action array).
-template <int FB, int VW, bool CL, bool MLP>
-#ifndef WF_TILE_MAXT
-#define WF_TILE_MAXT 512
-#define WF_TILE_MINB 2
-#endif
-__global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kernel(DevState s, StepCfg c, TilePar t, TileIO io) {
+// MLP: WF_POLICY_MLP steps (no reset mode, no action array).  FIN: final-state capture (tile_fin_kernel only).
+// tid_x: threadIdx.x, read in the kernel itself (where __launch_bounds__ bounds its range).
+template <int FB, int VW, bool CL, bool MLP, bool FIN>
+__device__ __forceinline__ void tile_body(const DevState& s, const StepCfg& c, const TilePar& t, const TileIO& io, int tid_x,
+                                          const FinalCapture& fin = FinalCapture{}) {
     extern __shared__ uint32_t qmem[];  // per-warp active-word queues (7 x 32 * VW words each); observation staging
     __shared__ int32_t sc[WF_NSCALARS];
     __shared__ int red[kRed];
@@ -1207,9 +1275,10 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
     __shared__ StepShared ss;
     __shared__ uint32_t spread3[256];  // bit i of the index -> bit 3i
     __shared__ uint2 tab8[256];        // bit i of the index -> byte i
+    int32_t* const fin_sh = FIN ? fin_shared() : nullptr;  // FIN: the step ended the episode; the record's slot
 
     Env e;
-    e.tid = threadIdx.x; e.T = t.T;
+    e.tid = tid_x; e.T = t.T;
     e.CS = CL ? (int)cluster_nctarank() : 1;
     e.rank = CL ? (int)cluster_ctarank() : 0;
     e.env = CL ? (int)cluster_id_x() : (int)blockIdx.x;
@@ -1306,6 +1375,7 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
                 if (io.done) io.done[(size_t)k * s.N + e.env] = is_done ? 1 : 0;
             }
             ss.reset_now = c.auto_reset && is_done;
+            if (FIN) fin_sh[0] = is_done;
         };
         // Per step: barrier X -> tick -> CTA barrier -> the partial sums go to the peers and every thread ARRIVES at cluster
         // barrier Y; warp 0 waits for it, adds the totals up, and thread 0 does finish + the agent phase of the next step,
@@ -1386,6 +1456,7 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
                     }
                     ss.reset_now = 0;
                     ss.slow = 0;
+                    if (FIN) fin_sh[0] = 0;
                     if (!MLP && k + 1 < io.K) agent_phase<false>(e, c, t, io, s, k + 1, do_tick, sc, ss, writer);
                 }
                 WF_TSTAMP(3);
@@ -1394,9 +1465,17 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
                 __syncthreads();
                 WF_TSTAMP(5);
             }
+            if constexpr (FIN) {
+                if (fin_sh[0]) capture_final<CL>(e, fin, k, sc, fin_sh, spread3, tab8, qmem, ovis, oax, oay);
+            }
             const bool late_agent = act && (ss.slow || ss.reset_now);
             if (ss.reset_now) {
                 reset_env<FB, CL>(e, s, c, t, nullptr, sc, ss, red, xch, par);
+                if (FIN && writer && tid == 0 && fin_sh[0] && (int64_t)(uint32_t)fin_sh[1] < fin.capacity) {  // the next start
+                    uint32_t* const rec = fin.records + (size_t)(uint32_t)fin_sh[1] * fin.words;
+                    rec[WF_F_NEXT_AX] = (uint32_t)sc[WF_S_AX];
+                    rec[WF_F_NEXT_AY] = (uint32_t)sc[WF_S_AY];
+                }
                 if (tid == 0) ss.obs_ctr = 0;
                 __syncthreads();
                 if (obs_k != nullptr)  // the new episode's first observation replaces the speculative one
@@ -1418,6 +1497,20 @@ __global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kerne
     __syncthreads();
     if (writer && tid < WF_NSCALARS) s.scal[(size_t)e.env * WF_NSCALARS + tid] = sc[tid];
     if (writer && tid < ST_N && ss.stat[tid]) atomicAdd(&s.stats[tid], (unsigned long long)ss.stat[tid]);
+}
+
+#ifndef WF_TILE_MAXT
+#define WF_TILE_MAXT 512
+#define WF_TILE_MINB 2
+#endif
+template <int FB, int VW, bool CL, bool MLP>
+__global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_rollout_kernel(DevState s, StepCfg c, TilePar t, TileIO io) {
+    tile_body<FB, VW, CL, MLP, false>(s, c, t, io, threadIdx.x);
+}
+// The same with final-state capture (wf_set_final_capture): a kernel of its own, so that tile_rollout_kernel keeps its code.
+template <int FB, int VW, bool CL, bool MLP>
+__global__ void __launch_bounds__(WF_TILE_MAXT, WF_TILE_MINB) tile_fin_kernel(DevState s, StepCfg c, TilePar t, TileIO io, FinalCapture fin) {
+    tile_body<FB, VW, CL, MLP, true>(s, c, t, io, threadIdx.x, fin);
 }
 
 // S := B & (fuel >= 2) in the env's current source plane, R re-flooded, n_burning recounted
@@ -1487,13 +1580,18 @@ static void choose_geometry(const DevState& s, int& T, int& CS) {
     if (cs_env == 1 || cs_env == 2 || cs_env == 4 || cs_env == 8 || cs_env == 16) CS = cs_env;
 }
 
-template <int FB, int VW, bool CL, bool MLP>
-static cudaError_t set_smem_attr() {
-    if (CL) {
-        cudaError_t e = cudaFuncSetAttribute(tile_rollout_kernel<FB, VW, CL, MLP>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+template <typename Kernel>
+static cudaError_t set_smem_attr_of(Kernel k, bool cl) {
+    if (cl) {
+        cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
         if (e != cudaSuccess) return e;
     }
-    return cudaFuncSetAttribute(tile_rollout_kernel<FB, VW, CL, MLP>, cudaFuncAttributeMaxDynamicSharedMemorySize, 512 * 4 * 28);
+    return cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 512 * 4 * 28);
+}
+template <int FB, int VW, bool CL, bool MLP>
+static cudaError_t set_smem_attr() {
+    cudaError_t e = set_smem_attr_of(tile_rollout_kernel<FB, VW, CL, MLP>, CL);
+    return e == cudaSuccess ? set_smem_attr_of(tile_fin_kernel<FB, VW, CL, MLP>, CL) : e;
 }
 template <bool MLP>
 static cudaError_t set_smem_attrs() {
@@ -1570,11 +1668,14 @@ static TilePar make_par(const TileState* t, const DevState& s, int obs_dtype) {
 }
 
 template <int FB, int VW, bool MLP>
-static cudaError_t launch(const TileState* t, const DevState& s, const StepCfg& c, const TileIO& io, cudaStream_t st) {
+static cudaError_t launch(const TileState* t, const DevState& s, const StepCfg& c, const TileIO& io, cudaStream_t st,
+                          const FinalCapture* fin) {
     const TilePar p = make_par(t, s, io.obs_dtype);
     const size_t smem = (size_t)t->T * VW * 28;  // per warp: 7 queue arrays of 32 * VW words (reused as observation staging)
+    const bool capture = fin != nullptr && fin->records != nullptr && !io.reset_mode;
     if (t->CS == 1) {
-        tile_rollout_kernel<FB, VW, false, MLP><<<s.N, t->T, smem, st>>>(s, c, p, io);
+        if (capture) tile_fin_kernel<FB, VW, false, MLP><<<s.N, t->T, smem, st>>>(s, c, p, io, *fin);
+        else tile_rollout_kernel<FB, VW, false, MLP><<<s.N, t->T, smem, st>>>(s, c, p, io);
         return cudaGetLastError();
     }
     cudaLaunchConfig_t cfg = {};
@@ -1596,21 +1697,23 @@ static cudaError_t launch(const TileState* t, const DevState& s, const StepCfg& 
             fprintf(stderr, "wf_tile: %d clusters of %d x %d threads in the grid, %d resident at once\n", s.N, t->CS, t->T, nc);
         said = true;
     }
+    if (capture) return cudaLaunchKernelEx(&cfg, tile_fin_kernel<FB, VW, true, MLP>, s, c, p, io, *fin);
     return cudaLaunchKernelEx(&cfg, tile_rollout_kernel<FB, VW, true, MLP>, s, c, p, io);
 }
 
 template <bool MLP>
-static cudaError_t launch_fb_vw(const TileState* t, const DevState& s, const StepCfg& c, const TileIO& io, cudaStream_t st) {
+static cudaError_t launch_fb_vw(const TileState* t, const DevState& s, const StepCfg& c, const TileIO& io, cudaStream_t st,
+                                const FinalCapture* fin) {
     const bool v4 = (s.HW % 4 == 0);
-    if (s.FB == 5) return v4 ? launch<5, 4, MLP>(t, s, c, io, st) : launch<5, 1, MLP>(t, s, c, io, st);
-    return v4 ? launch<8, 4, MLP>(t, s, c, io, st) : launch<8, 1, MLP>(t, s, c, io, st);
+    if (s.FB == 5) return v4 ? launch<5, 4, MLP>(t, s, c, io, st, fin) : launch<5, 1, MLP>(t, s, c, io, st, fin);
+    return v4 ? launch<8, 4, MLP>(t, s, c, io, st, fin) : launch<8, 1, MLP>(t, s, c, io, st, fin);
 }
 
 cudaError_t launch_tile_family(TileState* t, const DevState& s, const StepCfg& c, const TileIO& io,
-                               cudaStream_t stream, int64_t* launches) {
+                               cudaStream_t stream, int64_t* launches, const FinalCapture* fin) {
     *launches += 1;
-    if (io.policy == WF_POLICY_MLP && io.actions == nullptr && !io.reset_mode) return launch_fb_vw<true>(t, s, c, io, stream);
-    return launch_fb_vw<false>(t, s, c, io, stream);
+    if (io.policy == WF_POLICY_MLP && io.actions == nullptr && !io.reset_mode) return launch_fb_vw<true>(t, s, c, io, stream, fin);
+    return launch_fb_vw<false>(t, s, c, io, stream, fin);
 }
 
 #ifdef WF_TILE_TIMING

@@ -261,6 +261,81 @@ __device__ __forceinline__ void emit_obs(void* obs_step, int dtype, uint32_t aro
     }
 }
 
+// Final-state capture: one section of the records of the warp's envs.  Row x's `nrow` bits (r0, then r1, r2) belong at
+// bit x * nrow of env `sub`'s section, which is `nw` words long and starts on a word boundary; the warp assembles the
+// sections in its stream buffer and stores env e's to dst[e] (nullptr: that env writes no record).
+template <int L>
+__device__ __forceinline__ void fin_section(uint32_t* stream, int lane, int sub, int x, int W, int nrow, int nw, uint32_t r0,
+                                            uint32_t r1, uint32_t r2, uint32_t* dst0, uint32_t* dst1) {
+    constexpr int EPW = 32 / L;
+    __syncwarp();
+    for (int i = lane; i < kStreamWords; i += 32) stream[i] = 0u;
+    __syncwarp();
+    if (x < W) {
+        const int start = sub * nw * 32 + x * nrow, w0 = start >> 5, sh = start & 31;
+        atomicOr(&stream[w0], r0 << sh);
+        if (sh + nrow > 32) atomicOr(&stream[w0 + 1], __funnelshift_l(r0, r1, sh));
+        if (sh + nrow > 64) atomicOr(&stream[w0 + 2], __funnelshift_l(r1, r2, sh));
+        if (sh + nrow > 96) atomicOr(&stream[w0 + 3], __funnelshift_l(r2, 0u, sh));
+    }
+    __syncwarp();
+    for (int w = lane; w < EPW * nw; w += 32) {
+        const int e = w >= nw ? 1 : 0;
+        uint32_t* d = e ? dst1 : dst0;
+        if (d != nullptr) d[w - e * nw] = stream[w];
+    }
+}
+
+// The record of every env of the warp that returns done this step (`rec`), taken before the auto-reset; include/wildfire.h
+// has the layout.  Returns the header of this lane's env's record, or nullptr (no record, or past the capacity).
+template <int L, int FB>
+__device__ __forceinline__ uint32_t* capture_final(const Rows<FB>& r, const Agent& a, const FinalCapture& fin, bool rec, int k, int env,
+                                                int lane, int sub, int x, int W, int H, uint32_t validmask, uint32_t* stream,
+                                                const uint32_t* spread3) {
+    constexpr uint32_t FULL = 0xffffffffu;
+    uint32_t slot = 0xffffffffu;
+    if (rec && x == 0) slot = atomicAdd(fin.count, 1u);
+    slot = __shfl_sync(FULL, slot, sub * L);
+    uint32_t* const mine = (rec && (int64_t)slot < fin.capacity) ? fin.records + (size_t)slot * fin.words : nullptr;
+    uint32_t* const d0 = reinterpret_cast<uint32_t*>(__shfl_sync(FULL, reinterpret_cast<uintptr_t>(mine), 0));
+    uint32_t* const d1 = L == 16 ? reinterpret_cast<uint32_t*>(__shfl_sync(FULL, reinterpret_cast<uintptr_t>(mine), 16)) : nullptr;
+    if (mine != nullptr && x == 0) {
+        const int flags = (a.alive ? WF_FINAL_ALIVE : 0) | (a.vis ? WF_FINAL_VISIBLE : 0) | (a.dead ? WF_FINAL_DEAD : 0) |
+                          (a.digging ? WF_FINAL_DIGGING : 0);
+        uint4* h = reinterpret_cast<uint4*>(mine);
+        h[0] = make_uint4((uint32_t)k, (uint32_t)env, a.episode, a.t);
+        h[1] = make_uint4((uint32_t)a.ax, (uint32_t)a.ay, (uint32_t)flags, 0xffffffffu);
+        h[2] = make_uint4(0xffffffffu, 0u, 0u, 0u);
+        h[3] = make_uint4(0u, 0u, 0u, 0u);
+    }
+    // the terminal observation (World.get_state, as emit_obs builds it) ...
+    const uint32_t arow = (a.vis && x == a.ax) ? (1u << a.ay) : 0u, freerow = ~r.I & validmask;
+    auto piece = [&](int p) -> uint32_t {
+        return spread3[(arow >> (8 * p)) & 255u] | (spread3[(r.F >> (8 * p)) & 255u] << 1) | (spread3[(freerow >> (8 * p)) & 255u] << 2);
+    };
+    const uint32_t p0 = piece(0), p1 = piece(1);
+    uint32_t o0 = p0 | (p1 << 24), o1 = p1 >> 8, o2 = 0u;
+    if (L == 32 && H > 16) {
+        const uint32_t p2 = piece(2), p3 = piece(3);
+        o1 |= p2 << 16;
+        o2 = (p2 >> 16) | (p3 << 8);
+    }
+    const int pw = final_plane_words(W, H), po = fin.plane_off;
+    // (the section runs up to the planes, so the padding words after the observation are written as zeros too)
+    fin_section<L>(stream, lane, sub, x, W, 3 * H, po - WF_FINAL_OBS, o0, o1, o2, d0 ? d0 + WF_FINAL_OBS : nullptr,
+                   d1 ? d1 + WF_FINAL_OBS : nullptr);
+    // ... the type planes, and the zero padding at the end of the record
+    const uint32_t planes[4] = {r.F, r.BT, r.D, r.WT};
+#pragma unroll
+    for (int p = 0; p < 4; ++p)
+        fin_section<L>(stream, lane, sub, x, W, H, pw, planes[p], 0u, 0u, d0 ? d0 + po + p * pw : nullptr,
+                       d1 ? d1 + po + p * pw : nullptr);
+    if (mine != nullptr)
+        for (int w = po + 4 * pw + x; w < fin.words; w += L) mine[w] = 0u;
+    __syncwarp();
+    return mine;
+}
+
 // UNI: every wind of the handle has direction-independent heat quanta (e.g. wind vector (0, 0)): a cell
 // ignites when its TOTAL hit count reaches kmin, so `temp` is a 7-bit counter per cell, bit-sliced in
 // registers (planes HC0..HC6); heat transfer + ignition test are ~40 word-parallel logic instructions
@@ -289,7 +364,8 @@ __device__ __forceinline__ void st_release_gpu(uint32_t* p, uint32_t v) {
     asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
 
-template <int L, int FB, bool UNI, bool MLP, bool SRV, bool OB>
+// FIN: final-state capture (`fin`): the record of every episode that ends is written before the auto-reset.
+template <int L, int FB, bool UNI, bool MLP, bool SRV, bool OB, bool FIN = false>
 __device__ __forceinline__ void warp_body(const DevState& s, const StepCfg& c, const WarpIO& io, const SrvCtl& srv) {
     constexpr int EPW = 32 / L;  // envs per warp
     constexpr uint32_t FULL = 0xffffffffu;
@@ -850,8 +926,23 @@ __device__ __forceinline__ void warp_body(const DevState& s, const StepCfg& c, c
                 if (io.reward != nullptr) io.reward[(size_t)k * s.N + env] = rew;
                 if (io.done != nullptr) io.done[(size_t)k * s.N + env] = done ? 1 : 0;
             }
-            // ---- auto-reset (batched-env convention: the returned obs is the new episode's first)
-            if (c.auto_reset && act && done) {
+            if constexpr (FIN) {
+                // ---- final-state capture, then the auto-reset and the next episode's start cell in the record
+                uint32_t* fin_rec = nullptr;
+                if (__any_sync(FULL, act && done))
+                    fin_rec = capture_final<L, FB>(r, a, static_cast<const WarpFinIO&>(io).fin, act && done, k, env, lane, sub, x,
+                                                   W, H, validmask, stream_warp, spread3);
+                if (c.auto_reset && act && done) {
+                    reset_rows<L, FB, UNI>(r, a, s, c, nullptr, env, x, validmask);
+                    a.refresh_wind(s.wind);
+                    reach_ok = false;
+                    if (fin_rec != nullptr && x == 0) {
+                        fin_rec[WF_F_NEXT_AX] = (uint32_t)a.ax;
+                        fin_rec[WF_F_NEXT_AY] = (uint32_t)a.ay;
+                    }
+                }
+            } else if (c.auto_reset && act && done) {
+                // ---- auto-reset (batched-env convention: the returned obs is the new episode's first)
                 reset_rows<L, FB, UNI>(r, a, s, c, nullptr, env, x, validmask);
                 a.refresh_wind(s.wind);
                 reach_ok = false;
@@ -1048,6 +1139,11 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32)
 warp_kernel(DevState s, StepCfg c, WarpIO io) {
     warp_body<L, FB, UNI, MLP, false, OB>(s, c, io, SrvCtl{});
 }
+// The same with final-state capture (wf_set_final_capture): a kernel of its own, so that warp_kernel keeps its code.
+template <int L, int FB, bool UNI, bool MLP, bool OB>
+__global__ void __launch_bounds__(kWarpsPerBlock * 32) warp_fin_kernel(DevState s, StepCfg c, WarpFinIO io) {
+    warp_body<L, FB, UNI, MLP, false, OB, true>(s, c, io, SrvCtl{});
+}
 // The step server must be resident as a whole (cooperative launch): 128 registers at most.
 template <int L, int FB, bool UNI>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32, 16 / kWarpsPerBlock) warp_server_kernel(DevState s, StepCfg c, WarpIO io, SrvCtl srv) {
@@ -1056,7 +1152,7 @@ __global__ void __launch_bounds__(kWarpsPerBlock * 32, 16 / kWarpsPerBlock) warp
 
 // ---------------------------------------------------------------------------------------------
 // host launcher (called from wf_api.cu)
-cudaError_t launch_warp_family(const DevState& s, const StepCfg& c, const WarpIO& io, cudaStream_t stream) {
+cudaError_t launch_warp_family(const DevState& s, const StepCfg& c, const WarpIO& io, cudaStream_t stream, const FinalCapture* fin) {
     const int L = s.RS;
     const int epw = 32 / L;
     const int envs_per_block = kWarpsPerBlock * epw;
@@ -1067,10 +1163,17 @@ cudaError_t launch_warp_family(const DevState& s, const StepCfg& c, const WarpIO
                 io.mlp.group_envs % envs_per_block != 0))
         return cudaErrorInvalidValue;
     const bool ob = io.obs != nullptr && io.obs_dtype == WF_OBS_BITS;
-#define WF_LAUNCH(LL, FF, UU, MM)                                                   \
-    do {                                                                            \
-        if (ob) warp_kernel<LL, FF, UU, MM, true><<<grid, block, 0, stream>>>(s, c, io);  \
-        else warp_kernel<LL, FF, UU, MM, false><<<grid, block, 0, stream>>>(s, c, io);    \
+    const bool capture = fin != nullptr && fin->records != nullptr && !io.reset_mode;
+    WarpFinIO fio;
+    static_cast<WarpIO&>(fio) = io;
+    if (capture) fio.fin = *fin;
+#define WF_LAUNCH(LL, FF, UU, MM)                                                                         \
+    do {                                                                                                  \
+        if (capture) {                                                                                    \
+            if (ob) warp_fin_kernel<LL, FF, UU, MM, true><<<grid, block, 0, stream>>>(s, c, fio);         \
+            else warp_fin_kernel<LL, FF, UU, MM, false><<<grid, block, 0, stream>>>(s, c, fio);           \
+        } else if (ob) warp_kernel<LL, FF, UU, MM, true><<<grid, block, 0, stream>>>(s, c, io);           \
+        else warp_kernel<LL, FF, UU, MM, false><<<grid, block, 0, stream>>>(s, c, io);                    \
     } while (0)
     if (mlp) {
         if (L == 16 && s.FB == 5 && s.HB) WF_LAUNCH(16, 5, true, true);
