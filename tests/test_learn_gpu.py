@@ -266,11 +266,12 @@ def test_learn_batched_end_to_end(name, tmp_path):
 
 # ---------------------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("name", ["DQN", "DQN_SARSA"])
-def test_replay_ring_holds_the_rollouts_transitions(name):
-    """learn_batched's ring (_PackedReplayRing) over 6 launches of the mlp policy with auto-resets, wrapping twice: after
-    every launch each sampleable (s, a, r, s', a', done) equals the one of a uint8 rollout of the same seed re-driven
-    with the recorded actions (s = the frame before step t, the reset frame for t = 0; a' = the action of step t + 1),
-    the window holds at least memory_size transitions, and the demonstrations come back unchanged."""
+def test_replay_ring_of_one_group_holds_the_rollouts_transitions(name):
+    """learn_batched's ring (_PackedReplayRing with one group, i.e. one demonstration memory) over 6 launches of the mlp
+    policy with auto-resets, wrapping twice: after every launch each sampleable (s, a, r, s', a', done) equals the one of
+    a uint8 rollout of the same seed re-driven with the recorded actions (s = the frame before step t, the reset frame for
+    t = 0; a' = the action of step t + 1), the window holds at least memory_size transitions, and the demonstrations
+    come back unchanged."""
     from wildfire_control_python_b200.constants import DQN_DEFAULTS
     N, K, W, launches = 64, 16, 10, 6
     ag = _agent(name, W, W, seed=7)
@@ -281,7 +282,7 @@ def test_replay_ring_holds_the_rollouts_transitions(name):
     env = BatchedForestFire(N, obs_dtype="bits", auto_reset=True, seed=5, **keys)
     ref = BatchedForestFire(N, auto_reset=True, seed=5, **keys)
     memory_size = K * N
-    ring = A._PackedReplayRing(env, K, memory_size, ag.memory, ag._SARSA)
+    ring = A._PackedReplayRing(env, K, memory_size, [ag.memory], ag._SARSA)
     assert ring.T == 2 * K  # wraps after two launches
     obs = [ref.reset().clone()]  # obs[t + 1] = the frame of step t
     acts, rews, dones = [], [], []
@@ -298,10 +299,10 @@ def test_replay_ring_holds_the_rollouts_transitions(name):
         dones += list(d)
         steps = (launch + 1) * K
         lo, hi = max(0, steps - ring.T + 1), steps - (1 if ag._SARSA else 0)
-        assert ring.n_sampleable == (hi - lo) * N + D
+        assert ring.sampleable(0) == (hi - lo) * N + D
         if launch >= 2:
             assert (hi - lo) * N >= memory_size
-        s_row, sp_row, a, ap, r, d = ring.gather(torch.arange(ring.n_sampleable, device="cuda"))
+        s_row, sp_row, a, ap, r, d = ring.gather(torch.arange(ring.sampleable(0), device="cuda"))
         s_u8 = unpack_obs(ring.frames, W, W, s_row, torch.uint8)
         sp_u8 = unpack_obs(ring.frames, W, W, sp_row, torch.uint8)
         ts = range(lo, hi)

@@ -81,6 +81,28 @@ def test_learn_batched_refuses_a_checkpoint_of_another_run(tmp_path, field):
     assert path.read_bytes() == before  # a refused checkpoint is left as it was
 
 
+def test_learn_batched_refuses_a_checkpoint_of_the_per_agent_layout(tmp_path):
+    """A checkpoint in the layout learn_batched wrote before it shared learn_population's (one agent's modules under
+    ``agent``, one ``replay_generator``), whose fingerprint has no ``layout``: refused with ValueError naming that field
+    before anything is restored, and left as it was."""
+    path = tmp_path / "run.ckpt"
+    ag = _agent(demos=3)
+    fp = A._run_fingerprint("learn_batched", [ag], **BATCHED)
+    del fp["layout"]
+    cpu = lambda m: {k: v.cpu() for k, v in m.state_dict().items()}  # noqa: E731
+    A._RunCheckpoint(path, fp).save(dict(
+        env={"scalars": torch.zeros((64, 8), dtype=torch.int32)}, ring={"steps": 16},
+        replay_generator=torch.Generator().manual_seed(3).get_state(),
+        agent=dict(model=cpu(ag.model), target=cpu(ag.target), adam_t=0, adam_m=[], adam_v=[], until_sync=20,
+                   logs="{}", eps=1.0, eps_per_launch=[1.0], episodes_before_launch=[0]),
+        carry=torch.zeros(64, dtype=torch.float64), done_eps=0, rewards=[], deaths=[], elapsed=0.5))
+    before = path.read_bytes()
+    kw = dict(BATCHED)
+    n = kw.pop("n_episodes")
+    _refused("layout", lambda: _agent(demos=3).learn_batched(n, checkpoint=path, **kw))
+    assert path.read_bytes() == before
+
+
 def _population(n=3, **kw):
     settings = [dict(alpha=0.005, target_update=20), dict(alpha=0.002, target_update=7), dict(alpha=0.01, target_update=50)]
     return [_agent(demos=d, **settings[j], **kw) for j, d in zip(range(n), (4, 0, 2))]

@@ -117,9 +117,9 @@ def test_learn_population_resumed_after_every_launch(name, tmp_path):
         assert _result(pop[j], got[j]) == want[j], j
 
 
-def test_a_resume_without_the_replay_generator_diverges(tmp_path):
-    """The same stop and resume with the checkpoint's replay generator replaced by a freshly seeded one: the replays draw
-    other minibatches, and the weights and logs come out different."""
+def test_a_resume_with_a_freshly_seeded_replay_generator_diverges(tmp_path):
+    """The same stop and resume with the checkpoint's replay generator (learner 0's of the stacked layout) replaced by a
+    freshly seeded one: the replays draw other minibatches, and the weights and logs come out different."""
     memory, init = _demos("DQN", 10, 20)
 
     def make(out):
@@ -135,8 +135,8 @@ def test_a_resume_without_the_replay_generator_diverges(tmp_path):
         assert make(tmp_path / "resumed").learn_batched(300, checkpoint=path, time_limit=0, **kw) is None
         if not restore:
             ck = torch.load(path, weights_only=True)
-            assert ck["state"]["agent"]["adam_t"] > 0  # the first launch replayed: the generator has moved
-            ck["state"]["replay_generator"] = torch.Generator(device="cuda").manual_seed(3).get_state()
+            assert ck["state"]["adam_t"][0] > 0  # the first launch replayed: the generator has moved
+            ck["state"]["replay_generators"][0] = torch.Generator(device="cuda").manual_seed(3).get_state()
             torch.save(ck, path)
         ag = make(tmp_path / "resumed")
         got = _result(ag, ag.learn_batched(300, checkpoint=path, **kw))

@@ -429,11 +429,10 @@ class DQN:
         are not under-represented; an episode still undecided at the end of its rollout is dropped.
         Returns the number of environment steps simulated."""
         from .batched import BatchedForestFire
-        from .constants import DQN_DEFAULTS as _D
         if not num_of_episodes:
             return 0
-        keys = {k: v for k, v in self.METADATA.items() if k not in _D and k not in ("debug", "a_speed_iter", "seed", "auto_reset")}
-        env = BatchedForestFire(n_envs, device=self.device if self.device.type == "cuda" else None, auto_reset=True, seed=seed, **keys)
+        env = BatchedForestFire(n_envs, device=self.device if self.device.type == "cuda" else None, auto_reset=True, seed=seed,
+                                **_env_kwargs(self))
         bonus = self.METADATA["contained_bonus"]
         self.memory = self._new_memory(None)
         success, simulated = 0, 0
@@ -558,10 +557,8 @@ class DQN:
         ``record_maps=True`` (needs the in-kernel path): also return the final map of every evaluated episode, the string
         ``ForestFire.render(print_map=False)`` gives for its last state, in the order of the returns."""
         from .batched import BatchedForestFire
-        from .constants import DQN_DEFAULTS as _D
         eps = self.min_eps if eps is None else eps
-        keys = {k: v for k, v in self.METADATA.items() if k not in _D and k not in ("debug", "a_speed_iter", "seed", "auto_reset")}
-        env = BatchedForestFire(n_envs, device=self.device, auto_reset=True, seed=seed, **keys)
+        env = BatchedForestFire(n_envs, device=self.device, auto_reset=True, seed=seed, **_env_kwargs(self))
         if in_kernel is None:
             in_kernel = env.kernel_family == "warp"
         if record_maps and not in_kernel:
@@ -657,9 +654,7 @@ class DQN:
         from the previous call, starting at ``target_update``) is the number of replays left until the next refresh.
         ``model``, ``target`` and the optimiser's ``t``, ``m``, ``v`` are updated in place; returns the ``[n_replays]``
         float32 losses (a device tensor: nothing is synchronised)."""
-        from torch.nn.utils import parameters_to_vector
         from . import _lib
-        from .batched import _ptr
         if self.device.type != "cuda":
             raise _lib.WildfireError("fit_batches_fused needs a CUDA device (no CPU fallback)")
         n_replays = int(n_replays)
@@ -670,45 +665,13 @@ class DQN:
         frames = frames.to(dev).contiguous()
         if frames.dtype != torch.int32 or frames.dim() != 2:
             raise ValueError("frames must be an int32 [n_frames, words] tensor")
-        cols = [torch.as_tensor(x, device=dev).to(dt).contiguous()
-                for x, dt in ((s_row, torch.int64), (sp_row, torch.int64), (a, torch.int32), (ap, torch.int32),
-                              (r, torch.float32), (d, torch.uint8))]
+        cols = [torch.as_tensor(x, device=dev) for x in (s_row, sp_row, a, ap, r, d)]
         if any(c.shape != (n_replays * batch,) for c in cols):
             raise ValueError("s_row, sp_row, a, ap, r and d must be one-dimensional and of the same length")
-        s_row, sp_row, a, ap, r, d = cols
-        params = list(self.model.parameters())
-        states = [self.optimizer.state[p] for p in params]
-        t0 = states[0]["t"] if states[0] else 0
-        with torch.no_grad():
-            flat = parameters_to_vector(params).contiguous()
-            tgt = parameters_to_vector(self.target.parameters()).contiguous()
-            m = parameters_to_vector([st["m"] for st in states]) if t0 else torch.zeros_like(flat)
-            v = parameters_to_vector([st["v"] for st in states]) if t0 else torch.zeros_like(flat)
-        group = self.optimizer.param_groups[0]
-        te = int(self.target_update_freq)
-        phase = int(getattr(self, "_until_sync", te) if phase is None else phase)
-        hp = _lib.WfFitParams(gamma=float(self.gamma), lr=group["lr"], beta_1=group["beta_1"], beta_2=group["beta_2"],
-                              epsilon=group["epsilon"], clipvalue=math.inf if group["clipvalue"] is None else group["clipvalue"],
-                              adam_t=t0, target_every=te, phase=phase)
+        stack = _LearnerStack([self], [int(getattr(self, "_until_sync", self.target_update_freq) if phase is None else phase)])
         loss = torch.empty(n_replays, dtype=torch.float32, device=dev)
-        W, H = self.obs_shape[0], self.obs_shape[1]
-        fit = _lib.lib().wf_replay_fit if W <= 32 and H <= 32 else _lib.lib().wf_replay_fit_large
-        with torch.cuda.device(dev):
-            _lib.check(fit(
-                ctypes.byref(self._flat_shape(batch)), ctypes.byref(hp), n_replays, _ptr(flat), _ptr(tgt), _ptr(m), _ptr(v),
-                _ptr(frames), frames.shape[0], _ptr(s_row), _ptr(sp_row), _ptr(a), _ptr(ap) if self._SARSA else None,
-                _ptr(r), _ptr(d), _ptr(loss), ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
-        with torch.no_grad():
-            off = 0
-            for p, tp, st in zip(params, self.target.parameters(), states):
-                n = p.numel()
-                p.copy_(flat[off:off + n].view_as(p))
-                tp.copy_(tgt[off:off + n].view_as(p))
-                st["m"] = m[off:off + n].view_as(p).clone()
-                st["v"] = v[off:off + n].view_as(p).clone()
-                st["t"] = t0 + n_replays
-                off += n
-        self._until_sync = (phase - n_replays - 1) % te + 1
+        stack.replay_fit([0], frames, [cols], n_replays, loss)
+        stack.write_back(0)
         return loss
 
     def learn_batched(self, n_episodes, n_envs=1024, k_steps=16, replays_per_launch=None, batch_size=None, seed=0,
@@ -716,7 +679,7 @@ class DQN:
         """``learn`` over ``n_envs`` CUDA environments at once: the envs act with the eps-greedy Q-network evaluated inside
         the step kernel (``rollout(policy="mlp")``, ``k_steps`` steps per launch), each rollout writes its packed
         observations straight into a device replay ring, and after every launch ``replays_per_launch`` (default
-        ``k_steps``) replays of ``batch_size`` (default METADATA's) transitions run as one ``fit_batches_fused`` launch.
+        ``k_steps``) replays of ``batch_size`` (default METADATA's) transitions run in one launch, as in ``fit_batches_fused``.
         The in-kernel policy is refreshed on the device before every launch, with eps = min + (max - min) *
         exp(-rate * episodes completed so far) (``decay_epsilon``).
 
@@ -735,24 +698,17 @@ class DQN:
         ``_end_of_episode``'s map rule in the order it is logged, with the map string rendered from its final state, and
         DQN / DQN_DUEL log each episode's start cell (the SARSA classes do not, as in ``learn``).  Capture is an output
         only: trajectories, weights and the other logs are byte-identical to ``record_maps=False``.
-        ``eps_per_launch`` / ``episodes_before_launch`` record the schedule.  Any grid: ``fit_batches_fused`` runs the
-        replays in ``wf_replay_fit`` up to 32x32 and in ``wf_replay_fit_large`` on larger grids.  Returns the number of
-        environment steps simulated.
+        ``eps_per_launch`` / ``episodes_before_launch`` record the schedule.  Any grid: the replays run in ``wf_replay_fit``
+        up to 32x32 and in ``wf_replay_fit_large`` on larger grids.  Returns the number of environment steps simulated.
 
         ``checkpoint=PATH``: resume the run from that file if it exists (``ValueError`` if it was written by a run with
         another class, network shape, METADATA, demonstration count or other arguments); remove it once the logs are
         written.  ``time_limit=SECONDS`` (needs ``checkpoint``): checked after each launch's replays and episode
         accounting; once this call has run that long and the run is not finished, write the run's whole state to the
-        checkpoint (atomically) and return None without writing logs.  Calling again with the same arguments continues
-        exactly where the run stopped, with byte-identical results, from a freshly built agent too: the model, target,
-        optimiser state, ``_until_sync``, logs and eps schedule are overwritten from the file.  ``logs['total_time']`` is
-        the sum of the calls' times."""
-        from . import _lib
-        from .batched import BatchedForestFire
-        from .constants import DQN_DEFAULTS as _D
-        if time_limit is not None and checkpoint is None:
-            raise ValueError("time_limit needs a checkpoint file to save the run to")
-        t_run = time.time()
+        checkpoint (atomically) and return None without writing logs; the agent holds the state trained so far.  Calling
+        again with the same arguments continues exactly where the run stopped, with byte-identical results, from a freshly
+        built agent too: the model, target, optimiser state, ``_until_sync``, logs and eps schedule are overwritten from
+        the file.  ``logs['total_time']`` is the sum of the calls' times."""
         N, K = int(n_envs), int(k_steps)
         R = K if replays_per_launch is None else int(replays_per_launch)
         B = int(self.METADATA["batch_size"] if batch_size is None else batch_size)
@@ -760,87 +716,8 @@ class DQN:
         ckpt = _RunCheckpoint(checkpoint, _run_fingerprint("learn_batched", [self], n_episodes=n_episodes, n_envs=N, k_steps=K,
                                                            replays_per_launch=R, batch_size=B, seed=seed, replay_seed=rseed,
                                                            **({"record_maps": True} if record_maps else {})))
-        saved = ckpt.load()
-        keys = {k: v for k, v in self.METADATA.items() if k not in _D and k not in ("debug", "a_speed_iter", "seed", "auto_reset")}
-        env = BatchedForestFire(N, device=self.device, obs_dtype="bits", auto_reset=True, seed=seed, **keys)
-        death_penalty = float(self.METADATA["death_penalty"])
-        gen = torch.Generator(device=env.device).manual_seed(rseed)
-        self._until_sync = self.target_update_freq
-        self.logs["n_episodes"] = n_episodes
-        self.eps_per_launch, self.episodes_before_launch = [], []
-        rewards, deaths = [], []
-        carry = np.zeros(N)
-        done_eps, elapsed = 0, 0.0
-        try:
-            ring = _PackedReplayRing(env, K, int(self.METADATA["memory_size"]), self.memory, self._SARSA)
-            if record_maps:
-                sc = env.get_state()["scalars"]
-                maplog = _MapLog(self, sc[:, _lib.S_AX:_lib.S_AY + 1].cpu().numpy())
-            if saved is not None:
-                env.set_state(**saved["env"])
-                ring.load_state_dict(saved["ring"])
-                gen.set_state(saved["replay_generator"])
-                self._load_learner_state(saved["agent"])
-                carry, done_eps, elapsed = saved["carry"].numpy(), saved["done_eps"], saved["elapsed"]
-                rewards, deaths = saved["rewards"], saved["deaths"]
-                if record_maps:
-                    maplog.load(saved["maps"])
-            while len(rewards) < n_episodes:
-                self.eps = self.min_eps + (self.max_eps - self.min_eps) * np.exp(-self.eps_decay_rate * done_eps)
-                self.eps_per_launch.append(float(self.eps))
-                self.episodes_before_launch.append(done_eps)
-                net = self.model
-                env.set_policy_mlp_dev(net.dense_1.weight, net.dense_1.bias, net.dense_2.weight, net.dense_2.bias, eps=self.eps)
-                rew, done = ring.launch(finals=record_maps)
-                if R > 0 and ring.n_sampleable > B:
-                    self.fit_batches_fused(ring.frames, *ring.gather(ring.sample(R, B, gen)), R)
-                rd = torch.stack((rew, done.double())).cpu().numpy()
-                e_idx, k_idx, ret, carry = _episode_ends(carry, rd[0], rd[1] != 0)
-                order = np.lexsort((e_idx, k_idx))
-                at = _final_index(ring.finals) if record_maps else None
-                for i in order[: n_episodes - len(rewards)]:
-                    if record_maps:
-                        maplog.episode(len(rewards), float(ret[i]), e_idx[i], ring.finals, at, (int(k_idx[i]), int(e_idx[i])))
-                    rewards.append(float(ret[i]))
-                    deaths.append(bool(rd[0][k_idx[i], e_idx[i]] == death_penalty))
-                done_eps += len(e_idx)
-                if len(rewards) < n_episodes and time_limit is not None and time.time() - t_run >= time_limit:
-                    ckpt.save(dict(env=_env_state(env), ring=ring.state_dict(), replay_generator=gen.get_state(),
-                                   agent=self._learner_state(), carry=torch.from_numpy(carry), done_eps=done_eps,
-                                   rewards=rewards, deaths=deaths, elapsed=elapsed + time.time() - t_run,
-                                   **({"maps": maplog.state()} if record_maps else {})))
-                    return None
-            steps = ring.steps
-        finally:
-            env.close()
-        self.logs["total_rewards"] = rewards
-        self.logs["agent_deaths"] = deaths
-        if record_maps:
-            maplog.write(self)
-        self.logs["total_time"] = round(elapsed + time.time() - t_run, 3)
-        self.write_data()
-        ckpt.remove()
-        return steps * N
-
-    def _learner_state(self):
-        """What ``learn_batched`` checkpoints of this agent, on the CPU: model, target, ``KerasAdam`` step and moments,
-        ``_until_sync``, logs and eps schedule."""
-        params = list(self.model.parameters())
-        opt = [self.optimizer.state[p] for p in params]
-        t = opt[0]["t"] if opt[0] else 0
-        cpu = lambda sd: {k: v.cpu() for k, v in sd.items()}  # noqa: E731
-        return dict(model=cpu(self.model.state_dict()), target=cpu(self.target.state_dict()), adam_t=t,
-                    adam_m=[st["m"].cpu() for st in opt] if t else [], adam_v=[st["v"].cpu() for st in opt] if t else [],
-                    until_sync=self._until_sync, **_schedule_state(self))
-
-    def _load_learner_state(self, st):
-        self.model.load_state_dict(st["model"])  # copies into the existing parameters: the optimiser keeps them
-        self.target.load_state_dict(st["target"])
-        self.optimizer.state.clear()
-        for p, m, v in zip(self.model.parameters(), st["adam_m"], st["adam_v"]):
-            self.optimizer.state[p] = dict(t=st["adam_t"], m=m.to(p.device), v=v.to(p.device))
-        self._until_sync = st["until_sync"]
-        _load_schedule_state(self, st)
+        steps = _learn_on_device("learn_batched", [self], ckpt, n_episodes, N, K, R, B, seed, [rseed], time_limit, record_maps)
+        return None if steps is None else steps[0]
 
     def save_model(self, name):  # DQN.py:441-443
         path = os.path.join(self.out_dir, "Models", name)
@@ -877,16 +754,15 @@ class _PackedReplayRing:
     on-policy transition becomes sampleable one step later).  Held after ``steps`` steps: t in [lo, hi) with
     lo = max(0, steps - T + 1) (s of step lo is the oldest frame the ring holds) and hi = steps (steps - 1 with a').
     T is the smallest multiple of K, and at least 2K, for which T - 1 (T - 2 with a') steps of a group's G envs hold
-    ``memory_size`` transitions.  The demonstrations (``ReplayMemory`` entries, uint8; ``demos``: one memory per group, or
-    one memory for one group) are packed once and kept."""
+    ``memory_size`` transitions.  The demonstrations (``ReplayMemory`` entries, uint8; ``demos``: one memory per group, so
+    ``len(demos)`` groups) are packed once and kept."""
 
-    def __init__(self, env, k_steps, memory_size, demos, on_policy, groups=1):
+    def __init__(self, env, k_steps, memory_size, demos, on_policy):
         from .batched import pack_obs
         self.env, self.K, self.N, self.on_policy = env, int(k_steps), env.n_envs, bool(on_policy)
-        if not isinstance(demos, (list, tuple)):
-            demos = [demos]
-        if len(demos) != groups or self.N % groups:
-            raise ValueError("need one demonstration memory per group and equal groups of envs")
+        groups = len(demos)
+        if self.N % groups:
+            raise ValueError("the envs must form equal groups, one per demonstration memory")
         self.G = G = self.N // groups
         K, N, dev, words = self.K, self.N, env.device, env.obs_words
         need = -(-int(memory_size) // G) + 1 + int(self.on_policy)
@@ -947,10 +823,6 @@ class _PackedReplayRing:
         lo, hi = self.window
         return max(0, hi - lo) * self.G + self.D[group]
 
-    @property
-    def n_sampleable(self):
-        return self.sampleable(0)
-
     def sample(self, n_batches, batch, gen, group=0):
         """``n_batches`` batches, each drawn uniformly without replacement from the group's sampleable transitions:
         [n * batch]."""
@@ -979,10 +851,12 @@ class _PackedReplayRing:
 
 
 def _run_fingerprint(entry, agents, **args):
-    """What a checkpoint must agree on to continue a run: the entry point, the agents' class and network shape, every
-    agent's METADATA and demonstration count, and the call's arguments (as JSON values)."""
+    """What a checkpoint must agree on to continue a run: the layout of its state, the entry point, the agents' class and
+    network shape, every agent's METADATA and demonstration count, and the call's arguments (as JSON values)."""
     a0 = agents[0]
-    fp = dict(entry=entry, agent_class=type(a0).__name__, network=[list(p.shape) for p in a0.model.parameters()],
+    # layout: of the state _learn_on_device saves; a change to that state must change this number, so that older files
+    # are refused before anything is restored
+    fp = dict(layout=2, entry=entry, agent_class=type(a0).__name__, network=[list(p.shape) for p in a0.model.parameters()],
               agents=len(agents), METADATA=[a.METADATA for a in agents], demonstrations=[len(a.memory) for a in agents],
               **args)
     return json.loads(json.dumps(fp, default=_jsonable))
@@ -1054,6 +928,13 @@ def _env_state(env):
     return {k: v.cpu() for k, v in env.get_state().items() if k not in ("temp", "apos")}
 
 
+def _env_kwargs(agent):
+    """``BatchedForestFire`` keyword arguments for an agent's environment: its METADATA without the learner's settings
+    and the keys the batch sets itself."""
+    own = ("debug", "a_speed_iter", "seed", "auto_reset")
+    return {k: v for k, v in agent.METADATA.items() if k not in DQN_DEFAULTS and k not in own}
+
+
 def _schedule_state(ag):
     """An agent's logs and eps schedule, as a checkpoint stores them (the logs as the JSON ``write_data`` writes)."""
     return dict(logs=json.dumps(ag.logs, default=_jsonable), eps=float(ag.eps), eps_per_launch=list(ag.eps_per_launch),
@@ -1082,7 +963,7 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
     network and eps (``set_policy_mlp_flat_dev``).  The replay ring (``_PackedReplayRing``) keeps one column group and
     the demonstrations per learner; learner j draws its batches from its own window with its own generator, seeded with
     ``seed + j``.  The stacked [M, P] model, target and Adam moments are the state during the run and are written back
-    into each agent (modules, ``KerasAdam`` m, v and t, ``_until_sync``) at the end.
+    into each agent (modules, ``KerasAdam`` m, v and t, ``_until_sync``) when the call returns.
 
     Learner j logs its first ``n_episodes`` episodes exactly as ``learn_batched`` does (``eps_per_launch`` and
     ``episodes_before_launch`` included) and stops replaying after the launch in which it reaches them; its envs keep
@@ -1094,17 +975,12 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
     ``checkpoint`` and ``time_limit`` work as in ``learn_batched``: the file holds the stacked model, target and Adam
     state, each learner's Adam step, sync phase, generator, episode accounting, logs and eps schedule, the env batch and
     the replay ring, and its fingerprint covers the number of agents and each agent's METADATA and demonstration count.
-    A stopped call returns None and writes no logs.
+    A stopped call returns None and writes no logs; the agents hold the state trained so far.
 
     ``record_maps=True``: every learner also keeps ``maps``, ``best_reward`` and ``agent_pos`` as ``learn_batched(...,
     record_maps=True)`` does, equal to that run's byte for byte; the episodes of a learner that has finished are not
     rendered."""
-    from torch.nn.utils import parameters_to_vector
     from . import _lib
-    from .batched import BatchedForestFire, _ptr
-    from .constants import DQN_DEFAULTS as _D
-    if time_limit is not None and checkpoint is None:
-        raise ValueError("time_limit needs a checkpoint file to save the run to")
     agents = list(agents)
     M = len(agents)
     if not 1 <= M <= _lib.MAX_LEARNERS:
@@ -1126,33 +1002,43 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
         raise ValueError("envs_per_learner must be a positive multiple of 8")
     if any(a.device != a0.device for a in agents):
         raise ValueError("learn_population: every agent must be on the same device")
-    t_run = time.time()
     R = K if replays_per_launch is None else int(replays_per_launch)
     B = int(a0.METADATA["batch_size"] if batch_size is None else batch_size)
     ckpt = _RunCheckpoint(checkpoint, _run_fingerprint("learn_population", agents, n_episodes=n_episodes, envs_per_learner=G,
                                                        k_steps=K, replays_per_launch=R, batch_size=B, seed=seed,
                                                        **({"record_maps": True} if record_maps else {})))
+    return _learn_on_device("learn_population", agents, ckpt, n_episodes, G, K, R, B, seed, [int(seed) + j for j in range(M)],
+                            time_limit, record_maps)
+
+
+def _learn_on_device(entry, agents, ckpt, n_episodes, G, K, R, B, seed, replay_seeds, time_limit, record_maps):
+    """The training loop of ``DQN.learn_batched`` (one agent) and ``learn_population``: M = len(agents) learners of one
+    class, shape and environment METADATA on one ``"bits"`` handle of M * G auto-reset envs with Philox key ``seed``,
+    learner j on envs j*G ... j*G + G - 1 and replaying with a generator seeded with ``replay_seeds[j]``; ``K`` steps per
+    launch, then ``R`` replays of ``B`` transitions for each learner that has not finished.  ``ckpt``: the call's
+    ``_RunCheckpoint``.  Writes the trained state back into the agents whenever it returns; returns each learner's
+    env-step count, or None when ``time_limit`` stopped the call."""
+    from . import _lib
+    from .batched import BatchedForestFire
+    if time_limit is not None and ckpt.path is None:
+        raise ValueError("time_limit needs a checkpoint file to save the run to")
+    t_run = time.time()
     saved = ckpt.load()
+    M, a0 = len(agents), agents[0]
     if a0.device.type != "cuda":
-        raise _lib.WildfireError("learn_population needs a CUDA device (no CPU fallback)")
-    N = M * G
-    sarsa, dueling = a0._SARSA, hasattr(a0.model, "dense_3")
-    hidden = a0.model.dense_1.out_features
-    keys = {k: v for k, v in a0.METADATA.items() if k not in _D and k not in ("debug", "a_speed_iter", "seed", "auto_reset")}
-    env = BatchedForestFire(N, device=a0.device, obs_dtype="bits", auto_reset=True, seed=seed, **keys)
-    dev = env.device
+        raise _lib.WildfireError(f"{entry} needs a CUDA device (no CPU fallback)")
+    stack = _LearnerStack(agents, [int(a.target_update_freq) for a in agents])
+    state = [x.view(M, -1) for x in stack.flat]  # [M, P] model, target, m, v
+    # one network: wf_set_policy_mlp_dev reads dense_1 and dense_2 (the advantage stream of a dueling head) from row 0,
+    # and takes every grid and env count; several: wf_set_policy_mlp_nets_dev (<= 32x32, groups of a multiple of 8)
+    policy, off = [], 0
+    for p in list(a0.model.parameters())[:4]:
+        policy.append(stack.flat[0][off:off + p.numel()].view_as(p))
+        off += p.numel()
+    hidden, dueling = a0.model.dense_1.out_features, hasattr(a0.model, "dense_3")
+    env = BatchedForestFire(M * G, device=a0.device, obs_dtype="bits", auto_reset=True, seed=seed, **_env_kwargs(a0))
     death_penalty = float(a0.METADATA["death_penalty"])
-    gens = [torch.Generator(device=dev).manual_seed(int(seed) + j) for j in range(M)]
-    # the stacked state, as DQN.fit_batches_fused flattens it
-    with torch.no_grad():
-        adam_t = [(a.optimizer.state[next(a.model.parameters())] or {}).get("t", 0) for a in agents]
-        P = torch.stack([parameters_to_vector(a.model.parameters()) for a in agents]).contiguous()
-        Tg = torch.stack([parameters_to_vector(a.target.parameters()) for a in agents]).contiguous()
-        Mm = torch.stack([parameters_to_vector([a.optimizer.state[p]["m"] for p in a.model.parameters()]) if t else
-                          torch.zeros(P.shape[1], device=dev) for a, t in zip(agents, adam_t)]).contiguous()
-        Vv = torch.stack([parameters_to_vector([a.optimizer.state[p]["v"] for p in a.model.parameters()]) if t else
-                          torch.zeros(P.shape[1], device=dev) for a, t in zip(agents, adam_t)]).contiguous()
-    until_sync = [int(a.target_update_freq) for a in agents]
+    gens = [torch.Generator(device=env.device).manual_seed(s) for s in replay_seeds]
     rewards, deaths = [[] for _ in agents], [[] for _ in agents]
     carry = [np.zeros(G) for _ in agents]
     done_eps, steps, finished = [0] * M, [0] * M, [False] * M
@@ -1160,10 +1046,8 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
     for a in agents:
         a.logs["n_episodes"] = n_episodes
         a.eps_per_launch, a.episodes_before_launch = [], []
-    shape = a0._flat_shape(B)
-    stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
     try:
-        ring = _PackedReplayRing(env, K, int(a0.METADATA["memory_size"]), [a.memory for a in agents], sarsa, groups=M)
+        ring = _PackedReplayRing(env, K, int(a0.METADATA["memory_size"]), [a.memory for a in agents], a0._SARSA)
         if record_maps:
             starts = env.get_state()["scalars"][:, _lib.S_AX:_lib.S_AY + 1].cpu().numpy()
             maplogs = [_MapLog(a, starts[j * G:(j + 1) * G]) for j, a in enumerate(agents)]
@@ -1172,9 +1056,9 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
             ring.load_state_dict(saved["ring"])
             for g, st in zip(gens, saved["replay_generators"]):
                 g.set_state(st)
-            for x, k in ((P, "params"), (Tg, "target"), (Mm, "adam_m"), (Vv, "adam_v")):
+            for x, k in zip(state, ("params", "target", "adam_m", "adam_v")):
                 x.copy_(saved[k])
-            adam_t, until_sync = list(saved["adam_t"]), list(saved["until_sync"])
+            stack.adam_t, stack.until_sync = list(saved["adam_t"]), list(saved["until_sync"])
             carry = [c.numpy() for c in saved["carry"]]
             done_eps, steps, finished = list(saved["done_eps"]), list(saved["steps"]), list(saved["finished"])
             rewards, deaths, elapsed = saved["rewards"], saved["deaths"], saved["elapsed"]
@@ -1189,34 +1073,14 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
                     a.eps = a.min_eps + (a.max_eps - a.min_eps) * np.exp(-a.eps_decay_rate * done_eps[j])
                     a.eps_per_launch.append(float(a.eps))
                     a.episodes_before_launch.append(done_eps[j])
-            env.set_policy_mlp_flat_dev(P, hidden, dueling, [float(a.eps) for a in agents])
+            if M == 1:
+                env.set_policy_mlp_dev(*policy, eps=a0.eps)
+            else:
+                env.set_policy_mlp_flat_dev(state[0], hidden, dueling, [float(a.eps) for a in agents])
             rew, done = ring.launch(finals=record_maps)
             fit = [j for j in range(M) if not finished[j] and R > 0 and ring.sampleable(j) > B]
             if fit:
-                keep, desc = [], (_lib.WfFitLearner * len(fit))()
-                for i, j in enumerate(fit):
-                    a = agents[j]
-                    cols = [x.to(dt).contiguous() for x, dt in zip(ring.gather(ring.sample(R, B, gens[j], j), j),
-                                                                   (torch.int64, torch.int64, torch.int32, torch.int32,
-                                                                    torch.float32, torch.uint8))]
-                    keep.append(cols)
-                    grp = a.optimizer.param_groups[0]
-                    te = int(a.target_update_freq)
-                    hp = _lib.WfFitParams(gamma=float(a.gamma), lr=grp["lr"], beta_1=grp["beta_1"], beta_2=grp["beta_2"],
-                                          epsilon=grp["epsilon"],
-                                          clipvalue=math.inf if grp["clipvalue"] is None else grp["clipvalue"],
-                                          adam_t=adam_t[j], target_every=te, phase=until_sync[j])
-                    desc[i] = _lib.WfFitLearner(P[j].data_ptr(), Tg[j].data_ptr(), Mm[j].data_ptr(), Vv[j].data_ptr(),
-                                                cols[0].data_ptr(), cols[1].data_ptr(), cols[2].data_ptr(),
-                                                cols[3].data_ptr() if sarsa else None, cols[4].data_ptr(),
-                                                cols[5].data_ptr(), None, hp)
-                with torch.cuda.device(dev):
-                    _lib.check(_lib.lib().wf_replay_fit_many(ctypes.byref(shape), len(fit), desc, R, _ptr(ring.frames),
-                                                             ring.frames.shape[0], stream))
-                for j in fit:
-                    adam_t[j] += R
-                    te = int(agents[j].target_update_freq)
-                    until_sync[j] = (until_sync[j] - R - 1) % te + 1
+                stack.replay_fit(fit, ring.frames, [ring.gather(ring.sample(R, B, gens[j], j), j) for j in fit], R)
             rd = torch.stack((rew, done.double())).cpu().numpy()
             at = _final_index(ring.finals) if record_maps else None
             for j in range(M):
@@ -1235,39 +1099,109 @@ def learn_population(agents, n_episodes, envs_per_learner=64, k_steps=16, replay
                 if len(rewards[j]) >= n_episodes:
                     finished[j], steps[j] = True, ring.steps * G
             if not all(finished) and time_limit is not None and time.time() - t_run >= time_limit:
+                P, Tg, Mm, Vv = state
                 ckpt.save(dict(env=_env_state(env), ring=ring.state_dict(), replay_generators=[g.get_state() for g in gens],
-                               params=P.cpu(), target=Tg.cpu(), adam_m=Mm.cpu(), adam_v=Vv.cpu(), adam_t=adam_t,
-                               until_sync=until_sync, carry=[torch.from_numpy(c) for c in carry], done_eps=done_eps,
+                               params=P.cpu(), target=Tg.cpu(), adam_m=Mm.cpu(), adam_v=Vv.cpu(), adam_t=stack.adam_t,
+                               until_sync=stack.until_sync, carry=[torch.from_numpy(c) for c in carry], done_eps=done_eps,
                                steps=steps, finished=finished, rewards=rewards, deaths=deaths,
                                agents=[_schedule_state(a) for a in agents], elapsed=elapsed + time.time() - t_run,
                                **({"maps": [ml.state() for ml in maplogs]} if record_maps else {})))
-                return None
+                break
     finally:
         env.close()
+    for j in range(M):
+        stack.write_back(j)
+    if not all(finished):
+        return None
     total_time = round(elapsed + time.time() - t_run, 3)
-    with torch.no_grad():
-        for j, a in enumerate(agents):
-            params = list(a.model.parameters())
-            off = 0
-            for p, tp in zip(params, a.target.parameters()):
-                n = p.numel()
-                p.copy_(P[j, off:off + n].view_as(p))
-                tp.copy_(Tg[j, off:off + n].view_as(p))
-                if adam_t[j]:
-                    st = a.optimizer.state[p]
-                    st["m"] = Mm[j, off:off + n].view_as(p).clone()
-                    st["v"] = Vv[j, off:off + n].view_as(p).clone()
-                    st["t"] = adam_t[j]
-                off += n
-            a._until_sync = until_sync[j]
-            a.logs["total_rewards"] = rewards[j]
-            a.logs["agent_deaths"] = deaths[j]
-            if record_maps:
-                maplogs[j].write(a)
-            a.logs["total_time"] = total_time
-            a.write_data()
+    for j, a in enumerate(agents):
+        a.logs["total_rewards"] = rewards[j]
+        a.logs["agent_deaths"] = deaths[j]
+        if record_maps:
+            maplogs[j].write(a)
+        a.logs["total_time"] = total_time
+        a.write_data()
     ckpt.remove()
     return steps
+
+
+class _LearnerStack:
+    """The state of M agents that train together on the device: ``flat``, their model, target and ``KerasAdam`` m and v as
+    four float32 buffers of M * P floats, agent j's P floats from j * P on in the flat layout of ``wf_replay_fit``
+    (include/wildfire.h; zero moments for an agent not yet updated), and each agent's Adam step ``adam_t`` and
+    target-sync phase ``until_sync`` (replays left until the next refresh)."""
+
+    def __init__(self, agents, until_sync):
+        self.agents, self.until_sync = list(agents), list(until_sync)
+        self.adam_t = [(a.optimizer.state[next(a.model.parameters())] or {}).get("t", 0) for a in self.agents]
+        params = [list(a.model.parameters()) for a in self.agents]
+        opt = [[a.optimizer.state[p] for p in ps] for a, ps in zip(self.agents, params)]
+
+        def cat(tensors):  # each agent's tensors, in parameter order
+            return torch.cat([t.reshape(-1) for ts in tensors for t in ts])
+
+        with torch.no_grad():
+            self.flat = [cat(params), cat([list(a.target.parameters()) for a in self.agents])] + [
+                cat([[st[k] for st in sts] if t else [torch.zeros_like(p) for p in ps]
+                     for ps, sts, t in zip(params, opt, self.adam_t)]) for k in "mv"]
+        self.P = self.flat[0].numel() // len(self.agents)
+
+    def replay_fit(self, learners, frames, batches, n_replays, loss=None):
+        """``n_replays`` consecutive replays of each learner j in ``learners``, in one launch: learner ``learners[i]`` on
+        ``batches[i]`` = (s_row, sp_row, a, ap, r, d), int64, int64, int32, int32, float32 and uint8 CUDA tensors of
+        ``n_replays * batch`` transitions as ``fit_batches_fused`` takes them, rows of ``frames``.  One learner runs in
+        ``wf_replay_fit`` up to 32x32 and in ``wf_replay_fit_large`` above, several in ``wf_replay_fit_many``
+        (bit-identical to ``wf_replay_fit`` per learner).  ``loss``: the one learner's [n_replays] losses, or None."""
+        from . import _lib
+        from .batched import _ptr
+        a0, L, dev = self.agents[learners[0]], _lib.lib(), frames.device
+        shape = a0._flat_shape(len(batches[0][0]) // n_replays)
+        stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        batches = [[x.to(dt).contiguous() for x, dt in zip(b, (torch.int64, torch.int64, torch.int32, torch.int32,
+                                                                torch.float32, torch.uint8))] for b in batches]
+        hps, ptrs = [], []
+        for j, (s_row, sp_row, a, ap, r, d) in zip(learners, batches):
+            ag, grp = self.agents[j], self.agents[j].optimizer.param_groups[0]
+            clip = math.inf if grp["clipvalue"] is None else grp["clipvalue"]
+            hps.append(_lib.WfFitParams(gamma=float(ag.gamma), lr=grp["lr"], beta_1=grp["beta_1"], beta_2=grp["beta_2"],
+                                        epsilon=grp["epsilon"], clipvalue=clip, adam_t=self.adam_t[j],
+                                        target_every=int(ag.target_update_freq), phase=self.until_sync[j]))
+            ptrs.append([x.data_ptr() + x.element_size() * j * self.P for x in self.flat]
+                        + [s_row.data_ptr(), sp_row.data_ptr(), a.data_ptr(), ap.data_ptr() if a0._SARSA else None,
+                           r.data_ptr(), d.data_ptr()])
+        with torch.cuda.device(dev):
+            if len(learners) == 1:
+                W, H = a0.obs_shape[0], a0.obs_shape[1]
+                fit = L.wf_replay_fit if W <= 32 and H <= 32 else L.wf_replay_fit_large
+                _lib.check(fit(ctypes.byref(shape), ctypes.byref(hps[0]), n_replays, *ptrs[0][:4], _ptr(frames),
+                               frames.shape[0], *ptrs[0][4:], _ptr(loss), stream))
+            else:
+                desc = (_lib.WfFitLearner * len(learners))(*(_lib.WfFitLearner(*p, None, hp) for p, hp in zip(ptrs, hps)))
+                _lib.check(L.wf_replay_fit_many(ctypes.byref(shape), len(learners), desc, n_replays, _ptr(frames),
+                                                frames.shape[0], stream))
+        for j in learners:
+            te = int(self.agents[j].target_update_freq)
+            self.adam_t[j] += n_replays
+            self.until_sync[j] = (self.until_sync[j] - n_replays - 1) % te + 1
+
+    def write_back(self, j):
+        """Agent j's part of the stack back into agent j: its model and target, its ``KerasAdam`` m, v and t (once it has
+        been updated) and ``_until_sync``."""
+        a = self.agents[j]
+        P, Tg, Mm, Vv = self.flat
+        with torch.no_grad():
+            off = j * self.P
+            for p, tp in zip(a.model.parameters(), a.target.parameters()):
+                n = p.numel()
+                p.copy_(P[off:off + n].view_as(p))
+                tp.copy_(Tg[off:off + n].view_as(p))
+                if self.adam_t[j]:
+                    st = a.optimizer.state[p]
+                    st["m"] = Mm[off:off + n].view_as(p).clone()
+                    st["v"] = Vv[off:off + n].view_as(p).clone()
+                    st["t"] = self.adam_t[j]
+                off += n
+        a._until_sync = self.until_sync[j]
 
 
 def _map_rule(maps, best_reward, episode, total_reward, render):
